@@ -2,6 +2,7 @@
 """bench.py — Mrays/s of the per-pixel ray/scene hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c4|c3|c2|c1|c5|c5s]
+                    [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[3] "unitychan 3840x2160 64 spp", the configuration
 the metric's 1/2/4/8-GPU numbers are quoted on; it fits one GPU, so it is also the N=1 workload.
@@ -23,6 +24,17 @@ pixels per frame.  The frame is fixed, so scaling is "strong".  e2e at N > 1: ev
 tiles of accuBuffer + bitcolor into ONE shared host frame (POSIX shared memory, registered in every
 process) over its own PCIe link (rt_gpu_deliver_owned), instead of funnelling the frame through rank 0.
 
+Meshes: the reference's Data folder where oracle/Makefile has staged it (assets/_ref/Data), else stand-ins of the
+same names generated into a temporary directory (tests/standin_data.py: a textured ~22 k-triangle figure in place of
+unitychan); `config.assets` of the JSON line says which, and `config.workload` marks a stand-in run.  Numbers on the
+stand-ins measure the same code on other geometry: they are not comparable with the figures of BASELINE.json and
+README.md, which are on the reference's meshes.  Nothing is written into the repository.
+
+--dump-outputs DIR writes what the timed path computed in its last step, after the timing: the accumulation buffer
+(accuBuffer: RGB sum + pass count) and the display buffer (bitcolor, ARGB8 as 4 floats) of a fixed, seeded sample of
+2^20 pixels (every pixel of a smaller frame), their pixel indices, and the step's ray counts, as float32 / float64
+.npy files (40 MB at most).  The inputs depend on the arguments only, so two builds can be compared file by file.
+
 --impl reference times the UNMODIFIED reference (oracle/_ref/libref_oracle.so, compiled from
 /root/reference by oracle/Makefile) on all host cores, same scene / camera / seed, each step one
 pass (4 camera rays per pixel) over the full frame — a bounded sample of the 16-pass step; its rays are
@@ -35,6 +47,7 @@ import hashlib
 import json
 import os
 import sys
+import tempfile
 import threading
 import time
 
@@ -44,9 +57,22 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import numpy as np  # noqa: E402
 
-DATA = os.path.join(ROOT, "assets", "_ref", "Data")
+REF_DATA = os.path.join(ROOT, "assets", "_ref", "Data")
+DATA = REF_DATA
+ASSETS = "reference Data folder (assets/_ref/Data)"
 TILE = 32
 NUM_SMS = 148
+DUMP_PIXELS = 1 << 20
+_scratch = None
+
+
+def scratch_dir():
+    """A temporary directory of this process for generated inputs; removed at exit."""
+    global _scratch
+    if _scratch is None:
+        _scratch = tempfile.TemporaryDirectory(prefix="rtb200_bench_")
+    return _scratch.name
+
 
 WORKLOADS = {
     # name: (scene fn name, W, H, passes, antialias, max_bounce, mode, description)
@@ -124,11 +150,12 @@ def build_spec(workload):
         sys.path.insert(0, os.path.join(ROOT, "tools"))
         import make_c5
         copies = int(fn.split(":")[1])
-        out_dir = os.environ.get("RT_SCRATCH", "/tmp/rt_c5")
+        out_dir = os.environ.get("RT_SCRATCH") or scratch_dir()
         os.makedirs(out_dir, exist_ok=True)
-        out = os.path.join(out_dir, f"unitychan_x{copies}.obj")
+        src = os.path.join(DATA, "unitychan.obj")
+        out = os.path.join(out_dir, make_c5.cached_name(src, copies, W / H))
         if not os.path.exists(out):
-            make_c5.main(os.path.join(DATA, "unitychan.obj"), out, copies, W / H)
+            make_c5.main(src, out, copies, W / H)
         spec = [("mesh", out, ("blend", ("reflective", scenes.WHITE, 0.2), ("diffuse", scenes.WHITE), 1.0))]
         return spec, W, H, passes, aa, bounce, mode, desc
     return getattr(scenes, fn)(DATA), W, H, passes, aa, bounce, mode, desc
@@ -137,7 +164,9 @@ def build_spec(workload):
 def workload_config(args, W, H, passes, aa, bounce, desc):
     """`config` of the JSON line: the workload, identical in both arms (what differs per arm is outside it)."""
     return {
-        "workload": f"{args.workload}: {desc}",
+        "workload": f"{args.workload}: {desc}" + ("" if DATA == REF_DATA else
+                    " -- on STAND-IN meshes, not the reference's: not comparable with the figures of BASELINE.json / README.md"),
+        "assets": ASSETS,
         "frame": f"{W}x{H}", "passes_per_step": passes, "camera_rays_per_pixel": passes * (4 if aa else 1), "max_bounce": bounce,
         "camera": "eye (0,0,7), dir_z -0.5 (RayTracerProgram.cpp:133,164)", "seed": 0,
         "rng": "counter RNG shared by both arms (include/rt_rng.h; interposed for rand() in the reference, lock-free)",
@@ -450,6 +479,12 @@ def run_own(args):
     ms = ev0.elapsed_time(ev1)
     launches = ctx.launch_count - launches0
     c = ctx.counters()
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # the last timed frame, on rank 0 the whole frame (the gather has landed: barrier above)
+        select(args.steps - 1)
+        dumped = (ctx.readback(rt.RT_READ_ACCUM_RGBN_F32, W, H).reshape(npix, 4),
+                  ctx.readback(rt.RT_READ_DISPLAY_ARGB8, W, H).reshape(npix))
 
     # --- per-kernel-class durations: one more step with a single pipe (strictly one kernel at a time, same process,
     # same data, one CUDA event per launch on the launching stream), outside the timed region ---
@@ -678,6 +713,8 @@ def run_own(args):
         }
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline(args, spec, W, H, passes, aa, bounce, mode, c["rays"] / args.steps)
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, *dumped, stats / args.steps)
         print(json.dumps(line))
     # tear down in dependency order: collectives first (they are queued behind the context's streams),
     # then hand torch its own stream back before the context destroys the ones it borrowed
@@ -700,6 +737,22 @@ def run_own(args):
         dist.destroy_process_group()
     ctx.close()
     return 0
+
+
+def dump_outputs(out_dir, accum, display, stats_per_step):
+    """accum (npix, 4) f32 and display (npix,) ARGB8 of one frame -> DIR/*.npy, a fixed sample of DUMP_PIXELS pixels."""
+    npix = accum.shape[0]
+    if npix > DUMP_PIXELS:
+        index = np.sort(np.random.default_rng(0).choice(npix, DUMP_PIXELS, replace=False))
+    else:
+        index = np.arange(npix)
+    disp = display[index].astype(np.uint32)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pixel_index.npy"), index.astype(np.float64))
+    np.save(os.path.join(out_dir, "accum.npy"), np.ascontiguousarray(accum[index], np.float32))
+    np.save(os.path.join(out_dir, "display_argb.npy"), np.stack([(disp >> s) & 255 for s in (24, 16, 8, 0)], -1).astype(np.float32))
+    # rays and camera rays of one step, all ranks (node / triangle visit counts depend on how the walks were scheduled)
+    np.save(os.path.join(out_dir, "counters.npy"), stats_per_step.cpu().numpy()[[1, 5]].astype(np.float64))
 
 
 def cpu_baseline(args, spec, W, H, passes, aa, bounce, mode, gpu_rays_per_step):
@@ -748,11 +801,20 @@ def main():
     ap.add_argument("--no-overlap", action="store_true", help="one frame slot: a frame starts when the previous one has ended")
     ap.add_argument("--slots", type=int, default=0, help="frames in flight (1-4; default 4)")
     ap.add_argument("--profile-frames", type=int, default=0, help="(ncu) render this many plain frames and exit")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (sampled frame buffers, ray counts) to DIR/*.npy")
     args = ap.parse_args()
     if args.warmup < 3 and args.impl == "own":
         args.warmup = 3                     # timing rule: at least 3 warm-up steps
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        raise SystemExit("--dump-outputs writes the outputs of the own arm; it is not available with --impl reference")
+    global DATA, ASSETS
     if not os.path.isdir(DATA):
-        raise SystemExit("assets/_ref/Data missing: run __graft_entry__.build() where /root/reference exists")
+        import standin_data
+        DATA = standin_data.write(os.path.join(scratch_dir(), "Data"))
+        ASSETS = "generated stand-ins of the reference's meshes (tests/standin_data.py)"
     sys.exit(run_reference(args) if args.impl == "reference" else run_own(args))
 
 

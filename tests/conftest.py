@@ -1,13 +1,17 @@
 """Shared fixtures.  `-m "not gpu"` runs on a CPU-only box; `-m gpu` needs a B200.
 
 The checkers (oracle/) are used here only to CHECK: the product path (raytracerwin_b200) never
-imports them.  /root/reference is never read at test time: the reference's compiled hot path
-(oracle/_ref/*.so) and its staged assets (assets/_ref/Data) are build outputs that travel with
-the repository snapshot, and the committed fixtures under tests/golden/ cover the case where
-they are absent.
+imports them.  The reference's compiled hot path (oracle/_ref/*.so) and its Data folder
+(assets/_ref/Data) are build outputs of oracle/Makefile where the reference's sources are at hand.
+Without them:
+  * the scenes load generated stand-ins with the same file names (tests/standin_data.py), and the
+    golden fixtures are those of the stand-ins (tests/golden/standin/);
+  * the CPU tests that pin the restatement to the reference skip; the GPU tests compare the CUDA
+    path with the restatement instead (tests/port_reference.py), which those CPU tests pin.
 """
 import os
 import sys
+import warnings
 
 import numpy as np
 import pytest
@@ -49,28 +53,58 @@ def rt():
 
 
 @pytest.fixture(scope="session")
-def data_dir():
-    if not os.path.isdir(DATA_DIR):
-        pytest.skip("assets/_ref/Data not staged (run __graft_entry__.build() where /root/reference exists)")
-    return DATA_DIR
+def data_dir(tmp_path_factory):
+    """Meshes for the scenes of scenes.py: the reference's Data folder where staged, else generated stand-ins."""
+    if os.path.isdir(DATA_DIR):
+        return DATA_DIR
+    import standin_data
+    return standin_data.write(str(tmp_path_factory.mktemp("standin") / "Data"))
 
 
-@pytest.fixture(scope="session")
-def ref():
+_ORACLES = {}
+
+
+def _ref_oracle(counting):
+    """One RefOracle per library for the whole session."""
+    from oracle import bindings
+    if counting not in _ORACLES:
+        _ORACLES[counting] = bindings.RefOracle(counting=counting)
+    return _ORACLES[counting]
+
+
+def _port_reference(request):
+    """GPU tests only: the restatement in the reference's place (tests/port_reference.py)."""
+    from oracle import bindings
+    if request.node.get_closest_marker("gpu") is None or not bindings.port_available():
+        return None
+    import raytracerwin_b200
+    from port_reference import PortReference
+    raytracerwin_b200.load_library()
+    return PortReference(raytracerwin_b200, bindings.PortOracle())
+
+
+@pytest.fixture
+def ref(request):
     from oracle import bindings
     if not bindings.ref_available():
-        pytest.skip("oracle/_ref/libref_oracle.so not built")
-    return bindings.RefOracle()
+        stand_in = _port_reference(request)
+        if stand_in is None:
+            pytest.skip("oracle/_ref/libref_oracle.so not built")
+        return stand_in
+    return _ref_oracle(False)
 
 
-@pytest.fixture(scope="session")
-def ref_counting():
+@pytest.fixture
+def ref_counting(request):
     """The ray-counting twin of the reference (RayTracerScene.cpp built with -finstrument-functions): same
     results, and ref.render(...)["rays"] = the number of FindIntersectionWithScene calls it made."""
     from oracle import bindings
     if not os.path.exists(bindings.REF_COUNT_LIB):
-        pytest.skip("oracle/_ref/libref_oracle_count.so not built")
-    return bindings.RefOracle(counting=True)
+        stand_in = _port_reference(request)       # counts the same rays (tests/test_oracle_vs_ref.py)
+        if stand_in is None:
+            pytest.skip("oracle/_ref/libref_oracle_count.so not built")
+        return stand_in
+    return _ref_oracle(True)
 
 
 @pytest.fixture(scope="session")
@@ -86,6 +120,17 @@ def gpu(rt):
     ctx = rt.GpuContext(0)
     yield ctx
     ctx.close()
+
+
+def is_reference(ref, what):
+    """True where `ref` is the reference itself.  With the restatement in its place (port_reference.py), `what`
+    (output of the host scene layer: loader counts, tree, unit-vector table) would be compared with itself: the
+    caller leaves that comparison out, and the warning summary says so."""
+    if getattr(ref, "stands_in", False):
+        warnings.warn(f"{what}: not compared: no compiled reference (oracle/_ref), and the restatement in its place "
+                      "shares the host scene layer under test")
+        return False
+    return True
 
 
 def bits(a):

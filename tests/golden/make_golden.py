@@ -6,12 +6,19 @@ oracle/ref_harness.cpp with the shared counter RNG.  Run where /root/reference e
 
     python tests/golden/make_golden.py
 
+Without the reference, `--standin` writes the fixtures of the generated stand-in meshes
+(tests/standin_data.py) into tests/golden/standin/, at reduced sizes, through the plain-C restatement
+in the reference's place (tests/port_reference.py; tests/test_oracle_vs_ref.py pins it to the
+reference).  They pin the CUDA path and the host layer to what the restatement computed when they
+were written.  kat.npz holds no mesh and is not rewritten.
+
 Inputs are regenerated from fixed seeds by the tests; the fixtures hold inputs too where that is cheap,
 so a change of numpy's generators cannot silently invalidate them.
 """
 import hashlib
 import os
 import sys
+import tempfile
 
 import numpy as np
 
@@ -38,8 +45,25 @@ RENDERS = {
 }
 
 
+def main_standin():
+    import raytracerwin_b200 as rt
+    import standin_data
+    from oracle.bindings import PortOracle
+    from port_reference import PortReference
+    rt.load_library()
+    ref = PortReference(rt, PortOracle())
+    with tempfile.TemporaryDirectory() as tmp:
+        data = standin_data.write(os.path.join(tmp, "Data"))
+        write_mesh_fixtures(ref, data, os.path.join(HERE, "standin"), scale=2, n_rays=2000, n_uv=500)
+
+
 def main():
     ref = RefOracle()
+    kat(ref)
+    write_mesh_fixtures(ref, DATA, HERE)
+
+
+def kat(ref):
     rng = np.random.default_rng(3)
     n = 4000
     rays = random_rays(n, 11)
@@ -66,6 +90,10 @@ def main():
     out["display"] = ref.kat_display(rgb)
     np.savez_compressed(os.path.join(HERE, "kat.npz"), **out)
 
+
+def write_mesh_fixtures(ref, DATA, OUT, scale=1, n_rays=20000, n_uv=2000):
+    """Fixtures of scenes with meshes from DATA into OUT; image sides divided by `scale`."""
+    os.makedirs(OUT, exist_ok=True)
     # loader + BVH + primary hits per mesh
     for name in ("TorusKnot", "BlenderMonkey", "unitychan"):
         spec = [("mesh", f"{DATA}/{name}.obj", ("diffuse", scenes.WHITE))]
@@ -73,19 +101,20 @@ def main():
         counts = np.array(ref.mesh_counts(s, 0), np.int32)
         bounds, escape, tri, verts = ref.mesh_bvh(s, 0)
         d = ref.mesh_dump(s, 0)
-        W, H = 160, 120
-        r = ref.trace_primary(s, W, H, want_hit=True)
+        W, H = 160 // scale, 120 // scale
+        r = ref.trace_primary(s, W, H, want_hit=isinstance(ref, RefOracle))
         assert r["mismatches"] == 0
         digest = lambda a: np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), np.uint8)
-        np.savez_compressed(os.path.join(HERE, f"primary_{name}.npz"), counts=counts, W=W, H=H,
+        hit = {} if r["hit"] is None else dict(hit=r["hit"])
+        np.savez_compressed(os.path.join(OUT, f"primary_{name}.npz"), counts=counts, W=W, H=H, **hit,
                             bvh_bounds_sha=digest(bounds), bvh_escape_sha=digest(escape), bvh_tri_sha=digest(tri),
                             points_sha=digest(d["points"]), pidx_sha=digest(d["pidx"]), matid_sha=digest(d["matid"]),
-                            shape=r["shape"].astype(np.int8), tri=r["tri"], dist=r["dist"], hit=r["hit"],
+                            shape=r["shape"].astype(np.int8), tri=r["tri"], dist=r["dist"],
                             node_tests=r["node_tests"], tri_tests=r["tri_tests"])
         if name == "unitychan":
             # texture pixels (linearised by the reference at load): digest per slot + a few samples
             tex = {}
-            uv = (np.random.default_rng(5).random(size=(2000, 2)) * 3 - 1).astype(np.float32)
+            uv = (np.random.default_rng(5).random(size=(n_uv, 2)) * 3 - 1).astype(np.float32)
             k = 0
             for slot in range(16):
                 px = ref.mesh_texture(s, 0, slot)
@@ -96,29 +125,30 @@ def main():
                 tex[f"tex{k}_sha"] = digest(px)
                 tex[f"tex{k}_samples"] = ref.kat_texture_sample(s, 0, slot, uv)
                 k += 1
-            np.savez_compressed(os.path.join(HERE, "textures_unitychan.npz"), uv=uv, count=k, **tex)
+            np.savez_compressed(os.path.join(OUT, "textures_unitychan.npz"), uv=uv, count=k, **tex)
         ref.free_scene(s)
 
     # arbitrary rays through the default scene (all shape classes)
     s = ref.build_scene(scenes.default_scene(DATA))
-    rr = random_rays(20000, 7)
+    rr = random_rays(n_rays, 7)
     sh, tr, hit = ref.trace_rays(s, rr)
-    np.savez_compressed(os.path.join(HERE, "rays_default_scene.npz"), rays=rr, shape=sh.astype(np.int8), tri=tr, hit=hit)
+    np.savez_compressed(os.path.join(OUT, "rays_default_scene.npz"), rays=rr, shape=sh.astype(np.int8), tri=tr, hit=hit)
     ref.free_scene(s)
 
     # renders
     for name, (scene, W, H, mode, bounce, aa, passes, seed, table_seed) in RENDERS.items():
+        W, H = W // scale, H // scale
         if table_seed is not None:
             ref.init_unit_vectors(table_seed)
         s = ref.build_scene(getattr(scenes, scene)(DATA))
         r = ref.render(s, W, H, mode=mode, max_bounce=bounce, antialias=aa, pass_count=passes, seed=seed, nthreads=8, want_display=True)
-        np.savez_compressed(os.path.join(HERE, f"render_{name}.npz"), accum=r["accum"], display=r["display"],
+        np.savez_compressed(os.path.join(OUT, f"render_{name}.npz"), accum=r["accum"], display=r["display"],
                             params=np.array([W, H, mode, bounce, aa, passes, seed, -1 if table_seed is None else table_seed], np.int32))
         ref.free_scene(s)
         print(name, "done")
-    total = sum(os.path.getsize(os.path.join(HERE, f)) for f in os.listdir(HERE) if f.endswith(".npz"))
+    total = sum(os.path.getsize(os.path.join(OUT, f)) for f in os.listdir(OUT) if f.endswith(".npz"))
     print("fixtures:", total // 1024, "KiB")
 
 
 if __name__ == "__main__":
-    main()
+    main_standin() if "--standin" in sys.argv[1:] else main()

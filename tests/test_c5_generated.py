@@ -7,7 +7,7 @@ import sys
 import numpy as np
 import pytest
 
-from conftest import ROOT, bits
+from conftest import DATA_DIR, ROOT, bits
 
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 import make_c5  # noqa: E402
@@ -45,7 +45,10 @@ def test_generated_grid_gpu(tmp_path, rt, gpu, port, data_dir):
     spec = [("mesh", out, ("blend", ("reflective", WHITE, 0.2), ("diffuse", WHITE), 1.0))]
     sc = rt.Scene(spec)
     sc.set_unit_vectors(seed=1, count=1 << 20)
-    assert sc.mesh_counts(0)[3] == 12 * 16056
+    one = rt.Scene([("mesh", os.path.join(data_dir, "unitychan.obj"), ("diffuse", WHITE))]).mesh_counts(0)[3]
+    if data_dir == DATA_DIR:
+        assert one == 16056                                                   # the reference's unitychan
+    assert sc.mesh_counts(0)[3] == 12 * one
     gpu.upload_scene(sc)
     W, H = 640, 360
     for tr in (rt.RT_TRAVERSE_EXACT, rt.RT_TRAVERSE_CULLED):

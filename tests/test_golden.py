@@ -1,8 +1,12 @@
-"""Replays the committed golden fixtures (tests/golden/*.npz, generated from the UNMODIFIED reference by
-tests/golden/make_golden.py) against
+"""Replays the committed golden fixtures against
   * the plain-C restatement + the product's host scene layer     (CPU, always), and
   * the CUDA path through the C-ABI                                (-m gpu).
-These do not need oracle/_ref at run time."""
+These do not need oracle/_ref at run time.  Which fixtures (tests_golden_common.golden):
+  * tests/golden/*.npz, generated from the UNMODIFIED reference by tests/golden/make_golden.py, where the
+    reference's meshes are staged (assets/_ref/Data); kat.npz (no mesh) always;
+  * else tests/golden/standin/*.npz, the stand-in meshes (tests/standin_data.py) as the plain-C restatement
+    rendered them (make_golden.py --standin): they pin later changes to what the project computed then,
+    not to the reference."""
 import hashlib
 import os
 

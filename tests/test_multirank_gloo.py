@@ -12,7 +12,7 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 import scenes
-from conftest import DATA_DIR, ROOT, bits
+from conftest import ROOT, bits
 
 
 def _free_port():
@@ -23,7 +23,7 @@ def _free_port():
     return p
 
 
-def _worker(rank, world, port, W, H, T, out_path):
+def _worker(rank, world, port, W, H, T, data_dir, out_path):
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     os.environ["MASTER_ADDR"] = "127.0.0.1"
@@ -32,7 +32,7 @@ def _worker(rank, world, port, W, H, T, out_path):
     import raytracerwin_b200 as rt
     from raytracerwin_b200 import tiles
     from oracle.bindings import PortOracle
-    sc = rt.Scene(scenes.deterministic_mix(DATA_DIR))
+    sc = rt.Scene(scenes.deterministic_mix(data_dir))
     kw = dict(mode=rt.RT_MODE_PATH, max_bounce=4, antialias=0, traverse=rt.RT_TRAVERSE_EXACT)
     p = rt.make_params(W, H, tile_size=T, tile_count=world, tile_rank=rank, **kw)
     part = PortOracle().render(sc.desc, p)["accum"].reshape(-1, 4)
@@ -58,7 +58,7 @@ def _worker(rank, world, port, W, H, T, out_path):
 @pytest.mark.parametrize("world,W,H,T", [(2, 150, 70, 32), (3, 97, 61, 16)])
 def test_tile_sharded_render_reassembles(tmp_path, rt, port, data_dir, world, W, H, T):
     out = str(tmp_path / "frame.npy")
-    mp.spawn(_worker, args=(world, _free_port(), W, H, T, out), nprocs=world, join=True)
+    mp.spawn(_worker, args=(world, _free_port(), W, H, T, data_dir, out), nprocs=world, join=True)
     frame = np.load(out)
     sc = rt.Scene(scenes.deterministic_mix(data_dir))
     whole = port.render(sc.desc, rt.make_params(W, H, mode=rt.RT_MODE_PATH, max_bounce=4, antialias=0,
@@ -66,7 +66,7 @@ def test_tile_sharded_render_reassembles(tmp_path, rt, port, data_dir, world, W,
     np.testing.assert_array_equal(bits(frame), bits(whole))
 
 
-def _shared_frame_worker(rank, world, port, W, H, T, name, out_path):
+def _shared_frame_worker(rank, world, port, W, H, T, data_dir, name, out_path):
     """The N > 1 end-to-end host logic of bench.py: every rank attaches ONE shared host frame and puts its own tiles
     into it (on the GPU box rt_gpu_deliver_owned writes them over PCIe; here the checker's pixels are copied in)."""
     sys.path.insert(0, ROOT)
@@ -83,7 +83,7 @@ def _shared_frame_worker(rank, world, port, W, H, T, name, out_path):
     dist.barrier()
     if rank != 0:
         frame = bench.SharedFrame(name, npix, False)
-    sc = rt.Scene(scenes.deterministic_mix(DATA_DIR))
+    sc = rt.Scene(scenes.deterministic_mix(data_dir))
     p = rt.make_params(W, H, mode=rt.RT_MODE_PATH, max_bounce=4, antialias=0, traverse=rt.RT_TRAVERSE_EXACT,
                        tile_size=T, tile_count=world, tile_rank=rank)
     o = PortOracle().render(sc.desc, p, want_display=True)
@@ -101,7 +101,7 @@ def _shared_frame_worker(rank, world, port, W, H, T, name, out_path):
 def test_shared_host_frame_assembled_by_two_ranks(tmp_path, rt, port, data_dir):
     W, H, T, world = 150, 70, 32, 2
     out = str(tmp_path / "frame.npz")
-    mp.spawn(_shared_frame_worker, args=(world, _free_port(), W, H, T, f"rtb200_test_{os.getpid()}", out), nprocs=world, join=True)
+    mp.spawn(_shared_frame_worker, args=(world, _free_port(), W, H, T, data_dir, f"rtb200_test_{os.getpid()}", out), nprocs=world, join=True)
     got = np.load(out)
     sc = rt.Scene(scenes.deterministic_mix(data_dir))
     whole = port.render(sc.desc, rt.make_params(W, H, mode=rt.RT_MODE_PATH, max_bounce=4, antialias=0,

@@ -7,9 +7,21 @@ the ordinary loader.  Deterministic: no randomness.
 
 `usemtl`/`mtllib` lines are kept; the .mtl and its textures are expected next to OUT.obj (this script symlinks
 the source's .mtl and texture directory when they exist)."""
+import hashlib
 import math
 import os
 import sys
+
+
+def cached_name(src, copies, aspect=16.0 / 9.0):
+    """File name for the generated OBJ in a cache directory: keyed by the source mesh's and this script's
+    contents, the copy count and the aspect, so that a changed input never reuses an old file."""
+    h = hashlib.sha256()
+    for path in (src, os.path.abspath(__file__)):
+        with open(path, "rb") as f:
+            h.update(f.read())
+    h.update(f"{copies}:{float(aspect)!r}".encode())
+    return f"{os.path.splitext(os.path.basename(src))[0]}_x{copies}_{h.hexdigest()[:16]}.obj"
 
 
 def main(src, out, copies, aspect=16.0 / 9.0):
