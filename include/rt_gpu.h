@@ -13,6 +13,8 @@
  *   rt_gpu_render_tile   replaces ThreadWorker_Render(begin, end, MaxBounceCount, Option)
  *                        (RayTracerProgram.cpp:131-188), i.e. one RenderThreadTask (:79-95)
  *   rt_gpu_readback      replaces reading bitcolor[] / accuBuffer[] (:49,:77)
+ *   rt_gpu_query_rays    FindIntersectionWithScene (RayTracerScene.cpp:99-125) and the shadow query of
+ *                        CalculateLightColor (:152-164) on batches of the caller's rays in device memory
  *
  * Plain C: POD structs, pointers and sizes only.  No C++/STL/torch types cross the boundary.
  * Every entry returns 0 on success or a negative rt_status; rt_gpu_last_error() gives text.
@@ -230,6 +232,34 @@ int rt_gpu_reset_accum(rt_gpu_ctx* ctx, int32_t width, int32_t height);
 /* Enqueues one render task on the context's stream and returns immediately.
  * If the buffers do not match params->width/height they are reset first. */
 int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* params);
+
+/* ---- ray queries on device memory -------------------------------------------------------------
+ * Batches of the caller's own rays through the same wavefront kernels as render_tile (generate -> packet /
+ * lane-per-walk / long walk -> shade, one round per mesh a ray reaches), results in device memory: picking,
+ * visibility and shadow masks, cameras of one's own, bakes.  Results equal rt_gpu_trace_rays bit for bit. */
+enum {
+    RT_QUERY_NEAREST = 0,   /* RayTracerScene::FindIntersectionWithScene (RayTracerScene.cpp:99-125) */
+    RT_QUERY_ANY = 1        /* the shadow loop of CalculateLightColor (:152-164): any accepted hit within Distance */
+};
+
+typedef struct rt_ray_query {
+    const float* rays;      /* DEVICE, n x 7 floats {origin, direction, Distance}: the rays of rt_gpu_trace_rays */
+    int32_t n;
+    int32_t kind;           /* RT_QUERY_* */
+    int32_t traverse;       /* RT_TRAVERSE_* (same results either way) */
+    int32_t* shape;         /* DEVICE, n.  NEAREST: index of the shape hit, -1 = none;  ANY: 1 occluded, 0 not */
+    int32_t* tri;           /* DEVICE, n, may be NULL; NEAREST only: original triangle id, -1 for analytic shapes / miss */
+    float* hit;             /* DEVICE, n x 11, may be NULL; NEAREST only: HitPosition, HitNormal, Distance, SampledColor,
+                               SampledAlpha, zeros on a miss (rt_gpu_trace_rays' hit11) */
+} rt_ray_query;
+
+/* Enqueues the queries on `stream` (a cudaStream_t; NULL = the current frame slot's stream) and returns at once:
+ * the work is ordered after everything enqueued on `stream` before the call, and the outputs are complete for
+ * everything enqueued on it after.  Every pointer must be device memory of the context's GPU.  n == 0 is a no-op.
+ * Adds to the context's counters (rays; shadow_rays for RT_QUERY_ANY; slab / triangle tests, mesh walks and hits);
+ * those are read on the context's stream, so order it after `stream` before reading them.  Leaves the frame
+ * buffers, the frame slot and rt_gpu_last_render_ms alone. */
+int rt_gpu_query_rays(rt_gpu_ctx* ctx, const rt_ray_query* q, void* stream);
 
 /* Synchronises the stream, then copies `what` into caller memory (size-checked). */
 int rt_gpu_readback(rt_gpu_ctx* ctx, int what, void* dst, size_t bytes);

@@ -13,8 +13,8 @@ import os
 import numpy as np
 
 from . import _abi
-from ._abi import (rt_render_params, rt_counters, rt_scene_desc,  # noqa: F401
-                   RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY,
+from ._abi import (rt_render_params, rt_counters, rt_scene_desc, rt_ray_query,  # noqa: F401
+                   RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY, RT_QUERY_NEAREST, RT_QUERY_ANY,
                    RT_TRAVERSE_EXACT, RT_TRAVERSE_CULLED,
                    RT_READ_ACCUM_RGBN_F32, RT_READ_DISPLAY_ARGB8, RT_READ_PRIMARY_IDS_I32X2,
                    RT_READ_PRIMARY_DIST_F32, RT_READ_COUNTERS_U64, RT_READ_PREVIEW_RGBA_F32)
@@ -328,6 +328,44 @@ class GpuContext:
             self._h, rays.ctypes.data_as(_abi.PF), n, traverse,
             shape.ctypes.data_as(_abi.PI32), tri.ctypes.data_as(_abi.PI32), hit.ctypes.data_as(_abi.PF)))
         return shape, tri, hit
+
+    def query_rays(self, rays, any_hit=False, traverse=RT_TRAVERSE_CULLED, want_tri=None, want_hit=None):
+        """Nearest-hit or occlusion queries of a batch of rays held in device memory (rt_gpu_query_rays).
+
+        `rays`: contiguous float32 torch tensor (N, 7) {origin, direction, Distance} on cuda:<self.device>.
+        The queries are enqueued on torch.cuda.current_stream(self.device) and the call returns at once; the
+        results are usable on that stream without a host synchronisation.  Outputs are torch tensors on the same
+        device: nearest hit -> dict(shape=int32[N] (-1 = none), tri=int32[N] or None, hit=float32[N, 11] or None)
+        with rt_gpu_trace_rays' fields; any_hit -> int32[N], 1 where the ray is occluded.  want_tri / want_hit
+        default to True for nearest-hit queries and to False for occlusion queries (which have neither).
+        The context's counters are read on its own stream: synchronise before reading them."""
+        import torch
+        if not isinstance(rays, torch.Tensor):
+            raise ValueError(f"rays must be a torch tensor on cuda:{self.device}, not {type(rays).__name__}")
+        dev = torch.device("cuda", self.device)
+        if rays.device != dev:
+            raise ValueError(f"rays are on {rays.device}, the context is on {dev}")
+        if rays.dtype != torch.float32:
+            raise ValueError(f"rays must be float32, not {rays.dtype}")
+        if rays.dim() != 2 or rays.shape[1] != 7:
+            raise ValueError(f"rays must have shape (N, 7), not {tuple(rays.shape)}")
+        if not rays.is_contiguous():
+            raise ValueError("rays must be contiguous")
+        n = rays.shape[0]
+        want_tri = not any_hit if want_tri is None else want_tri
+        want_hit = not any_hit if want_hit is None else want_hit
+        shape = torch.empty(n, dtype=torch.int32, device=dev)
+        tri = torch.empty(n, dtype=torch.int32, device=dev) if want_tri else None
+        hit = torch.empty((n, 11), dtype=torch.float32, device=dev) if want_hit else None
+        q = rt_ray_query(rays.data_ptr(), n, RT_QUERY_ANY if any_hit else RT_QUERY_NEAREST, traverse, shape.data_ptr(),
+                         None if tri is None else tri.data_ptr(), None if hit is None else hit.data_ptr())
+        # torch names the legacy default stream 0, which rt_gpu_query_rays would take for the context's own stream:
+        # pass it as cudaStreamLegacy (1) instead
+        stream = torch.cuda.current_stream(dev).cuda_stream or 1
+        self._check(self._lib.rt_gpu_query_rays(self._h, C.byref(q), stream))
+        if any_hit:
+            return shape
+        return dict(shape=shape, tri=tri, hit=hit)
 
     def build_bvh(self, points, point_idx):
         """KdTree::Build on the device: (nodes, tris, depth, device ms) with the dtypes of Scene.flat_mesh."""

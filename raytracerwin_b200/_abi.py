@@ -14,6 +14,7 @@ RT_LIGHT_POINT, RT_LIGHT_DIRECTIONAL = 0, 1
 RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY = range(4)
 RT_TRAVERSE_EXACT, RT_TRAVERSE_CULLED = 0, 1
 RT_READ_ACCUM_RGBN_F32, RT_READ_DISPLAY_ARGB8, RT_READ_PRIMARY_IDS_I32X2, RT_READ_PRIMARY_DIST_F32, RT_READ_COUNTERS_U64, RT_READ_PREVIEW_RGBA_F32 = range(6)
+RT_QUERY_NEAREST, RT_QUERY_ANY = 0, 1
 RT_GPU_ABI_VERSION = 2
 RT_GPU_FRAME_SLOTS = 4
 
@@ -86,6 +87,11 @@ class rt_counters(C.Structure):
         return {n: int(getattr(self, n)) for n, _ in self._fields_ }
 
 
+class rt_ray_query(C.Structure):
+    _fields_ = [("rays", C.c_void_p), ("n", C.c_int32), ("kind", C.c_int32), ("traverse", C.c_int32),
+                ("shape", C.c_void_p), ("tri", C.c_void_p), ("hit", C.c_void_p)]
+
+
 STRUCT_SIZES = {"rt_shape": 80, "rt_material": 28, "rt_bvh_node": 32, "rt_tri": 64, "rt_shade": 64,
                 "rt_light": 28, "rt_render_params": 56, "rt_counters": 72}
 
@@ -137,6 +143,7 @@ GPU_PROTOTYPES = {
     "rt_gpu_get_frame_slot": (I, [VP]),
     "rt_gpu_time_kernels": (I, [VP, I32]),
     "rt_gpu_build_bvh": (I, [VP, VP, I32, VP, I32, VP, VP, PI32, PF]),
+    "rt_gpu_query_rays": (I, [VP, C.POINTER(rt_ray_query), VP]),
     "rt_gpu_trace_rays": (I, [VP, PF, I32, I32, PI32, PI32, PF]),
     "rt_gpu_kat": (I, [VP, I32, VP, VP, I32, I32, VP, VP]),
     "rt_gpu_kat_texture": (I, [VP, I32, VP, I32, VP]),

@@ -197,8 +197,18 @@ static cudaError_t launch_shade(int mode, unsigned grid, cudaStream_t st, const 
     case RT_MODE_PREVIEW: rt_shade_kernel<CULL, RT_MODE_PREVIEW><<<grid, 256, 0, st>>>(sc, a, w, round); break;
     case RT_MODE_WHITTED: rt_shade_kernel<CULL, RT_MODE_WHITTED><<<grid, 256, 0, st>>>(sc, a, w, round); break;
     case RT_MODE_PRIMARY: rt_shade_kernel<CULL, RT_MODE_PRIMARY><<<grid, 256, 0, st>>>(sc, a, w, round); break;
+    case RT_QMODE_NEAREST: rt_shade_kernel<CULL, RT_QMODE_NEAREST><<<grid, 256, 0, st>>>(sc, a, w, round); break;
+    case RT_QMODE_ANY: rt_shade_kernel<CULL, RT_QMODE_ANY><<<grid, 256, 0, st>>>(sc, a, w, round); break;
     default: return cudaErrorInvalidValue;
     }
+    return cudaGetLastError();
+}
+
+template <bool CULL>
+static cudaError_t launch_query_generate(int qmode, unsigned grid, cudaStream_t st, const DevScene& sc, const RenderArgs& a, const WaveArgs& w)
+{
+    if (qmode == RT_QMODE_ANY) rt_query_generate_kernel<CULL, RT_QMODE_ANY><<<grid, 256, 0, st>>>(sc, a, w);
+    else rt_query_generate_kernel<CULL, RT_QMODE_NEAREST><<<grid, 256, 0, st>>>(sc, a, w);
     return cudaGetLastError();
 }
 
@@ -231,6 +241,201 @@ static cudaError_t grow(T** ptr, size_t* cap, size_t need)
     cudaError_t e = cudaMalloc((void**)ptr, need * sizeof(T));
     if (e == cudaSuccess) *cap = need;
     return e;
+}
+
+// resident CTAs per SM of the walk kernels (persistent grids), queried once
+static int init_walk_grid(rt_gpu_ctx* ctx)
+{
+    if (ctx->walk_blocks_per_sm != 0) return RT_OK;
+    int b0 = 0, b1 = 0;
+    RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b0, rt_walk_kernel<true, true>, 256, 0));
+    RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b1, rt_walk_kernel<false, true>, 256, 0));
+    ctx->walk_blocks_per_sm = b0 < b1 ? b0 : b1;
+    RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->octo_blocks_per_sm, rt_walk_octo_kernel, 256, 0));
+    if (ctx->octo_blocks_per_sm < 1) return fail(ctx, RT_ERR_CUDA, "8-wide walk kernel does not fit on an SM");
+    if (ctx->walk_blocks_per_sm < 1) return fail(ctx, RT_ERR_CUDA, "walk kernel does not fit on an SM");
+    return RT_OK;
+}
+
+// Path pools (one per pipe; render_tile and rt_gpu_query_rays share them).  plan_pools: the records a batch of
+// `batch` items may use — all of them up to the per-pipe maximum, fewer when the pools have to grow and half of
+// the free device memory cannot hold that many (a smaller pool only costs retry passes or smaller query chunks).
+// grow_pools then makes the pools at least that large, with `levels` unwinding levels and the Whitted fields if
+// asked; it only ever grows them, and synchronises only when it does.
+static int plan_pools(rt_gpu_ctx* ctx, size_t batch, size_t levels, bool whitted, size_t* out_want)
+{
+    size_t pool_want = batch < ctx->max_pool_paths ? batch : ctx->max_pool_paths;
+    if (pool_want > ctx->pool_cap || levels > ctx->pool_levels || (whitted && !ctx->pool_whitted))
+    {
+        // (only when the pools have to grow: the memory query costs a driver round trip)
+        // keep all pools together within ~half of the device memory that is free right now (deep bounce
+        // budgets make a path record large: 36 B per level); a smaller pool only costs retry passes
+        const size_t lv = levels > ctx->pool_levels ? levels : ctx->pool_levels;
+        const size_t per_path = 9 * 16 + ((whitted || ctx->pool_whitted) ? 64 : 0) + lv * 36 + 12;
+        size_t free_b = 0, total_b = 0;
+        RT_CUDA(cudaMemGetInfo(&free_b, &total_b));
+        const size_t have_b = free_b + ctx->pool_cap * (9 * 16 + (ctx->pool_whitted ? 64 : 0) + ctx->pool_levels * 36 + 12) * RT_PIPES;
+        const size_t fit = have_b / 2 / RT_PIPES / per_path;
+        if (pool_want > fit) pool_want = fit > 255 ? (fit & ~(size_t)255) : fit;
+        if (pool_want < (batch < 4096 ? batch : (size_t)4096)) return fail(ctx, RT_ERR_NOMEM, "not enough device memory for the path pools");
+    }
+    *out_want = pool_want;
+    return RT_OK;
+}
+
+static int grow_pools(rt_gpu_ctx* ctx, size_t pool_want, size_t levels, bool whitted)
+{
+    if (!(pool_want > ctx->pool_cap || levels > ctx->pool_levels || (whitted && !ctx->pool_whitted))) return RT_OK;
+    RT_CUDA(cudaStreamSynchronize(ctx->stream));
+    const bool same_shape = levels <= ctx->pool_levels && (!whitted || ctx->pool_whitted);
+    const size_t cap = (same_shape && ctx->pool_cap > pool_want) ? ctx->pool_cap : pool_want;
+    const size_t lv = levels > ctx->pool_levels ? levels : ctx->pool_levels;
+    const bool wh = whitted || ctx->pool_whitted;
+    for (int k = 0; k < RT_PIPES; k++)
+    {
+        rt_gpu_ctx::Pipe& pp = ctx->pipes[k];
+        RT_CUDA(cudaStreamSynchronize(pp.stream));
+        for (void* q : pp.allocs) cudaFree(q);
+        pp.allocs.clear();
+        auto alloc = [&](size_t bytes, void** out) -> cudaError_t {
+            cudaError_t e = cudaMalloc(out, bytes);
+            if (e == cudaSuccess) pp.allocs.push_back(*out);
+            return e;
+        };
+        PathPool& pl = pp.pool;
+        memset(&pl, 0, sizeof pl);
+        RT_CUDA(alloc(cap * 16, (void**)&pl.ro)); RT_CUDA(alloc(cap * 16, (void**)&pl.rd));
+        RT_CUDA(alloc(cap * 16, (void**)&pl.cur)); RT_CUDA(alloc(cap * 16, (void**)&pl.bp));
+        RT_CUDA(alloc(cap * 16, (void**)&pl.h0)); RT_CUDA(alloc(cap * 16, (void**)&pl.h1));
+        RT_CUDA(alloc(cap * 16, (void**)&pl.h2)); RT_CUDA(alloc(cap * 16, (void**)&pl.pa));
+        RT_CUDA(alloc(cap * 16, (void**)&pl.pb));
+        if (wh)
+        {
+            RT_CUDA(alloc(cap * 16, (void**)&pl.w0)); RT_CUDA(alloc(cap * 16, (void**)&pl.w1));
+            RT_CUDA(alloc(cap * 16, (void**)&pl.w2)); RT_CUDA(alloc(cap * 16, (void**)&pl.w3));
+        }
+        RT_CUDA(alloc(cap * lv * 16, (void**)&pl.st0)); RT_CUDA(alloc(cap * lv * 16, (void**)&pl.st1));
+        RT_CUDA(alloc(cap * lv * 4, (void**)&pl.st2));
+        RT_CUDA(alloc(cap * 4, (void**)&pp.queue[0])); RT_CUDA(alloc(cap * 4, (void**)&pp.queue[1]));
+        RT_CUDA(alloc(cap * 4, (void**)&pp.longq));
+        RT_CUDA(alloc(cap * 4, (void**)&pp.slowq));
+        pl.cap = (unsigned)cap;
+    }
+    ctx->pool_cap = cap; ctx->pool_levels = lv; ctx->pool_whitted = wh;
+    return RT_OK;
+}
+
+// the wavefront arguments of one pipe: its pool, queues and round counters, and the scheduling knobs
+static WaveArgs pipe_wave_args(const rt_gpu_ctx* ctx, const rt_gpu_ctx::Pipe& pp, int packets)
+{
+    WaveArgs w;
+    memset(&w, 0, sizeof w);
+    w.pool = pp.pool;
+    w.queue[0] = pp.queue[0]; w.queue[1] = pp.queue[1];
+    w.counts = pp.round_counters; w.heads = pp.round_counters + RT_MAX_ROUNDS + 1;
+    w.longq = pp.longq; w.lcounts = w.heads + RT_MAX_ROUNDS; w.lheads = w.lcounts + RT_MAX_ROUNDS;
+    w.slowq = pp.slowq; w.scounts = w.lheads + RT_MAX_ROUNDS; w.sheads = w.scounts + RT_MAX_ROUNDS;
+    w.packet_probe = ctx->tune_packet_probe; w.packet_min_lanes = ctx->tune_packet_min_lanes;
+    w.long_limit = ctx->tune_long_limit; w.small_round = ctx->tune_small_round;
+    w.thin_count = ctx->tune_thin_count; w.thin_limit = ctx->tune_thin_limit;
+    w.packets = packets;
+    w.min_lanes = ctx->tune_min_lanes; w.leaf_wait = ctx->tune_leaf_wait; w.window = ctx->tune_window;
+    return w;
+}
+
+// Work forked from a caller's stream onto the pipes: any error return before the join leaves pipes with work in
+// flight that the caller's stream has not been ordered after; wait for them on the way out, so that a later reset /
+// readback / upload cannot race them.
+struct PipeGuard
+{
+    rt_gpu_ctx* ctx;
+    bool used[RT_PIPES];
+    bool joined;
+    ~PipeGuard()
+    {
+        if (joined) return;
+        for (int k = 0; k < RT_PIPES; k++)
+            if (used[k]) cudaStreamSynchronize(ctx->pipes[k].stream);
+    }
+};
+
+// One round of the wavefront on a pipe: the mesh walks of the round's queue (rounds below `packet_rounds` as packets,
+// then the walks they hand back lane by lane; later rounds lane by lane or on the 8-wide tree), the long walks parked
+// on the way, then the shade kernel in `mode`.  small_pass / thin: the reduced grids of render_tile's retry passes
+// and of late rounds with frames in flight.  mark(class, stream) tags each launch for rt_gpu_time_kernels(ctx, 2);
+// `timed` lets the walk brackets of rt_gpu_time_kernels(ctx, 1) be recorded.
+template <typename Mark>
+static int enqueue_round(rt_gpu_ctx* ctx, rt_gpu_ctx::Pipe& pp, const RenderArgs& a, const WaveArgs& w, int mode, int round,
+                         bool cull, int packet_rounds, bool has_mesh, bool small_pass, bool thin, unsigned walk_grid,
+                         unsigned shade_grid, bool timed, Mark& mark)
+{
+    const unsigned sms = (unsigned)ctx->num_sms;
+    if (has_mesh)
+    {
+        if (timed && ctx->time_walks)
+        {
+            while ((int)ctx->kev.size() < ctx->kev_used + 2)
+            {
+                cudaEvent_t e = nullptr;
+                RT_CUDA(cudaEventCreate(&e));
+                ctx->kev.push_back(e);
+            }
+            RT_CUDA(cudaEventRecord(ctx->kev[ctx->kev_used], pp.stream));
+        }
+        if (round < packet_rounds)
+        {
+            // packets first; what they hand back (incoherent ones) goes on lane by lane
+            RT_CUDA(mark(RT_KERNEL_PACKET_WALK, pp.stream));
+            if (cull) rt_walk_packet_kernel<true><<<small_pass ? sms : walk_grid, 256, 0, pp.stream>>>(ctx->scene, a, w, round);
+            else rt_walk_packet_kernel<false><<<small_pass ? sms : walk_grid, 256, 0, pp.stream>>>(ctx->scene, a, w, round);
+            RT_CUDA(cudaGetLastError());
+            ctx->launches++;
+            RT_CUDA(mark(RT_KERNEL_WALK, pp.stream));
+            RT_CUDA(launch_walk(cull, ctx->tune_top_stage, small_pass ? sms : walk_grid, pp.stream, ctx->scene, a, w, round, 1));
+        }
+        else if (cull && ctx->tune_octo)
+        {
+            // bounce / shadow rounds of the culled traversal: the 8-wide tree
+            RT_CUDA(mark(RT_KERNEL_WALK, pp.stream));
+            rt_walk_octo_kernel<<<(unsigned)(ctx->num_sms * ctx->octo_blocks_per_sm), 256, 0, pp.stream>>>(ctx->scene, a, w, round);
+        }
+        else
+        {
+            RT_CUDA(mark(RT_KERNEL_WALK, pp.stream));
+            RT_CUDA(launch_walk(cull, ctx->tune_top_stage, small_pass ? sms : (thin ? walk_grid / 4u : walk_grid), pp.stream, ctx->scene, a, w, round, 0));
+        }
+        RT_CUDA(cudaGetLastError());
+        const bool time_long = ctx->tune_time_long;     // tooling: bracket walk + long walk
+        if (timed && ctx->time_walks && !time_long)
+        {
+            RT_CUDA(cudaEventRecord(ctx->kev[ctx->kev_used + 1], pp.stream));
+            ctx->kev_used += 2;
+        }
+        ctx->launches++;
+        // the walks that kernel parked as too long, one warp each
+        RT_CUDA(mark(RT_KERNEL_LONG_WALK, pp.stream));
+        {
+            const int group = ctx->tune_long_group;
+            const unsigned lgrid = (unsigned)ctx->num_sms * ((thin || small_pass) ? 1u : (unsigned)RT_LONG_BLOCKS);
+#define RT_LAUNCH_LONG(G) (cull ? rt_longwalk_kernel<true, G><<<lgrid, 256, 0, pp.stream>>>(ctx->scene, a, w, round) \
+                                : rt_longwalk_kernel<false, G><<<lgrid, 256, 0, pp.stream>>>(ctx->scene, a, w, round))
+            if (group == 32) RT_LAUNCH_LONG(32); else if (group == 16) RT_LAUNCH_LONG(16); else RT_LAUNCH_LONG(8);
+#undef RT_LAUNCH_LONG
+        }
+        RT_CUDA(cudaGetLastError());
+        if (timed && ctx->time_walks && time_long)
+        {
+            RT_CUDA(cudaEventRecord(ctx->kev[ctx->kev_used + 1], pp.stream));
+            ctx->kev_used += 2;
+        }
+        ctx->launches++;
+    }
+    RT_CUDA(mark(RT_KERNEL_SHADE, pp.stream));
+    const unsigned sgrid = small_pass ? (sms < shade_grid ? sms : shade_grid) : (thin ? (shade_grid + 7u) / 8u : shade_grid);
+    RT_CUDA(cull ? launch_shade<true>(mode, sgrid, pp.stream, ctx->scene, a, w, round)
+                 : launch_shade<false>(mode, sgrid, pp.stream, ctx->scene, a, w, round));
+    ctx->launches++;
+    return RT_OK;
 }
 
 extern "C" {
@@ -812,16 +1017,8 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
             return RT_OK;
         }
 
-        if (ctx->walk_blocks_per_sm == 0)
-        {
-            int b0 = 0, b1 = 0;
-            RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b0, rt_walk_kernel<true, true>, 256, 0));
-            RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b1, rt_walk_kernel<false, true>, 256, 0));
-            ctx->walk_blocks_per_sm = b0 < b1 ? b0 : b1;
-            RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->octo_blocks_per_sm, rt_walk_octo_kernel, 256, 0));
-            if (ctx->octo_blocks_per_sm < 1) return fail(ctx, RT_ERR_CUDA, "8-wide walk kernel does not fit on an SM");
-            if (ctx->walk_blocks_per_sm < 1) return fail(ctx, RT_ERR_CUDA, "walk kernel does not fit on an SM");
-        }
+        int rc = init_walk_grid(ctx);
+        if (rc != RT_OK) return rc;
         // rounds: one mesh walk per round; a path needs at most (segments) x (mesh shapes) walks
         int mesh_shapes = 0;
         for (int i = 0; i < ctx->scene.num_shapes; i++) mesh_shapes += ctx->host_shape_is_mesh[i] ? 1 : 0;
@@ -882,67 +1079,14 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
         const unsigned long long items_per_chunk = (unsigned long long)passes_per_chunk * a.spp * a.num_blocks * 32ull;
         const int npipes = ctx->tune_pipes;
         const size_t batch = (size_t)((items_per_chunk + 255ull) & ~255ull);
-        size_t pool_want = batch < ctx->max_pool_paths ? batch : ctx->max_pool_paths;
-        const size_t levels_want = p->mode == RT_MODE_PATH ? (size_t)(p->max_bounce > 0 ? p->max_bounce : 1) : 1;
-        if (pool_want > ctx->pool_cap || levels_want > ctx->pool_levels || (p->mode == RT_MODE_WHITTED && !ctx->pool_whitted))
-        {
-            // (only when the pools have to grow: the memory query costs a driver round trip)
-            // keep all pools together within ~half of the device memory that is free right now (deep bounce
-            // budgets make a path record large: 36 B per level); a smaller pool only costs retry passes
-            const size_t levels_now = p->mode == RT_MODE_PATH ? (size_t)(p->max_bounce > 0 ? p->max_bounce : 1) : 1;
-            const size_t lv = levels_now > ctx->pool_levels ? levels_now : ctx->pool_levels;
-            const size_t per_path = 9 * 16 + ((p->mode == RT_MODE_WHITTED || ctx->pool_whitted) ? 64 : 0) + lv * 36 + 12;
-            size_t free_b = 0, total_b = 0;
-            RT_CUDA(cudaMemGetInfo(&free_b, &total_b));
-            const size_t have_b = free_b + ctx->pool_cap * (9 * 16 + (ctx->pool_whitted ? 64 : 0) + ctx->pool_levels * 36 + 12) * RT_PIPES;
-            const size_t fit = have_b / 2 / RT_PIPES / per_path;
-            if (pool_want > fit) pool_want = fit > 255 ? (fit & ~(size_t)255) : fit;
-            if (pool_want < (batch < 4096 ? batch : (size_t)4096)) return fail(ctx, RT_ERR_NOMEM, "not enough device memory for the path pools");
-        }
+        const size_t levels = p->mode == RT_MODE_PATH ? (size_t)(p->max_bounce > 0 ? p->max_bounce : 1) : 1;
+        const bool whitted = p->mode == RT_MODE_WHITTED;
+        size_t pool_want = 0;
+        if ((rc = plan_pools(ctx, batch, levels, whitted, &pool_want)) != RT_OK) return rc;
         const int retries = (int)((batch + pool_want - 1) / pool_want) - 1;
         if (retries >= RT_MAX_RETRIES) return fail(ctx, RT_ERR_NOMEM, "path pool too small for this frame (raise the pool size)");
         {
-            const size_t levels = p->mode == RT_MODE_PATH ? (size_t)(p->max_bounce > 0 ? p->max_bounce : 1) : 1;
-            const bool whitted = p->mode == RT_MODE_WHITTED;
-            if (pool_want > ctx->pool_cap || levels > ctx->pool_levels || (whitted && !ctx->pool_whitted))
-            {
-                RT_CUDA(cudaStreamSynchronize(ctx->stream));
-                const bool same_shape = levels <= ctx->pool_levels && (!whitted || ctx->pool_whitted);
-                const size_t cap = (same_shape && ctx->pool_cap > pool_want) ? ctx->pool_cap : pool_want;
-                const size_t lv = levels > ctx->pool_levels ? levels : ctx->pool_levels;
-                const bool wh = whitted || ctx->pool_whitted;
-                for (int k = 0; k < RT_PIPES; k++)
-                {
-                    rt_gpu_ctx::Pipe& pp = ctx->pipes[k];
-                    RT_CUDA(cudaStreamSynchronize(pp.stream));
-                    for (void* q : pp.allocs) cudaFree(q);
-                    pp.allocs.clear();
-                    auto alloc = [&](size_t bytes, void** out) -> cudaError_t {
-                        cudaError_t e = cudaMalloc(out, bytes);
-                        if (e == cudaSuccess) pp.allocs.push_back(*out);
-                        return e;
-                    };
-                    PathPool& pl = pp.pool;
-                    memset(&pl, 0, sizeof pl);
-                    RT_CUDA(alloc(cap * 16, (void**)&pl.ro)); RT_CUDA(alloc(cap * 16, (void**)&pl.rd));
-                    RT_CUDA(alloc(cap * 16, (void**)&pl.cur)); RT_CUDA(alloc(cap * 16, (void**)&pl.bp));
-                    RT_CUDA(alloc(cap * 16, (void**)&pl.h0)); RT_CUDA(alloc(cap * 16, (void**)&pl.h1));
-                    RT_CUDA(alloc(cap * 16, (void**)&pl.h2)); RT_CUDA(alloc(cap * 16, (void**)&pl.pa));
-                    RT_CUDA(alloc(cap * 16, (void**)&pl.pb));
-                    if (wh)
-                    {
-                        RT_CUDA(alloc(cap * 16, (void**)&pl.w0)); RT_CUDA(alloc(cap * 16, (void**)&pl.w1));
-                        RT_CUDA(alloc(cap * 16, (void**)&pl.w2)); RT_CUDA(alloc(cap * 16, (void**)&pl.w3));
-                    }
-                    RT_CUDA(alloc(cap * lv * 16, (void**)&pl.st0)); RT_CUDA(alloc(cap * lv * 16, (void**)&pl.st1));
-                    RT_CUDA(alloc(cap * lv * 4, (void**)&pl.st2));
-                    RT_CUDA(alloc(cap * 4, (void**)&pp.queue[0])); RT_CUDA(alloc(cap * 4, (void**)&pp.queue[1]));
-                    RT_CUDA(alloc(cap * 4, (void**)&pp.longq));
-                    RT_CUDA(alloc(cap * 4, (void**)&pp.slowq));
-                    pl.cap = (unsigned)cap;
-                }
-                ctx->pool_cap = cap; ctx->pool_levels = lv; ctx->pool_whitted = wh;
-            }
+            if ((rc = grow_pools(ctx, pool_want, levels, whitted)) != RT_OK) return rc;
             for (int k = 0; k < RT_PIPES; k++)
             {
                 rt_gpu_ctx::Pipe& pp = ctx->pipes[k];
@@ -967,20 +1111,7 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
         // itself; the only cross-pipe order is fold(k) before fold(k+1) (AddPixel sums in pass order), so
         // the thin, latency-bound last rounds of chunk k overlap the dense first rounds of chunk k+1.
         RT_CUDA(cudaEventRecord(ctx->fork, ctx->stream));
-        // Any error return from here on leaves pipes with work in flight that the context stream has not been
-        // ordered after: wait for them on the way out, so that a later reset / readback / upload cannot race them.
-        struct PipeGuard
-        {
-            rt_gpu_ctx* ctx;
-            bool used[RT_PIPES];
-            bool joined;
-            ~PipeGuard()
-            {
-                if (joined) return;
-                for (int k = 0; k < RT_PIPES; k++)
-                    if (used[k]) cudaStreamSynchronize(ctx->pipes[k].stream);
-            }
-        } guard = { ctx, { false }, false };
+        PipeGuard guard = { ctx, { false }, false };
         bool (&used)[RT_PIPES] = guard.used;
         int chunk_index = 0, last_pipe = -1;
         // With frame slots in use consecutive calls rotate through the pipes, so that the next frame's chunks do
@@ -997,18 +1128,7 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
             a.num_items = (unsigned)((unsigned long long)a.num_samples * a.num_blocks * 32ull);
             a.samples = pp.samples;
             {
-                WaveArgs w;
-                memset(&w, 0, sizeof w);
-                w.pool = pp.pool;
-                w.queue[0] = pp.queue[0]; w.queue[1] = pp.queue[1];
-                w.counts = pp.round_counters; w.heads = pp.round_counters + RT_MAX_ROUNDS + 1;
-                w.longq = pp.longq; w.lcounts = w.heads + RT_MAX_ROUNDS; w.lheads = w.lcounts + RT_MAX_ROUNDS;
-                w.slowq = pp.slowq; w.scounts = w.lheads + RT_MAX_ROUNDS; w.sheads = w.scounts + RT_MAX_ROUNDS;
-                w.packet_probe = ctx->tune_packet_probe; w.packet_min_lanes = ctx->tune_packet_min_lanes;
-                w.long_limit = ctx->tune_long_limit; w.small_round = ctx->tune_small_round;
-                w.thin_count = ctx->tune_thin_count; w.thin_limit = ctx->tune_thin_limit;
-                w.packets = packet_rounds > 0 && mesh_shapes > 0 ? 1 : 0;
-                w.min_lanes = ctx->tune_min_lanes; w.leaf_wait = ctx->tune_leaf_wait; w.window = ctx->tune_window;
+                WaveArgs w = pipe_wave_args(ctx, pp, packet_rounds > 0 && mesh_shapes > 0 ? 1 : 0);
                 w.item_begin = 0u;
                 w.item_count = a.num_items;
                 unsigned gen_grid = (a.num_blocks * 32u + 255u) / 256u;
@@ -1056,71 +1176,9 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
                         const bool thin = ctx->tune_thin_from_round > 0 ? round >= ctx->tune_thin_from_round
                                         : (ctx->slots_touched >= 3 && npipes > 1 && ctx->tune_thin_from_round == 0 && seen_counts && round < RT_SEEN_ROUNDS &&
                                            seen_counts[round] < ctx->tune_thin_grid_count);
-                        if (mesh_shapes > 0)
-                        {
-                            if (ctx->time_walks)
-                            {
-                                while ((int)ctx->kev.size() < ctx->kev_used + 2)
-                                {
-                                    cudaEvent_t e = nullptr;
-                                    RT_CUDA(cudaEventCreate(&e));
-                                    ctx->kev.push_back(e);
-                                }
-                                RT_CUDA(cudaEventRecord(ctx->kev[ctx->kev_used], pp.stream));
-                            }
-                            if (round < packet_rounds)
-                            {
-                                // packets first; what they hand back (incoherent ones) goes on lane by lane
-                                RT_CUDA(mark(RT_KERNEL_PACKET_WALK, pp.stream));
-                                if (cull) rt_walk_packet_kernel<true><<<small_pass ? sms : walk_grid, 256, 0, pp.stream>>>(ctx->scene, a, w, round);
-                                else rt_walk_packet_kernel<false><<<small_pass ? sms : walk_grid, 256, 0, pp.stream>>>(ctx->scene, a, w, round);
-                                RT_CUDA(cudaGetLastError());
-                                ctx->launches++;
-                                RT_CUDA(mark(RT_KERNEL_WALK, pp.stream));
-                                RT_CUDA(launch_walk(cull, ctx->tune_top_stage, small_pass ? sms : walk_grid, pp.stream, ctx->scene, a, w, round, 1));
-                            }
-                            else if (cull && ctx->tune_octo)
-                            {
-                                // bounce / shadow rounds of the culled traversal: the 8-wide tree
-                                RT_CUDA(mark(RT_KERNEL_WALK, pp.stream));
-                                rt_walk_octo_kernel<<<(unsigned)(ctx->num_sms * ctx->octo_blocks_per_sm), 256, 0, pp.stream>>>(ctx->scene, a, w, round);
-                            }
-                            else
-                            {
-                                RT_CUDA(mark(RT_KERNEL_WALK, pp.stream));
-                                RT_CUDA(launch_walk(cull, ctx->tune_top_stage, small_pass ? sms : (thin ? walk_grid / 4u : walk_grid), pp.stream, ctx->scene, a, w, round, 0));
-                            }
-                            RT_CUDA(cudaGetLastError());
-                            const bool time_long = ctx->tune_time_long;     // tooling: bracket walk + long walk
-                            if (ctx->time_walks && !time_long)
-                            {
-                                RT_CUDA(cudaEventRecord(ctx->kev[ctx->kev_used + 1], pp.stream));
-                                ctx->kev_used += 2;
-                            }
-                            ctx->launches++;
-                            // the walks that kernel parked as too long, one warp each
-                            RT_CUDA(mark(RT_KERNEL_LONG_WALK, pp.stream));
-                            {
-                                const int group = ctx->tune_long_group;
-                                const unsigned lgrid = (unsigned)ctx->num_sms * ((thin || small_pass) ? 1u : (unsigned)RT_LONG_BLOCKS);
-    #define RT_LAUNCH_LONG(G) (cull ? rt_longwalk_kernel<true, G><<<lgrid, 256, 0, pp.stream>>>(ctx->scene, a, w, round) \
-                                    : rt_longwalk_kernel<false, G><<<lgrid, 256, 0, pp.stream>>>(ctx->scene, a, w, round))
-                                if (group == 32) RT_LAUNCH_LONG(32); else if (group == 16) RT_LAUNCH_LONG(16); else RT_LAUNCH_LONG(8);
-    #undef RT_LAUNCH_LONG
-                            }
-                            RT_CUDA(cudaGetLastError());
-                            if (ctx->time_walks && time_long)
-                            {
-                                RT_CUDA(cudaEventRecord(ctx->kev[ctx->kev_used + 1], pp.stream));
-                                ctx->kev_used += 2;
-                            }
-                            ctx->launches++;
-                        }
-                        RT_CUDA(mark(RT_KERNEL_SHADE, pp.stream));
-                        const unsigned sgrid = small_pass ? (sms < shade_grid ? sms : shade_grid) : (thin ? (shade_grid + 7u) / 8u : shade_grid);
-                        RT_CUDA(cull ? launch_shade<true>(p->mode, sgrid, pp.stream, ctx->scene, a, w, round)
-                                     : launch_shade<false>(p->mode, sgrid, pp.stream, ctx->scene, a, w, round));
-                        ctx->launches++;
+                        if ((rc = enqueue_round(ctx, pp, a, w, p->mode, round, cull, packet_rounds, mesh_shapes > 0, small_pass, thin,
+                                                walk_grid, shade_grid, true, mark)) != RT_OK)
+                            return rc;
                     }
                     if (pass == 0 && pp.seen_counts)
                     {
@@ -1159,6 +1217,102 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
         guard.joined = true;
         ctx->pipe_cursor = (pipe_base + chunk_index) % npipes;
         RT_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
+        return RT_OK;
+    });
+}
+
+// A batch of ray queries runs through the render's wavefront: query generate, then one round per mesh a ray can
+// reach (walks + long walks + shade in a query mode), on the pipes' pools and queues.  The batch is cut into pieces
+// that fit a pool (aligned to 32 rays, so that round-0 packets stay 32 consecutive rays of the caller's order) and the
+// pieces are dealt round-robin to the pipes, so that the tail of one overlaps the next.  Nothing that a later render
+// reads is touched: frame buffers and slot, ev0 / ev1, the pipe cursor and the round sizes remembered per pipe (the
+// quarter grids they steer are for frames in flight; a query round gets the full grids).
+int rt_gpu_query_rays(rt_gpu_ctx* ctx, const rt_ray_query* q, void* stream)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        if (!q) return fail(ctx, RT_ERR_INVALID, "rt_gpu_query_rays: query is null");
+        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_query_rays before rt_gpu_upload_scene");
+        if (q->n < 0) return fail(ctx, RT_ERR_INVALID, "rt_gpu_query_rays: negative ray count");
+        if (q->kind != RT_QUERY_NEAREST && q->kind != RT_QUERY_ANY) return fail(ctx, RT_ERR_INVALID, "rt_gpu_query_rays: unknown query kind");
+        if (q->traverse != RT_TRAVERSE_EXACT && q->traverse != RT_TRAVERSE_CULLED) return fail(ctx, RT_ERR_INVALID, "rt_gpu_query_rays: unknown traverse");
+        if (q->kind == RT_QUERY_ANY && (q->tri || q->hit))
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_query_rays: tri and hit are results of RT_QUERY_NEAREST only");
+        if (q->n == 0) return RT_OK;
+        if (!q->rays || !q->shape) return fail(ctx, RT_ERR_INVALID, "rt_gpu_query_rays: rays and shape are required");
+        RT_CUDA(cudaSetDevice(ctx->device));
+        const void* ptrs[4] = { q->rays, q->shape, q->tri, q->hit };
+        const char* names[4] = { "rays", "shape", "tri", "hit" };
+        for (int k = 0; k < 4; k++)
+        {
+            if (!ptrs[k]) continue;
+            cudaPointerAttributes at;
+            memset(&at, 0, sizeof at);
+            const cudaError_t e = cudaPointerGetAttributes(&at, ptrs[k]);
+            if (e != cudaSuccess) cudaGetLastError();
+            if (e != cudaSuccess || (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != ctx->device)
+                return fail(ctx, RT_ERR_INVALID, std::string("rt_gpu_query_rays: ") + names[k] + " is not device memory of the context's GPU");
+        }
+        int mesh_shapes = 0;
+        for (int i = 0; i < ctx->scene.num_shapes; i++) mesh_shapes += ctx->host_shape_is_mesh[i] ? 1 : 0;
+        const int rounds = mesh_shapes;                 // a query walks each mesh whose bounds it enters at most once
+        if (rounds >= RT_MAX_ROUNDS) return fail(ctx, RT_ERR_INVALID, "rt_gpu_query_rays: mesh shapes exceed the round table");
+        int rc = init_walk_grid(ctx);
+        if (rc != RT_OK) return rc;
+        const size_t n = (size_t)q->n;
+        size_t pool_want = 0;
+        if ((rc = plan_pools(ctx, (n + 255) & ~(size_t)255, 1, false, &pool_want)) != RT_OK) return rc;
+        if ((rc = grow_pools(ctx, pool_want, 1, false)) != RT_OK) return rc;
+        const size_t piece = pool_want & ~(size_t)31;   // path_alloc_packet takes 32 ids per warp with a live ray
+
+        const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+        const bool cull = q->traverse == RT_TRAVERSE_CULLED;
+        const int qmode = q->kind == RT_QUERY_ANY ? RT_QMODE_ANY : RT_QMODE_NEAREST;
+        const int packet_rounds = ctx->tune_packet_rounds >= 0 ? ctx->tune_packet_rounds : 1;
+        const unsigned walk_grid = (unsigned)(ctx->num_sms * ctx->walk_blocks_per_sm);
+        const int npipes = ctx->tune_pipes;
+        auto no_mark = [](int, cudaStream_t) -> cudaError_t { return cudaSuccess; };
+        RenderArgs a;
+        memset(&a, 0, sizeof a);
+        a.mode = qmode;
+        a.counters = ctx->counters;
+        a.exact = cull ? 0 : 1;
+        a.all_bounded = ctx->all_bounded ? 1 : 0;
+
+        RT_CUDA(cudaEventRecord(ctx->fork, st));
+        PipeGuard guard = { ctx, { false }, false };
+        int index = 0;
+        for (size_t begin = 0; begin < n; begin += piece, index++)
+        {
+            const size_t count = n - begin < piece ? n - begin : piece;
+            const int pipe = index % npipes;
+            rt_gpu_ctx::Pipe& pp = ctx->pipes[pipe];
+            if (!guard.used[pipe]) { RT_CUDA(cudaStreamWaitEvent(pp.stream, ctx->fork, 0)); guard.used[pipe] = true; }
+            a.q_rays = q->rays + 7 * begin;
+            a.q_count = (int)count;
+            a.q_shape = q->shape + begin;
+            a.q_tri = q->tri ? q->tri + begin : nullptr;
+            a.q_hit = q->hit ? q->hit + 11 * begin : nullptr;
+            WaveArgs w = pipe_wave_args(ctx, pp, packet_rounds > 0 && mesh_shapes > 0 ? 1 : 0);
+            w.item_count = (unsigned)count;
+            unsigned gen_grid = (unsigned)((count + 255) / 256);
+            if (gen_grid > (unsigned)ctx->num_sms * 8u) gen_grid = (unsigned)ctx->num_sms * 8u;
+            unsigned shade_grid = (unsigned)((count + 255) / 256);
+            if (shade_grid > (unsigned)ctx->num_sms * 16u) shade_grid = (unsigned)ctx->num_sms * 16u;
+            RT_CUDA(cudaMemsetAsync(pp.round_counters, 0, (6 * RT_MAX_ROUNDS + 1) * sizeof(unsigned), pp.stream));
+            RT_CUDA(cull ? launch_query_generate<true>(qmode, gen_grid, pp.stream, ctx->scene, a, w)
+                         : launch_query_generate<false>(qmode, gen_grid, pp.stream, ctx->scene, a, w));
+            ctx->launches++;
+            for (int round = 0; round < rounds; round++)
+                if ((rc = enqueue_round(ctx, pp, a, w, qmode, round, cull, packet_rounds, true, false, false,
+                                        walk_grid, shade_grid, false, no_mark)) != RT_OK)
+                    return rc;
+            RT_CUDA(cudaEventRecord(pp.done, pp.stream));
+        }
+        // join: `stream` continues after every pipe
+        for (int k = 0; k < RT_PIPES; k++)
+            if (guard.used[k]) RT_CUDA(cudaStreamWaitEvent(st, ctx->pipes[k].done, 0));
+        guard.joined = true;
         return RT_OK;
     });
 }

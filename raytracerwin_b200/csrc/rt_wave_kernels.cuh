@@ -110,12 +110,39 @@ __device__ __forceinline__ unsigned path_alloc_packet(unsigned* counter, bool wa
 // on the way back up its recursion.  The path runs the recursion forwards and keeps (att, colour,
 // emissive) per level in the pool so the fold runs in exactly the reference's order and rounding;
 // pass-through levels (:79-85, final = 0 + L_next) only set a bit.
+// A completed ray query (RT_QMODE_*): its result at the ray's place in the batch, with the fields and the
+// zeros-on-a-miss of rt_trace_rays_kernel (rt_hooks.cu).
+template <int MODE>
+__device__ __forceinline__ void query_result(const RenderArgs& a, int i, const Query& q)
+{
+    const int shape = q.hit_shape;
+    if (MODE == RT_QMODE_ANY) { a.q_shape[i] = shape >= 0 ? 1 : 0; return; }
+    a.q_shape[i] = shape;
+    if (a.q_tri) a.q_tri[i] = shape >= 0 ? q.tri : -1;
+    if (a.q_hit)
+    {
+        float* o = a.q_hit + 11 * (size_t)i;
+        if (shape >= 0)
+        {
+            o[0] = q.h.pos.x; o[1] = q.h.pos.y; o[2] = q.h.pos.z; o[3] = q.h.nrm.x; o[4] = q.h.nrm.y; o[5] = q.h.nrm.z;
+            o[6] = q.h.dist; o[7] = q.h.color.x; o[8] = q.h.color.y; o[9] = q.h.color.z; o[10] = q.h.alpha;
+        }
+        else
+            for (int k = 0; k < 11; k++) o[k] = 0.0f;
+    }
+}
+
 // Returns true when the path continues with `next` (query not yet begun); otherwise the path has
 // ended and its sample has been written.
 template <int MODE>
 __device__ __forceinline__ bool shade_query(const DevScene& sc, const RenderArgs& a, const PathPool& pool, unsigned id,
                                             const Query& q, PathState& s, Ray& next, bool& next_any)
 {
+    if (MODE == RT_QMODE_NEAREST || MODE == RT_QMODE_ANY)
+    {
+        query_result<MODE>(a, s.pixel, q);
+        return false;
+    }
     bool done = false, newseg = false;
     next_any = false;
     float3 L = V3(0, 0, 0);
@@ -404,6 +431,56 @@ rt_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w)
             // pool full: the item is turned away untouched (its counters too) and generated again by the retry pass
             if (full) cnt = before;
             queue_push(w.retry_out, w.retry_out_count, full, ((smp * a.num_blocks + bl) << 5) | (unsigned)lane_in_block);
+        }
+    }
+    flush_counters(cnt, a.counters, a.exact);
+}
+
+// ---- kernel Q: generate for a batch of ray queries (rt_gpu_query_rays) ---------------------------------------------
+// What rt_generate_kernel does up to its queue push, for the caller's rays: one thread per ray (grid-stride, whole
+// warps together), the shape list up to the first mesh whose bounds the ray enters.  A query that needs no walk — it
+// missed everything, hit only analytic shapes, or an analytic shape occluded it — writes its result on the spot; the
+// rest become pool records (pa.x = the ray's place in the batch) in round 0, allocated in packets of 32 so that a
+// round-0 packet is 32 consecutive rays of the caller's order.  The host hands a batch over in pieces that fit the
+// pool: no item is ever turned away here.
+template <bool CULL, int MODE>
+__global__ void __launch_bounds__(256, 2)
+rt_query_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w)
+{
+    Counters cnt = { 0, 0, 0, 0, 0, 0 };
+    const unsigned n = (unsigned)a.q_count;
+    const unsigned rounded = (n + 31u) & ~31u;
+    const unsigned stride = gridDim.x * blockDim.x;
+    for (unsigned t = blockIdx.x * blockDim.x + threadIdx.x; t < rounded; t += stride)
+    {
+        bool live = false;
+        Query q;
+        PathState s;
+        int state = ST_IDLE;
+        if (t < n)
+        {
+            const float* p = a.q_rays + 7 * (size_t)t;
+            Ray r; r.o = V3(p[0], p[1], p[2]); r.d = V3(p[3], p[4], p[5]); r.dist = p[6];
+            query_begin(q, r, MODE == RT_QMODE_ANY, cnt);
+            state = ST_SHAPES;
+            query_shapes<CULL>(sc, q, state, cnt);
+            live = state == ST_TRAVERSE;
+            if (!live) query_result<MODE>(a, (int)t, q);
+            s.pixel = (int)t; s.slot = 0; s.rng.key = 0; s.rng.n = 0;
+            s.depth_left = 0; s.sp = 0; s.pass_mask = 0; s.light = 0; s.seg_dist = r.dist;
+        }
+        unsigned spare = 0xffffffffu;
+        const unsigned id = path_alloc_packet(w.counts + 0, live, spare);
+        if (spare < w.pool.cap)
+        {
+            // filler of a packet: an entry every kernel skips
+            w.pool.cur[spare] = make_int4(0, -1, ST_IDLE, 0);
+            w.queue[0][spare] = spare;
+        }
+        if (live)
+        {
+            pool_store<MODE>(w.pool, id, q, state, s);
+            w.queue[0][id] = id;
         }
     }
     flush_counters(cnt, a.counters, a.exact);

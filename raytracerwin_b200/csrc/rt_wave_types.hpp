@@ -38,7 +38,19 @@ struct RenderArgs
     unsigned long long* counters;
     int exact;                  // traverse == RT_TRAVERSE_EXACT: node_tests/tri_tests are the visits
     int all_bounded;            // every shape has culling bounds (no plane): rays that miss them all see the sky
+    // ray queries (rt_gpu_query_rays, modes RT_QMODE_*): the caller's rays and result arrays, indexed by the ray's
+    // place in the batch (PathState::pixel); q_tri / q_hit may be null
+    const float* q_rays;
+    int q_count;
+    int* q_shape;
+    int* q_tri;
+    float* q_hit;
 };
+
+// Internal modes of the wavefront kernels next to the RT_MODE_* of the ABI: a batch of ray queries.  A completed
+// query writes its result and ends (no shading); ANY is the shadow query (pool record bit 256).
+#define RT_QMODE_NEAREST 4
+#define RT_QMODE_ANY 5
 
 __device__ __forceinline__ bool owns_pixel(const RenderArgs& a, int x, int y)
 {
