@@ -15,6 +15,8 @@
  *   rt_gpu_readback      replaces reading bitcolor[] / accuBuffer[] (:49,:77)
  *   rt_gpu_query_rays    FindIntersectionWithScene (RayTracerScene.cpp:99-125) and the shadow query of
  *                        CalculateLightColor (:152-164) on batches of the caller's rays in device memory
+ *   rt_gpu_radiance_rays RayTracerScene::RayTrace (RayTracerScene.cpp:31-97), its preview branch, or the Whitted
+ *                        composition, on batches of the caller's rays in device memory (own cameras, probes, bakes)
  *
  * Plain C: POD structs, pointers and sizes only.  No C++/STL/torch types cross the boundary.
  * Every entry returns 0 on success or a negative rt_status; rt_gpu_last_error() gives text.
@@ -260,6 +262,34 @@ typedef struct rt_ray_query {
  * those are read on the context's stream, so order it after `stream` before reading them.  Leaves the frame
  * buffers, the frame slot and rt_gpu_last_render_ms alone. */
 int rt_gpu_query_rays(rt_gpu_ctx* ctx, const rt_ray_query* q, void* stream);
+
+/* Radiance of the caller's rays: what render_tile computes for one camera ray, started from ray i of the batch
+ * instead — the path of RayTrace (RT_MODE_PATH), its UseBaseColor branch (RT_MODE_PREVIEW) or the Whitted composition
+ * (RT_MODE_WHITTED).  Ray i draws rand() from the stream rt_rng_key(seed, stream_i, sample) (include/rt_rng.h),
+ * starting at draw first_draw.  So render_tile's sample (pixel p, sample s) is reproduced bit for bit by its camera
+ * ray with stream_i = p, sample = s and first_draw = 0 (un-jittered) or 2 (a jittered ray has drawn its two offsets). */
+typedef struct rt_radiance_query {
+    const float* rays;          /* DEVICE, n x 7 {origin, direction, Distance} (as rt_ray_query), 4-byte aligned */
+    int32_t n;
+    int32_t mode;               /* RT_MODE_PATH, RT_MODE_PREVIEW or RT_MODE_WHITTED */
+    int32_t max_bounce;         /* MaxBounceTimes counting this segment, in [0, 32]; PATH/PREVIEW: 0 = black (RayTrace(ray, 0));
+                                   WHITTED ignores it */
+    int32_t traverse;           /* RT_TRAVERSE_* (same results either way) */
+    uint32_t seed;              /* ray i draws rand() from rt_rng_key(seed, stream_i, sample), starting at draw first_draw */
+    uint32_t sample;
+    const uint32_t* rng_stream; /* DEVICE, n, may be NULL: stream_i = rng_stream_base + i */
+    uint32_t rng_stream_base;
+    uint32_t first_draw;        /* draws already consumed (2 = a jittered camera ray of render_tile) */
+    float* rgba;                /* DEVICE, n x 4, 16-byte aligned: the radiance RayTrace / the Whitted composition returns, .w = 0 */
+} rt_radiance_query;
+
+/* Stream, ordering and pointer rules of rt_gpu_query_rays; n == 0 is a no-op.  Adds to the counters rays, shadow_rays
+ * (Whitted light rays), slab / triangle tests, mesh walks and hits; camera_rays is not touched.  Leaves the frame
+ * buffers, the frame slot and rt_gpu_last_render_ms alone.  RT_ERR_INVALID for another mode, max_bounce outside
+ * [0, 32], (segments) x (mesh shapes) walks per path beyond the round table (as render_tile counts them), NULL or
+ * misaligned rays / rgba, pointers that are not device memory of the context's GPU, and RT_MODE_PATH on a scene with
+ * Diffuse materials but no unit-vector table. */
+int rt_gpu_radiance_rays(rt_gpu_ctx* ctx, const rt_radiance_query* q, void* stream);
 
 /* Synchronises the stream, then copies `what` into caller memory (size-checked). */
 int rt_gpu_readback(rt_gpu_ctx* ctx, int what, void* dst, size_t bytes);

@@ -13,7 +13,7 @@ import os
 import numpy as np
 
 from . import _abi
-from ._abi import (rt_render_params, rt_counters, rt_scene_desc, rt_ray_query,  # noqa: F401
+from ._abi import (rt_render_params, rt_counters, rt_scene_desc, rt_ray_query, rt_radiance_query,  # noqa: F401
                    RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY, RT_QUERY_NEAREST, RT_QUERY_ANY,
                    RT_TRAVERSE_EXACT, RT_TRAVERSE_CULLED,
                    RT_READ_ACCUM_RGBN_F32, RT_READ_DISPLAY_ARGB8, RT_READ_PRIMARY_IDS_I32X2,
@@ -329,6 +329,29 @@ class GpuContext:
             shape.ctypes.data_as(_abi.PI32), tri.ctypes.data_as(_abi.PI32), hit.ctypes.data_as(_abi.PF)))
         return shape, tri, hit
 
+    def _device_tensor(self, name, t, dtype, shape):
+        """Checks that `t` is a contiguous torch tensor of `dtype` and `shape` (None = any length) on this GPU."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        if not isinstance(t, torch.Tensor):
+            raise ValueError(f"{name} must be a torch tensor on {dev}, not {type(t).__name__}")
+        if t.device != dev:
+            raise ValueError(f"{name} on {t.device}, but the context is on {dev}")
+        if t.dtype != dtype:
+            raise ValueError(f"{name} must be {dtype}, not {t.dtype}")
+        if t.dim() != len(shape) or any(s is not None and t.shape[k] != s for k, s in enumerate(shape)):
+            want = tuple("N" if s is None else s for s in shape)
+            raise ValueError(f"{name} must have shape {want}, not {tuple(t.shape)}")
+        if not t.is_contiguous():
+            raise ValueError(f"{name} must be contiguous")
+
+    @staticmethod
+    def _torch_stream(dev):
+        import torch
+        # torch names the legacy default stream 0, which the C calls would take for the context's own stream:
+        # pass it as cudaStreamLegacy (1) instead
+        return torch.cuda.current_stream(dev).cuda_stream or 1
+
     def query_rays(self, rays, any_hit=False, traverse=RT_TRAVERSE_CULLED, want_tri=None, want_hit=None):
         """Nearest-hit or occlusion queries of a batch of rays held in device memory (rt_gpu_query_rays).
 
@@ -340,17 +363,8 @@ class GpuContext:
         default to True for nearest-hit queries and to False for occlusion queries (which have neither).
         The context's counters are read on its own stream: synchronise before reading them."""
         import torch
-        if not isinstance(rays, torch.Tensor):
-            raise ValueError(f"rays must be a torch tensor on cuda:{self.device}, not {type(rays).__name__}")
+        self._device_tensor("rays", rays, torch.float32, (None, 7))
         dev = torch.device("cuda", self.device)
-        if rays.device != dev:
-            raise ValueError(f"rays are on {rays.device}, the context is on {dev}")
-        if rays.dtype != torch.float32:
-            raise ValueError(f"rays must be float32, not {rays.dtype}")
-        if rays.dim() != 2 or rays.shape[1] != 7:
-            raise ValueError(f"rays must have shape (N, 7), not {tuple(rays.shape)}")
-        if not rays.is_contiguous():
-            raise ValueError("rays must be contiguous")
         n = rays.shape[0]
         want_tri = not any_hit if want_tri is None else want_tri
         want_hit = not any_hit if want_hit is None else want_hit
@@ -359,13 +373,39 @@ class GpuContext:
         hit = torch.empty((n, 11), dtype=torch.float32, device=dev) if want_hit else None
         q = rt_ray_query(rays.data_ptr(), n, RT_QUERY_ANY if any_hit else RT_QUERY_NEAREST, traverse, shape.data_ptr(),
                          None if tri is None else tri.data_ptr(), None if hit is None else hit.data_ptr())
-        # torch names the legacy default stream 0, which rt_gpu_query_rays would take for the context's own stream:
-        # pass it as cudaStreamLegacy (1) instead
-        stream = torch.cuda.current_stream(dev).cuda_stream or 1
-        self._check(self._lib.rt_gpu_query_rays(self._h, C.byref(q), stream))
+        self._check(self._lib.rt_gpu_query_rays(self._h, C.byref(q), self._torch_stream(dev)))
         if any_hit:
             return shape
         return dict(shape=shape, tri=tri, hit=hit)
+
+    def radiance_rays(self, rays, mode=RT_MODE_PATH, max_bounce=10, seed=0, sample=0, rng_stream=None,
+                      rng_stream_base=0, first_draw=0, traverse=RT_TRAVERSE_CULLED, out=None):
+        """Radiance of a batch of rays held in device memory (rt_gpu_radiance_rays): RayTrace's path (RT_MODE_PATH), its
+        preview colour (RT_MODE_PREVIEW) or the Whitted composition (RT_MODE_WHITTED) of each ray, as render_tile
+        computes it for a camera ray.
+
+        `rays`: contiguous float32 torch tensor (N, 7) {origin, direction, Distance} on cuda:<self.device>.  Ray i draws
+        its random numbers from rt_rng_key(seed, stream_i, sample) starting at draw `first_draw`, with stream_i =
+        rng_stream[i] (an int32 (N,) tensor on the same device whose bits are the stream ids) or rng_stream_base + i.
+        `out`: optional contiguous float32 (N, 4) tensor on the same device to write into.  Enqueued on
+        torch.cuda.current_stream(self.device); returns the float32 (N, 4) tensor {r, g, b, 0}, usable on that stream
+        without a host synchronisation.  The context's counters are read on its own stream: synchronise before
+        reading them."""
+        import torch
+        self._device_tensor("rays", rays, torch.float32, (None, 7))
+        dev = torch.device("cuda", self.device)
+        n = rays.shape[0]
+        if rng_stream is not None:
+            self._device_tensor("rng_stream", rng_stream, torch.int32, (n,))
+        if out is None:
+            out = torch.empty((n, 4), dtype=torch.float32, device=dev)
+        else:
+            self._device_tensor("out", out, torch.float32, (n, 4))
+        q = rt_radiance_query(rays.data_ptr(), n, mode, max_bounce, traverse, seed & 0xFFFFFFFF, sample & 0xFFFFFFFF,
+                              None if rng_stream is None else rng_stream.data_ptr(), rng_stream_base & 0xFFFFFFFF,
+                              first_draw & 0xFFFFFFFF, out.data_ptr())
+        self._check(self._lib.rt_gpu_radiance_rays(self._h, C.byref(q), self._torch_stream(dev)))
+        return out
 
     def build_bvh(self, points, point_idx):
         """KdTree::Build on the device: (nodes, tris, depth, device ms) with the dtypes of Scene.flat_mesh."""

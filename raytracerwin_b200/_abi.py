@@ -92,6 +92,12 @@ class rt_ray_query(C.Structure):
                 ("shape", C.c_void_p), ("tri", C.c_void_p), ("hit", C.c_void_p)]
 
 
+class rt_radiance_query(C.Structure):
+    _fields_ = [("rays", C.c_void_p), ("n", C.c_int32), ("mode", C.c_int32), ("max_bounce", C.c_int32),
+                ("traverse", C.c_int32), ("seed", C.c_uint32), ("sample", C.c_uint32), ("rng_stream", C.c_void_p),
+                ("rng_stream_base", C.c_uint32), ("first_draw", C.c_uint32), ("rgba", C.c_void_p)]
+
+
 STRUCT_SIZES = {"rt_shape": 80, "rt_material": 28, "rt_bvh_node": 32, "rt_tri": 64, "rt_shade": 64,
                 "rt_light": 28, "rt_render_params": 56, "rt_counters": 72}
 
@@ -144,6 +150,7 @@ GPU_PROTOTYPES = {
     "rt_gpu_time_kernels": (I, [VP, I32]),
     "rt_gpu_build_bvh": (I, [VP, VP, I32, VP, I32, VP, VP, PI32, PF]),
     "rt_gpu_query_rays": (I, [VP, C.POINTER(rt_ray_query), VP]),
+    "rt_gpu_radiance_rays": (I, [VP, C.POINTER(rt_radiance_query), VP]),
     "rt_gpu_trace_rays": (I, [VP, PF, I32, I32, PI32, PI32, PF]),
     "rt_gpu_kat": (I, [VP, I32, VP, VP, I32, I32, VP, VP]),
     "rt_gpu_kat_texture": (I, [VP, I32, VP, I32, VP]),

@@ -441,7 +441,10 @@ __device__ __forceinline__ float cull_pad_for(const Ray& r, const RayPre& pre, f
     const float growth = scale * 1.52587890625e-05f;
     const float mi_x = pre.ex ? fabsf(pre.inv.x) : 0.0f, mi_y = pre.ey ? fabsf(pre.inv.y) : 0.0f, mi_z = pre.ez ? fabsf(pre.inv.z) : 0.0f;
     float pad = growth * fmaxf(fmaxf(mi_x, mi_y), mi_z) + growth;
-    if (!(pad <= FLT_MAX)) pad = FLT_MAX;      // NaN/inf: never cull
+    // NaN/inf: never cull.  Nor with a negative Distance (a bounce after a hit beyond the segment's end: the
+    // capsule test does not compare with Distance, and |d| > 1 makes a triangle's distance exceed it): the reference
+    // then accepts triangles BEHIND the origin, and an accepted hit makes Distance positive again
+    if (!(pad <= FLT_MAX) || !(r.dist >= 0.0f)) pad = FLT_MAX;
     return pad;
 }
 

@@ -205,10 +205,17 @@ static cudaError_t launch_shade(int mode, unsigned grid, cudaStream_t st, const 
 }
 
 template <bool CULL>
-static cudaError_t launch_query_generate(int qmode, unsigned grid, cudaStream_t st, const DevScene& sc, const RenderArgs& a, const WaveArgs& w)
+static cudaError_t launch_query_generate(int mode, unsigned grid, cudaStream_t st, const DevScene& sc, const RenderArgs& a, const WaveArgs& w)
 {
-    if (qmode == RT_QMODE_ANY) rt_query_generate_kernel<CULL, RT_QMODE_ANY><<<grid, 256, 0, st>>>(sc, a, w);
-    else rt_query_generate_kernel<CULL, RT_QMODE_NEAREST><<<grid, 256, 0, st>>>(sc, a, w);
+    switch (mode)
+    {
+    case RT_QMODE_NEAREST: rt_query_generate_kernel<CULL, RT_QMODE_NEAREST><<<grid, 256, 0, st>>>(sc, a, w); break;
+    case RT_QMODE_ANY: rt_query_generate_kernel<CULL, RT_QMODE_ANY><<<grid, 256, 0, st>>>(sc, a, w); break;
+    case RT_MODE_PATH: rt_query_generate_kernel<CULL, RT_MODE_PATH><<<grid, 256, 0, st>>>(sc, a, w); break;
+    case RT_MODE_PREVIEW: rt_query_generate_kernel<CULL, RT_MODE_PREVIEW><<<grid, 256, 0, st>>>(sc, a, w); break;
+    case RT_MODE_WHITTED: rt_query_generate_kernel<CULL, RT_MODE_WHITTED><<<grid, 256, 0, st>>>(sc, a, w); break;
+    default: return cudaErrorInvalidValue;
+    }
     return cudaGetLastError();
 }
 
@@ -435,6 +442,67 @@ static int enqueue_round(rt_gpu_ctx* ctx, rt_gpu_ctx::Pipe& pp, const RenderArgs
     RT_CUDA(cull ? launch_shade<true>(mode, sgrid, pp.stream, ctx->scene, a, w, round)
                  : launch_shade<false>(mode, sgrid, pp.stream, ctx->scene, a, w, round));
     ctx->launches++;
+    return RT_OK;
+}
+
+// rt_gpu_query_rays / rt_gpu_radiance_rays take device memory of the context's GPU only
+static bool on_device(const rt_gpu_ctx* ctx, const void* ptr)
+{
+    cudaPointerAttributes at;
+    memset(&at, 0, sizeof at);
+    const cudaError_t e = cudaPointerGetAttributes(&at, ptr);
+    if (e != cudaSuccess) cudaGetLastError();
+    return e == cudaSuccess && (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && at.device == ctx->device;
+}
+
+// A batch of n caller rays through the render's wavefront, ordered on `st`: query generate in `mode`, then `rounds`
+// rounds (walks + long walks + shade in `mode`) on the pipes' pools and queues.  The batch is cut into pieces of
+// `piece` rays (a multiple of 32 that fits a pool, so that round-0 packets stay 32 consecutive rays of the caller's
+// order) and the pieces are dealt round-robin to the pipes, so that the tail of one overlaps the next.
+// set_piece(a, begin, count) points the argument block at the piece's part of the caller's arrays.  Nothing that a
+// later render reads is touched: frame buffers and slot, ev0 / ev1, the pipe cursor and the round sizes remembered
+// per pipe (the quarter grids they steer are for frames in flight; a query round gets the full grids).
+template <typename SetPiece>
+static int enqueue_ray_batch(rt_gpu_ctx* ctx, RenderArgs& a, size_t n, size_t piece, int mode, int rounds, bool has_mesh,
+                             bool cull, cudaStream_t st, SetPiece set_piece)
+{
+    const int packet_rounds = ctx->tune_packet_rounds >= 0 ? ctx->tune_packet_rounds : 1;
+    const unsigned walk_grid = (unsigned)(ctx->num_sms * ctx->walk_blocks_per_sm);
+    const int npipes = ctx->tune_pipes;
+    auto no_mark = [](int, cudaStream_t) -> cudaError_t { return cudaSuccess; };
+    RT_CUDA(cudaEventRecord(ctx->fork, st));
+    PipeGuard guard = { ctx, { false }, false };
+    int index = 0;
+    for (size_t begin = 0; begin < n; begin += piece, index++)
+    {
+        const size_t count = n - begin < piece ? n - begin : piece;
+        const int pipe = index % npipes;
+        rt_gpu_ctx::Pipe& pp = ctx->pipes[pipe];
+        if (!guard.used[pipe]) { RT_CUDA(cudaStreamWaitEvent(pp.stream, ctx->fork, 0)); guard.used[pipe] = true; }
+        a.q_count = (int)count;
+        set_piece(a, begin, count);
+        WaveArgs w = pipe_wave_args(ctx, pp, packet_rounds > 0 && has_mesh ? 1 : 0);
+        w.item_count = (unsigned)count;
+        unsigned gen_grid = (unsigned)((count + 255) / 256);
+        if (gen_grid > (unsigned)ctx->num_sms * 8u) gen_grid = (unsigned)ctx->num_sms * 8u;
+        unsigned shade_grid = (unsigned)((count + 255) / 256);
+        if (shade_grid > (unsigned)ctx->num_sms * 16u) shade_grid = (unsigned)ctx->num_sms * 16u;
+        RT_CUDA(cudaMemsetAsync(pp.round_counters, 0, (6 * RT_MAX_ROUNDS + 1) * sizeof(unsigned), pp.stream));
+        RT_CUDA(cull ? launch_query_generate<true>(mode, gen_grid, pp.stream, ctx->scene, a, w)
+                     : launch_query_generate<false>(mode, gen_grid, pp.stream, ctx->scene, a, w));
+        ctx->launches++;
+        for (int round = 0; round < rounds; round++)
+        {
+            const int rc = enqueue_round(ctx, pp, a, w, mode, round, cull, packet_rounds, has_mesh, false, false,
+                                         walk_grid, shade_grid, false, no_mark);
+            if (rc != RT_OK) return rc;
+        }
+        RT_CUDA(cudaEventRecord(pp.done, pp.stream));
+    }
+    // join: `st` continues after every pipe
+    for (int k = 0; k < RT_PIPES; k++)
+        if (guard.used[k]) RT_CUDA(cudaStreamWaitEvent(st, ctx->pipes[k].done, 0));
+    guard.joined = true;
     return RT_OK;
 }
 
@@ -1221,12 +1289,8 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
     });
 }
 
-// A batch of ray queries runs through the render's wavefront: query generate, then one round per mesh a ray can
-// reach (walks + long walks + shade in a query mode), on the pipes' pools and queues.  The batch is cut into pieces
-// that fit a pool (aligned to 32 rays, so that round-0 packets stay 32 consecutive rays of the caller's order) and the
-// pieces are dealt round-robin to the pipes, so that the tail of one overlaps the next.  Nothing that a later render
-// reads is touched: frame buffers and slot, ev0 / ev1, the pipe cursor and the round sizes remembered per pipe (the
-// quarter grids they steer are for frames in flight; a query round gets the full grids).
+// A batch of ray queries runs through the render's wavefront (enqueue_ray_batch): query generate, then one round per
+// mesh a ray can reach, with the shade kernel in a query mode.
 int rt_gpu_query_rays(rt_gpu_ctx* ctx, const rt_ray_query* q, void* stream)
 {
     return rt_guard(ctx, [&]() -> int {
@@ -1244,15 +1308,8 @@ int rt_gpu_query_rays(rt_gpu_ctx* ctx, const rt_ray_query* q, void* stream)
         const void* ptrs[4] = { q->rays, q->shape, q->tri, q->hit };
         const char* names[4] = { "rays", "shape", "tri", "hit" };
         for (int k = 0; k < 4; k++)
-        {
-            if (!ptrs[k]) continue;
-            cudaPointerAttributes at;
-            memset(&at, 0, sizeof at);
-            const cudaError_t e = cudaPointerGetAttributes(&at, ptrs[k]);
-            if (e != cudaSuccess) cudaGetLastError();
-            if (e != cudaSuccess || (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != ctx->device)
+            if (ptrs[k] && !on_device(ctx, ptrs[k]))
                 return fail(ctx, RT_ERR_INVALID, std::string("rt_gpu_query_rays: ") + names[k] + " is not device memory of the context's GPU");
-        }
         int mesh_shapes = 0;
         for (int i = 0; i < ctx->scene.num_shapes; i++) mesh_shapes += ctx->host_shape_is_mesh[i] ? 1 : 0;
         const int rounds = mesh_shapes;                 // a query walks each mesh whose bounds it enters at most once
@@ -1268,52 +1325,88 @@ int rt_gpu_query_rays(rt_gpu_ctx* ctx, const rt_ray_query* q, void* stream)
         const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
         const bool cull = q->traverse == RT_TRAVERSE_CULLED;
         const int qmode = q->kind == RT_QUERY_ANY ? RT_QMODE_ANY : RT_QMODE_NEAREST;
-        const int packet_rounds = ctx->tune_packet_rounds >= 0 ? ctx->tune_packet_rounds : 1;
-        const unsigned walk_grid = (unsigned)(ctx->num_sms * ctx->walk_blocks_per_sm);
-        const int npipes = ctx->tune_pipes;
-        auto no_mark = [](int, cudaStream_t) -> cudaError_t { return cudaSuccess; };
         RenderArgs a;
         memset(&a, 0, sizeof a);
         a.mode = qmode;
         a.counters = ctx->counters;
         a.exact = cull ? 0 : 1;
         a.all_bounded = ctx->all_bounded ? 1 : 0;
+        return enqueue_ray_batch(ctx, a, n, piece, qmode, rounds, mesh_shapes > 0, cull, st,
+                                 [&](RenderArgs& pa, size_t begin, size_t) {
+                                     pa.q_rays = q->rays + 7 * begin;
+                                     pa.q_shape = q->shape + begin;
+                                     pa.q_tri = q->tri ? q->tri + begin : nullptr;
+                                     pa.q_hit = q->hit ? q->hit + 11 * begin : nullptr;
+                                 });
+    });
+}
 
-        RT_CUDA(cudaEventRecord(ctx->fork, st));
-        PipeGuard guard = { ctx, { false }, false };
-        int index = 0;
-        for (size_t begin = 0; begin < n; begin += piece, index++)
-        {
-            const size_t count = n - begin < piece ? n - begin : piece;
-            const int pipe = index % npipes;
-            rt_gpu_ctx::Pipe& pp = ctx->pipes[pipe];
-            if (!guard.used[pipe]) { RT_CUDA(cudaStreamWaitEvent(pp.stream, ctx->fork, 0)); guard.used[pipe] = true; }
-            a.q_rays = q->rays + 7 * begin;
-            a.q_count = (int)count;
-            a.q_shape = q->shape + begin;
-            a.q_tri = q->tri ? q->tri + begin : nullptr;
-            a.q_hit = q->hit ? q->hit + 11 * begin : nullptr;
-            WaveArgs w = pipe_wave_args(ctx, pp, packet_rounds > 0 && mesh_shapes > 0 ? 1 : 0);
-            w.item_count = (unsigned)count;
-            unsigned gen_grid = (unsigned)((count + 255) / 256);
-            if (gen_grid > (unsigned)ctx->num_sms * 8u) gen_grid = (unsigned)ctx->num_sms * 8u;
-            unsigned shade_grid = (unsigned)((count + 255) / 256);
-            if (shade_grid > (unsigned)ctx->num_sms * 16u) shade_grid = (unsigned)ctx->num_sms * 16u;
-            RT_CUDA(cudaMemsetAsync(pp.round_counters, 0, (6 * RT_MAX_ROUNDS + 1) * sizeof(unsigned), pp.stream));
-            RT_CUDA(cull ? launch_query_generate<true>(qmode, gen_grid, pp.stream, ctx->scene, a, w)
-                         : launch_query_generate<false>(qmode, gen_grid, pp.stream, ctx->scene, a, w));
-            ctx->launches++;
-            for (int round = 0; round < rounds; round++)
-                if ((rc = enqueue_round(ctx, pp, a, w, qmode, round, cull, packet_rounds, true, false, false,
-                                        walk_grid, shade_grid, false, no_mark)) != RT_OK)
-                    return rc;
-            RT_CUDA(cudaEventRecord(pp.done, pp.stream));
-        }
-        // join: `stream` continues after every pipe
-        for (int k = 0; k < RT_PIPES; k++)
-            if (guard.used[k]) RT_CUDA(cudaStreamWaitEvent(st, ctx->pipes[k].done, 0));
-        guard.joined = true;
-        return RT_OK;
+// Radiance of a batch of rays: the render's path (or preview / Whitted composition) from the caller's rays instead of
+// the camera's.  The query generate kernel starts each path; the walk, long-walk and shade kernels run in the plain
+// render mode, and the sample of ray i lands at rgba[i]: the piece's part of rgba is its sample buffer, one frame of
+// `count` x 1 pixels, sample slot 0.
+int rt_gpu_radiance_rays(rt_gpu_ctx* ctx, const rt_radiance_query* q, void* stream)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        if (!q) return fail(ctx, RT_ERR_INVALID, "rt_gpu_radiance_rays: query is null");
+        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_radiance_rays before rt_gpu_upload_scene");
+        if (q->n < 0) return fail(ctx, RT_ERR_INVALID, "rt_gpu_radiance_rays: negative ray count");
+        if (q->mode != RT_MODE_PATH && q->mode != RT_MODE_PREVIEW && q->mode != RT_MODE_WHITTED)
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_radiance_rays: mode must be RT_MODE_PATH, RT_MODE_PREVIEW or RT_MODE_WHITTED");
+        if (q->traverse != RT_TRAVERSE_EXACT && q->traverse != RT_TRAVERSE_CULLED) return fail(ctx, RT_ERR_INVALID, "rt_gpu_radiance_rays: unknown traverse");
+        if (q->max_bounce < 0 || q->max_bounce > RT_MAX_PATH_DEPTH) return fail(ctx, RT_ERR_INVALID, "rt_gpu_radiance_rays: max_bounce must be in [0, 32]");
+        if (q->mode == RT_MODE_PATH && ctx->needs_table && ctx->scene.num_unit_vectors == 0)
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_radiance_rays: scene has Diffuse materials but no unit-vector table (rt_host_set_unit_vectors)");
+        // rounds: one mesh walk per round; a path needs at most (segments) x (mesh shapes) walks (as render_tile counts)
+        int mesh_shapes = 0;
+        for (int i = 0; i < ctx->scene.num_shapes; i++) mesh_shapes += ctx->host_shape_is_mesh[i] ? 1 : 0;
+        const int segments = q->mode == RT_MODE_PATH ? (q->max_bounce > 0 ? q->max_bounce : 1)
+                           : q->mode == RT_MODE_WHITTED ? 1 + ctx->scene.num_lights : 1;
+        const int rounds = segments * (mesh_shapes > 0 ? mesh_shapes : 1);
+        if (rounds >= RT_MAX_ROUNDS) return fail(ctx, RT_ERR_INVALID, "rt_gpu_radiance_rays: segments x mesh shapes exceed the round table");
+        if (q->n == 0) return RT_OK;
+        if (!q->rays || !q->rgba) return fail(ctx, RT_ERR_INVALID, "rt_gpu_radiance_rays: rays and rgba are required");
+        RT_CUDA(cudaSetDevice(ctx->device));
+        const void* ptrs[3] = { q->rays, q->rng_stream, q->rgba };
+        const char* names[3] = { "rays", "rng_stream", "rgba" };
+        for (int k = 0; k < 3; k++)
+            if (ptrs[k] && !on_device(ctx, ptrs[k]))
+                return fail(ctx, RT_ERR_INVALID, std::string("rt_gpu_radiance_rays: ") + names[k] + " is not device memory of the context's GPU");
+        // (the samples are written as float4)
+        if ((uintptr_t)q->rgba % 16 != 0 || (uintptr_t)q->rays % 4 != 0 || (uintptr_t)q->rng_stream % 4 != 0)
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_radiance_rays: rgba must be 16-byte aligned, rays and rng_stream 4-byte aligned");
+        int rc = init_walk_grid(ctx);
+        if (rc != RT_OK) return rc;
+        const size_t n = (size_t)q->n;
+        const size_t levels = q->mode == RT_MODE_PATH ? (size_t)(q->max_bounce > 0 ? q->max_bounce : 1) : 1;
+        const bool whitted = q->mode == RT_MODE_WHITTED;
+        size_t pool_want = 0;
+        if ((rc = plan_pools(ctx, (n + 255) & ~(size_t)255, levels, whitted, &pool_want)) != RT_OK) return rc;
+        if ((rc = grow_pools(ctx, pool_want, levels, whitted)) != RT_OK) return rc;
+        const size_t piece = pool_want & ~(size_t)31;   // path_alloc_packet takes 32 ids per warp with a live ray
+
+        const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+        const bool cull = q->traverse == RT_TRAVERSE_CULLED;
+        RenderArgs a;
+        memset(&a, 0, sizeof a);
+        a.mode = q->mode;
+        a.max_bounce = q->max_bounce;
+        a.seed = q->seed;
+        a.q_sample = q->sample;
+        a.q_first_draw = q->first_draw;
+        a.height = 1;
+        a.counters = ctx->counters;
+        a.exact = cull ? 0 : 1;
+        a.all_bounded = ctx->all_bounded ? 1 : 0;
+        return enqueue_ray_batch(ctx, a, n, piece, q->mode, rounds, mesh_shapes > 0, cull, st,
+                                 [&](RenderArgs& pa, size_t begin, size_t count) {
+                                     pa.q_rays = q->rays + 7 * begin;
+                                     pa.q_stream = q->rng_stream ? q->rng_stream + begin : nullptr;
+                                     pa.q_stream_base = q->rng_stream_base + (uint32_t)begin;
+                                     pa.samples = reinterpret_cast<float4*>(q->rgba + 4 * begin);
+                                     pa.width = (int)count;
+                                 });
     });
 }
 

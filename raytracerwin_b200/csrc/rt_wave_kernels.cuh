@@ -443,10 +443,15 @@ rt_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w)
 // rest become pool records (pa.x = the ray's place in the batch) in round 0, allocated in packets of 32 so that a
 // round-0 packet is 32 consecutive rays of the caller's order.  The host hands a batch over in pieces that fit the
 // pool: no item is ever turned away here.
+// Radiance queries (rt_gpu_radiance_rays, MODE = RT_MODE_PATH / PREVIEW / WHITTED) start a whole path instead, as
+// rt_generate_kernel does after its camera ray: the ray's own RNG stream, the bounce budget, the sky on the spot for
+// a ray that hit nothing and has no mesh to walk, and a round-0 record for every other ray (analytic hits included:
+// the shade kernel shades them).  The sample of ray i is a.samples[i] (the host points it at the caller's rgba).
 template <bool CULL, int MODE>
 __global__ void __launch_bounds__(256, 2)
 rt_query_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w)
 {
+    constexpr bool radiance = MODE == RT_MODE_PATH || MODE == RT_MODE_PREVIEW || MODE == RT_MODE_WHITTED;
     Counters cnt = { 0, 0, 0, 0, 0, 0 };
     const unsigned n = (unsigned)a.q_count;
     const unsigned rounded = (n + 31u) & ~31u;
@@ -461,13 +466,40 @@ rt_query_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w
         {
             const float* p = a.q_rays + 7 * (size_t)t;
             Ray r; r.o = V3(p[0], p[1], p[2]); r.d = V3(p[3], p[4], p[5]); r.dist = p[6];
-            query_begin(q, r, MODE == RT_QMODE_ANY, cnt);
-            state = ST_SHAPES;
-            query_shapes<CULL>(sc, q, state, cnt);
-            live = state == ST_TRAVERSE;
-            if (!live) query_result<MODE>(a, (int)t, q);
-            s.pixel = (int)t; s.slot = 0; s.rng.key = 0; s.rng.n = 0;
+            s.pixel = (int)t; s.slot = 0;
             s.depth_left = 0; s.sp = 0; s.pass_mask = 0; s.light = 0; s.seg_dist = r.dist;
+            if (radiance)
+            {
+                const uint32_t stream_id = a.q_stream ? a.q_stream[t] : a.q_stream_base + t;
+                s.rng.key = rt_rng_key(a.seed, stream_id, a.q_sample); s.rng.n = a.q_first_draw;
+                s.depth_left = a.max_bounce;
+                s.w_pos = s.w_nrm = s.w_surface = s.w_sum = V3(0, 0, 0);
+                // RayTrace(ray, 0) returns black before any query (RayTracerScene.cpp:39-42)
+                if (MODE != RT_MODE_WHITTED && a.max_bounce == 0) a.samples[t] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+                else
+                {
+                    query_begin(q, r, false, cnt);
+                    state = ST_SHAPES;
+                    query_shapes<CULL>(sc, q, state, cnt);
+                    live = true;
+                    if (state == ST_SHADE && q.hit_shape == -1)
+                    {
+                        // nothing hit and no mesh to walk: RayTrace's miss branch (RayTracerScene.cpp:90-94)
+                        const float3 L = sky_color(r.d);
+                        a.samples[t] = make_float4(L.x, L.y, L.z, 0.0f);
+                        live = false;
+                    }
+                }
+            }
+            else
+            {
+                query_begin(q, r, MODE == RT_QMODE_ANY, cnt);
+                state = ST_SHAPES;
+                query_shapes<CULL>(sc, q, state, cnt);
+                live = state == ST_TRAVERSE;
+                if (!live) query_result<MODE>(a, (int)t, q);
+                s.rng.key = 0; s.rng.n = 0;
+            }
         }
         unsigned spare = 0xffffffffu;
         const unsigned id = path_alloc_packet(w.counts + 0, live, spare);
@@ -479,7 +511,11 @@ rt_query_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w
         }
         if (live)
         {
-            pool_store<MODE>(w.pool, id, q, state, s);
+            // (rt_generate_kernel's rule: a path ray whose only remaining chance is this last mesh is retired with the
+            // sky colour by the walk kernel itself if the walk finds nothing)
+            const bool sky_on_miss = (MODE == RT_MODE_PATH || MODE == RT_MODE_PREVIEW) && state == ST_TRAVERSE &&
+                                     q.hit_shape == -1 && q.si == sc.num_shapes - 1;
+            pool_store<MODE>(w.pool, id, q, state, s, sky_on_miss);
             w.queue[0][id] = id;
         }
     }
@@ -1253,7 +1289,7 @@ rt_longwalk_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, int 
             pad3.x = pre.ex ? growth * fabsf(pre.inv.x) + growth : FLT_MAX;
             pad3.y = pre.ey ? growth * fabsf(pre.inv.y) + growth : FLT_MAX;
             pad3.z = pre.ez ? growth * fabsf(pre.inv.z) + growth : FLT_MAX;
-            cull = finite3(r.o) && finite3(r.d) && growth < FLT_MAX;
+            cull = finite3(r.o) && finite3(r.d) && growth < FLT_MAX && r.dist >= 0.0f;    // (see cull_pad_for)
         }
         int i = __float_as_int(bp.w), best = cur.y;
         float3 bpos = xyz(bp);

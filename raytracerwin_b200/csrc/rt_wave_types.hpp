@@ -45,6 +45,12 @@ struct RenderArgs
     int* q_shape;
     int* q_tri;
     float* q_hit;
+    // radiance queries (rt_gpu_radiance_rays, modes RT_MODE_PATH / PREVIEW / WHITTED): ray i draws from
+    // rt_rng_key(seed, stream_i, q_sample) starting at draw q_first_draw, stream_i = q_stream[i] or q_stream_base + i
+    const uint32_t* q_stream;
+    uint32_t q_stream_base;
+    uint32_t q_sample;
+    uint32_t q_first_draw;
 };
 
 // Internal modes of the wavefront kernels next to the RT_MODE_* of the ABI: a batch of ray queries.  A completed
