@@ -17,6 +17,8 @@
  *                        CalculateLightColor (:152-164) on batches of the caller's rays in device memory
  *   rt_gpu_radiance_rays RayTracerScene::RayTrace (RayTracerScene.cpp:31-97), its preview branch, or the Whitted
  *                        composition, on batches of the caller's rays in device memory (own cameras, probes, bakes)
+ *   rt_gpu_update_mesh   new mesh geometry from device memory (tree rebuilt on the device) and moved analytic
+ *   rt_gpu_update_shapes shapes, without a new upload and without draining frames in flight
  *
  * Plain C: POD structs, pointers and sizes only.  No C++/STL/torch types cross the boundary.
  * Every entry returns 0 on success or a negative rt_status; rt_gpu_last_error() gives text.
@@ -290,6 +292,44 @@ typedef struct rt_radiance_query {
  * misaligned rays / rgba, pointers that are not device memory of the context's GPU, and RT_MODE_PATH on a scene with
  * Diffuse materials but no unit-vector table. */
 int rt_gpu_radiance_rays(rt_gpu_ctx* ctx, const rt_radiance_query* q, void* stream);
+
+/* ---- scene updates on device memory ---------------------------------------------------------------
+ * Geometry that moves (skinning, physics, a probe's surroundings) without a new rt_gpu_upload_scene.  After an
+ * update, every later render, query and radiance call returns exactly what it would after a fresh upload of the same
+ * scene with the mesh built by rt_host_add_mesh_arrays(points, point_idx, normals, normal_idx, ...) (the uploaded
+ * texture coordinates and texture slot of each triangle stay), or with the shape records given.
+ * Ordering: calls made on the context before an update see the old scene, calls made after it the new one, on any
+ * frame slot and any stream, with no host synchronisation by the caller.  The update reads its inputs in `stream`'s
+ * order (a cudaStream_t; NULL = the current frame slot's stream) and does not wait for frames in flight; it publishes
+ * on the device once the calls enqueued before it have finished with the old scene, and later calls wait for that on
+ * their streams.  Errors (RT_ERR_INVALID) leave the scene exactly as it was. */
+typedef struct rt_mesh_update {
+    const float* points;       /* DEVICE, num_points x 3, 4-byte aligned */
+    int32_t num_points;
+    const int32_t* point_idx;  /* DEVICE, num_tris x 3: triangle t = original triangle id t */
+    int32_t num_tris;          /* must equal the uploaded mesh's num_tris */
+    const float* normals;      /* DEVICE, num_normals x 3, or NULL: every corner gets its triangle's cross(p1-p0, p2-p0) */
+    int32_t num_normals;
+    const int32_t* normal_idx; /* DEVICE, num_tris x 3, or NULL (exactly when normals is NULL) */
+} rt_mesh_update;
+
+/* New geometry for the mesh of mesh shape `shape`: the tree is rebuilt on the device (rt_gpu_build_bvh's rules), the
+ * shading records, the shape's bounds (RAabb::Expand over all points) and the culling margin are recomputed.  The
+ * builder reads one count per tree level on the host, so the call RETURNS ONCE THE BUILD IS COMPLETE: it waits for
+ * `stream`'s earlier work and the build, not for renders on other streams.  The first update of a mesh allocates a
+ * spare set of its arrays (192 B per triangle).  RT_ERR_INVALID for NULL, misaligned or non-device pointers, a shape
+ * that is not a mesh or whose mesh another shape also references, num_tris other than the uploaded count, an
+ * uploaded mesh whose node count is not 2 * num_tris - 1 (a description the host layer never produces),
+ * num_points <= 0, normals without normal_idx or the reverse, and a point or normal index out of range (found on the
+ * device, before anything is published); RT_ERR_NO_SCENE before an upload. */
+int rt_gpu_update_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, void* stream);
+
+/* Copies `count` caller records (host memory, consumed before return) over shapes [first, first + count): moved
+ * spheres, planes, capsules and triangles, other materials.  type, mesh and has_bounds must equal the uploaded
+ * record's and material must be in range (RT_ERR_INVALID otherwise); of a mesh record only `material` is taken (its
+ * bounds are those of the mesh's current geometry).  Ordering as rt_gpu_update_mesh.  The records travel as kernel
+ * parameters, so the call returns at once: it never waits on the host for frames in flight. */
+int rt_gpu_update_shapes(rt_gpu_ctx* ctx, const rt_shape* shapes, int32_t first, int32_t count, void* stream);
 
 /* Synchronises the stream, then copies `what` into caller memory (size-checked). */
 int rt_gpu_readback(rt_gpu_ctx* ctx, int what, void* dst, size_t bytes);

@@ -2,7 +2,8 @@
  *
  * Not part of the drop-in boundary (include/rt_gpu.h): nothing here replaces a reference interface.  They read
  * the per-round bookkeeping of the wavefront after a render call made with rt_gpu_time_kernels(ctx, 1), so that
- * the round structure can be inspected without a profiler.  Every function synchronises the context. */
+ * the round structure can be inspected without a profiler; rt_gpu_debug_read_mesh reads a mesh's device arrays back.
+ * Every function synchronises the context. */
 #ifndef RT_GPU_DEBUG_H
 #define RT_GPU_DEBUG_H
 
@@ -23,6 +24,13 @@ int rt_gpu_debug_timeline(rt_gpu_ctx* ctx, float* begin_ms, float* end_ms, int32
 
 /* Long-walk queue sizes per round of the last batch on pipe 0. */
 int rt_gpu_debug_long(rt_gpu_ctx* ctx, uint32_t* lcounts, int32_t max_rounds);
+
+/* The current device arrays of mesh `mesh` (after every update enqueued so far): nodes (the uploaded num_nodes records,
+ * 2 * num_tris - 1 for a tree of its triangles and after any update; inner nodes
+ * with the right child in `tri` as the device keeps them), tris and shade (num_tris each, shade in LEAF order), the
+ * bounds {min xyz, max xyz} of the shape that references it and its culling margin.  Any output may be NULL. */
+int rt_gpu_debug_read_mesh(rt_gpu_ctx* ctx, int32_t mesh, rt_bvh_node* nodes, rt_tri* tris, rt_shade* shade, float* bounds6,
+                           float* cull_scale);
 
 #ifdef __cplusplus
 }

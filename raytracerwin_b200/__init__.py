@@ -13,7 +13,7 @@ import os
 import numpy as np
 
 from . import _abi
-from ._abi import (rt_render_params, rt_counters, rt_scene_desc, rt_ray_query, rt_radiance_query,  # noqa: F401
+from ._abi import (rt_render_params, rt_counters, rt_scene_desc, rt_ray_query, rt_radiance_query, rt_mesh_update,  # noqa: F401
                    RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY, RT_QUERY_NEAREST, RT_QUERY_ANY,
                    RT_TRAVERSE_EXACT, RT_TRAVERSE_CULLED,
                    RT_READ_ACCUM_RGBN_F32, RT_READ_DISPLAY_ARGB8, RT_READ_PRIMARY_IDS_I32X2,
@@ -37,6 +37,7 @@ def load_library():
         lib = C.CDLL(path)
         _abi.bind(lib, _abi.GPU_PROTOTYPES)
         _abi.bind(lib, _abi.HOST_PROTOTYPES)
+        _abi.bind(lib, _abi.DEBUG_PROTOTYPES)
         _lib = lib
     return _lib
 
@@ -241,6 +242,9 @@ class GpuContext:
     def upload_scene(self, scene):
         desc = scene.desc if isinstance(scene, Scene) else scene
         self._check(self._lib.rt_gpu_upload_scene(self._h, desc))
+        d = desc if isinstance(desc, rt_scene_desc) else getattr(desc, "contents", None)
+        self._uploaded_tris = {} if d is None else {i: (int(d.meshes[i].num_tris), int(d.meshes[i].num_nodes))
+                                                     for i in range(d.num_meshes)}
 
     def reset_accum(self, width, height):
         self._check(self._lib.rt_gpu_reset_accum(self._h, width, height))
@@ -406,6 +410,62 @@ class GpuContext:
                               first_draw & 0xFFFFFFFF, out.data_ptr())
         self._check(self._lib.rt_gpu_radiance_rays(self._h, C.byref(q), self._torch_stream(dev)))
         return out
+
+    def update_mesh(self, shape, points, point_idx, normals=None, normal_idx=None):
+        """New geometry for mesh shape `shape` from device memory (rt_gpu_update_mesh): the tree is rebuilt on the GPU.
+
+        `points` float32 (P, 3), `point_idx` int32 (T, 3) with T the uploaded triangle count, optional `normals`
+        float32 (Q, 3) with `normal_idx` int32 (T, 3) (without them every corner gets its triangle's geometric normal);
+        contiguous torch tensors on cuda:<self.device>.  Enqueued on torch.cuda.current_stream(self.device): the inputs
+        are read in that stream's order.  Returns once the build is complete (it waits for that stream's earlier work,
+        not for frames in flight); calls made after it see the new geometry, calls made before it the old one."""
+        import torch
+        self._device_tensor("points", points, torch.float32, (None, 3))
+        self._device_tensor("point_idx", point_idx, torch.int32, (None, 3))
+        if (normals is None) != (normal_idx is None):
+            raise ValueError("normals and normal_idx come together")
+        if normals is not None:
+            self._device_tensor("normals", normals, torch.float32, (None, 3))
+            self._device_tensor("normal_idx", normal_idx, torch.int32, (point_idx.shape[0], 3))
+        u = rt_mesh_update(points.data_ptr(), points.shape[0], point_idx.data_ptr(), point_idx.shape[0],
+                           None if normals is None else normals.data_ptr(), 0 if normals is None else normals.shape[0],
+                           None if normal_idx is None else normal_idx.data_ptr())
+        self._check(self._lib.rt_gpu_update_mesh(self._h, shape, C.byref(u),
+                                                 self._torch_stream(torch.device("cuda", self.device))))
+
+    def update_shapes(self, scene, first=0, count=None):
+        """Copies the flattened records [first, first + count) of host Scene `scene` over the uploaded shapes
+        (rt_gpu_update_shapes): moved analytic shapes, other materials.  Enqueued on torch.cuda.current_stream."""
+        import torch
+        desc = scene.desc.contents
+        count = desc.num_shapes - first if count is None else count
+        if first < 0 or count < 0 or first + count > desc.num_shapes:
+            raise ValueError(f"shapes [{first}, {first + count}) outside the scene's {desc.num_shapes}")
+        recs = C.cast(C.addressof(desc.shapes.contents) + first * C.sizeof(_abi.rt_shape), C.POINTER(_abi.rt_shape)) \
+            if count else None
+        self._check(self._lib.rt_gpu_update_shapes(self._h, recs, first, count,
+                                                   self._torch_stream(torch.device("cuda", self.device))))
+
+    def read_mesh(self, mesh):
+        """The device arrays of uploaded mesh `mesh` as they are now (rt_gpu_debug_read_mesh; synchronises): nodes,
+        tris and shade (leaf order) with the dtypes of Scene.flat_mesh, bounds float32 (6,), cull_scale."""
+        n, num_nodes = self._mesh_sizes(mesh)
+        node_dt = np.dtype([("bmin", "<f4", 3), ("escape", "<i4"), ("bmax", "<f4", 3), ("tri", "<i4")])
+        tri_dt = np.dtype([("p0", "<f4", 3), ("index", "<i4"), ("p1", "<f4", 3), ("pad0", "<f4"),
+                           ("p2", "<f4", 3), ("pad1", "<f4"), ("n", "<f4", 3), ("pad2", "<f4")])
+        shade_dt = np.dtype([("n0", "<f4", 3), ("n1", "<f4", 3), ("n2", "<f4", 3),
+                             ("uv0", "<f4", 2), ("uv1", "<f4", 2), ("uv2", "<f4", 2), ("texture", "<i4")])
+        nodes, tris, shade = np.zeros(num_nodes, node_dt), np.zeros(n, tri_dt), np.zeros(n, shade_dt)
+        bounds, scale = np.zeros(6, np.float32), C.c_float()
+        self._check(self._lib.rt_gpu_debug_read_mesh(self._h, mesh, nodes.ctypes.data, tris.ctypes.data, shade.ctypes.data,
+                                                     bounds.ctypes.data, C.byref(scale)))
+        return nodes, tris, shade, bounds, np.float32(scale.value)
+
+    def _mesh_sizes(self, mesh):
+        n = getattr(self, "_uploaded_tris", {}).get(mesh)
+        if n is None:
+            raise ValueError(f"mesh {mesh} of the uploaded scene is unknown")
+        return n
 
     def build_bvh(self, points, point_idx):
         """KdTree::Build on the device: (nodes, tris, depth, device ms) with the dtypes of Scene.flat_mesh."""

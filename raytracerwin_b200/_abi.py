@@ -98,6 +98,11 @@ class rt_radiance_query(C.Structure):
                 ("rng_stream_base", C.c_uint32), ("first_draw", C.c_uint32), ("rgba", C.c_void_p)]
 
 
+class rt_mesh_update(C.Structure):
+    _fields_ = [("points", C.c_void_p), ("num_points", C.c_int32), ("point_idx", C.c_void_p), ("num_tris", C.c_int32),
+                ("normals", C.c_void_p), ("num_normals", C.c_int32), ("normal_idx", C.c_void_p)]
+
+
 STRUCT_SIZES = {"rt_shape": 80, "rt_material": 28, "rt_bvh_node": 32, "rt_tri": 64, "rt_shade": 64,
                 "rt_light": 28, "rt_render_params": 56, "rt_counters": 72}
 
@@ -151,6 +156,8 @@ GPU_PROTOTYPES = {
     "rt_gpu_build_bvh": (I, [VP, VP, I32, VP, I32, VP, VP, PI32, PF]),
     "rt_gpu_query_rays": (I, [VP, C.POINTER(rt_ray_query), VP]),
     "rt_gpu_radiance_rays": (I, [VP, C.POINTER(rt_radiance_query), VP]),
+    "rt_gpu_update_mesh": (I, [VP, I32, C.POINTER(rt_mesh_update), VP]),
+    "rt_gpu_update_shapes": (I, [VP, C.POINTER(rt_shape), I32, I32, VP]),
     "rt_gpu_trace_rays": (I, [VP, PF, I32, I32, PI32, PI32, PF]),
     "rt_gpu_kat": (I, [VP, I32, VP, VP, I32, I32, VP, VP]),
     "rt_gpu_kat_texture": (I, [VP, I32, VP, I32, VP]),
@@ -187,6 +194,11 @@ HOST_PROTOTYPES = {
     "rt_host_free": (None, [VP]),
     "rt_host_write_png_argb": (I, [C.c_char_p, VP, I32, I32]),
     "rt_host_program_run": (I, [VP, I, I32, I32, I32, I32, U32, C.c_char_p, C.POINTER(C.c_double), C.POINTER(C.c_uint64)]),
+}
+
+# include/rt_gpu_debug.h (tooling; bound by load_library as well)
+DEBUG_PROTOTYPES = {
+    "rt_gpu_debug_read_mesh": (I, [VP, I32, VP, VP, VP, VP, PF]),
 }
 
 LIB_NAME = "librt_b200.so"

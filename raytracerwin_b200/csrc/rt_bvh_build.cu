@@ -22,6 +22,7 @@
 #include <vector>
 
 #include "rt_gpu.h"
+#include "rt_bvh_core.hpp"
 
 // library-internal helpers of rt_gpu.cu (the context is opaque here too)
 __attribute__((visibility("hidden"))) int rt_ctx_device(rt_gpu_ctx* ctx);
@@ -389,6 +390,42 @@ struct Buf
     }
 };
 
+// The scratch block: level counters, then every per-triangle array of the build, each 256-byte aligned
+struct Carve
+{
+    char* base; size_t off;
+    template <typename T> T* take(size_t n)
+    {
+        T* p = (T*)(base + off);
+        off += ((n ? n : 1) * sizeof(T) + 255) & ~(size_t)255;
+        return p;
+    }
+};
+
+struct Scratch
+{
+    int* counts;                                             // next_count, max_count, flag, -
+    float *cx, *cy, *cz, *gx, *gy, *gz; int *order[2], *sop[2]; Seg* segs[2];
+    unsigned long long *kmin, *kmax; float *mean, *big_sum; int *axis, *nl, *flags, *pre, *sums;
+};
+
+size_t carve(void* base, int T, Scratch* s)
+{
+    Scratch tmp;
+    if (!s) s = &tmp;
+    Carve c = { (char*)base, 0 };
+    s->counts = c.take<int>(4);
+    s->cx = c.take<float>(T); s->cy = c.take<float>(T); s->cz = c.take<float>(T);
+    s->gx = c.take<float>(T); s->gy = c.take<float>(T); s->gz = c.take<float>(T);
+    for (int k = 0; k < 2; k++) { s->order[k] = c.take<int>(T); s->sop[k] = c.take<int>(T); s->segs[k] = c.take<Seg>(T); }
+    s->big_sum = c.take<float>(3 * (size_t)T);
+    s->kmin = c.take<unsigned long long>(3 * (size_t)T); s->kmax = c.take<unsigned long long>(3 * (size_t)T);
+    s->mean = c.take<float>(T); s->axis = c.take<int>(T); s->nl = c.take<int>(T);
+    s->flags = c.take<int>(T); s->pre = c.take<int>((size_t)T + 1);
+    s->sums = c.take<int>((size_t)(T + SCAN_BLOCK - 1) / SCAN_BLOCK + 1);
+    return c.off;
+}
+
 } // namespace
 
 #define BV_CUDA(call)                                                                       \
@@ -400,6 +437,57 @@ struct Buf
             return RT_ERR_CUDA;                                                             \
         }                                                                                   \
     } while (0)
+
+size_t rt_bvh_scratch_bytes(int num_tris) { return carve(nullptr, num_tris, nullptr); }
+int* rt_bvh_scratch_flag(void* scratch) { return (int*)scratch + 2; }
+
+int rt_bvh_build_core(rt_gpu_ctx* ctx, const float* dP, const int* dI, int T, cudaStream_t st, void* scratch, int* host_counts,
+                      bool check_flag, const char* message, rt_bvh_node* dnodes, rt_tri* dtris, int* out_depth)
+{
+    Scratch s;
+    carve(scratch, T, &s);
+    const int tb = 256, pg = (T + tb - 1) / tb;
+    const int nb = (T + SCAN_BLOCK - 1) / SCAN_BLOCK;
+    k_centroids<<<pg, tb, 0, st>>>(dP, dI, T, s.cx, s.cy, s.cz, s.order[0], s.sop[0]);
+    const Seg root = { 0, T, 0 };
+    BV_CUDA(cudaMemcpyAsync(s.segs[0], &root, sizeof root, cudaMemcpyHostToDevice, st));
+    int num_segs = 1, depth = 0, cur = 0, level_max = T;
+    while (num_segs > 0)
+    {
+        depth++;
+        Level L;
+        L.P = dP; L.I = dI; L.cx = s.cx; L.cy = s.cy; L.cz = s.cz; L.gx = s.gx; L.gy = s.gy; L.gz = s.gz;
+        L.order = s.order[cur]; L.order_next = s.order[cur ^ 1];
+        L.seg_of_pos = s.sop[cur]; L.seg_of_pos_next = s.sop[cur ^ 1];
+        L.segs = s.segs[cur]; L.segs_next = s.segs[cur ^ 1];
+        L.num_segs = num_segs; L.next_count = s.counts;
+        L.kmin = s.kmin; L.kmax = s.kmax; L.mean = s.mean; L.axis = s.axis; L.nl = s.nl; L.flags = s.flags; L.pre = s.pre;
+        L.nodes = dnodes; L.tris = dtris; L.T = T; L.big_sum = s.big_sum; L.max_count = s.counts + 1;
+        BV_CUDA(cudaMemsetAsync(s.counts, 0, 2 * sizeof(int), st));
+        k_init_keys<<<(3 * num_segs + tb - 1) / tb, tb, 0, st>>>(s.kmin, s.kmax, 3 * num_segs);
+        k_bounds<<<pg, tb, 0, st>>>(L);
+        k_gather<<<pg, tb, 0, st>>>(L);
+        if (level_max > BIG_SEG) k_sum_big<<<num_segs, 64, 0, st>>>(L);
+        k_nodes<<<(num_segs + 63) / 64, 64, 0, st>>>(L);
+        k_flags<<<pg, tb, 0, st>>>(L);
+        k_block_sums<<<nb, SCAN_BLOCK, 0, st>>>(s.flags, T, s.sums);
+        k_scan_sums<<<1, SCAN_BLOCK, 0, st>>>(s.sums, nb);
+        k_block_scan<<<nb, SCAN_BLOCK, 0, st>>>(s.flags, T, s.sums, s.pre);
+        k_children<<<(num_segs + tb - 1) / tb, tb, 0, st>>>(L);
+        k_scatter<<<pg, tb, 0, st>>>(L);
+        BV_CUDA(cudaGetLastError());
+        // one read per level: the next level's segment count and largest segment (and, first, the caller's flag)
+        const bool first = depth == 1 && check_flag;
+        BV_CUDA(cudaMemcpyAsync(host_counts, s.counts, (first ? 3 : 2) * sizeof(int), cudaMemcpyDeviceToHost, st));
+        BV_CUDA(cudaStreamSynchronize(st));
+        if (first && host_counts[2] != 0) { rt_ctx_set_error(ctx, message); return RT_ERR_INVALID; }
+        num_segs = host_counts[0]; level_max = host_counts[1];
+        cur ^= 1;
+        if (depth > 4096) { rt_ctx_set_error(ctx, "rt_gpu_build_bvh: runaway depth"); return RT_ERR_CUDA; }
+    }
+    if (out_depth) *out_depth = depth;
+    return RT_OK;
+}
 
 extern "C" int rt_gpu_build_bvh(rt_gpu_ctx* ctx, const float* points, int32_t num_points, const int32_t* indices,
                                 int32_t num_tris, rt_bvh_node* out_nodes, rt_tri* out_tris, int32_t* out_depth, float* out_ms)
@@ -425,62 +513,18 @@ extern "C" int rt_gpu_build_bvh(rt_gpu_ctx* ctx, const float* points, int32_t nu
     cudaStream_t st = (cudaStream_t)rt_gpu_stream(ctx);
     const int T = num_tris;
     Buf buf;
-    float* dP; int* dI; float *cx, *cy, *cz, *gx, *gy, *gz; int *order[2], *sop[2]; Seg* segs[2]; int* next_count;
-    unsigned long long *kmin, *kmax; float *mean, *big_sum; int *axis, *nl, *flags, *pre, *sums, *max_count; rt_bvh_node* dnodes; rt_tri* dtris;
+    float* dP; int* dI; char* scratch; rt_bvh_node* dnodes; rt_tri* dtris;
     BV_CUDA(buf.alloc(&dP, 3 * (size_t)num_points)); BV_CUDA(buf.alloc(&dI, 3 * (size_t)T));
-    BV_CUDA(buf.alloc(&cx, T)); BV_CUDA(buf.alloc(&cy, T)); BV_CUDA(buf.alloc(&cz, T));
-    BV_CUDA(buf.alloc(&gx, T)); BV_CUDA(buf.alloc(&gy, T)); BV_CUDA(buf.alloc(&gz, T));
-    for (int k = 0; k < 2; k++) { BV_CUDA(buf.alloc(&order[k], T)); BV_CUDA(buf.alloc(&sop[k], T)); BV_CUDA(buf.alloc(&segs[k], T)); }
-    BV_CUDA(buf.alloc(&next_count, 1)); BV_CUDA(buf.alloc(&max_count, 1)); BV_CUDA(buf.alloc(&big_sum, 3 * (size_t)T));
-    BV_CUDA(buf.alloc(&kmin, 3 * (size_t)T)); BV_CUDA(buf.alloc(&kmax, 3 * (size_t)T));
-    BV_CUDA(buf.alloc(&mean, T)); BV_CUDA(buf.alloc(&axis, T)); BV_CUDA(buf.alloc(&nl, T));
-    BV_CUDA(buf.alloc(&flags, T)); BV_CUDA(buf.alloc(&pre, (size_t)T + 1));
-    const int nb = (T + SCAN_BLOCK - 1) / SCAN_BLOCK;
-    BV_CUDA(buf.alloc(&sums, (size_t)nb + 1));
+    BV_CUDA(buf.alloc(&scratch, rt_bvh_scratch_bytes(T)));
     BV_CUDA(buf.alloc(&dnodes, 2 * (size_t)T)); BV_CUDA(buf.alloc(&dtris, T));
     BV_CUDA(cudaMemcpyAsync(dP, points, 3 * (size_t)num_points * sizeof(float), cudaMemcpyHostToDevice, st));
     BV_CUDA(cudaMemcpyAsync(dI, indices, 3 * (size_t)T * sizeof(int), cudaMemcpyHostToDevice, st));
     cudaEvent_t e0, e1;
     BV_CUDA(cudaEventCreate(&e0)); BV_CUDA(cudaEventCreate(&e1));
     BV_CUDA(cudaEventRecord(e0, st));
-    const int tb = 256, pg = (T + tb - 1) / tb;
-    k_centroids<<<pg, tb, 0, st>>>(dP, dI, T, cx, cy, cz, order[0], sop[0]);
-    const Seg root = { 0, T, 0 };
-    BV_CUDA(cudaMemcpyAsync(segs[0], &root, sizeof root, cudaMemcpyHostToDevice, st));
-    int num_segs = 1, depth = 0, cur = 0, level_max = T;
-    while (num_segs > 0)
-    {
-        depth++;
-        Level L;
-        L.P = dP; L.I = dI; L.cx = cx; L.cy = cy; L.cz = cz; L.gx = gx; L.gy = gy; L.gz = gz;
-        L.order = order[cur]; L.order_next = order[cur ^ 1];
-        L.seg_of_pos = sop[cur]; L.seg_of_pos_next = sop[cur ^ 1];
-        L.segs = segs[cur]; L.segs_next = segs[cur ^ 1];
-        L.num_segs = num_segs; L.next_count = next_count;
-        L.kmin = kmin; L.kmax = kmax; L.mean = mean; L.axis = axis; L.nl = nl; L.flags = flags; L.pre = pre;
-        L.nodes = dnodes; L.tris = dtris; L.T = T; L.big_sum = big_sum; L.max_count = max_count;
-        BV_CUDA(cudaMemsetAsync(next_count, 0, sizeof(int), st));
-        BV_CUDA(cudaMemsetAsync(max_count, 0, sizeof(int), st));
-        k_init_keys<<<(3 * num_segs + tb - 1) / tb, tb, 0, st>>>(kmin, kmax, 3 * num_segs);
-        k_bounds<<<pg, tb, 0, st>>>(L);
-        k_gather<<<pg, tb, 0, st>>>(L);
-        if (level_max > BIG_SEG) k_sum_big<<<num_segs, 64, 0, st>>>(L);
-        k_nodes<<<(num_segs + 63) / 64, 64, 0, st>>>(L);
-        k_flags<<<pg, tb, 0, st>>>(L);
-        k_block_sums<<<nb, SCAN_BLOCK, 0, st>>>(flags, T, sums);
-        k_scan_sums<<<1, SCAN_BLOCK, 0, st>>>(sums, nb);
-        k_block_scan<<<nb, SCAN_BLOCK, 0, st>>>(flags, T, sums, pre);
-        k_children<<<(num_segs + tb - 1) / tb, tb, 0, st>>>(L);
-        k_scatter<<<pg, tb, 0, st>>>(L);
-        BV_CUDA(cudaGetLastError());
-        int next = 0, mc = 0;
-        BV_CUDA(cudaMemcpyAsync(&next, next_count, sizeof(int), cudaMemcpyDeviceToHost, st));
-        BV_CUDA(cudaMemcpyAsync(&mc, max_count, sizeof(int), cudaMemcpyDeviceToHost, st));
-        BV_CUDA(cudaStreamSynchronize(st));
-        num_segs = next; level_max = mc;
-        cur ^= 1;
-        if (depth > 4096) { rt_ctx_set_error(ctx, "rt_gpu_build_bvh: runaway depth"); return RT_ERR_CUDA; }
-    }
+    int counts[4] = { 0, 0, 0, 0 }, depth = 0;
+    const int rc = rt_bvh_build_core(ctx, dP, dI, T, st, scratch, counts, false, nullptr, dnodes, dtris, &depth);
+    if (rc != RT_OK) { cudaEventDestroy(e0); cudaEventDestroy(e1); return rc; }
     BV_CUDA(cudaEventRecord(e1, st));
     BV_CUDA(cudaMemcpyAsync(out_nodes, dnodes, (2 * (size_t)T - 1) * sizeof(rt_bvh_node), cudaMemcpyDeviceToHost, st));
     BV_CUDA(cudaMemcpyAsync(out_tris, dtris, (size_t)T * sizeof(rt_tri), cudaMemcpyDeviceToHost, st));

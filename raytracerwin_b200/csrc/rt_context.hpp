@@ -120,7 +120,37 @@ struct rt_gpu_ctx
     int tune_few_chunks = 0;                    // RT_FEW_CHUNKS: pass chunks of a call of few camera rays (0: 2, or 1 with frame slots)
     size_t tune_sample_budget = 0;              // RT_SAMPLE_BUDGET_MB at create (0: by call size)
     bool tune_time_long = false;                // RT_TIME_LONG at create: timed brackets span walk + long walk
+
+    // ---- scene updates (rt_gpu_update_mesh / rt_gpu_update_shapes) ----
+    // What the updates check and swap, per uploaded shape and mesh.  A mesh's arrays are double-buffered from its first
+    // update on: an update builds into the spare set and publishes it; the published set becomes the spare.
+    std::vector<rt_shape> host_shapes;          // the records as uploaded (materials follow rt_gpu_update_shapes)
+    int host_num_materials = 0;
+    struct MeshArrays { rt_bvh_node* nodes; rt_tri* tris; rt_shade* shade; };
+    struct MeshState
+    {
+        int num_tris = 0;
+        int num_nodes = 0;                      // as uploaded: an update builds 2 * num_tris - 1
+        int users = 0;                          // shapes that reference the mesh
+        MeshArrays cur = { nullptr, nullptr, nullptr };      // published (shade in leaf order)
+        MeshArrays spare = { nullptr, nullptr, nullptr };    // allocated by the first update
+    };
+    std::vector<MeshState> mesh_state;
+    // Recorded by every update after it has published; every later scene reader waits for it on its stream.  Live from
+    // the first update of an upload on (no update: no event, no wait).
+    cudaEvent_t scene_event = nullptr;
+    bool scene_event_live = false;
+    cudaEvent_t join_event = nullptr;           // one record per context stream when an update publishes
+    void* update_scratch = nullptr;             // the builder's scratch block and the update's temporaries (only grows)
+    size_t update_scratch_cap = 0;
+    int* update_counts = nullptr;               // PINNED HOST: the builder's per-level read
 };
+
+// A scene reader enqueued on `st` runs after the last published update
+static inline cudaError_t wait_scene(const rt_gpu_ctx* ctx, cudaStream_t st)
+{
+    return ctx->scene_event_live ? cudaStreamWaitEvent(st, ctx->scene_event, 0) : cudaSuccess;
+}
 
 extern thread_local std::string g_create_error;
 

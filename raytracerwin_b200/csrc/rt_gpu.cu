@@ -28,6 +28,7 @@
 // The whole file is compiled with -fmad=false; see rt_device.cuh.
 #include "rt_context.hpp"
 #include "rt_wave_kernels.cuh"
+#include "rt_bvh_core.hpp"
 
 thread_local std::string g_create_error;
 
@@ -107,6 +108,139 @@ __global__ void rt_shade_leaf_order_kernel(const float4* __restrict__ tris, cons
     const int index = __float_as_int(tris[4 * (size_t)k].w);        // rt_tri.index: the triangle's place in the original order
 #pragma unroll
     for (int j = 0; j < 4; j++) out[4 * (size_t)k + j] = shade[4 * (size_t)index + j];
+}
+
+// ---- scene updates (rt_gpu_update_mesh) ----
+// Bit flags of the update's input check (the builder's scratch flag)
+#define RT_UPD_BAD_POINT_INDEX 1
+#define RT_UPD_BAD_NORMAL_INDEX 2
+
+// Checks every point / normal index and copies the point indices into `safe` with bad ones replaced by 0, so that the
+// builder never reads outside `points` even before the host has seen the flag (the build is then thrown away).
+__global__ void rt_update_check_kernel(const int* __restrict__ pidx, int num_points, const int* __restrict__ nidx, int num_normals,
+                                       int n, int* __restrict__ safe, int* __restrict__ flag)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int v = pidx[i], bad = 0;
+    if (v < 0 || v >= num_points) { v = 0; bad |= RT_UPD_BAD_POINT_INDEX; }
+    safe[i] = v;
+    if (nidx) { const int w = nidx[i]; if (w < 0 || w >= num_normals) bad |= RT_UPD_BAD_NORMAL_INDEX; }
+    if (bad) atomicOr(flag, bad);
+}
+
+// Shading records in ORIGINAL triangle order: the new normals (normals[nidx], or every corner the triangle's
+// unnormalised geometric normal as host/mesh_loader.cpp computes it), uv and texture slot from the published record.
+// Published leaf record j belongs to triangle cur_tris[j].index.
+__global__ void rt_update_shade_kernel(const float4* __restrict__ cur_tris, const float* __restrict__ cur_shade,
+                                       const float* __restrict__ points, const int* __restrict__ pidx,
+                                       const float* __restrict__ normals, const int* __restrict__ nidx, float* __restrict__ out, int n)
+{
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const int t = __float_as_int(cur_tris[4 * (size_t)j].w);
+    const float* src = cur_shade + 16 * (size_t)j;
+    float* dst = out + 16 * (size_t)t;
+    if (normals)
+        for (int k = 0; k < 3; k++)
+        {
+            const float* v = normals + 3 * (size_t)nidx[3 * (size_t)t + k];
+            dst[3 * k] = v[0]; dst[3 * k + 1] = v[1]; dst[3 * k + 2] = v[2];
+        }
+    else
+    {
+        const float* p0 = points + 3 * (size_t)pidx[3 * (size_t)t];
+        const float* p1 = points + 3 * (size_t)pidx[3 * (size_t)t + 1];
+        const float* p2 = points + 3 * (size_t)pidx[3 * (size_t)t + 2];
+        const float ax = p1[0] - p0[0], ay = p1[1] - p0[1], az = p1[2] - p0[2];
+        const float bx = p2[0] - p0[0], by = p2[1] - p0[1], bz = p2[2] - p0[2];
+        const float nx = ay * bz - az * by, ny = az * bx - ax * bz, nz = ax * by - ay * bx;
+        for (int k = 0; k < 3; k++) { dst[3 * k] = nx; dst[3 * k + 1] = ny; dst[3 * k + 2] = nz; }
+    }
+    for (int k = 9; k < 16; k++) dst[k] = src[k];           // uv0 uv1 uv2 texture
+}
+
+// RAabb::Expand over the points in array order as 64-bit keys: value order in the high word (-0 == +0, as `<`
+// sees them), the point index in the low word so that ties go to the FIRST occurrence (min: index, max: ~index).
+__device__ __forceinline__ unsigned upd_ord_bits(float v)
+{
+    unsigned b = __float_as_uint(v);
+    if (v == 0.0f) b = 0u;
+    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+}
+
+__global__ void rt_update_bounds_kernel(const float* __restrict__ points, int num_points, unsigned long long* keys)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned long long mn[3] = { ~0ull, ~0ull, ~0ull }, mx[3] = { 0ull, 0ull, 0ull };
+    if (i < num_points)
+        for (int c = 0; c < 3; c++)
+        {
+            const float v = points[3 * (size_t)i + c];
+            if (v != v) continue;                                   // NaN never wins a < or > test
+            const unsigned long long o = (unsigned long long)upd_ord_bits(v) << 32;
+            mn[c] = o | (unsigned)i; mx[c] = o | (0xFFFFFFFFu - (unsigned)i);
+        }
+    for (int c = 0; c < 3; c++)
+    {
+        for (int o = 16; o > 0; o >>= 1)
+        {
+            const unsigned long long a = __shfl_xor_sync(0xffffffffu, mn[c], o), b = __shfl_xor_sync(0xffffffffu, mx[c], o);
+            if (a < mn[c]) mn[c] = a;
+            if (b > mx[c]) mx[c] = b;
+        }
+        if ((threadIdx.x & 31) == 0)
+        {
+            if (mn[c] != ~0ull) atomicMin(keys + c, mn[c]);
+            if (mx[c] != 0ull) atomicMax(keys + 3 + c, mx[c]);
+        }
+    }
+}
+
+// The publication of an update (one thread, after the join): the mesh's record points at the new arrays, with the
+// culling margin of the new root (as upload computes it) and without the 8-wide copy; the shape gets the new bounds.
+// Kernels read both records at run time.
+__global__ void rt_update_publish_kernel(DevMesh* meshes, int mesh, rt_shape* shapes, int shape, const rt_bvh_node* nodes,
+                                         const rt_tri* tris, const rt_shade* shade, const unsigned long long* keys, const float* points)
+{
+    float scale = 0.0f;
+    for (int k = 0; k < 3; k++)
+    {
+        scale = fmaxf(scale, fabsf(nodes[0].bmin[k]));
+        scale = fmaxf(scale, fabsf(nodes[0].bmax[k]));
+    }
+    DevMesh& m = meshes[mesh];
+    m.nodes = (const float4*)nodes; m.tris = (const float4*)tris; m.shade = (const float4*)shade;
+    m.octo = nullptr;
+    m.cull_scale = scale;
+    rt_shape& s = shapes[shape];
+    for (int c = 0; c < 3; c++)
+    {
+        float lo = FLT_MAX, hi = -FLT_MAX;                       // RAabb's empty box
+        if (keys[c] != ~0ull)
+        {
+            const float v = points[3 * (size_t)(unsigned)(keys[c] & 0xFFFFFFFFull) + c];
+            if (v < lo) lo = v;
+        }
+        if (keys[3 + c] != 0ull)
+        {
+            const float v = points[3 * (size_t)(0xFFFFFFFFu - (unsigned)(keys[3 + c] & 0xFFFFFFFFull)) + c];
+            if (v > hi) hi = v;
+        }
+        s.bounds_min[c] = lo; s.bounds_max[c] = hi;
+    }
+}
+
+// rt_gpu_update_shapes: caller records over the device's; a mesh record gives its material only.  The records travel
+// as the kernel's parameter (copied at launch: no staging buffer, nothing for the host to wait for).
+#define RT_SHAPES_PER_LAUNCH 48                       // 48 x 80 B: within the classic 4 KB parameter space
+struct ShapeBatch { rt_shape rec[RT_SHAPES_PER_LAUNCH]; };
+__global__ void rt_update_shapes_kernel(rt_shape* shapes, ShapeBatch src, int count)
+{
+    const int k = threadIdx.x;
+    if (k >= count) return;
+    if (src.rec[k].type == RT_SHAPE_MESH) shapes[k].material = src.rec[k].material;
+    else shapes[k] = src.rec[k];
 }
 
 static void free_scene(rt_gpu_ctx* ctx)
@@ -470,6 +604,7 @@ static int enqueue_ray_batch(rt_gpu_ctx* ctx, RenderArgs& a, size_t n, size_t pi
     const unsigned walk_grid = (unsigned)(ctx->num_sms * ctx->walk_blocks_per_sm);
     const int npipes = ctx->tune_pipes;
     auto no_mark = [](int, cudaStream_t) -> cudaError_t { return cudaSuccess; };
+    RT_CUDA(wait_scene(ctx, st));
     RT_CUDA(cudaEventRecord(ctx->fork, st));
     PipeGuard guard = { ctx, { false }, false };
     int index = 0;
@@ -575,8 +710,12 @@ int rt_gpu_destroy(rt_gpu_ctx* ctx)
         if (!ctx) return RT_OK;
         cudaSetDevice(ctx->device);
         sync_all_streams(ctx);
+        if (ctx->scene_event_live) cudaEventSynchronize(ctx->scene_event);
         free_scene(ctx);
         free_frame(ctx);
+        cudaFree(ctx->update_scratch);
+        if (ctx->update_counts) cudaFreeHost(ctx->update_counts);
+        for (cudaEvent_t e : { ctx->scene_event, ctx->join_event }) if (e) cudaEventDestroy(e);
         for (int k = 0; k < RT_FRAME_SLOTS; k++)
         {
             if (k == ctx->slot) continue;
@@ -682,7 +821,10 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
 
         RT_CUDA(cudaSetDevice(ctx->device));
         RT_CUDA(sync_all_streams(ctx));
+        if (ctx->scene_event_live) RT_CUDA(cudaEventSynchronize(ctx->scene_event));    // an update on a caller's stream
+        ctx->scene_event_live = false;
         free_scene(ctx);
+        ctx->host_shapes.clear(); ctx->mesh_state.clear();
 
         DevScene d;
         memset(&d, 0, sizeof d);
@@ -786,6 +928,10 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
                 RT_CUDA(cudaGetLastError());
             }
             dm.nodes = (const float4*)dn; dm.tris = (const float4*)dt; dm.shade = (const float4*)dsh;
+            ctx->mesh_state.emplace_back();
+            ctx->mesh_state.back().num_tris = m.num_tris;
+            ctx->mesh_state.back().num_nodes = m.num_nodes;
+            ctx->mesh_state.back().cur = rt_gpu_ctx::MeshArrays{ dn, dt, (rt_shade*)dsh };
             dm.octo = nullptr;
             if (m.num_nodes > 0 && ctx->tune_octo)
             {
@@ -941,6 +1087,10 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
         for (int i = 0; i < s->num_shapes; i++) ctx->host_shape_is_mesh[i] = s->shapes[i].type == RT_SHAPE_MESH ? 1 : 0;
         ctx->all_bounded = true;
         for (int i = 0; i < s->num_shapes; i++) if (!s->shapes[i].has_bounds) ctx->all_bounded = false;
+        ctx->host_shapes.assign(s->shapes, s->shapes + s->num_shapes);
+        ctx->host_num_materials = s->num_materials;
+        for (int i = 0; i < s->num_shapes; i++)
+            if (s->shapes[i].type == RT_SHAPE_MESH) ctx->mesh_state[s->shapes[i].mesh].users++;
         return RT_OK;
     });
 }
@@ -1019,6 +1169,7 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
             int rc = rt_gpu_reset_accum(ctx, p->width, p->height);
             if (rc != RT_OK) return rc;
         }
+        RT_CUDA(wait_scene(ctx, ctx->stream));
         RT_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
         ctx->timed = true;
         ctx->kev_used = 0;
@@ -1407,6 +1558,181 @@ int rt_gpu_radiance_rays(rt_gpu_ctx* ctx, const rt_radiance_query* q, void* stre
                                      pa.samples = reinterpret_cast<float4*>(q->rgba + 4 * begin);
                                      pa.width = (int)count;
                                  });
+    });
+}
+
+// Every stream of the context that runs scene readers (the frame slots' streams and the pipes, onto which render calls
+// and queries fork) has finished what was enqueued on it before this call, in `st`'s order: the join of an update.
+static int join_scene_readers(rt_gpu_ctx* ctx, cudaStream_t st)
+{
+    if (!ctx->join_event) RT_CUDA(cudaEventCreateWithFlags(&ctx->join_event, cudaEventDisableTiming));
+    auto join = [&](cudaStream_t s) -> cudaError_t {
+        if (!s || s == st) return cudaSuccess;
+        cudaError_t e = cudaEventRecord(ctx->join_event, s);
+        return e == cudaSuccess ? cudaStreamWaitEvent(st, ctx->join_event, 0) : e;
+    };
+    RT_CUDA(join(ctx->stream));
+    for (int k = 0; k < RT_FRAME_SLOTS; k++)
+        if (k != ctx->slot) RT_CUDA(join(ctx->parked[k].stream));
+    for (int k = 0; k < RT_PIPES; k++) RT_CUDA(join(ctx->pipes[k].stream));
+    return RT_OK;
+}
+
+static int publish_done(rt_gpu_ctx* ctx, cudaStream_t st)
+{
+    if (!ctx->scene_event) RT_CUDA(cudaEventCreateWithFlags(&ctx->scene_event, cudaEventDisableTiming));
+    RT_CUDA(cudaEventRecord(ctx->scene_event, st));
+    ctx->scene_event_live = true;
+    return RT_OK;
+}
+
+// Stream-ordered device memory that lives as long as the context or the scene
+static int alloc_on(rt_gpu_ctx* ctx, void** out, size_t bytes, cudaStream_t st)
+{
+    *out = nullptr;
+    RT_CUDA(cudaMallocAsync(out, bytes, st));
+    return RT_OK;
+}
+
+static inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+int rt_gpu_update_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, void* stream)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_update_mesh before rt_gpu_upload_scene");
+        if (!u) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: update is null");
+        if (shape < 0 || shape >= (int)ctx->host_shapes.size() || ctx->host_shapes[shape].type != RT_SHAPE_MESH)
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: shape is not a mesh shape of the scene");
+        const int mi = ctx->host_shapes[shape].mesh;
+        rt_gpu_ctx::MeshState& ms = ctx->mesh_state[mi];
+        if (ms.users != 1) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: another shape references the same mesh");
+        if (ms.num_tris <= 0 || u->num_tris != ms.num_tris)
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: num_tris differs from the uploaded mesh's");
+        // the update publishes a tree of 2T-1 nodes in an array of that size; the walks read num_nodes as uploaded
+        if (ms.num_nodes != 2 * ms.num_tris - 1)
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: the uploaded mesh's node count is not 2 * num_tris - 1 (not a tree of its triangles)");
+        if ((long long)ms.num_tris * 3 >= 0xFFFFFFFFll) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: too many triangles");
+        if (u->num_points <= 0) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: num_points must be positive");
+        if (!u->points || !u->point_idx) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: points and point_idx are required");
+        if ((u->normals == nullptr) != (u->normal_idx == nullptr))
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: normals and normal_idx come together");
+        if (u->normals && u->num_normals <= 0) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: num_normals must be positive");
+        const void* ptrs[4] = { u->points, u->point_idx, u->normals, u->normal_idx };
+        const char* names[4] = { "points", "point_idx", "normals", "normal_idx" };
+        for (int k = 0; k < 4; k++)
+            if (ptrs[k] && (uintptr_t)ptrs[k] % 4 != 0)
+                return fail(ctx, RT_ERR_INVALID, std::string("rt_gpu_update_mesh: ") + names[k] + " must be 4-byte aligned");
+        RT_CUDA(cudaSetDevice(ctx->device));
+        for (int k = 0; k < 4; k++)
+            if (ptrs[k] && !on_device(ctx, ptrs[k]))
+                return fail(ctx, RT_ERR_INVALID, std::string("rt_gpu_update_mesh: ") + names[k] + " is not device memory of the context's GPU");
+        const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+        const int T = ms.num_tris;
+        // the spare set and the scratch block were last read by work the previous update waited for
+        RT_CUDA(wait_scene(ctx, st));
+        int rc;
+        if (!ms.spare.nodes)
+        {
+            rt_gpu_ctx::MeshArrays a = { nullptr, nullptr, nullptr };
+            if ((rc = alloc_on(ctx, (void**)&a.nodes, (2 * (size_t)T - 1) * sizeof(rt_bvh_node), st)) != RT_OK) return rc;
+            ctx->scene_allocs.push_back(a.nodes);
+            if ((rc = alloc_on(ctx, (void**)&a.tris, (size_t)T * sizeof(rt_tri), st)) != RT_OK) return rc;
+            ctx->scene_allocs.push_back(a.tris);
+            if ((rc = alloc_on(ctx, (void**)&a.shade, (size_t)T * sizeof(rt_shade), st)) != RT_OK) return rc;
+            ctx->scene_allocs.push_back(a.shade);
+            ctx->scene_bytes += (2 * (size_t)T - 1) * sizeof(rt_bvh_node) + (size_t)T * (sizeof(rt_tri) + sizeof(rt_shade));
+            ms.spare = a;
+        }
+        // scratch: the builder's block, safe point indices (3T), shading records in original order (T), bounds keys (6)
+        const size_t build_bytes = align256(rt_bvh_scratch_bytes(T));
+        const size_t idx_off = build_bytes, shade_off = idx_off + align256(3 * (size_t)T * sizeof(int));
+        const size_t keys_off = shade_off + align256((size_t)T * sizeof(rt_shade));
+        const size_t need = keys_off + 6 * sizeof(unsigned long long);
+        if (need > ctx->update_scratch_cap)
+        {
+            if (ctx->update_scratch) RT_CUDA(cudaFreeAsync(ctx->update_scratch, st));
+            ctx->update_scratch = nullptr; ctx->update_scratch_cap = 0;
+            if ((rc = alloc_on(ctx, &ctx->update_scratch, need, st)) != RT_OK) return rc;
+            ctx->update_scratch_cap = need;
+        }
+        if (!ctx->update_counts) RT_CUDA(cudaHostAlloc((void**)&ctx->update_counts, 4 * sizeof(int), cudaHostAllocDefault));
+        char* scratch = (char*)ctx->update_scratch;
+        int* safe_idx = (int*)(scratch + idx_off);
+        rt_shade* shade_tmp = (rt_shade*)(scratch + shade_off);
+        unsigned long long* keys = (unsigned long long*)(scratch + keys_off);
+        int* flag = rt_bvh_scratch_flag(scratch);
+
+        const int n3 = 3 * T;
+        RT_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), st));
+        rt_update_check_kernel<<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(u->point_idx, u->num_points, u->normal_idx,
+                                                                              u->normals ? u->num_normals : 0, n3, safe_idx, flag);
+        RT_CUDA(cudaGetLastError());
+        ctx->launches++;
+        rc = rt_bvh_build_core(ctx, u->points, safe_idx, T, st, scratch, ctx->update_counts, true,
+                               "rt_gpu_update_mesh: point or normal index out of range", ms.spare.nodes, ms.spare.tris, nullptr);
+        if (rc != RT_OK) return rc;
+        rt_patch_right_child<<<(unsigned)((2 * T - 1 + 255) / 256), 256, 0, st>>>(ms.spare.nodes, 2 * T - 1);
+        rt_update_shade_kernel<<<(unsigned)((T + 255) / 256), 256, 0, st>>>((const float4*)ms.cur.tris, (const float*)ms.cur.shade,
+                                                                            u->points, safe_idx, u->normals, u->normal_idx, (float*)shade_tmp, T);
+        rt_shade_leaf_order_kernel<<<(unsigned)((T + 255) / 256), 256, 0, st>>>((const float4*)ms.spare.tris, (const float4*)shade_tmp,
+                                                                                (float4*)ms.spare.shade, T);
+        RT_CUDA(cudaMemsetAsync(keys, 0xFF, 3 * sizeof(unsigned long long), st));
+        RT_CUDA(cudaMemsetAsync(keys + 3, 0, 3 * sizeof(unsigned long long), st));
+        rt_update_bounds_kernel<<<(unsigned)((u->num_points + 255) / 256), 256, 0, st>>>(u->points, u->num_points, keys);
+        RT_CUDA(cudaGetLastError());
+        ctx->launches += 4;
+        // publish once every call enqueued before this one has finished reading the old arrays
+        if ((rc = join_scene_readers(ctx, st)) != RT_OK) return rc;
+        rt_update_publish_kernel<<<1, 1, 0, st>>>(const_cast<DevMesh*>(ctx->scene.meshes), mi, const_cast<rt_shape*>(ctx->scene.shapes),
+                                                  shape, ms.spare.nodes, ms.spare.tris, ms.spare.shade, keys, u->points);
+        RT_CUDA(cudaGetLastError());
+        ctx->launches++;
+        if ((rc = publish_done(ctx, st)) != RT_OK) return rc;
+        std::swap(ms.cur, ms.spare);
+        // the shared-memory stage holds mesh 0's uploaded top levels; a pointer test cannot tell the ping-pong's arrays apart
+        if (mi == 0) ctx->scene.top_of = nullptr;
+        return RT_OK;
+    });
+}
+
+int rt_gpu_update_shapes(rt_gpu_ctx* ctx, const rt_shape* shapes, int32_t first, int32_t count, void* stream)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_update_shapes before rt_gpu_upload_scene");
+        const int num = (int)ctx->host_shapes.size();
+        if (first < 0 || count < 0 || first > num || count > num - first)
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_shapes: [first, first + count) is not a range of the scene's shapes");
+        if (count == 0) return RT_OK;
+        if (!shapes) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_shapes: shapes is null");
+        for (int k = 0; k < count; k++)
+        {
+            const rt_shape& r = shapes[k];
+            const rt_shape& up = ctx->host_shapes[first + k];
+            if (r.type != up.type || r.mesh != up.mesh || r.has_bounds != up.has_bounds)
+                return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_shapes: type, mesh and has_bounds must stay those of the upload");
+            if (r.material < -1 || r.material >= ctx->host_num_materials)
+                return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_shapes: material index out of range");
+        }
+        RT_CUDA(cudaSetDevice(ctx->device));
+        const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+        RT_CUDA(wait_scene(ctx, st));
+        int rc = join_scene_readers(ctx, st);
+        if (rc != RT_OK) return rc;
+        for (int b = 0; b < count; b += RT_SHAPES_PER_LAUNCH)
+        {
+            const int n = count - b < RT_SHAPES_PER_LAUNCH ? count - b : RT_SHAPES_PER_LAUNCH;
+            ShapeBatch batch;
+            memset(&batch, 0, sizeof batch);
+            memcpy(batch.rec, shapes + b, (size_t)n * sizeof(rt_shape));
+            rt_update_shapes_kernel<<<1, RT_SHAPES_PER_LAUNCH, 0, st>>>(const_cast<rt_shape*>(ctx->scene.shapes) + first + b, batch, n);
+            RT_CUDA(cudaGetLastError());
+            ctx->launches++;
+        }
+        if ((rc = publish_done(ctx, st)) != RT_OK) return rc;
+        for (int k = 0; k < count; k++) ctx->host_shapes[first + k].material = shapes[k].material;
+        return RT_OK;
     });
 }
 

@@ -160,6 +160,42 @@ int rt_gpu_debug_long(rt_gpu_ctx* ctx, uint32_t* lcounts, int32_t max_rounds)
     return RT_OK;
 }
 
+int rt_gpu_debug_read_mesh(rt_gpu_ctx* ctx, int32_t mesh, rt_bvh_node* nodes, rt_tri* tris, rt_shade* shade, float* bounds6,
+                           float* cull_scale)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_debug_read_mesh before rt_gpu_upload_scene");
+        if (mesh < 0 || mesh >= ctx->scene.num_meshes) return fail(ctx, RT_ERR_INVALID, "rt_gpu_debug_read_mesh: mesh out of range");
+        RT_CUDA(cudaSetDevice(ctx->device));
+        if (ctx->scene_event_live) RT_CUDA(cudaEventSynchronize(ctx->scene_event));
+        RT_CUDA(cudaStreamSynchronize(ctx->stream));
+        // the record the kernels read, not the host's bookkeeping
+        DevMesh m;
+        RT_CUDA(cudaMemcpyAsync(&m, ctx->scene.meshes + mesh, sizeof m, cudaMemcpyDeviceToHost, ctx->stream));
+        RT_CUDA(cudaStreamSynchronize(ctx->stream));
+        const size_t T = (size_t)m.num_tris;
+        if (nodes && m.num_nodes > 0)
+            RT_CUDA(cudaMemcpyAsync(nodes, m.nodes, (size_t)m.num_nodes * sizeof(rt_bvh_node), cudaMemcpyDeviceToHost, ctx->stream));
+        if (tris && T) RT_CUDA(cudaMemcpyAsync(tris, m.tris, T * sizeof(rt_tri), cudaMemcpyDeviceToHost, ctx->stream));
+        if (shade && T) RT_CUDA(cudaMemcpyAsync(shade, m.shade, T * sizeof(rt_shade), cudaMemcpyDeviceToHost, ctx->stream));
+        if (bounds6)
+        {
+            int si = -1;
+            for (size_t k = 0; k < ctx->host_shapes.size() && si < 0; k++)
+                if (ctx->host_shapes[k].type == RT_SHAPE_MESH && ctx->host_shapes[k].mesh == mesh) si = (int)k;
+            if (si < 0) return fail(ctx, RT_ERR_INVALID, "rt_gpu_debug_read_mesh: no shape references the mesh");
+            rt_shape rec;
+            RT_CUDA(cudaMemcpyAsync(&rec, ctx->scene.shapes + si, sizeof rec, cudaMemcpyDeviceToHost, ctx->stream));
+            RT_CUDA(cudaStreamSynchronize(ctx->stream));
+            for (int c = 0; c < 3; c++) { bounds6[c] = rec.bounds_min[c]; bounds6[3 + c] = rec.bounds_max[c]; }
+        }
+        RT_CUDA(cudaStreamSynchronize(ctx->stream));
+        if (cull_scale) *cull_scale = m.cull_scale;
+        return RT_OK;
+    });
+}
+
 int rt_gpu_trace_rays(rt_gpu_ctx* ctx, const float* rays, int32_t n, int32_t traverse, int32_t* shape, int32_t* tri, float* hit11)
 {
     return rt_guard(ctx, [&]() -> int {
@@ -174,6 +210,7 @@ int rt_gpu_trace_rays(rt_gpu_ctx* ctx, const float* rays, int32_t n, int32_t tra
         if (e == cudaSuccess) e = cudaMalloc((void**)&dtri, (size_t)n * sizeof(int));
         if (e == cudaSuccess) e = cudaMalloc((void**)&dhit, (size_t)n * 11 * sizeof(float));
         if (e == cudaSuccess) e = cudaMemcpyAsync(drays, rays, (size_t)n * 7 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+        if (e == cudaSuccess) e = wait_scene(ctx, ctx->stream);
         if (e == cudaSuccess)
         {
             const int exact = traverse == RT_TRAVERSE_EXACT ? 1 : 0;

@@ -1,10 +1,14 @@
-"""Host vs device build of the reference's tree for the bench scenes (SURVEY 8f-1).  python tools/time_bvh.py [c3 c5s c5]"""
+"""Host vs device build of the reference's tree for the bench scenes (SURVEY 8f-1).  python tools/time_bvh.py [c3 c5s c5]
+Uses bench.py's generated stand-ins when the reference's meshes are not staged."""
 import json, os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np
 import raytracerwin_b200 as rt
 import bench
+if not os.path.isdir(bench.DATA):                  # the reference's meshes are not staged: bench.py's stand-ins
+    import standin_data
+    bench.DATA = standin_data.write(os.path.join(bench.scratch_dir(), "Data"))
 ctx = rt.GpuContext(0)
 for wl in (sys.argv[1:] or ["c3", "c5s", "c5"]):
     spec, *_ = bench.build_spec(wl)
