@@ -19,6 +19,7 @@
  *                        composition, on batches of the caller's rays in device memory (own cameras, probes, bakes)
  *   rt_gpu_update_mesh   new mesh geometry from device memory (tree rebuilt on the device) and moved analytic
  *   rt_gpu_update_shapes shapes, without a new upload and without draining frames in flight
+ *   rt_gpu_refit_mesh    new points under a mesh's published tree (boxes recomputed, topology kept), with no host wait
  *
  * Plain C: POD structs, pointers and sizes only.  No C++/STL/torch types cross the boundary.
  * Every entry returns 0 on success or a negative rt_status; rt_gpu_last_error() gives text.
@@ -323,6 +324,29 @@ typedef struct rt_mesh_update {
  * num_points <= 0, normals without normal_idx or the reverse, and a point or normal index out of range (found on the
  * device, before anything is published); RT_ERR_NO_SCENE before an upload. */
 int rt_gpu_update_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, void* stream);
+
+/* A REFIT of the mesh of mesh shape `shape` to new points (per-frame deformation: skinning, cloth, physics): the
+ * mesh's PUBLISHED tree (the uploaded one, or the one the last rt_gpu_update_mesh built) keeps its topology, that is
+ * its node array, escapes, right-child words and leaf order; leaf slot j keeps triangle t = tris[j].index.  Recomputed:
+ *   tris[j]      the record both builders emit for t from points[point_idx[3t+k]]: pads 0, n = cross(p1-p0, p2-p0),
+ *                normalised (1.0f / sqrtf) iff |n|^2 >= FLT_EPSILON;
+ *   leaf boxes   from FLT_MAX / -FLT_MAX, expanded with p0, p1, p2 in that order by < / >;
+ *   inner boxes  the left child's box, a component taken from the right child's only where strictly smaller (min) or
+ *                strictly larger (max): RAabb::Expand over the subtree's corners in leaf order.  This equals the
+ *                builder's box in value, not always in the sign of a zero bound;
+ *   shading records, the shape's bounds and the culling margin exactly as rt_gpu_update_mesh.
+ * After a refit, every later call returns what a fresh upload of the scene with these arrays returns.  Ordering and
+ * the spare set as rt_gpu_update_mesh, but the call RETURNS AT ONCE: no host read, no synchronisation, no blocking
+ * allocation.  `status`: DEVICE int32 or NULL, written in `stream`'s order: 0 when the refit was published, otherwise
+ * the bits of the index check (1 = a point index out of range, 2 = a normal index out of range).  The mesh's arrays,
+ * the shape's bounds and the culling margin are then left as they were, and every later call returns what it returned
+ * before.  Such a refit still publishes (a copy of the arrays), so, as after an update, an RT_OCTO mesh walks its binary
+ * tree from then on and for mesh 0 RT_TOP_STAGE is turned off; both give the same bits.  RT_ERR_INVALID (nothing
+ * enqueued) as rt_gpu_update_mesh's host-side checks, for a misaligned or non-device `status`, and for an uploaded
+ * tree that is not a full binary tree over all its nodes whose leaves name every triangle slot exactly once (the host
+ * layer always produces one; after an rt_gpu_update_mesh the builder's tree is one); RT_ERR_NO_SCENE before an
+ * upload. */
+int rt_gpu_refit_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, int32_t* status, void* stream);
 
 /* Copies `count` caller records (host memory, consumed before return) over shapes [first, first + count): moved
  * spheres, planes, capsules and triangles, other materials.  type, mesh and has_bounds must equal the uploaded

@@ -420,6 +420,29 @@ class GpuContext:
         are read in that stream's order.  Returns once the build is complete (it waits for that stream's earlier work,
         not for frames in flight); calls made after it see the new geometry, calls made before it the old one."""
         import torch
+        self._mesh_update_tensors(points, point_idx, normals, normal_idx)
+        u = self._mesh_update(points, point_idx, normals, normal_idx)
+        self._check(self._lib.rt_gpu_update_mesh(self._h, shape, C.byref(u),
+                                                 self._torch_stream(torch.device("cuda", self.device))))
+
+    def refit_mesh(self, shape, points, point_idx, normals=None, normal_idx=None):
+        """New points under the published tree of mesh shape `shape` (rt_gpu_refit_mesh): the topology stays, the triangle
+        records, node boxes, shading records, bounds and culling margin are recomputed.  Arguments as update_mesh.
+
+        Enqueued on torch.cuda.current_stream(self.device) and returns at once, with no host wait.  Returns the int32
+        (1,) status tensor on the device, written in that stream's order: 0 when the refit was published, otherwise
+        1 (a point index out of range) | 2 (a normal index out of range), and the mesh is left as it was.  Reading
+        it is the caller's choice (it synchronises)."""
+        import torch
+        self._mesh_update_tensors(points, point_idx, normals, normal_idx)
+        dev = torch.device("cuda", self.device)
+        status = torch.empty(1, dtype=torch.int32, device=dev)
+        u = self._mesh_update(points, point_idx, normals, normal_idx)
+        self._check(self._lib.rt_gpu_refit_mesh(self._h, shape, C.byref(u), status.data_ptr(), self._torch_stream(dev)))
+        return status
+
+    def _mesh_update_tensors(self, points, point_idx, normals, normal_idx):
+        import torch
         self._device_tensor("points", points, torch.float32, (None, 3))
         self._device_tensor("point_idx", point_idx, torch.int32, (None, 3))
         if (normals is None) != (normal_idx is None):
@@ -427,11 +450,12 @@ class GpuContext:
         if normals is not None:
             self._device_tensor("normals", normals, torch.float32, (None, 3))
             self._device_tensor("normal_idx", normal_idx, torch.int32, (point_idx.shape[0], 3))
-        u = rt_mesh_update(points.data_ptr(), points.shape[0], point_idx.data_ptr(), point_idx.shape[0],
-                           None if normals is None else normals.data_ptr(), 0 if normals is None else normals.shape[0],
-                           None if normal_idx is None else normal_idx.data_ptr())
-        self._check(self._lib.rt_gpu_update_mesh(self._h, shape, C.byref(u),
-                                                 self._torch_stream(torch.device("cuda", self.device))))
+
+    @staticmethod
+    def _mesh_update(points, point_idx, normals, normal_idx):
+        return rt_mesh_update(points.data_ptr(), points.shape[0], point_idx.data_ptr(), point_idx.shape[0],
+                              None if normals is None else normals.data_ptr(), 0 if normals is None else normals.shape[0],
+                              None if normal_idx is None else normal_idx.data_ptr())
 
     def update_shapes(self, scene, first=0, count=None):
         """Copies the flattened records [first, first + count) of host Scene `scene` over the uploaded shapes

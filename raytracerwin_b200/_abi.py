@@ -157,6 +157,7 @@ GPU_PROTOTYPES = {
     "rt_gpu_query_rays": (I, [VP, C.POINTER(rt_ray_query), VP]),
     "rt_gpu_radiance_rays": (I, [VP, C.POINTER(rt_radiance_query), VP]),
     "rt_gpu_update_mesh": (I, [VP, I32, C.POINTER(rt_mesh_update), VP]),
+    "rt_gpu_refit_mesh": (I, [VP, I32, C.POINTER(rt_mesh_update), VP, VP]),
     "rt_gpu_update_shapes": (I, [VP, C.POINTER(rt_shape), I32, I32, VP]),
     "rt_gpu_trace_rays": (I, [VP, PF, I32, I32, PI32, PI32, PF]),
     "rt_gpu_kat": (I, [VP, I32, VP, VP, I32, I32, VP, VP]),

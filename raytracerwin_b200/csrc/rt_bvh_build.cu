@@ -217,22 +217,7 @@ __global__ void k_nodes(Level L)
     {
         const int t = L.order[sg.begin];
         const float* p0 = L.P + 3 * (size_t)L.I[3 * t], * p1 = L.P + 3 * (size_t)L.I[3 * t + 1], * p2 = L.P + 3 * (size_t)L.I[3 * t + 2];
-        rt_tri r;
-        r.p0[0] = p0[0]; r.p0[1] = p0[1]; r.p0[2] = p0[2]; r.index = t;
-        r.p1[0] = p1[0]; r.p1[1] = p1[1]; r.p1[2] = p1[2]; r.pad0 = 0.0f;
-        r.p2[0] = p2[0]; r.p2[1] = p2[1]; r.p2[2] = p2[2]; r.pad1 = 0.0f;
-        // face normal exactly as the host builder / RRay.cpp:138-145
-        const float ax = p1[0] - p0[0], ay = p1[1] - p0[1], az = p1[2] - p0[2];
-        const float bx = p2[0] - p0[0], by = p2[1] - p0[1], bz = p2[2] - p0[2];
-        float nx = ay * bz - az * by, ny = az * bx - ax * bz, nz = ax * by - ay * bx;
-        const float sqr = nx * nx + ny * ny + nz * nz;
-        if (!(fabsf(sqr) < FLT_EPSILON))
-        {
-            const float inv = 1.0f / sqrtf(sqr);
-            nx *= inv; ny *= inv; nz *= inv;
-        }
-        r.n[0] = nx; r.n[1] = ny; r.n[2] = nz; r.pad2 = 0.0f;
-        L.tris[sg.begin] = r;
+        L.tris[sg.begin] = rt_tri_record(p0, p1, p2, t);
         L.axis[s] = -1;
         return;
     }

@@ -2,6 +2,7 @@
 // host copies, rt_gpu_update_mesh (rt_gpu.cu) runs it on device inputs into a mesh's spare arrays.
 #pragma once
 #include <cuda_runtime.h>
+#include <float.h>
 #include <stddef.h>
 
 #include "rt_gpu.h"
@@ -19,3 +20,25 @@ __attribute__((visibility("hidden"))) int* rt_bvh_scratch_flag(void* scratch);
 __attribute__((visibility("hidden"))) int rt_bvh_build_core(rt_gpu_ctx* ctx, const float* points, const int* indices, int num_tris,
                                                             cudaStream_t st, void* scratch, int* host_counts, bool check_flag,
                                                             const char* message, rt_bvh_node* nodes, rt_tri* tris, int* out_depth);
+
+// The leaf record of triangle t with corners p0, p1, p2, as the host builder emits it: pads 0 and the face normal
+// exactly as RRay.cpp:138-145 computes it (cross(p1-p0, p2-p0), normalised unless |n|^2 < FLT_EPSILON).  The builder's
+// k_nodes and rt_gpu_refit_mesh both write it.
+static __device__ __forceinline__ rt_tri rt_tri_record(const float* p0, const float* p1, const float* p2, int t)
+{
+    rt_tri r;
+    r.p0[0] = p0[0]; r.p0[1] = p0[1]; r.p0[2] = p0[2]; r.index = t;
+    r.p1[0] = p1[0]; r.p1[1] = p1[1]; r.p1[2] = p1[2]; r.pad0 = 0.0f;
+    r.p2[0] = p2[0]; r.p2[1] = p2[1]; r.p2[2] = p2[2]; r.pad1 = 0.0f;
+    const float ax = p1[0] - p0[0], ay = p1[1] - p0[1], az = p1[2] - p0[2];
+    const float bx = p2[0] - p0[0], by = p2[1] - p0[1], bz = p2[2] - p0[2];
+    float nx = ay * bz - az * by, ny = az * bx - ax * bz, nz = ax * by - ay * bx;
+    const float sqr = nx * nx + ny * ny + nz * nz;
+    if (!(fabsf(sqr) < FLT_EPSILON))
+    {
+        const float inv = 1.0f / sqrtf(sqr);
+        nx *= inv; ny *= inv; nz *= inv;
+    }
+    r.n[0] = nx; r.n[1] = ny; r.n[2] = nz; r.pad2 = 0.0f;
+    return r;
+}

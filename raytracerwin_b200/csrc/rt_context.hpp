@@ -132,6 +132,9 @@ struct rt_gpu_ctx
         int num_tris = 0;
         int num_nodes = 0;                      // as uploaded: an update builds 2 * num_tris - 1
         int users = 0;                          // shapes that reference the mesh
+        // The published tree is a full binary tree over all its nodes whose leaves name every triangle slot exactly once
+        // (checked at upload, true after an update): what rt_gpu_refit_mesh needs to reach and rewrite every node.
+        bool refittable = false;
         MeshArrays cur = { nullptr, nullptr, nullptr };      // published (shade in leaf order)
         MeshArrays spare = { nullptr, nullptr, nullptr };    // allocated by the first update
     };

@@ -243,6 +243,139 @@ __global__ void rt_update_shapes_kernel(rt_shape* shapes, ShapeBatch src, int co
     else shapes[k] = src.rec[k];
 }
 
+// ---- mesh refits (rt_gpu_refit_mesh) ----
+// No host read sees the check's flag, so every later kernel runs on clamped copies of BOTH index arrays (bad ones
+// replaced by 0): nothing reads outside `points` or `normals`; with the flag set the result is thrown away below.
+__global__ void rt_refit_check_kernel(const int* __restrict__ pidx, int num_points, const int* __restrict__ nidx, int num_normals,
+                                      int n, int* __restrict__ safe_p, int* __restrict__ safe_n, int* __restrict__ flag)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int v = pidx[i], bad = 0;
+    if (v < 0 || v >= num_points) { v = 0; bad |= RT_UPD_BAD_POINT_INDEX; }
+    safe_p[i] = v;
+    if (nidx)
+    {
+        int w = nidx[i];
+        if (w < 0 || w >= num_normals) { w = 0; bad |= RT_UPD_BAD_NORMAL_INDEX; }
+        safe_n[i] = w;
+    }
+    if (bad) atomicOr(flag, bad);
+}
+
+// Parent links of the published tree (left child i+1, right child in the inner node's `tri` word, -2 - index; the root
+// has none), the node of each leaf slot, and zeroed arrival counters.  rt_gpu_refit_mesh runs only on a full binary
+// tree over all its nodes whose leaves name every slot once (MeshState::refittable), so every link is set and every
+// node is reached by a climb.
+__global__ void rt_refit_links_kernel(const rt_bvh_node* __restrict__ nodes, int n, int* __restrict__ parent,
+                                      int* __restrict__ leaf_node, int* __restrict__ arrivals)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    arrivals[i] = 0;
+    if (i == 0) parent[0] = -1;
+    const int tri = nodes[i].tri;
+    if (tri >= 0)
+    {
+        leaf_node[tri] = i;
+        return;
+    }
+    parent[i + 1] = i;
+    parent[-2 - tri] = i;
+}
+
+__device__ __forceinline__ void refit_store_node(float4* nodes, int i, const float* mn, int escape, const float* mx, int tri)
+{
+    nodes[2 * (size_t)i] = make_float4(mn[0], mn[1], mn[2], __int_as_float(escape));
+    nodes[2 * (size_t)i + 1] = make_float4(mx[0], mx[1], mx[2], __int_as_float(tri));
+}
+
+// One thread per leaf slot j: the triangle record of t = cur_tris[j].index from the new corners and the leaf's box
+// (RAabb's empty box expanded with p0, p1, p2 by < / >, as the host builder's loop over a one-triangle node), then
+// up the tree: the SECOND child to arrive at an inner node combines both children's boxes, always left then right
+// (a component of the right child's box only where strictly smaller / larger), so the result does not depend on which
+// child finished first.  Escape and `tri` words are the published ones.
+__global__ void rt_refit_kernel(const float4* __restrict__ cur_tris, const float4* __restrict__ cur_nodes,
+                                const float* __restrict__ points, const int* __restrict__ pidx, const int* __restrict__ leaf_node,
+                                const int* __restrict__ parent, int* arrivals, rt_tri* __restrict__ tris, float4* nodes, int T)
+{
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= T) return;
+    const int t = __float_as_int(cur_tris[4 * (size_t)j].w);
+    const rt_tri r = rt_tri_record(points + 3 * (size_t)pidx[3 * (size_t)t], points + 3 * (size_t)pidx[3 * (size_t)t + 1],
+                                   points + 3 * (size_t)pidx[3 * (size_t)t + 2], t);
+    tris[j] = r;
+    int i = leaf_node[j];
+    float mn[3] = { FLT_MAX, FLT_MAX, FLT_MAX }, mx[3] = { -FLT_MAX, -FLT_MAX, -FLT_MAX };
+    const float* corner[3] = { r.p0, r.p1, r.p2 };
+    for (int k = 0; k < 3; k++)
+        for (int c = 0; c < 3; c++)
+        {
+            if (corner[k][c] < mn[c]) mn[c] = corner[k][c];
+            if (corner[k][c] > mx[c]) mx[c] = corner[k][c];
+        }
+    float4 w0 = cur_nodes[2 * (size_t)i], w1 = cur_nodes[2 * (size_t)i + 1];
+    refit_store_node(nodes, i, mn, __float_as_int(w0.w), mx, __float_as_int(w1.w));
+    for (;;)
+    {
+        __threadfence();                                    // this node's box before the arrival that publishes it
+        const int p = parent[i];
+        if (p < 0) return;
+        if (atomicAdd(arrivals + p, 1) == 0) return;        // the sibling is still on its way: it carries on
+        __threadfence();
+        w0 = cur_nodes[2 * (size_t)p]; w1 = cur_nodes[2 * (size_t)p + 1];
+        const int right = -2 - __float_as_int(w1.w);
+        const float4 l0 = __ldcg(nodes + 2 * (size_t)(p + 1)), l1 = __ldcg(nodes + 2 * (size_t)(p + 1) + 1);
+        const float4 r0 = __ldcg(nodes + 2 * (size_t)right), r1 = __ldcg(nodes + 2 * (size_t)right + 1);
+        mn[0] = l0.x; mn[1] = l0.y; mn[2] = l0.z; mx[0] = l1.x; mx[1] = l1.y; mx[2] = l1.z;
+        if (r0.x < mn[0]) mn[0] = r0.x;
+        if (r0.y < mn[1]) mn[1] = r0.y;
+        if (r0.z < mn[2]) mn[2] = r0.z;
+        if (r1.x > mx[0]) mx[0] = r1.x;
+        if (r1.y > mx[1]) mx[1] = r1.y;
+        if (r1.z > mx[2]) mx[2] = r1.z;
+        refit_store_node(nodes, p, mn, __float_as_int(w0.w), mx, __float_as_int(w1.w));
+        i = p;
+    }
+}
+
+// A refit whose index check failed publishes an exact copy of the published set (the host's ping-pong swaps on
+// every call, so the spare set must hold the live arrays afterwards) and keeps the shape's bounds and the mesh's
+// culling margin, saved here for rt_refit_finish_kernel.  Without the flag every block leaves at once.
+__global__ void rt_refit_restore_kernel(const int* __restrict__ flag, const float4* __restrict__ cur_nodes,
+                                        const float4* __restrict__ cur_tris, const float4* __restrict__ cur_shade, float4* nodes,
+                                        float4* tris, float4* shade, int n, int T, const DevMesh* mesh, const rt_shape* shape,
+                                        float* saved)
+{
+    if (*flag == 0) return;
+    const size_t a = 2 * (size_t)n, b = 4 * (size_t)T;
+    for (size_t k = blockIdx.x * (size_t)blockDim.x + threadIdx.x; k < a + 2 * b; k += (size_t)gridDim.x * blockDim.x)
+    {
+        if (k < a) nodes[k] = cur_nodes[k];
+        else if (k < a + b) tris[k - a] = cur_tris[k - a];
+        else shade[k - a - b] = cur_shade[k - a - b];
+    }
+    if (blockIdx.x == 0 && threadIdx.x < 3)
+    {
+        saved[threadIdx.x] = shape->bounds_min[threadIdx.x];
+        saved[3 + threadIdx.x] = shape->bounds_max[threadIdx.x];
+        if (threadIdx.x == 0) saved[6] = mesh->cull_scale;
+    }
+}
+
+// After rt_update_publish_kernel: a failed check gets the saved bounds and margin back; the status goes to the caller.
+__global__ void rt_refit_finish_kernel(const int* __restrict__ flag, int* status, DevMesh* mesh, rt_shape* shape,
+                                       const float* __restrict__ saved)
+{
+    const int f = *flag;
+    if (f)
+    {
+        for (int c = 0; c < 3; c++) { shape->bounds_min[c] = saved[c]; shape->bounds_max[c] = saved[3 + c]; }
+        mesh->cull_scale = saved[6];
+    }
+    if (status) *status = f;
+}
+
 static void free_scene(rt_gpu_ctx* ctx)
 {
     for (cudaTextureObject_t t : ctx->texobjs) cudaDestroyTextureObject(t);
@@ -778,6 +911,9 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
             if (sh.material >= s->num_materials) return fail(ctx, RT_ERR_INVALID, "shape material index out of range");
             if (sh.type == RT_SHAPE_MESH && (sh.mesh < 0 || sh.mesh >= s->num_meshes)) return fail(ctx, RT_ERR_INVALID, "shape mesh index out of range");
         }
+        // a tree the upload accepts may still leave nodes out of the root's range, give an inner node an empty right
+        // range, or name a triangle slot twice; a refit reaches every node only when none of that happens
+        std::vector<char> refittable((size_t)s->num_meshes, 0);
         for (int i = 0; i < s->num_meshes; i++)
         {
             const rt_mesh& m = s->meshes[i];
@@ -803,6 +939,19 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
                         return fail(ctx, RT_ERR_INVALID, "malformed BVH node (subtrees do not nest)");
                 }
                 else if (nd.escape != k + 1) return fail(ctx, RT_ERR_INVALID, "malformed BVH node (leaf with a subtree)");
+            }
+            if (m.num_nodes > 0 && m.nodes[0].escape == m.num_nodes)
+            {
+                std::vector<char> named((size_t)m.num_tris, 0);
+                bool full = true;
+                int leaves = 0;
+                for (int k = 0; k < m.num_nodes && full; k++)
+                {
+                    const rt_bvh_node& nd = m.nodes[k];
+                    if (nd.tri < 0) full = m.nodes[k + 1].escape < nd.escape;
+                    else { full = !named[nd.tri]; named[nd.tri] = 1; leaves++; }
+                }
+                refittable[i] = full && leaves == m.num_tris;
             }
             for (int k = 0; k < m.num_tris; k++)
             {
@@ -931,6 +1080,7 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
             ctx->mesh_state.emplace_back();
             ctx->mesh_state.back().num_tris = m.num_tris;
             ctx->mesh_state.back().num_nodes = m.num_nodes;
+            ctx->mesh_state.back().refittable = refittable[i] != 0;
             ctx->mesh_state.back().cur = rt_gpu_ctx::MeshArrays{ dn, dt, (rt_shade*)dsh };
             dm.octo = nullptr;
             if (m.num_nodes > 0 && ctx->tune_octo)
@@ -1596,66 +1746,89 @@ static int alloc_on(rt_gpu_ctx* ctx, void** out, size_t bytes, cudaStream_t st)
 
 static inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
+// The host-side checks of rt_gpu_update_mesh and rt_gpu_refit_mesh (`fn` names the call in the messages); the shape's
+// mesh goes to *mesh.
+static int check_mesh_update(rt_gpu_ctx* ctx, const char* fn, int32_t shape, const rt_mesh_update* u, int* mesh)
+{
+    const std::string f(fn);
+    if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, f + " before rt_gpu_upload_scene");
+    if (!u) return fail(ctx, RT_ERR_INVALID, f + ": update is null");
+    if (shape < 0 || shape >= (int)ctx->host_shapes.size() || ctx->host_shapes[shape].type != RT_SHAPE_MESH)
+        return fail(ctx, RT_ERR_INVALID, f + ": shape is not a mesh shape of the scene");
+    const int mi = ctx->host_shapes[shape].mesh;
+    const rt_gpu_ctx::MeshState& ms = ctx->mesh_state[mi];
+    if (ms.users != 1) return fail(ctx, RT_ERR_INVALID, f + ": another shape references the same mesh");
+    if (ms.num_tris <= 0 || u->num_tris != ms.num_tris)
+        return fail(ctx, RT_ERR_INVALID, f + ": num_tris differs from the uploaded mesh's");
+    // the update publishes a tree of 2T-1 nodes in an array of that size; the walks read num_nodes as uploaded
+    if (ms.num_nodes != 2 * ms.num_tris - 1)
+        return fail(ctx, RT_ERR_INVALID, f + ": the uploaded mesh's node count is not 2 * num_tris - 1 (not a tree of its triangles)");
+    if ((long long)ms.num_tris * 3 >= 0xFFFFFFFFll) return fail(ctx, RT_ERR_INVALID, f + ": too many triangles");
+    if (u->num_points <= 0) return fail(ctx, RT_ERR_INVALID, f + ": num_points must be positive");
+    if (!u->points || !u->point_idx) return fail(ctx, RT_ERR_INVALID, f + ": points and point_idx are required");
+    if ((u->normals == nullptr) != (u->normal_idx == nullptr))
+        return fail(ctx, RT_ERR_INVALID, f + ": normals and normal_idx come together");
+    if (u->normals && u->num_normals <= 0) return fail(ctx, RT_ERR_INVALID, f + ": num_normals must be positive");
+    const void* ptrs[4] = { u->points, u->point_idx, u->normals, u->normal_idx };
+    const char* names[4] = { "points", "point_idx", "normals", "normal_idx" };
+    for (int k = 0; k < 4; k++)
+        if (ptrs[k] && (uintptr_t)ptrs[k] % 4 != 0)
+            return fail(ctx, RT_ERR_INVALID, f + ": " + names[k] + " must be 4-byte aligned");
+    RT_CUDA(cudaSetDevice(ctx->device));
+    for (int k = 0; k < 4; k++)
+        if (ptrs[k] && !on_device(ctx, ptrs[k]))
+            return fail(ctx, RT_ERR_INVALID, f + ": " + names[k] + " is not device memory of the context's GPU");
+    *mesh = mi;
+    return RT_OK;
+}
+
+// The spare set of a mesh's arrays (first update or refit) and the updates' scratch block (only grows), on `st` after
+// wait_scene: the spare set and the scratch were last read by work the previous update waited for.
+static int alloc_spare(rt_gpu_ctx* ctx, rt_gpu_ctx::MeshState& ms, cudaStream_t st)
+{
+    if (ms.spare.nodes) return RT_OK;
+    const size_t T = (size_t)ms.num_tris;
+    rt_gpu_ctx::MeshArrays a = { nullptr, nullptr, nullptr };
+    int rc;
+    if ((rc = alloc_on(ctx, (void**)&a.nodes, (2 * T - 1) * sizeof(rt_bvh_node), st)) != RT_OK) return rc;
+    ctx->scene_allocs.push_back(a.nodes);
+    if ((rc = alloc_on(ctx, (void**)&a.tris, T * sizeof(rt_tri), st)) != RT_OK) return rc;
+    ctx->scene_allocs.push_back(a.tris);
+    if ((rc = alloc_on(ctx, (void**)&a.shade, T * sizeof(rt_shade), st)) != RT_OK) return rc;
+    ctx->scene_allocs.push_back(a.shade);
+    ctx->scene_bytes += (2 * T - 1) * sizeof(rt_bvh_node) + T * (sizeof(rt_tri) + sizeof(rt_shade));
+    ms.spare = a;
+    return RT_OK;
+}
+
+static int grow_update_scratch(rt_gpu_ctx* ctx, size_t need, cudaStream_t st)
+{
+    if (need <= ctx->update_scratch_cap) return RT_OK;
+    if (ctx->update_scratch) RT_CUDA(cudaFreeAsync(ctx->update_scratch, st));
+    ctx->update_scratch = nullptr; ctx->update_scratch_cap = 0;
+    const int rc = alloc_on(ctx, &ctx->update_scratch, need, st);
+    if (rc != RT_OK) return rc;
+    ctx->update_scratch_cap = need;
+    return RT_OK;
+}
+
 int rt_gpu_update_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, void* stream)
 {
     return rt_guard(ctx, [&]() -> int {
         if (!ctx) return RT_ERR_INVALID;
-        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_update_mesh before rt_gpu_upload_scene");
-        if (!u) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: update is null");
-        if (shape < 0 || shape >= (int)ctx->host_shapes.size() || ctx->host_shapes[shape].type != RT_SHAPE_MESH)
-            return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: shape is not a mesh shape of the scene");
-        const int mi = ctx->host_shapes[shape].mesh;
+        int mi = -1;
+        int rc = check_mesh_update(ctx, "rt_gpu_update_mesh", shape, u, &mi);
+        if (rc != RT_OK) return rc;
         rt_gpu_ctx::MeshState& ms = ctx->mesh_state[mi];
-        if (ms.users != 1) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: another shape references the same mesh");
-        if (ms.num_tris <= 0 || u->num_tris != ms.num_tris)
-            return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: num_tris differs from the uploaded mesh's");
-        // the update publishes a tree of 2T-1 nodes in an array of that size; the walks read num_nodes as uploaded
-        if (ms.num_nodes != 2 * ms.num_tris - 1)
-            return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: the uploaded mesh's node count is not 2 * num_tris - 1 (not a tree of its triangles)");
-        if ((long long)ms.num_tris * 3 >= 0xFFFFFFFFll) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: too many triangles");
-        if (u->num_points <= 0) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: num_points must be positive");
-        if (!u->points || !u->point_idx) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: points and point_idx are required");
-        if ((u->normals == nullptr) != (u->normal_idx == nullptr))
-            return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: normals and normal_idx come together");
-        if (u->normals && u->num_normals <= 0) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_mesh: num_normals must be positive");
-        const void* ptrs[4] = { u->points, u->point_idx, u->normals, u->normal_idx };
-        const char* names[4] = { "points", "point_idx", "normals", "normal_idx" };
-        for (int k = 0; k < 4; k++)
-            if (ptrs[k] && (uintptr_t)ptrs[k] % 4 != 0)
-                return fail(ctx, RT_ERR_INVALID, std::string("rt_gpu_update_mesh: ") + names[k] + " must be 4-byte aligned");
-        RT_CUDA(cudaSetDevice(ctx->device));
-        for (int k = 0; k < 4; k++)
-            if (ptrs[k] && !on_device(ctx, ptrs[k]))
-                return fail(ctx, RT_ERR_INVALID, std::string("rt_gpu_update_mesh: ") + names[k] + " is not device memory of the context's GPU");
         const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
         const int T = ms.num_tris;
-        // the spare set and the scratch block were last read by work the previous update waited for
         RT_CUDA(wait_scene(ctx, st));
-        int rc;
-        if (!ms.spare.nodes)
-        {
-            rt_gpu_ctx::MeshArrays a = { nullptr, nullptr, nullptr };
-            if ((rc = alloc_on(ctx, (void**)&a.nodes, (2 * (size_t)T - 1) * sizeof(rt_bvh_node), st)) != RT_OK) return rc;
-            ctx->scene_allocs.push_back(a.nodes);
-            if ((rc = alloc_on(ctx, (void**)&a.tris, (size_t)T * sizeof(rt_tri), st)) != RT_OK) return rc;
-            ctx->scene_allocs.push_back(a.tris);
-            if ((rc = alloc_on(ctx, (void**)&a.shade, (size_t)T * sizeof(rt_shade), st)) != RT_OK) return rc;
-            ctx->scene_allocs.push_back(a.shade);
-            ctx->scene_bytes += (2 * (size_t)T - 1) * sizeof(rt_bvh_node) + (size_t)T * (sizeof(rt_tri) + sizeof(rt_shade));
-            ms.spare = a;
-        }
+        if ((rc = alloc_spare(ctx, ms, st)) != RT_OK) return rc;
         // scratch: the builder's block, safe point indices (3T), shading records in original order (T), bounds keys (6)
         const size_t build_bytes = align256(rt_bvh_scratch_bytes(T));
         const size_t idx_off = build_bytes, shade_off = idx_off + align256(3 * (size_t)T * sizeof(int));
         const size_t keys_off = shade_off + align256((size_t)T * sizeof(rt_shade));
-        const size_t need = keys_off + 6 * sizeof(unsigned long long);
-        if (need > ctx->update_scratch_cap)
-        {
-            if (ctx->update_scratch) RT_CUDA(cudaFreeAsync(ctx->update_scratch, st));
-            ctx->update_scratch = nullptr; ctx->update_scratch_cap = 0;
-            if ((rc = alloc_on(ctx, &ctx->update_scratch, need, st)) != RT_OK) return rc;
-            ctx->update_scratch_cap = need;
-        }
+        if ((rc = grow_update_scratch(ctx, keys_off + 6 * sizeof(unsigned long long), st)) != RT_OK) return rc;
         if (!ctx->update_counts) RT_CUDA(cudaHostAlloc((void**)&ctx->update_counts, 4 * sizeof(int), cudaHostAllocDefault));
         char* scratch = (char*)ctx->update_scratch;
         int* safe_idx = (int*)(scratch + idx_off);
@@ -1690,7 +1863,84 @@ int rt_gpu_update_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, 
         ctx->launches++;
         if ((rc = publish_done(ctx, st)) != RT_OK) return rc;
         std::swap(ms.cur, ms.spare);
+        ms.refittable = true;                   // the builder's tree
         // the shared-memory stage holds mesh 0's uploaded top levels; a pointer test cannot tell the ping-pong's arrays apart
+        if (mi == 0) ctx->scene.top_of = nullptr;
+        return RT_OK;
+    });
+}
+
+// The published topology with new points: O(T) stream-ordered kernels and no host read, so the call returns at once.
+// A bad index cannot stop the call on the host; the device publishes a copy of the live set instead (see
+// rt_refit_restore_kernel), so the ping-pong stays consistent either way.
+int rt_gpu_refit_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, int32_t* status, void* stream)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        int mi = -1;
+        int rc = check_mesh_update(ctx, "rt_gpu_refit_mesh", shape, u, &mi);
+        if (rc != RT_OK) return rc;
+        if (status && ((uintptr_t)status % 4 != 0 || !on_device(ctx, status)))
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_refit_mesh: status must be 4-byte aligned device memory of the context's GPU");
+        rt_gpu_ctx::MeshState& ms = ctx->mesh_state[mi];
+        if (!ms.refittable)
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_refit_mesh: the uploaded tree is not a full binary tree whose leaves name every "
+                                             "triangle slot once (rt_gpu_update_mesh builds one)");
+        const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+        const int T = ms.num_tris, N = 2 * T - 1;
+        RT_CUDA(wait_scene(ctx, st));
+        if ((rc = alloc_spare(ctx, ms, st)) != RT_OK) return rc;
+        // scratch: flag, safe point and normal indices (3T each), shading records in original order (T), bounds keys
+        // (6), saved bounds and margin (7 floats), parent links (N) + leaf nodes (T), arrival counters (N)
+        const size_t pidx_off = 256, nidx_off = pidx_off + align256(3 * (size_t)T * sizeof(int));
+        const size_t shade_off = nidx_off + align256(3 * (size_t)T * sizeof(int));
+        const size_t keys_off = shade_off + align256((size_t)T * sizeof(rt_shade));
+        const size_t saved_off = keys_off + 6 * sizeof(unsigned long long);
+        const size_t links_off = align256(saved_off + 7 * sizeof(float));
+        const size_t arrivals_off = links_off + align256(((size_t)N + T) * sizeof(int));
+        if ((rc = grow_update_scratch(ctx, arrivals_off + (size_t)N * sizeof(int), st)) != RT_OK) return rc;
+        char* scratch = (char*)ctx->update_scratch;
+        int* flag = (int*)scratch;
+        int* safe_p = (int*)(scratch + pidx_off);
+        int* safe_n = u->normals ? (int*)(scratch + nidx_off) : nullptr;
+        rt_shade* shade_tmp = (rt_shade*)(scratch + shade_off);
+        unsigned long long* keys = (unsigned long long*)(scratch + keys_off);
+        float* saved = (float*)(scratch + saved_off);
+        int* parent = (int*)(scratch + links_off);
+        int* leaf_node = parent + N;
+        int* arrivals = (int*)(scratch + arrivals_off);
+        DevMesh* dmesh = const_cast<DevMesh*>(ctx->scene.meshes) + mi;
+        rt_shape* dshape = const_cast<rt_shape*>(ctx->scene.shapes) + shape;
+        const unsigned gT = (unsigned)((T + 255) / 256), gN = (unsigned)((N + 255) / 256);
+
+        const int n3 = 3 * T;
+        RT_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), st));
+        rt_refit_check_kernel<<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(u->point_idx, u->num_points, u->normal_idx,
+                                                                             u->normals ? u->num_normals : 0, n3, safe_p, safe_n, flag);
+        rt_refit_links_kernel<<<gN, 256, 0, st>>>(ms.cur.nodes, N, parent, leaf_node, arrivals);
+        rt_refit_kernel<<<gT, 256, 0, st>>>((const float4*)ms.cur.tris, (const float4*)ms.cur.nodes, u->points, safe_p, leaf_node,
+                                            parent, arrivals, ms.spare.tris, (float4*)ms.spare.nodes, T);
+        rt_update_shade_kernel<<<gT, 256, 0, st>>>((const float4*)ms.cur.tris, (const float*)ms.cur.shade, u->points, safe_p,
+                                                   u->normals, safe_n, (float*)shade_tmp, T);
+        rt_shade_leaf_order_kernel<<<gT, 256, 0, st>>>((const float4*)ms.spare.tris, (const float4*)shade_tmp, (float4*)ms.spare.shade, T);
+        RT_CUDA(cudaMemsetAsync(keys, 0xFF, 3 * sizeof(unsigned long long), st));
+        RT_CUDA(cudaMemsetAsync(keys + 3, 0, 3 * sizeof(unsigned long long), st));
+        rt_update_bounds_kernel<<<(unsigned)((u->num_points + 255) / 256), 256, 0, st>>>(u->points, u->num_points, keys);
+        rt_refit_restore_kernel<<<(unsigned)ctx->num_sms * 4u, 256, 0, st>>>(
+            flag, (const float4*)ms.cur.nodes, (const float4*)ms.cur.tris, (const float4*)ms.cur.shade, (float4*)ms.spare.nodes,
+            (float4*)ms.spare.tris, (float4*)ms.spare.shade, N, T, dmesh, dshape, saved);
+        RT_CUDA(cudaGetLastError());
+        ctx->launches += 7;
+        // publish once every call enqueued before this one has finished reading the old arrays
+        if ((rc = join_scene_readers(ctx, st)) != RT_OK) return rc;
+        rt_update_publish_kernel<<<1, 1, 0, st>>>(const_cast<DevMesh*>(ctx->scene.meshes), mi, const_cast<rt_shape*>(ctx->scene.shapes),
+                                                  shape, ms.spare.nodes, ms.spare.tris, ms.spare.shade, keys, u->points);
+        rt_refit_finish_kernel<<<1, 1, 0, st>>>(flag, status, dmesh, dshape, saved);
+        RT_CUDA(cudaGetLastError());
+        ctx->launches += 2;
+        if ((rc = publish_done(ctx, st)) != RT_OK) return rc;
+        std::swap(ms.cur, ms.spare);
+        // as rt_gpu_update_mesh: the stage holds mesh 0's uploaded top levels
         if (mi == 0) ctx->scene.top_of = nullptr;
         return RT_OK;
     });

@@ -1,7 +1,7 @@
 """Per-kernel registers, spills, stack and shared memory of two -Xptxas -v logs (the Makefile keeps them in
 raytracerwin_b200/csrc/build/ptxas*.log), matched by mangled name with nvcc's per-build hash of anonymous namespaces
-removed.  Prints every kernel of the first log with its line in the second and whether it changed, then kernels only
-the second log has.
+removed (it depends on the source's path, so trees built in different directories compare too).  Prints every kernel
+of the first log with its line in the second and whether it changed, then kernels only the second log has.
 
    python tools/ptxas_compare.py OLD.log NEW.log
 """
@@ -14,7 +14,7 @@ def parse(path):
     for line in open(path):
         m = re.search(r"Compiling entry function '(\S+)'", line)
         if m:
-            cur = re.sub(r"_cu_[0-9a-f]{8}", "_cu_", m.group(1))
+            cur = re.sub(r"(_cu_|_GLOBAL__N__)[0-9a-f]{8}", r"\1", m.group(1))
             out[cur] = []
         elif cur and ("Used" in line or "spill" in line) and "Function properties" not in line:
             out[cur].append(re.sub(r"^ptxas info\s*:\s*", "", line.strip()))
