@@ -20,6 +20,8 @@
  *   rt_gpu_update_mesh   new mesh geometry from device memory (tree rebuilt on the device) and moved analytic
  *   rt_gpu_update_shapes shapes, without a new upload and without draining frames in flight
  *   rt_gpu_refit_mesh    new points under a mesh's published tree (boxes recomputed, topology kept), with no host wait
+ *   rt_gpu_replace_mesh  a new mesh of any triangle count, with texture coordinates and texture slots, from device memory
+ *                        (levels of detail, procedural and streamed geometry) without a new upload
  *
  * Plain C: POD structs, pointers and sizes only.  No C++/STL/torch types cross the boundary.
  * Every entry returns 0 on success or a negative rt_status; rt_gpu_last_error() gives text.
@@ -308,7 +310,7 @@ typedef struct rt_mesh_update {
     const float* points;       /* DEVICE, num_points x 3, 4-byte aligned */
     int32_t num_points;
     const int32_t* point_idx;  /* DEVICE, num_tris x 3: triangle t = original triangle id t */
-    int32_t num_tris;          /* must equal the uploaded mesh's num_tris */
+    int32_t num_tris;          /* must equal the mesh's num_tris (as uploaded, or as the last rt_gpu_replace_mesh gave it) */
     const float* normals;      /* DEVICE, num_normals x 3, or NULL: every corner gets its triangle's cross(p1-p0, p2-p0) */
     int32_t num_normals;
     const int32_t* normal_idx; /* DEVICE, num_tris x 3, or NULL (exactly when normals is NULL) */
@@ -319,7 +321,7 @@ typedef struct rt_mesh_update {
  * builder reads one count per tree level on the host, so the call RETURNS ONCE THE BUILD IS COMPLETE: it waits for
  * `stream`'s earlier work and the build, not for renders on other streams.  The first update of a mesh allocates a
  * spare set of its arrays (192 B per triangle).  RT_ERR_INVALID for NULL, misaligned or non-device pointers, a shape
- * that is not a mesh or whose mesh another shape also references, num_tris other than the uploaded count, an
+ * that is not a mesh or whose mesh another shape also references, num_tris other than the mesh's count, an
  * uploaded mesh whose node count is not 2 * num_tris - 1 (a description the host layer never produces),
  * num_points <= 0, normals without normal_idx or the reverse, and a point or normal index out of range (found on the
  * device, before anything is published); RT_ERR_NO_SCENE before an upload. */
@@ -347,6 +349,33 @@ int rt_gpu_update_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, 
  * layer always produces one; after an rt_gpu_update_mesh the builder's tree is one); RT_ERR_NO_SCENE before an
  * upload. */
 int rt_gpu_refit_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, int32_t* status, void* stream);
+
+/* A REPLACE of the mesh of mesh shape `shape`: new geometry of ANY triangle count, with its own texture coordinates and
+ * texture slots (switching a level of detail, marching cubes or other geometry generated on the GPU, fracture,
+ * streaming).  After a replace, every later call returns what a fresh upload returns of the scene in which the mesh is
+ * rt_host_add_mesh_arrays(points, normals, texcoords, point_idx, normal_idx, texcoord_idx, num_tris) with
+ * rt_shade.texture of triangle t = texture[t], the mesh keeps its uploaded rt_texture slots, and the shape's bounds are
+ * RAabb::Expand over all the points.  Triangle ids that queries return are the new triangle order.  Ordering, blocking
+ * (the call returns once the build is complete), RT_OCTO and RT_TOP_STAGE as rt_gpu_update_mesh.  The uploaded mesh must
+ * have at least one triangle; its node count and tree shape do not matter.  Afterwards the mesh is updatable and
+ * refittable with the new count, and later updates and refits keep the new uv and slots.
+ * Memory: the spare set is reused when it holds at least num_tris triangles, otherwise a set of num_tris is allocated
+ * (stream-ordered on `stream`) and a spare set an earlier update allocated is released; capacity only grows.
+ * RT_ERR_INVALID (the scene left exactly as it was) for rt_gpu_update_mesh's host-side checks other than the count and
+ * node-count tests, num_tris <= 0, texcoords without texcoord_idx or the reverse, num_texcoords <= 0 with texcoords,
+ * misaligned or non-device texcoords / texcoord_idx / texture, and, found on the device before anything is published, a
+ * point, normal or texcoord index out of range or a texture slot the upload would refuse (>= the mesh's texture count,
+ * or a slot without pixels; negative slots are untextured and pass); RT_ERR_NO_SCENE before an upload. */
+typedef struct rt_mesh_replace {
+    rt_mesh_update geometry;      /* rt_mesh_update's rules, except that num_tris is the NEW triangle count (>= 1) */
+    const float* texcoords;       /* DEVICE, num_texcoords x 2 {u, v}, 4-byte aligned, or NULL: every corner gets uv (0, 0) */
+    int32_t num_texcoords;
+    const int32_t* texcoord_idx;  /* DEVICE, num_tris x 3, or NULL (exactly when texcoords is NULL) */
+    const int32_t* texture;       /* DEVICE, num_tris, or NULL (-1 everywhere): rt_shade.texture of triangle t, a slot of
+                                     the mesh's UPLOADED textures */
+} rt_mesh_replace;
+
+int rt_gpu_replace_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_replace* r, void* stream);
 
 /* Copies `count` caller records (host memory, consumed before return) over shapes [first, first + count): moved
  * spheres, planes, capsules and triangles, other materials.  type, mesh and has_bounds must equal the uploaded

@@ -14,6 +14,7 @@ import numpy as np
 
 from . import _abi
 from ._abi import (rt_render_params, rt_counters, rt_scene_desc, rt_ray_query, rt_radiance_query, rt_mesh_update,  # noqa: F401
+                   rt_mesh_replace,
                    RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY, RT_QUERY_NEAREST, RT_QUERY_ANY,
                    RT_TRAVERSE_EXACT, RT_TRAVERSE_CULLED,
                    RT_READ_ACCUM_RGBN_F32, RT_READ_DISPLAY_ARGB8, RT_READ_PRIMARY_IDS_I32X2,
@@ -245,6 +246,8 @@ class GpuContext:
         d = desc if isinstance(desc, rt_scene_desc) else getattr(desc, "contents", None)
         self._uploaded_tris = {} if d is None else {i: (int(d.meshes[i].num_tris), int(d.meshes[i].num_nodes))
                                                      for i in range(d.num_meshes)}
+        self._shape_mesh = {} if d is None else {i: int(d.shapes[i].mesh) for i in range(d.num_shapes)
+                                                  if d.shapes[i].type == _abi.RT_SHAPE_MESH}
 
     def reset_accum(self, width, height):
         self._check(self._lib.rt_gpu_reset_accum(self._h, width, height))
@@ -440,6 +443,35 @@ class GpuContext:
         u = self._mesh_update(points, point_idx, normals, normal_idx)
         self._check(self._lib.rt_gpu_refit_mesh(self._h, shape, C.byref(u), status.data_ptr(), self._torch_stream(dev)))
         return status
+
+    def replace_mesh(self, shape, points, point_idx, normals=None, normal_idx=None, texcoords=None, texcoord_idx=None,
+                     texture=None):
+        """A new mesh of any triangle count for mesh shape `shape` (rt_gpu_replace_mesh): levels of detail, geometry
+        generated on the GPU, fracture.  The tree is built on the GPU.
+
+        `points` float32 (P, 3), `point_idx` int32 (T, 3) with any T >= 1, optional `normals` float32 (Q, 3) with
+        `normal_idx` int32 (T, 3) (as update_mesh), optional `texcoords` float32 (U, 2) {u, v} with `texcoord_idx` int32
+        (T, 3) (without them every corner gets uv (0, 0)), optional `texture` int32 (T,): the texture slot of each
+        triangle among the mesh's uploaded textures (-1 = untextured, the default); contiguous torch tensors on
+        cuda:<self.device>.  Ordering and blocking as update_mesh; triangle ids in query results are the new order."""
+        import torch
+        self._mesh_update_tensors(points, point_idx, normals, normal_idx)
+        T = point_idx.shape[0]
+        if (texcoords is None) != (texcoord_idx is None):
+            raise ValueError("texcoords and texcoord_idx come together")
+        if texcoords is not None:
+            self._device_tensor("texcoords", texcoords, torch.float32, (None, 2))
+            self._device_tensor("texcoord_idx", texcoord_idx, torch.int32, (T, 3))
+        if texture is not None:
+            self._device_tensor("texture", texture, torch.int32, (T,))
+        mesh = getattr(self, "_shape_mesh", {}).get(shape)
+        r = rt_mesh_replace(self._mesh_update(points, point_idx, normals, normal_idx),
+                            None if texcoords is None else texcoords.data_ptr(), 0 if texcoords is None else texcoords.shape[0],
+                            None if texcoord_idx is None else texcoord_idx.data_ptr(),
+                            None if texture is None else texture.data_ptr())
+        self._check(self._lib.rt_gpu_replace_mesh(self._h, shape, C.byref(r),
+                                                  self._torch_stream(torch.device("cuda", self.device))))
+        self._uploaded_tris[mesh] = (T, 2 * T - 1)            # read_mesh sizes its arrays by the published counts
 
     def _mesh_update_tensors(self, points, point_idx, normals, normal_idx):
         import torch

@@ -103,6 +103,11 @@ class rt_mesh_update(C.Structure):
                 ("normals", C.c_void_p), ("num_normals", C.c_int32), ("normal_idx", C.c_void_p)]
 
 
+class rt_mesh_replace(C.Structure):
+    _fields_ = [("geometry", rt_mesh_update), ("texcoords", C.c_void_p), ("num_texcoords", C.c_int32),
+                ("texcoord_idx", C.c_void_p), ("texture", C.c_void_p)]
+
+
 STRUCT_SIZES = {"rt_shape": 80, "rt_material": 28, "rt_bvh_node": 32, "rt_tri": 64, "rt_shade": 64,
                 "rt_light": 28, "rt_render_params": 56, "rt_counters": 72}
 
@@ -158,6 +163,7 @@ GPU_PROTOTYPES = {
     "rt_gpu_radiance_rays": (I, [VP, C.POINTER(rt_radiance_query), VP]),
     "rt_gpu_update_mesh": (I, [VP, I32, C.POINTER(rt_mesh_update), VP]),
     "rt_gpu_refit_mesh": (I, [VP, I32, C.POINTER(rt_mesh_update), VP, VP]),
+    "rt_gpu_replace_mesh": (I, [VP, I32, C.POINTER(rt_mesh_replace), VP]),
     "rt_gpu_update_shapes": (I, [VP, C.POINTER(rt_shape), I32, I32, VP]),
     "rt_gpu_trace_rays": (I, [VP, PF, I32, I32, PI32, PI32, PF]),
     "rt_gpu_kat": (I, [VP, I32, VP, VP, I32, I32, VP, VP]),

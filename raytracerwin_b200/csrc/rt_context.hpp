@@ -121,22 +121,25 @@ struct rt_gpu_ctx
     size_t tune_sample_budget = 0;              // RT_SAMPLE_BUDGET_MB at create (0: by call size)
     bool tune_time_long = false;                // RT_TIME_LONG at create: timed brackets span walk + long walk
 
-    // ---- scene updates (rt_gpu_update_mesh / rt_gpu_update_shapes) ----
+    // ---- scene updates (rt_gpu_update_mesh / rt_gpu_refit_mesh / rt_gpu_replace_mesh / rt_gpu_update_shapes) ----
     // What the updates check and swap, per uploaded shape and mesh.  A mesh's arrays are double-buffered from its first
     // update on: an update builds into the spare set and publishes it; the published set becomes the spare.
     std::vector<rt_shape> host_shapes;          // the records as uploaded (materials follow rt_gpu_update_shapes)
     int host_num_materials = 0;
-    struct MeshArrays { rt_bvh_node* nodes; rt_tri* tris; rt_shade* shade; };
+    // One set of a mesh's arrays: room for `cap` triangles (2 * cap - 1 nodes).  `pooled`: from cudaMallocAsync by an
+    // update, released with cudaFreeAsync when a larger set replaces it; the uploaded set (cudaMalloc) stays in
+    // scene_allocs until the next upload or destroy.
+    struct MeshArrays { rt_bvh_node* nodes; rt_tri* tris; rt_shade* shade; int cap; bool pooled; };
     struct MeshState
     {
-        int num_tris = 0;
+        int num_tris = 0;                       // published counts: as uploaded, then those of the last replace
         int num_nodes = 0;                      // as uploaded: an update builds 2 * num_tris - 1
         int users = 0;                          // shapes that reference the mesh
         // The published tree is a full binary tree over all its nodes whose leaves name every triangle slot exactly once
         // (checked at upload, true after an update): what rt_gpu_refit_mesh needs to reach and rewrite every node.
         bool refittable = false;
-        MeshArrays cur = { nullptr, nullptr, nullptr };      // published (shade in leaf order)
-        MeshArrays spare = { nullptr, nullptr, nullptr };    // allocated by the first update
+        MeshArrays cur = { nullptr, nullptr, nullptr, 0, false };      // published (shade in leaf order)
+        MeshArrays spare = { nullptr, nullptr, nullptr, 0, false };    // allocated by the first update
     };
     std::vector<MeshState> mesh_state;
     // Recorded by every update after it has published; every later scene reader waits for it on its stream.  Live from

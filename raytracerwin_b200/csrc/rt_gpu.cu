@@ -110,15 +110,21 @@ __global__ void rt_shade_leaf_order_kernel(const float4* __restrict__ tris, cons
     for (int j = 0; j < 4; j++) out[4 * (size_t)k + j] = shade[4 * (size_t)index + j];
 }
 
-// ---- scene updates (rt_gpu_update_mesh) ----
+// ---- scene updates (rt_gpu_update_mesh, rt_gpu_replace_mesh) ----
 // Bit flags of the update's input check (the builder's scratch flag)
 #define RT_UPD_BAD_POINT_INDEX 1
 #define RT_UPD_BAD_NORMAL_INDEX 2
+#define RT_UPD_BAD_TEXCOORD_INDEX 4
+#define RT_UPD_BAD_TEXTURE 8
 
-// Checks every point / normal index and copies the point indices into `safe` with bad ones replaced by 0, so that the
-// builder never reads outside `points` even before the host has seen the flag (the build is then thrown away).
+// Checks every point / normal / texcoord index and copies the point and texcoord indices into `safe` / `safe_t` with
+// bad ones replaced by 0, so that no later kernel reads outside `points` or `texcoords` even before the host has seen
+// the flag (the build is then thrown away).  A replace also gives one texture slot per triangle: one the upload would
+// refuse (>= the mesh's slot count, or a slot without pixels) is bad; negative slots pass.
 __global__ void rt_update_check_kernel(const int* __restrict__ pidx, int num_points, const int* __restrict__ nidx, int num_normals,
-                                       int n, int* __restrict__ safe, int* __restrict__ flag)
+                                       const int* __restrict__ tidx, int num_texcoords, const int* __restrict__ texture,
+                                       const DevMesh* __restrict__ mesh, int n, int* __restrict__ safe, int* __restrict__ safe_t,
+                                       int* __restrict__ flag)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -126,21 +132,25 @@ __global__ void rt_update_check_kernel(const int* __restrict__ pidx, int num_poi
     if (v < 0 || v >= num_points) { v = 0; bad |= RT_UPD_BAD_POINT_INDEX; }
     safe[i] = v;
     if (nidx) { const int w = nidx[i]; if (w < 0 || w >= num_normals) bad |= RT_UPD_BAD_NORMAL_INDEX; }
+    if (tidx)
+    {
+        int w = tidx[i];
+        if (w < 0 || w >= num_texcoords) { w = 0; bad |= RT_UPD_BAD_TEXCOORD_INDEX; }
+        safe_t[i] = w;
+    }
+    if (texture && i % 3 == 0)
+    {
+        const int slot = texture[i / 3];
+        if (slot >= mesh->num_textures || (slot >= 0 && mesh->textures[slot].width == 0)) bad |= RT_UPD_BAD_TEXTURE;
+    }
     if (bad) atomicOr(flag, bad);
 }
 
-// Shading records in ORIGINAL triangle order: the new normals (normals[nidx], or every corner the triangle's
-// unnormalised geometric normal as host/mesh_loader.cpp computes it), uv and texture slot from the published record.
-// Published leaf record j belongs to triangle cur_tris[j].index.
-__global__ void rt_update_shade_kernel(const float4* __restrict__ cur_tris, const float* __restrict__ cur_shade,
-                                       const float* __restrict__ points, const int* __restrict__ pidx,
-                                       const float* __restrict__ normals, const int* __restrict__ nidx, float* __restrict__ out, int n)
+// The corner normals of triangle t into dst[0..8]: normals[nidx], or every corner the triangle's unnormalised geometric
+// normal as host/mesh_loader.cpp computes it.
+__device__ __forceinline__ void upd_corner_normals(float* dst, int t, const float* __restrict__ points, const int* __restrict__ pidx,
+                                                   const float* __restrict__ normals, const int* __restrict__ nidx)
 {
-    const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n) return;
-    const int t = __float_as_int(cur_tris[4 * (size_t)j].w);
-    const float* src = cur_shade + 16 * (size_t)j;
-    float* dst = out + 16 * (size_t)t;
     if (normals)
         for (int k = 0; k < 3; k++)
         {
@@ -157,7 +167,45 @@ __global__ void rt_update_shade_kernel(const float4* __restrict__ cur_tris, cons
         const float nx = ay * bz - az * by, ny = az * bx - ax * bz, nz = ax * by - ay * bx;
         for (int k = 0; k < 3; k++) { dst[3 * k] = nx; dst[3 * k + 1] = ny; dst[3 * k + 2] = nz; }
     }
+}
+
+// Shading records in ORIGINAL triangle order: the new normals, uv and texture slot from the published record.
+// Published leaf record j belongs to triangle cur_tris[j].index.
+__global__ void rt_update_shade_kernel(const float4* __restrict__ cur_tris, const float* __restrict__ cur_shade,
+                                       const float* __restrict__ points, const int* __restrict__ pidx,
+                                       const float* __restrict__ normals, const int* __restrict__ nidx, float* __restrict__ out, int n)
+{
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const int t = __float_as_int(cur_tris[4 * (size_t)j].w);
+    const float* src = cur_shade + 16 * (size_t)j;
+    float* dst = out + 16 * (size_t)t;
+    upd_corner_normals(dst, t, points, pidx, normals, nidx);
     for (int k = 9; k < 16; k++) dst[k] = src[k];           // uv0 uv1 uv2 texture
+}
+
+// A replace's shading records in original order: normals as rt_update_shade_kernel, uv copied from
+// texcoords[tidx] (bits as given; (0, 0) without texcoords), the slot from `texture` (-1 without).
+__global__ void rt_replace_shade_kernel(const float* __restrict__ points, const int* __restrict__ pidx,
+                                        const float* __restrict__ normals, const int* __restrict__ nidx,
+                                        const float* __restrict__ texcoords, const int* __restrict__ tidx,
+                                        const int* __restrict__ texture, float* __restrict__ out, int n)
+{
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    float* dst = out + 16 * (size_t)t;
+    upd_corner_normals(dst, t, points, pidx, normals, nidx);
+    for (int k = 0; k < 3; k++)
+    {
+        float u = 0.0f, v = 0.0f;
+        if (texcoords)
+        {
+            const float* uv = texcoords + 2 * (size_t)tidx[3 * (size_t)t + k];
+            u = uv[0]; v = uv[1];
+        }
+        dst[9 + 2 * k] = u; dst[10 + 2 * k] = v;
+    }
+    dst[15] = __int_as_float(texture ? texture[t] : -1);
 }
 
 // RAabb::Expand over the points in array order as 64-bit keys: value order in the high word (-0 == +0, as `<`
@@ -197,11 +245,12 @@ __global__ void rt_update_bounds_kernel(const float* __restrict__ points, int nu
     }
 }
 
-// The publication of an update (one thread, after the join): the mesh's record points at the new arrays, with the
-// culling margin of the new root (as upload computes it) and without the 8-wide copy; the shape gets the new bounds.
-// Kernels read both records at run time.
+// The publication of an update (one thread, after the join): the mesh's record points at the new arrays of num_tris
+// triangles and 2 * num_tris - 1 nodes, with the culling margin of the new root (as upload computes it) and without the
+// 8-wide copy; the shape gets the new bounds.  Kernels read both records at run time.
 __global__ void rt_update_publish_kernel(DevMesh* meshes, int mesh, rt_shape* shapes, int shape, const rt_bvh_node* nodes,
-                                         const rt_tri* tris, const rt_shade* shade, const unsigned long long* keys, const float* points)
+                                         const rt_tri* tris, const rt_shade* shade, int num_tris, const unsigned long long* keys,
+                                         const float* points)
 {
     float scale = 0.0f;
     for (int k = 0; k < 3; k++)
@@ -212,6 +261,7 @@ __global__ void rt_update_publish_kernel(DevMesh* meshes, int mesh, rt_shape* sh
     DevMesh& m = meshes[mesh];
     m.nodes = (const float4*)nodes; m.tris = (const float4*)tris; m.shade = (const float4*)shade;
     m.octo = nullptr;
+    m.num_tris = num_tris; m.num_nodes = 2 * num_tris - 1;
     m.cull_scale = scale;
     rt_shape& s = shapes[shape];
     for (int c = 0; c < 3; c++)
@@ -1081,7 +1131,8 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
             ctx->mesh_state.back().num_tris = m.num_tris;
             ctx->mesh_state.back().num_nodes = m.num_nodes;
             ctx->mesh_state.back().refittable = refittable[i] != 0;
-            ctx->mesh_state.back().cur = rt_gpu_ctx::MeshArrays{ dn, dt, (rt_shade*)dsh };
+            // room for min(T, (N + 1) / 2) triangles when a replace builds into this set after it has become the spare
+            ctx->mesh_state.back().cur = rt_gpu_ctx::MeshArrays{ dn, dt, (rt_shade*)dsh, std::min(m.num_tris, (m.num_nodes + 1) / 2), false };
             dm.octo = nullptr;
             if (m.num_nodes > 0 && ctx->tune_octo)
             {
@@ -1746,9 +1797,10 @@ static int alloc_on(rt_gpu_ctx* ctx, void** out, size_t bytes, cudaStream_t st)
 
 static inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
-// The host-side checks of rt_gpu_update_mesh and rt_gpu_refit_mesh (`fn` names the call in the messages); the shape's
-// mesh goes to *mesh.
-static int check_mesh_update(rt_gpu_ctx* ctx, const char* fn, int32_t shape, const rt_mesh_update* u, int* mesh)
+// The host-side checks of rt_gpu_update_mesh, rt_gpu_refit_mesh and rt_gpu_replace_mesh (`fn` names the call in the
+// messages); the shape's mesh goes to *mesh.  An update and a refit keep the published count (`same_count`); a replace
+// takes any positive count and publishes a tree of its own, so the published node count does not matter to it.
+static int check_mesh_update(rt_gpu_ctx* ctx, const char* fn, int32_t shape, const rt_mesh_update* u, bool same_count, int* mesh)
 {
     const std::string f(fn);
     if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, f + " before rt_gpu_upload_scene");
@@ -1758,12 +1810,20 @@ static int check_mesh_update(rt_gpu_ctx* ctx, const char* fn, int32_t shape, con
     const int mi = ctx->host_shapes[shape].mesh;
     const rt_gpu_ctx::MeshState& ms = ctx->mesh_state[mi];
     if (ms.users != 1) return fail(ctx, RT_ERR_INVALID, f + ": another shape references the same mesh");
-    if (ms.num_tris <= 0 || u->num_tris != ms.num_tris)
-        return fail(ctx, RT_ERR_INVALID, f + ": num_tris differs from the uploaded mesh's");
-    // the update publishes a tree of 2T-1 nodes in an array of that size; the walks read num_nodes as uploaded
-    if (ms.num_nodes != 2 * ms.num_tris - 1)
-        return fail(ctx, RT_ERR_INVALID, f + ": the uploaded mesh's node count is not 2 * num_tris - 1 (not a tree of its triangles)");
-    if ((long long)ms.num_tris * 3 >= 0xFFFFFFFFll) return fail(ctx, RT_ERR_INVALID, f + ": too many triangles");
+    if (same_count)
+    {
+        if (ms.num_tris <= 0 || u->num_tris != ms.num_tris)
+            return fail(ctx, RT_ERR_INVALID, f + ": num_tris differs from the uploaded mesh's");
+        // the update publishes a tree of 2T-1 nodes in an array of that size; the walks read num_nodes as uploaded
+        if (ms.num_nodes != 2 * ms.num_tris - 1)
+            return fail(ctx, RT_ERR_INVALID, f + ": the uploaded mesh's node count is not 2 * num_tris - 1 (not a tree of its triangles)");
+    }
+    else
+    {
+        if (ms.num_tris <= 0) return fail(ctx, RT_ERR_INVALID, f + ": the uploaded mesh has no triangles");
+        if (u->num_tris <= 0) return fail(ctx, RT_ERR_INVALID, f + ": num_tris must be positive");
+    }
+    if ((long long)u->num_tris * 3 >= 0xFFFFFFFFll) return fail(ctx, RT_ERR_INVALID, f + ": too many triangles");
     if (u->num_points <= 0) return fail(ctx, RT_ERR_INVALID, f + ": num_points must be positive");
     if (!u->points || !u->point_idx) return fail(ctx, RT_ERR_INVALID, f + ": points and point_idx are required");
     if ((u->normals == nullptr) != (u->normal_idx == nullptr))
@@ -1782,13 +1842,29 @@ static int check_mesh_update(rt_gpu_ctx* ctx, const char* fn, int32_t shape, con
     return RT_OK;
 }
 
-// The spare set of a mesh's arrays (first update or refit) and the updates' scratch block (only grows), on `st` after
-// wait_scene: the spare set and the scratch were last read by work the previous update waited for.
-static int alloc_spare(rt_gpu_ctx* ctx, rt_gpu_ctx::MeshState& ms, cudaStream_t st)
+static inline size_t mesh_set_bytes(size_t T)
 {
-    if (ms.spare.nodes) return RT_OK;
-    const size_t T = (size_t)ms.num_tris;
-    rt_gpu_ctx::MeshArrays a = { nullptr, nullptr, nullptr };
+    return (2 * T - 1) * sizeof(rt_bvh_node) + T * (sizeof(rt_tri) + sizeof(rt_shade));
+}
+
+// A spare set of a mesh's arrays with room for `tris` triangles, on `st` after wait_scene: the spare set and the
+// scratch were last read by work the previous update waited for, so a spare that is too small can be released here.
+// Capacity only grows: a smaller count builds into the larger set.
+static int alloc_spare(rt_gpu_ctx* ctx, rt_gpu_ctx::MeshState& ms, int tris, cudaStream_t st)
+{
+    if (ms.spare.nodes && ms.spare.cap >= tris) return RT_OK;
+    if (ms.spare.pooled)
+    {
+        for (void* p : { (void*)ms.spare.nodes, (void*)ms.spare.tris, (void*)ms.spare.shade })
+        {
+            RT_CUDA(cudaFreeAsync(p, st));
+            ctx->scene_allocs.erase(std::find(ctx->scene_allocs.begin(), ctx->scene_allocs.end(), p));
+        }
+        ctx->scene_bytes -= mesh_set_bytes((size_t)ms.spare.cap);
+    }
+    ms.spare = rt_gpu_ctx::MeshArrays{ nullptr, nullptr, nullptr, 0, false };
+    const size_t T = (size_t)tris;
+    rt_gpu_ctx::MeshArrays a = { nullptr, nullptr, nullptr, tris, true };
     int rc;
     if ((rc = alloc_on(ctx, (void**)&a.nodes, (2 * T - 1) * sizeof(rt_bvh_node), st)) != RT_OK) return rc;
     ctx->scene_allocs.push_back(a.nodes);
@@ -1796,7 +1872,7 @@ static int alloc_spare(rt_gpu_ctx* ctx, rt_gpu_ctx::MeshState& ms, cudaStream_t 
     ctx->scene_allocs.push_back(a.tris);
     if ((rc = alloc_on(ctx, (void**)&a.shade, T * sizeof(rt_shade), st)) != RT_OK) return rc;
     ctx->scene_allocs.push_back(a.shade);
-    ctx->scene_bytes += (2 * T - 1) * sizeof(rt_bvh_node) + T * (sizeof(rt_tri) + sizeof(rt_shade));
+    ctx->scene_bytes += mesh_set_bytes(T);
     ms.spare = a;
     return RT_OK;
 }
@@ -1812,61 +1888,117 @@ static int grow_update_scratch(rt_gpu_ctx* ctx, size_t need, cudaStream_t st)
     return RT_OK;
 }
 
+// The body of rt_gpu_update_mesh and rt_gpu_replace_mesh after their host checks: the device check, a tree of
+// r->geometry.num_tris triangles built into the spare set, the shading records (uv and slot from the published records
+// for an update, from the caller's arrays for a `replace`), bounds and margin, then the publish of the arrays and the
+// counts after every earlier scene reader.  Returns once the build is complete.
+static int rebuild_mesh(rt_gpu_ctx* ctx, const char* fn, int32_t shape, int mi, const rt_mesh_replace* r, bool replace, cudaStream_t st)
+{
+    const rt_mesh_update* u = &r->geometry;
+    rt_gpu_ctx::MeshState& ms = ctx->mesh_state[mi];
+    const int T = u->num_tris;
+    RT_CUDA(wait_scene(ctx, st));
+    int rc;
+    if ((rc = alloc_spare(ctx, ms, T, st)) != RT_OK) return rc;
+    // scratch: the builder's block, safe point indices (3T), safe texcoord indices (3T, a replace with texcoords only),
+    // shading records in original order (T), bounds keys (6)
+    const size_t build_bytes = align256(rt_bvh_scratch_bytes(T));
+    const size_t idx_off = build_bytes, tidx_off = idx_off + align256(3 * (size_t)T * sizeof(int));
+    const size_t shade_off = tidx_off + (r->texcoord_idx ? align256(3 * (size_t)T * sizeof(int)) : 0);
+    const size_t keys_off = shade_off + align256((size_t)T * sizeof(rt_shade));
+    if ((rc = grow_update_scratch(ctx, keys_off + 6 * sizeof(unsigned long long), st)) != RT_OK) return rc;
+    if (!ctx->update_counts) RT_CUDA(cudaHostAlloc((void**)&ctx->update_counts, 4 * sizeof(int), cudaHostAllocDefault));
+    char* scratch = (char*)ctx->update_scratch;
+    int* safe_idx = (int*)(scratch + idx_off);
+    int* safe_tidx = r->texcoord_idx ? (int*)(scratch + tidx_off) : nullptr;
+    rt_shade* shade_tmp = (rt_shade*)(scratch + shade_off);
+    unsigned long long* keys = (unsigned long long*)(scratch + keys_off);
+    int* flag = rt_bvh_scratch_flag(scratch);
+
+    const int n3 = 3 * T;
+    const unsigned gT = (unsigned)((T + 255) / 256);
+    RT_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), st));
+    rt_update_check_kernel<<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(u->point_idx, u->num_points, u->normal_idx,
+                                                                          u->normals ? u->num_normals : 0, r->texcoord_idx,
+                                                                          r->num_texcoords, r->texture, ctx->scene.meshes + mi,
+                                                                          n3, safe_idx, safe_tidx, flag);
+    RT_CUDA(cudaGetLastError());
+    ctx->launches++;
+    const std::string message = std::string(fn) + (replace ? ": point, normal or texcoord index or texture slot out of range"
+                                                           : ": point or normal index out of range");
+    rc = rt_bvh_build_core(ctx, u->points, safe_idx, T, st, scratch, ctx->update_counts, true, message.c_str(),
+                           ms.spare.nodes, ms.spare.tris, nullptr);
+    if (rc != RT_OK)
+    {
+        if (rc == RT_ERR_INVALID && replace)
+        {
+            const int bad = ctx->update_counts[2];
+            std::string what;
+            for (auto b : { std::make_pair(RT_UPD_BAD_POINT_INDEX, "point index"), std::make_pair(RT_UPD_BAD_NORMAL_INDEX, "normal index"),
+                            std::make_pair(RT_UPD_BAD_TEXCOORD_INDEX, "texcoord index"), std::make_pair(RT_UPD_BAD_TEXTURE, "texture slot") })
+                if (bad & b.first) what += (what.empty() ? " " : ", ") + std::string(b.second);
+            ctx->err = std::string(fn) + ": out of range:" + what;
+        }
+        return rc;
+    }
+    rt_patch_right_child<<<(unsigned)((2 * T - 1 + 255) / 256), 256, 0, st>>>(ms.spare.nodes, 2 * T - 1);
+    if (replace)
+        rt_replace_shade_kernel<<<gT, 256, 0, st>>>(u->points, safe_idx, u->normals, u->normal_idx, r->texcoords, safe_tidx,
+                                                    r->texture, (float*)shade_tmp, T);
+    else
+        rt_update_shade_kernel<<<gT, 256, 0, st>>>((const float4*)ms.cur.tris, (const float*)ms.cur.shade, u->points, safe_idx,
+                                                   u->normals, u->normal_idx, (float*)shade_tmp, T);
+    rt_shade_leaf_order_kernel<<<gT, 256, 0, st>>>((const float4*)ms.spare.tris, (const float4*)shade_tmp, (float4*)ms.spare.shade, T);
+    RT_CUDA(cudaMemsetAsync(keys, 0xFF, 3 * sizeof(unsigned long long), st));
+    RT_CUDA(cudaMemsetAsync(keys + 3, 0, 3 * sizeof(unsigned long long), st));
+    rt_update_bounds_kernel<<<(unsigned)((u->num_points + 255) / 256), 256, 0, st>>>(u->points, u->num_points, keys);
+    RT_CUDA(cudaGetLastError());
+    ctx->launches += 4;
+    // publish once every call enqueued before this one has finished reading the old arrays
+    if ((rc = join_scene_readers(ctx, st)) != RT_OK) return rc;
+    rt_update_publish_kernel<<<1, 1, 0, st>>>(const_cast<DevMesh*>(ctx->scene.meshes), mi, const_cast<rt_shape*>(ctx->scene.shapes),
+                                              shape, ms.spare.nodes, ms.spare.tris, ms.spare.shade, T, keys, u->points);
+    RT_CUDA(cudaGetLastError());
+    ctx->launches++;
+    if ((rc = publish_done(ctx, st)) != RT_OK) return rc;
+    std::swap(ms.cur, ms.spare);
+    ms.num_tris = T; ms.num_nodes = 2 * T - 1;
+    ms.refittable = true;                   // the builder's tree
+    // the shared-memory stage holds mesh 0's uploaded top levels; a pointer test cannot tell the ping-pong's arrays apart
+    if (mi == 0) ctx->scene.top_of = nullptr;
+    return RT_OK;
+}
+
 int rt_gpu_update_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, void* stream)
 {
     return rt_guard(ctx, [&]() -> int {
         if (!ctx) return RT_ERR_INVALID;
         int mi = -1;
-        int rc = check_mesh_update(ctx, "rt_gpu_update_mesh", shape, u, &mi);
+        const int rc = check_mesh_update(ctx, "rt_gpu_update_mesh", shape, u, true, &mi);
         if (rc != RT_OK) return rc;
-        rt_gpu_ctx::MeshState& ms = ctx->mesh_state[mi];
-        const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-        const int T = ms.num_tris;
-        RT_CUDA(wait_scene(ctx, st));
-        if ((rc = alloc_spare(ctx, ms, st)) != RT_OK) return rc;
-        // scratch: the builder's block, safe point indices (3T), shading records in original order (T), bounds keys (6)
-        const size_t build_bytes = align256(rt_bvh_scratch_bytes(T));
-        const size_t idx_off = build_bytes, shade_off = idx_off + align256(3 * (size_t)T * sizeof(int));
-        const size_t keys_off = shade_off + align256((size_t)T * sizeof(rt_shade));
-        if ((rc = grow_update_scratch(ctx, keys_off + 6 * sizeof(unsigned long long), st)) != RT_OK) return rc;
-        if (!ctx->update_counts) RT_CUDA(cudaHostAlloc((void**)&ctx->update_counts, 4 * sizeof(int), cudaHostAllocDefault));
-        char* scratch = (char*)ctx->update_scratch;
-        int* safe_idx = (int*)(scratch + idx_off);
-        rt_shade* shade_tmp = (rt_shade*)(scratch + shade_off);
-        unsigned long long* keys = (unsigned long long*)(scratch + keys_off);
-        int* flag = rt_bvh_scratch_flag(scratch);
+        const rt_mesh_replace r = { *u, nullptr, 0, nullptr, nullptr };
+        return rebuild_mesh(ctx, "rt_gpu_update_mesh", shape, mi, &r, false, stream ? (cudaStream_t)stream : ctx->stream);
+    });
+}
 
-        const int n3 = 3 * T;
-        RT_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), st));
-        rt_update_check_kernel<<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(u->point_idx, u->num_points, u->normal_idx,
-                                                                              u->normals ? u->num_normals : 0, n3, safe_idx, flag);
-        RT_CUDA(cudaGetLastError());
-        ctx->launches++;
-        rc = rt_bvh_build_core(ctx, u->points, safe_idx, T, st, scratch, ctx->update_counts, true,
-                               "rt_gpu_update_mesh: point or normal index out of range", ms.spare.nodes, ms.spare.tris, nullptr);
+int rt_gpu_replace_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_replace* r, void* stream)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        const char* fn = "rt_gpu_replace_mesh";
+        if (!r) return fail(ctx, ctx->has_scene ? RT_ERR_INVALID : RT_ERR_NO_SCENE, std::string(fn) + ": replace is null");
+        int mi = -1;
+        int rc = check_mesh_update(ctx, fn, shape, &r->geometry, false, &mi);
         if (rc != RT_OK) return rc;
-        rt_patch_right_child<<<(unsigned)((2 * T - 1 + 255) / 256), 256, 0, st>>>(ms.spare.nodes, 2 * T - 1);
-        rt_update_shade_kernel<<<(unsigned)((T + 255) / 256), 256, 0, st>>>((const float4*)ms.cur.tris, (const float*)ms.cur.shade,
-                                                                            u->points, safe_idx, u->normals, u->normal_idx, (float*)shade_tmp, T);
-        rt_shade_leaf_order_kernel<<<(unsigned)((T + 255) / 256), 256, 0, st>>>((const float4*)ms.spare.tris, (const float4*)shade_tmp,
-                                                                                (float4*)ms.spare.shade, T);
-        RT_CUDA(cudaMemsetAsync(keys, 0xFF, 3 * sizeof(unsigned long long), st));
-        RT_CUDA(cudaMemsetAsync(keys + 3, 0, 3 * sizeof(unsigned long long), st));
-        rt_update_bounds_kernel<<<(unsigned)((u->num_points + 255) / 256), 256, 0, st>>>(u->points, u->num_points, keys);
-        RT_CUDA(cudaGetLastError());
-        ctx->launches += 4;
-        // publish once every call enqueued before this one has finished reading the old arrays
-        if ((rc = join_scene_readers(ctx, st)) != RT_OK) return rc;
-        rt_update_publish_kernel<<<1, 1, 0, st>>>(const_cast<DevMesh*>(ctx->scene.meshes), mi, const_cast<rt_shape*>(ctx->scene.shapes),
-                                                  shape, ms.spare.nodes, ms.spare.tris, ms.spare.shade, keys, u->points);
-        RT_CUDA(cudaGetLastError());
-        ctx->launches++;
-        if ((rc = publish_done(ctx, st)) != RT_OK) return rc;
-        std::swap(ms.cur, ms.spare);
-        ms.refittable = true;                   // the builder's tree
-        // the shared-memory stage holds mesh 0's uploaded top levels; a pointer test cannot tell the ping-pong's arrays apart
-        if (mi == 0) ctx->scene.top_of = nullptr;
-        return RT_OK;
+        if ((r->texcoords == nullptr) != (r->texcoord_idx == nullptr))
+            return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": texcoords and texcoord_idx come together");
+        if (r->texcoords && r->num_texcoords <= 0) return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": num_texcoords must be positive");
+        const void* ptrs[3] = { r->texcoords, r->texcoord_idx, r->texture };
+        const char* names[3] = { "texcoords", "texcoord_idx", "texture" };
+        for (int k = 0; k < 3; k++)
+            if (ptrs[k] && ((uintptr_t)ptrs[k] % 4 != 0 || !on_device(ctx, ptrs[k])))
+                return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": " + names[k] + " must be 4-byte aligned device memory of the context's GPU");
+        return rebuild_mesh(ctx, fn, shape, mi, r, true, stream ? (cudaStream_t)stream : ctx->stream);
     });
 }
 
@@ -1878,7 +2010,7 @@ int rt_gpu_refit_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, i
     return rt_guard(ctx, [&]() -> int {
         if (!ctx) return RT_ERR_INVALID;
         int mi = -1;
-        int rc = check_mesh_update(ctx, "rt_gpu_refit_mesh", shape, u, &mi);
+        int rc = check_mesh_update(ctx, "rt_gpu_refit_mesh", shape, u, true, &mi);
         if (rc != RT_OK) return rc;
         if (status && ((uintptr_t)status % 4 != 0 || !on_device(ctx, status)))
             return fail(ctx, RT_ERR_INVALID, "rt_gpu_refit_mesh: status must be 4-byte aligned device memory of the context's GPU");
@@ -1889,7 +2021,7 @@ int rt_gpu_refit_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, i
         const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
         const int T = ms.num_tris, N = 2 * T - 1;
         RT_CUDA(wait_scene(ctx, st));
-        if ((rc = alloc_spare(ctx, ms, st)) != RT_OK) return rc;
+        if ((rc = alloc_spare(ctx, ms, T, st)) != RT_OK) return rc;
         // scratch: flag, safe point and normal indices (3T each), shading records in original order (T), bounds keys
         // (6), saved bounds and margin (7 floats), parent links (N) + leaf nodes (T), arrival counters (N)
         const size_t pidx_off = 256, nidx_off = pidx_off + align256(3 * (size_t)T * sizeof(int));
@@ -1934,7 +2066,7 @@ int rt_gpu_refit_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, i
         // publish once every call enqueued before this one has finished reading the old arrays
         if ((rc = join_scene_readers(ctx, st)) != RT_OK) return rc;
         rt_update_publish_kernel<<<1, 1, 0, st>>>(const_cast<DevMesh*>(ctx->scene.meshes), mi, const_cast<rt_shape*>(ctx->scene.shapes),
-                                                  shape, ms.spare.nodes, ms.spare.tris, ms.spare.shade, keys, u->points);
+                                                  shape, ms.spare.nodes, ms.spare.tris, ms.spare.shade, T, keys, u->points);
         rt_refit_finish_kernel<<<1, 1, 0, st>>>(flag, status, dmesh, dshape, saved);
         RT_CUDA(cudaGetLastError());
         ctx->launches += 2;
