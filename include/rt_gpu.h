@@ -12,6 +12,7 @@
  *                        (RayTracerScene.cpp:14-18) and PseudoRandomUnitVectors (Math.cpp:17-19)
  *   rt_gpu_render_tile   replaces ThreadWorker_Render(begin, end, MaxBounceCount, Option)
  *                        (RayTracerProgram.cpp:131-188), i.e. one RenderThreadTask (:79-95)
+ *   rt_gpu_render_view   render_tile from a camera of the call's own: eye, orientation and image plane per call
  *   rt_gpu_readback      replaces reading bitcolor[] / accuBuffer[] (:49,:77)
  *   rt_gpu_query_rays    FindIntersectionWithScene (RayTracerScene.cpp:99-125) and the shadow query of
  *                        CalculateLightColor (:152-164) on batches of the caller's rays in device memory
@@ -239,6 +240,33 @@ int rt_gpu_reset_accum(rt_gpu_ctx* ctx, int32_t width, int32_t height);
 /* Enqueues one render task on the context's stream and returns immediately.
  * If the buffers do not match params->width/height they are reset first. */
 int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* params);
+
+/* ---- cameras -----------------------------------------------------------------------------------
+ * A camera of one render call: the eye, the orientation and the image plane, in place of the uploaded scene's
+ * eye / dir_z / ray_distance and the reference's fixed view down -z.  Nothing is kept: the next call without a
+ * camera renders the uploaded view again. */
+typedef struct rt_camera {
+    float eye[3];          /* origin of every camera ray */
+    float right[3];        /* world direction of camera-space +x (the reference's dx axis) */
+    float up[3];           /* world direction of camera-space +y (dy) */
+    float back[3];         /* world direction of camera-space +z: the camera looks along -back when dir_z < 0 */
+    float dir_z;           /* camera-space z of the image plane (the reference's -0.5; sets the field of view) */
+    float ray_distance;    /* Distance of camera rays (bounce segments are not affected) */
+} rt_camera;
+
+/* rt_gpu_render_tile with the camera rays of `camera`.  camera == NULL is exactly rt_gpu_render_tile(ctx, params);
+ * every other rule of render_tile applies unchanged (frame slot, pass chunks, tiles, counters, last_render_ms,
+ * kernel-class timing; enqueues and returns).
+ * The camera ray of (pixel, sub-sample): v = (dx + ox, dy + oy, dir_z) with dx, dy, ox, oy and their rand() draws
+ * those of render_tile (RayTracerProgram.cpp:133-165).  If right, up and back are exactly (1,0,0), (0,1,0), (0,0,1)
+ * (compared as floats, so -0 is 0) the direction is normalized(v): the reference's generator with the camera's eye,
+ * dir_z and distance.  Otherwise w[c] = (v.x*right[c] + v.y*up[c]) + v.z*back[c], in fp32, one rounding per
+ * operation in that order, and the direction is normalized(w) (RVec3::GetNormalizedVec3: short vectors unchanged).
+ * The basis need not be orthonormal; the image keeps the reference's mirroring in x.  Different frame slots may
+ * render different cameras at the same time, and tiled ranks that pass the same camera assemble the same frame.
+ * RT_ERR_INVALID, with nothing enqueued, for a non-finite field, a basis whose determinant (in double) is 0, and
+ * every error of render_tile. */
+int rt_gpu_render_view(rt_gpu_ctx* ctx, const rt_render_params* params, const rt_camera* camera);
 
 /* ---- ray queries on device memory -------------------------------------------------------------
  * Batches of the caller's own rays through the same wavefront kernels as render_tile (generate -> packet /

@@ -14,7 +14,7 @@ import numpy as np
 
 from . import _abi
 from ._abi import (rt_render_params, rt_counters, rt_scene_desc, rt_ray_query, rt_radiance_query, rt_mesh_update,  # noqa: F401
-                   rt_mesh_replace,
+                   rt_mesh_replace, rt_camera,
                    RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY, RT_QUERY_NEAREST, RT_QUERY_ANY,
                    RT_TRAVERSE_EXACT, RT_TRAVERSE_CULLED,
                    RT_READ_ACCUM_RGBN_F32, RT_READ_DISPLAY_ARGB8, RT_READ_PRIMARY_IDS_I32X2,
@@ -209,6 +209,37 @@ def make_params(width, height, mode=RT_MODE_PATH, max_bounce=10, pass_begin=0, p
     return p
 
 
+def camera(eye, right, up, back, dir_z=-0.5, ray_distance=1000.0):
+    """An rt_camera from raw values (rt_gpu_render_view takes them as they are; the basis need not be orthonormal)."""
+    c = rt_camera()
+    c.eye, c.right, c.up, c.back = _f3(eye), _f3(right), _f3(up), _f3(back)
+    c.dir_z, c.ray_distance = float(dir_z), float(ray_distance)
+    return c
+
+
+def look_at(eye, target, up=(0.0, 1.0, 0.0), dir_z=-0.5, ray_distance=1000.0):
+    """An rt_camera at `eye` looking at `target` (with dir_z < 0), `up` as near camera-space +y as it can be:
+    back = normalize(eye - target), right = normalize(cross(up, back)), up' = cross(back, right), in float64 and
+    rounded to float32.  look_at((0, 0, 7), (0, 0, 0)) is the uploaded default view: the identity basis.
+    Raises ValueError for target == eye and for an `up` parallel to the view direction."""
+    e, t, u = (np.asarray(v, np.float64).reshape(3) for v in (eye, target, up))
+    if not (np.isfinite(e).all() and np.isfinite(t).all() and np.isfinite(u).all()):
+        raise ValueError("look_at: eye, target and up must be finite")
+    back = e - t
+    n = np.linalg.norm(back)
+    if n == 0.0:
+        raise ValueError("look_at: target == eye")
+    back = back / n
+    right = np.cross(u, back)
+    n = np.linalg.norm(right)
+    if n <= 1e-12 * max(np.linalg.norm(u), 1e-300):
+        raise ValueError("look_at: up is parallel to the view direction")
+    right = right / n
+    up2 = np.cross(back, right)
+    f = lambda v: v.astype(np.float32)
+    return camera(f(e), f(right), f(up2), f(back), dir_z, ray_distance)
+
+
 class GpuContext:
     """One rt_gpu_ctx: a scene resident on one B200 plus its device framebuffers."""
 
@@ -255,8 +286,15 @@ class GpuContext:
     def reset_counters(self):
         self._check(self._lib.rt_gpu_reset_counters(self._h))
 
-    def render_tile(self, params):
-        self._check(self._lib.rt_gpu_render_tile(self._h, C.byref(params)))
+    def render_tile(self, params, camera=None):
+        """Enqueues one render task (rt_gpu_render_tile); with an rt_camera (look_at, camera) its camera rays are that
+        camera's (rt_gpu_render_view)."""
+        if camera is None:
+            self._check(self._lib.rt_gpu_render_tile(self._h, C.byref(params)))
+        else:
+            if not isinstance(camera, rt_camera):
+                raise TypeError(f"camera must be an rt_camera (look_at, camera), not {type(camera).__name__}")
+            self._check(self._lib.rt_gpu_render_view(self._h, C.byref(params), C.byref(camera)))
 
     def synchronize(self):
         self._check(self._lib.rt_gpu_synchronize(self._h))

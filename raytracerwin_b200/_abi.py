@@ -108,6 +108,10 @@ class rt_mesh_replace(C.Structure):
                 ("texcoord_idx", C.c_void_p), ("texture", C.c_void_p)]
 
 
+class rt_camera(C.Structure):
+    _fields_ = [("eye", f3), ("right", f3), ("up", f3), ("back", f3), ("dir_z", C.c_float), ("ray_distance", C.c_float)]
+
+
 STRUCT_SIZES = {"rt_shape": 80, "rt_material": 28, "rt_bvh_node": 32, "rt_tri": 64, "rt_shade": 64,
                 "rt_light": 28, "rt_render_params": 56, "rt_counters": 72}
 
@@ -129,6 +133,7 @@ GPU_PROTOTYPES = {
     "rt_gpu_upload_scene": (I, [VP, C.POINTER(rt_scene_desc)]),
     "rt_gpu_reset_accum": (I, [VP, I32, I32]),
     "rt_gpu_render_tile": (I, [VP, C.POINTER(rt_render_params)]),
+    "rt_gpu_render_view": (I, [VP, C.POINTER(rt_render_params), C.POINTER(rt_camera)]),
     "rt_gpu_readback": (I, [VP, I, VP, C.c_size_t]),
     "rt_gpu_synchronize": (I, [VP]),
     "rt_gpu_last_render_ms": (I, [VP, PF]),

@@ -847,9 +847,10 @@ __device__ __forceinline__ void camera_base(int width, int height, int x, int y,
     dy = -(float)(y - height / 2) / (float)(height * 2);
 }
 
-__device__ __forceinline__ Ray camera_ray_from_base(const DevScene& sc, int width, float dx, float dy, int sub, Rng& rng)
+// the sub-sample's offset and its two Random() draws (none for sub < 0)
+__device__ __forceinline__ void camera_jitter(int width, int sub, Rng& rng, float& ox, float& oy)
 {
-    float ox = 0.0f, oy = 0.0f;
+    ox = 0.0f; oy = 0.0f;
     if (sub >= 0)
     {
         const float inv_pixel_radius = 1.0f / (float)(width * 4);
@@ -859,9 +860,34 @@ __device__ __forceinline__ Ray camera_ray_from_base(const DevScene& sc, int widt
         ox += (rng_random(rng) - 0.5f) * offset_radius;
         oy += (rng_random(rng) - 0.5f) * offset_radius;
     }
+}
+
+__device__ __forceinline__ Ray camera_ray_from_base(const DevScene& sc, int width, float dx, float dy, int sub, Rng& rng)
+{
+    float ox, oy;
+    camera_jitter(width, sub, rng, ox, oy);
     Ray r;
     r.o = V3(sc.eye[0], sc.eye[1], sc.eye[2]);
     r.d = normalized3(V3(dx + ox, dy + oy, sc.dir_z));
+    r.dist = sc.ray_distance;
+    return r;
+}
+
+// rt_gpu_render_view's turned camera (rt_camera's basis; its eye, dir_z and distance travel in the DevScene)
+struct ViewBasis { float right[3], up[3], back[3]; };
+
+// camera_ray_from_base with v = (dx + ox, dy + oy, dir_z) taken into the world by the basis before it is normalized:
+// w[c] = (v.x*right[c] + v.y*up[c]) + v.z*back[c], one rounding per operation (-fmad=false), in that order
+__device__ __forceinline__ Ray camera_ray_view(const DevScene& sc, const ViewBasis& b, int width, float dx, float dy, int sub, Rng& rng)
+{
+    float ox, oy;
+    camera_jitter(width, sub, rng, ox, oy);
+    const float3 v = V3(dx + ox, dy + oy, sc.dir_z);
+    float w[3];
+    for (int c = 0; c < 3; c++) w[c] = (v.x * b.right[c] + v.y * b.up[c]) + v.z * b.back[c];
+    Ray r;
+    r.o = V3(sc.eye[0], sc.eye[1], sc.eye[2]);
+    r.d = normalized3(V3(w[0], w[1], w[2]));
     r.dist = sc.ray_distance;
     return r;
 }

@@ -491,9 +491,23 @@ static int upload(rt_gpu_ctx* ctx, const T* src, size_t count, T** out)
     return RT_OK;
 }
 
+// view: the basis of a turned camera (rt_gpu_render_view), nullptr for the reference's generator
 template <bool CULL>
-static cudaError_t launch_generate(int mode, unsigned grid, cudaStream_t st, const DevScene& sc, const RenderArgs& a, const WaveArgs& w)
+static cudaError_t launch_generate(int mode, unsigned grid, cudaStream_t st, const DevScene& sc, const RenderArgs& a, const WaveArgs& w,
+                                   const ViewBasis* view)
 {
+    if (view)
+    {
+        switch (mode)
+        {
+        case RT_MODE_PATH: rt_generate_view_kernel<CULL, RT_MODE_PATH><<<grid, 256, 0, st>>>(sc, a, w, *view); break;
+        case RT_MODE_PREVIEW: rt_generate_view_kernel<CULL, RT_MODE_PREVIEW><<<grid, 256, 0, st>>>(sc, a, w, *view); break;
+        case RT_MODE_WHITTED: rt_generate_view_kernel<CULL, RT_MODE_WHITTED><<<grid, 256, 0, st>>>(sc, a, w, *view); break;
+        case RT_MODE_PRIMARY: rt_generate_view_kernel<CULL, RT_MODE_PRIMARY><<<grid, 256, 0, st>>>(sc, a, w, *view); break;
+        default: return cudaErrorInvalidValue;
+        }
+        return cudaGetLastError();
+    }
     switch (mode)
     {
     case RT_MODE_PATH: rt_generate_kernel<CULL, RT_MODE_PATH><<<grid, 256, 0, st>>>(sc, a, w); break;
@@ -1347,12 +1361,33 @@ int rt_gpu_reset_accum(rt_gpu_ctx* ctx, int32_t width, int32_t height)
     });
 }
 
-int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
+// rt_camera's checks: every field finite and a basis of nonzero determinant (in double)
+static const char* bad_camera(const rt_camera* c)
+{
+    const float* f[] = { c->eye, c->right, c->up, c->back, &c->dir_z, &c->ray_distance };
+    const int n[] = { 3, 3, 3, 3, 1, 1 };
+    for (int k = 0; k < 6; k++)
+        for (int i = 0; i < n[k]; i++)
+            if (!std::isfinite(f[k][i])) return "camera has a non-finite field";
+    const double a0 = c->right[0], a1 = c->right[1], a2 = c->right[2];
+    const double b0 = c->up[0], b1 = c->up[1], b2 = c->up[2];
+    const double c0 = c->back[0], c1 = c->back[1], c2 = c->back[2];
+    const double det = a0 * (b1 * c2 - b2 * c1) - a1 * (b0 * c2 - b2 * c0) + a2 * (b0 * c1 - b1 * c0);
+    if (det == 0.0) return "camera basis is singular (right, up and back are linearly dependent)";
+    return nullptr;
+}
+
+// rt_gpu_render_tile and rt_gpu_render_view: cam == nullptr renders the uploaded view.  A camera replaces the eye,
+// dir_z and distance of the scene the generate kernel reads; a basis other than the identity selects its view variant.
+static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* cam)
 {
     return rt_guard(ctx, [&]() -> int {
         if (!ctx) return RT_ERR_INVALID;
         if (!p) return fail(ctx, RT_ERR_INVALID, "params is null");
-        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_render_tile before rt_gpu_upload_scene");
+        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, cam ? "rt_gpu_render_view before rt_gpu_upload_scene"
+                                                                   : "rt_gpu_render_tile before rt_gpu_upload_scene");
+        if (cam)
+            if (const char* why = bad_camera(cam)) return fail(ctx, RT_ERR_INVALID, why);
         if (p->width <= 0 || p->height <= 0 || (long long)p->width * p->height > 0x7fffffffLL) return fail(ctx, RT_ERR_INVALID, "bad frame size");
         const int npix = p->width * p->height;
         if (p->start < 0 || p->end >= npix) return fail(ctx, RT_ERR_INVALID, "pixel range outside the frame");
@@ -1522,6 +1557,22 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
             }
         }
         const bool cull = p->traverse == RT_TRAVERSE_CULLED;
+        DevScene gen_scene = ctx->scene;
+        ViewBasis basis;
+        const ViewBasis* view = nullptr;
+        if (cam)
+        {
+            for (int k = 0; k < 3; k++) gen_scene.eye[k] = cam->eye[k];
+            gen_scene.dir_z = cam->dir_z; gen_scene.ray_distance = cam->ray_distance;
+            bool identity = true;
+            for (int k = 0; k < 3; k++)
+            {
+                basis.right[k] = cam->right[k]; basis.up[k] = cam->up[k]; basis.back[k] = cam->back[k];
+                identity = identity && cam->right[k] == (k == 0 ? 1.0f : 0.0f) && cam->up[k] == (k == 1 ? 1.0f : 0.0f) &&
+                           cam->back[k] == (k == 2 ? 1.0f : 0.0f);
+            }
+            if (!identity) view = &basis;
+        }
         // the round whose queue is still in camera order is walked as packets (bounce and shadow rays of later
         // rounds are not coherent enough: measured slower, see DESIGN.md)
         const int packet_rounds = ctx->tune_packet_rounds >= 0 ? ctx->tune_packet_rounds : 1;
@@ -1578,8 +1629,8 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
                     RT_CUDA(mark(RT_KERNEL_OTHER, pp.stream));
                     RT_CUDA(cudaMemsetAsync(pp.round_counters, 0, (6 * RT_MAX_ROUNDS + 1) * sizeof(unsigned), pp.stream));
                     RT_CUDA(mark(RT_KERNEL_GENERATE, pp.stream));
-                    RT_CUDA(cull ? launch_generate<true>(p->mode, small_pass ? sms : gen_grid, pp.stream, ctx->scene, a, w)
-                                 : launch_generate<false>(p->mode, small_pass ? sms : gen_grid, pp.stream, ctx->scene, a, w));
+                    RT_CUDA(cull ? launch_generate<true>(p->mode, small_pass ? sms : gen_grid, pp.stream, gen_scene, a, w, view)
+                                 : launch_generate<false>(p->mode, small_pass ? sms : gen_grid, pp.stream, gen_scene, a, w, view));
                     ctx->launches++;
                     // (tooling: RT_FINISH_ROUND = k > 0 runs rounds >= k in the finishing kernel, -1 every round)
                     const int wave_rounds = ctx->tune_finish_round < 0 ? 0
@@ -1639,6 +1690,16 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
         RT_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
         return RT_OK;
     });
+}
+
+int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
+{
+    return render(ctx, p, nullptr);
+}
+
+int rt_gpu_render_view(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* camera)
+{
+    return render(ctx, p, camera);
 }
 
 // A batch of ray queries runs through the render's wavefront (enqueue_ray_batch): query generate, then one round per

@@ -267,9 +267,9 @@ __device__ __forceinline__ bool shade_query(const DevScene& sc, const RenderArgs
 // then the shape list up to the first mesh whose bounds the ray enters.  A ray that ends there having
 // hit nothing — most of them: they miss every bound and see the sky — is retired on the spot; the
 // rest become paths: pool record + an entry in the round-0 queue, compacted per warp by ballot.
-template <bool CULL, int MODE>
-__global__ void __launch_bounds__(256, RT_GEN_BLOCKS)
-rt_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w)
+// VIEW: the camera rays of rt_gpu_render_view's turned camera (camera_ray_view), everything else unchanged.
+template <bool CULL, int MODE, bool VIEW>
+__device__ __forceinline__ void generate_items(const DevScene& sc, const RenderArgs& a, const WaveArgs& w, const ViewBasis& view)
 {
     Counters cnt = { 0, 0, 0, 0, 0, 0 };
     // One thread per PIXEL of the work list (8x4 block, lane), looping over the chunk's samples: the
@@ -328,7 +328,8 @@ rt_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w)
                 const int sub = a.antialias ? (int)(smp & 3u) : -1;
                 s.rng.key = rt_rng_key_sample(pixel_key, (uint32_t)(a.antialias ? pass * 4 + sub : pass));
                 s.rng.n = 0;
-                const Ray cam = camera_ray_from_base(sc, a.width, base_dx, base_dy, MODE == RT_MODE_PRIMARY ? -1 : sub, s.rng);
+                const Ray cam = VIEW ? camera_ray_view(sc, view, a.width, base_dx, base_dy, MODE == RT_MODE_PRIMARY ? -1 : sub, s.rng)
+                                     : camera_ray_from_base(sc, a.width, base_dx, base_dy, MODE == RT_MODE_PRIMARY ? -1 : sub, s.rng);
                 cnt.camera_rays++;
                 s.depth_left = a.max_bounce; s.sp = 0; s.pass_mask = 0; s.light = 0; s.seg_dist = cam.dist;
                 s.w_pos = s.w_nrm = s.w_surface = s.w_sum = V3(0, 0, 0);
@@ -434,6 +435,20 @@ rt_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w)
         }
     }
     flush_counters(cnt, a.counters, a.exact);
+}
+
+template <bool CULL, int MODE>
+__global__ void __launch_bounds__(256, RT_GEN_BLOCKS)
+rt_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w)
+{
+    generate_items<CULL, MODE, false>(sc, a, w, ViewBasis());
+}
+
+template <bool CULL, int MODE>
+__global__ void __launch_bounds__(256, RT_GEN_BLOCKS)
+rt_generate_view_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, const ViewBasis view)
+{
+    generate_items<CULL, MODE, true>(sc, a, w, view);
 }
 
 // ---- kernel Q: generate for a batch of ray queries (rt_gpu_query_rays) ---------------------------------------------
