@@ -76,7 +76,10 @@ typedef struct rt_shape {
     float radius;           /* sphere / capsule Radius */
 } rt_shape;
 
-/* One node of a material tree (Blend/Combine reference children by index). */
+/* One node of a material graph (Blend/Combine reference children by index; nodes may be shared).  rt_gpu_upload_scene
+ * refuses (RT_ERR_INVALID) a graph with a cycle and one in which some path from ANY node down to a leaf passes more
+ * than 8 Combine nodes (the device's frame stack of Combines; Blend nodes do not count), whether or not a shape uses
+ * that node, since rt_gpu_update_shapes may point a shape at it later. */
 typedef struct rt_material {
     int32_t type;           /* RT_MAT_* */
     int32_t child_a;        /* Blend: BlendMaterialA, Combine: MaterialA; else -1 */

@@ -968,11 +968,48 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
                     return fail(ctx, RT_ERR_INVALID, "material child index out of range");
             if (m.type == RT_MAT_DIFFUSE || m.type == RT_MAT_CHECKER) needs_table = true;
         }
+        // material_eval walks a graph with no visit bound and holds RT_MAX_MATERIAL_DEPTH Combine frames, so from every
+        // node (rt_gpu_update_shapes may point a shape at any of them) each path down to a leaf must be finite and pass at
+        // most that many Combines.  Depth-first with an explicit stack (it holds exactly the current path) and each
+        // node's depth computed once: O(materials) however deep a caller's graph is.
+        {
+            const int n = s->num_materials;
+            std::vector<int8_t> state((size_t)n, 0);     // 0 unseen, 1 on the current path, 2 done
+            std::vector<int32_t> combines((size_t)n, 0);  // most Combine nodes on a path from the node down to a leaf
+            std::vector<int32_t> path;
+            for (int root = 0; root < n; root++)
+            {
+                if (state[root]) continue;
+                state[root] = 1; path.push_back(root);
+                while (!path.empty())
+                {
+                    const int i = path.back();
+                    const rt_material& m = s->materials[i];
+                    if (m.type == RT_MAT_BLEND || m.type == RT_MAT_COMBINE)
+                    {
+                        int next = -1;
+                        for (int c : { m.child_a, m.child_b })
+                        {
+                            if (state[c] == 1)
+                                return fail(ctx, RT_ERR_INVALID, "material graph has a cycle through node " + std::to_string(c));
+                            if (state[c] == 0) { next = c; break; }
+                        }
+                        if (next >= 0) { state[next] = 1; path.push_back(next); continue; }
+                        combines[i] = std::max(combines[m.child_a], combines[m.child_b]) + (m.type == RT_MAT_COMBINE);
+                        if (combines[i] > RT_MAX_MATERIAL_DEPTH)
+                            return fail(ctx, RT_ERR_INVALID, "material node " + std::to_string(i) + " nests Combine nodes "
+                                        + std::to_string(combines[i]) + " deep (at most "
+                                        + std::to_string(RT_MAX_MATERIAL_DEPTH) + ")");
+                    }
+                    state[i] = 2; path.pop_back();
+                }
+            }
+        }
         for (int i = 0; i < s->num_shapes; i++)
         {
             const rt_shape& sh = s->shapes[i];
             if (sh.type < RT_SHAPE_SPHERE || sh.type > RT_SHAPE_TRIANGLE) return fail(ctx, RT_ERR_INVALID, "unknown shape type");
-            if (sh.material >= s->num_materials) return fail(ctx, RT_ERR_INVALID, "shape material index out of range");
+            if (sh.material < -1 || sh.material >= s->num_materials) return fail(ctx, RT_ERR_INVALID, "shape material index out of range");
             if (sh.type == RT_SHAPE_MESH && (sh.mesh < 0 || sh.mesh >= s->num_meshes)) return fail(ctx, RT_ERR_INVALID, "shape mesh index out of range");
         }
         // a tree the upload accepts may still leave nodes out of the root's range, give an inner node an empty right
