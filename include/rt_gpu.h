@@ -23,6 +23,8 @@
  *   rt_gpu_refit_mesh    new points under a mesh's published tree (boxes recomputed, topology kept), with no host wait
  *   rt_gpu_replace_mesh  a new mesh of any triangle count, with texture coordinates and texture slots, from device memory
  *                        (levels of detail, procedural and streamed geometry) without a new upload
+ *   rt_gpu_update_materials  material nodes edited in place or appended, rt_gpu_update_lights a new light list and
+ *   rt_gpu_update_texture    a rectangle of texels from device memory: the scene's appearance without a new upload
  *
  * Plain C: POD structs, pointers and sizes only.  No C++/STL/torch types cross the boundary.
  * Every entry returns 0 on success or a negative rt_status; rt_gpu_last_error() gives text.
@@ -414,6 +416,43 @@ int rt_gpu_replace_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_replace* r
  * bounds are those of the mesh's current geometry).  Ordering as rt_gpu_update_mesh.  The records travel as kernel
  * parameters, so the call returns at once: it never waits on the host for frames in flight. */
 int rt_gpu_update_shapes(rt_gpu_ctx* ctx, const rt_shape* shapes, int32_t first, int32_t count, void* stream);
+
+/* Appearance updates: material nodes, lights and texels, for material editors, light placement, video or painted
+ * textures and bakes that write back into a texture.  Ordering as rt_gpu_update_shapes: calls made before see the old
+ * appearance, calls made after the new one, on any frame slot and stream, with no host synchronisation; the call
+ * returns at once (no host wait, no blocking allocation).  Every error is found on the host: RT_ERR_INVALID with nothing
+ * enqueued and the scene exactly as it was, RT_ERR_NO_SCENE before an upload.  After any sequence of them every later
+ * call returns what a fresh rt_gpu_upload_scene of the edited description returns.
+ *
+ * rt_gpu_update_materials copies `count` caller records (host memory, consumed before return) over material nodes
+ * [first, first + count).  first <= the current node count; a range past its end APPENDS nodes (the count only grows).
+ * The graph as it will be afterwards must pass the upload's checks (type, children in range, no cycle, at most 8 Combine
+ * nodes on any path from any node), so an update that closes a cycle through nodes it does not touch is refused.  A
+ * Diffuse or Checker node on a scene without unit vectors makes later RT_MODE_PATH calls refuse, as after such an
+ * upload; the update itself succeeds.  rt_gpu_update_shapes takes material indices below the new count. */
+int rt_gpu_update_materials(rt_gpu_ctx* ctx, const rt_material* materials, int32_t first, int32_t count, void* stream);
+
+/* Replaces the whole light list with `count` >= 0 caller records (host memory, consumed before return); the count may
+ * differ from the uploaded one.  Later RT_MODE_WHITTED calls size their rounds (1 + lights) by the new count. */
+int rt_gpu_update_lights(rt_gpu_ctx* ctx, const rt_light* lights, int32_t count, void* stream);
+
+/* A rectangle of texels of one uploaded texture slot, from device memory.  Texel (x + i, y + j) of the slot becomes
+ * rgba[j][i], or {lut[r], lut[g], lut[b], channels == 4 ? lut[256 + a] : 1.0f} of the 8-bit texel (what the upload
+ * expands; rt_host_texel_lut gives the loader's table).  Slot sizes and atlas places do not change. */
+typedef struct rt_texture_update {
+    int32_t x, y, width, height;  /* rectangle of the slot's texels to overwrite, inside its uploaded size */
+    const float* rgba;            /* DEVICE, `height` rows of width x {r,g,b,a} linear floats, `pitch` bytes apart; or NULL */
+    size_t pitch;                 /* >= width * 16 */
+    const uint8_t* texels8;       /* DEVICE, height x width x channels bytes, tightly packed; or NULL (exactly one of the two) */
+    int32_t channels;             /* 3 or 4 with texels8 */
+    const float* lut;             /* DEVICE, 512 floats with texels8: rt_texture's table */
+} rt_texture_update;
+
+/* Texture `slot` of mesh `mesh`.  width or height 0 is a no-op after the checks.  RT_ERR_INVALID for an unknown mesh or
+ * slot, a slot that had no pixels at upload, a rectangle outside the slot, both or neither of rgba / texels8, channels
+ * other than 3 or 4 with texels8, a pitch below width * 16 or not a multiple of 4, rgba or lut not 4-byte aligned, and a
+ * source or lut that is not device memory of the context's GPU. */
+int rt_gpu_update_texture(rt_gpu_ctx* ctx, int32_t mesh, int32_t slot, const rt_texture_update* t, void* stream);
 
 /* Synchronises the stream, then copies `what` into caller memory (size-checked). */
 int rt_gpu_readback(rt_gpu_ctx* ctx, int what, void* dst, size_t bytes);

@@ -32,6 +32,15 @@ int rt_gpu_debug_long(rt_gpu_ctx* ctx, uint32_t* lcounts, int32_t max_rounds);
 int rt_gpu_debug_read_mesh(rt_gpu_ctx* ctx, int32_t mesh, rt_bvh_node* nodes, rt_tri* tris, rt_shade* shade, float* bounds6,
                            float* cull_scale);
 
+/* The material and light records the kernels read now (after every update enqueued so far): the first min(count, cap)
+ * of each (either array may be NULL), and counts2 = {material count, light count}. */
+int rt_gpu_debug_read_appearance(rt_gpu_ctx* ctx, rt_material* materials, int32_t mat_cap, rt_light* lights, int32_t light_cap,
+                                 int32_t* counts2);
+
+/* The texels of texture `slot` of mesh `mesh` as the atlas holds them now: height x width x {r,g,b,a} floats (the slot's
+ * uploaded size). */
+int rt_gpu_debug_read_texture(rt_gpu_ctx* ctx, int32_t mesh, int32_t slot, float* rgba);
+
 #ifdef __cplusplus
 }
 #endif

@@ -79,6 +79,9 @@ int rt_host_mesh_texture_info(rt_host_scene* s, int shape, int slot, int32_t wh[
 int rt_host_mesh_texture_pixels(rt_host_scene* s, int shape, int slot, float* out);
 
 /* Stand-alone helpers */
+/* The 512-entry table of rt_texture.lut that the PNG loader builds (lut[c] = powf(c / 255, 2.2f) by this host's powf,
+ * lut[256 + c] = c / 255): 8-bit texels fed through it to rt_gpu_update_texture equal the loader's texels bit for bit. */
+int rt_host_texel_lut(float* out512);
 int rt_host_decode_png(const char* path, int32_t wh[2], int32_t* channels, uint8_t** out_pixels);
 void rt_host_free(void* p);
 int rt_host_write_png_argb(const char* path, const uint32_t* argb, int32_t width, int32_t height);

@@ -14,7 +14,7 @@ import numpy as np
 
 from . import _abi
 from ._abi import (rt_render_params, rt_counters, rt_scene_desc, rt_ray_query, rt_radiance_query, rt_mesh_update,  # noqa: F401
-                   rt_mesh_replace, rt_camera,
+                   rt_mesh_replace, rt_camera, rt_texture_update, rt_material, rt_light,
                    RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY, RT_QUERY_NEAREST, RT_QUERY_ANY,
                    RT_TRAVERSE_EXACT, RT_TRAVERSE_CULLED,
                    RT_READ_ACCUM_RGBN_F32, RT_READ_DISPLAY_ARGB8, RT_READ_PRIMARY_IDS_I32X2,
@@ -190,6 +190,15 @@ class Scene:
         return nodes.view(node_dt), tris.view(tri_dt), shade.view(shade_dt)
 
 
+def texel_lut():
+    """The PNG loader's 512-entry texel table (rt_texture.lut) as float32 (512,): [c] = powf(c / 255, 2.2f) for r, g, b,
+    [256 + c] = c / 255 for alpha.  8-bit texels fed through it to GpuContext.update_texture match the loader's."""
+    out = np.zeros(512, np.float32)
+    if load_library().rt_host_texel_lut(out.ctypes.data_as(_abi.PF)) != 0:
+        raise RtError(load_library().rt_host_last_error().decode())
+    return out
+
+
 def use_device_bvh_builder(ctx):
     """Meshes loaded from now on get their tree built on `ctx`'s GPU (None: back to the host builder)."""
     load_library().rt_host_use_device_bvh_builder(ctx.handle if ctx is not None else None)
@@ -279,6 +288,9 @@ class GpuContext:
                                                      for i in range(d.num_meshes)}
         self._shape_mesh = {} if d is None else {i: int(d.shapes[i].mesh) for i in range(d.num_shapes)
                                                   if d.shapes[i].type == _abi.RT_SHAPE_MESH}
+        self._texture_sizes = {} if d is None else {
+            (i, k): (int(t.height), int(t.width)) for i in range(d.num_meshes) for k in range(d.meshes[i].num_textures)
+            for t in (d.meshes[i].textures[k],) if bool(t.rgba) or bool(t.texels8)}
 
     def reset_accum(self, width, height):
         self._check(self._lib.rt_gpu_reset_accum(self._h, width, height))
@@ -539,6 +551,91 @@ class GpuContext:
             if count else None
         self._check(self._lib.rt_gpu_update_shapes(self._h, recs, first, count,
                                                    self._torch_stream(torch.device("cuda", self.device))))
+
+    def update_materials(self, materials, first=0, count=None):
+        """Material nodes edited or appended (rt_gpu_update_materials).  `materials`: a host Scene, whose flattened records
+        [first, first + count) are copied over nodes [first, first + count) (count: to the end of its records), or a
+        sequence of rt_material written to nodes [first, first + count) (count: its length).  A range past the current
+        node count appends nodes.  Enqueued on torch.cuda.current_stream; returns at once."""
+        import torch
+        if isinstance(materials, Scene):
+            desc = materials.desc.contents
+            count = desc.num_materials - first if count is None else count
+            if first < 0 or count < 0 or first + count > desc.num_materials:
+                raise ValueError(f"materials [{first}, {first + count}) outside the scene's {desc.num_materials}")
+            recs = C.cast(C.addressof(desc.materials.contents) + first * C.sizeof(rt_material), C.POINTER(rt_material)) \
+                if count else None
+        else:
+            seq = list(materials)
+            count = len(seq) if count is None else count
+            if count < 0 or count > len(seq):
+                raise ValueError(f"count {count} outside the {len(seq)} records given")
+            if not all(isinstance(m, rt_material) for m in seq):
+                raise TypeError("materials must be a Scene or a sequence of rt_material")
+            recs = (rt_material * max(count, 1))(*seq[:count])
+        self._check(self._lib.rt_gpu_update_materials(self._h, recs, first, count,
+                                                      self._torch_stream(torch.device("cuda", self.device))))
+
+    def update_lights(self, lights):
+        """A new light list (rt_gpu_update_lights): a host Scene's lights, or (kind, pos_or_dir, color) tuples as
+        Scene.set_lights takes them.  Enqueued on torch.cuda.current_stream; returns at once."""
+        import torch
+        if isinstance(lights, Scene):
+            desc = lights.desc.contents
+            n, recs = desc.num_lights, desc.lights if desc.num_lights else None
+        else:
+            seq = [rt_light(int(kind), _f3(v), _f3(color)) for kind, v, color in lights]
+            n, recs = len(seq), (rt_light * max(len(seq), 1))(*seq)
+        self._check(self._lib.rt_gpu_update_lights(self._h, recs, n, self._torch_stream(torch.device("cuda", self.device))))
+
+    def update_texture(self, mesh, slot, texels, x=0, y=0, lut=None):
+        """Overwrites the rectangle at (x, y) of texture `slot` of mesh `mesh` (rt_gpu_update_texture).  `texels`: a
+        contiguous torch tensor on cuda:<self.device>, float32 (h, w, 4) linear {r, g, b, a}, or uint8 (h, w, 3 | 4) codes
+        turned into texels through `lut` (float32 (512,) on the same device; default texel_lut(), the PNG loader's table).
+        Enqueued on torch.cuda.current_stream; returns at once.  An empty tensor is a no-op."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        if not isinstance(texels, torch.Tensor) or texels.dim() != 3:
+            raise ValueError("texels must be a torch tensor of shape (h, w, 4) float32 or (h, w, 3 | 4) uint8")
+        h, w, c = texels.shape
+        u = rt_texture_update(int(x), int(y), w, h)
+        if texels.dtype == torch.float32:
+            self._device_tensor("texels", texels, torch.float32, (h, w, 4))
+            u.rgba, u.pitch = texels.data_ptr(), w * 16
+        elif texels.dtype == torch.uint8:
+            if c not in (3, 4):
+                raise ValueError(f"uint8 texels must have 3 or 4 channels, not {c}")
+            self._device_tensor("texels", texels, torch.uint8, (h, w, c))
+            if lut is None:
+                if getattr(self, "_lut", None) is None:
+                    self._lut = torch.from_numpy(texel_lut()).to(dev)
+                lut = self._lut
+            self._device_tensor("lut", lut, torch.float32, (512,))
+            u.texels8, u.channels, u.lut = texels.data_ptr(), c, lut.data_ptr()
+        else:
+            raise ValueError(f"texels must be float32 or uint8, not {texels.dtype}")
+        if texels.numel() == 0:
+            return                     # an empty rectangle is a no-op (and an empty tensor has no address to pass)
+        self._check(self._lib.rt_gpu_update_texture(self._h, mesh, slot, C.byref(u), self._torch_stream(dev)))
+
+    def read_appearance(self):
+        """The material and light records the device holds now (rt_gpu_debug_read_appearance; synchronises): ctypes
+        arrays (rt_material * M, rt_light * L)."""
+        counts = (C.c_int32 * 2)()
+        self._check(self._lib.rt_gpu_debug_read_appearance(self._h, None, 0, None, 0, counts))
+        mats, lights = (rt_material * counts[0])(), (rt_light * counts[1])()
+        self._check(self._lib.rt_gpu_debug_read_appearance(self._h, mats, counts[0], lights, counts[1], counts))
+        return mats, lights
+
+    def read_texture(self, mesh, slot):
+        """The texels of texture `slot` of mesh `mesh` as the device holds them now (rt_gpu_debug_read_texture;
+        synchronises): float32 (h, w, 4)."""
+        size = getattr(self, "_texture_sizes", {}).get((mesh, slot))
+        if size is None:
+            raise ValueError(f"texture slot {slot} of mesh {mesh} has no pixels in the uploaded scene")
+        out = np.zeros(size + (4,), np.float32)
+        self._check(self._lib.rt_gpu_debug_read_texture(self._h, mesh, slot, out.ctypes.data))
+        return out
 
     def read_mesh(self, mesh):
         """The device arrays of uploaded mesh `mesh` as they are now (rt_gpu_debug_read_mesh; synchronises): nodes,

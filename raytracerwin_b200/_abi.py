@@ -108,6 +108,12 @@ class rt_mesh_replace(C.Structure):
                 ("texcoord_idx", C.c_void_p), ("texture", C.c_void_p)]
 
 
+class rt_texture_update(C.Structure):
+    _fields_ = [("x", C.c_int32), ("y", C.c_int32), ("width", C.c_int32), ("height", C.c_int32),
+                ("rgba", C.c_void_p), ("pitch", C.c_size_t), ("texels8", C.c_void_p), ("channels", C.c_int32),
+                ("lut", C.c_void_p)]
+
+
 class rt_camera(C.Structure):
     _fields_ = [("eye", f3), ("right", f3), ("up", f3), ("back", f3), ("dir_z", C.c_float), ("ray_distance", C.c_float)]
 
@@ -170,6 +176,9 @@ GPU_PROTOTYPES = {
     "rt_gpu_refit_mesh": (I, [VP, I32, C.POINTER(rt_mesh_update), VP, VP]),
     "rt_gpu_replace_mesh": (I, [VP, I32, C.POINTER(rt_mesh_replace), VP]),
     "rt_gpu_update_shapes": (I, [VP, C.POINTER(rt_shape), I32, I32, VP]),
+    "rt_gpu_update_materials": (I, [VP, C.POINTER(rt_material), I32, I32, VP]),
+    "rt_gpu_update_lights": (I, [VP, C.POINTER(rt_light), I32, VP]),
+    "rt_gpu_update_texture": (I, [VP, I32, I32, C.POINTER(rt_texture_update), VP]),
     "rt_gpu_trace_rays": (I, [VP, PF, I32, I32, PI32, PI32, PF]),
     "rt_gpu_kat": (I, [VP, I32, VP, VP, I32, I32, VP, VP]),
     "rt_gpu_kat_texture": (I, [VP, I32, VP, I32, VP]),
@@ -202,7 +211,8 @@ HOST_PROTOTYPES = {
     "rt_host_mesh_dump": (I, [VP, I, VP, VP, VP, VP, VP, VP, VP]),
     "rt_host_mesh_texture_info": (I, [VP, I, I, C.c_int32 * 2]),
     "rt_host_mesh_texture_pixels": (I, [VP, I, I, VP]),
-    "rt_host_decode_png": (I, [C.c_char_p, C.c_int32 * 2, C.POINTER(C.c_int32), C.POINTER(C.POINTER(C.c_uint8))]),
+    "rt_host_texel_lut": (I, [PF]),
+    "rt_host_decode_png":(I, [C.c_char_p, C.c_int32 * 2, C.POINTER(C.c_int32), C.POINTER(C.POINTER(C.c_uint8))]),
     "rt_host_free": (None, [VP]),
     "rt_host_write_png_argb": (I, [C.c_char_p, VP, I32, I32]),
     "rt_host_program_run": (I, [VP, I, I32, I32, I32, I32, U32, C.c_char_p, C.POINTER(C.c_double), C.POINTER(C.c_uint64)]),
@@ -211,6 +221,8 @@ HOST_PROTOTYPES = {
 # include/rt_gpu_debug.h (tooling; bound by load_library as well)
 DEBUG_PROTOTYPES = {
     "rt_gpu_debug_read_mesh": (I, [VP, I32, VP, VP, VP, VP, PF]),
+    "rt_gpu_debug_read_appearance": (I, [VP, C.POINTER(rt_material), I32, C.POINTER(rt_light), I32, PI32]),
+    "rt_gpu_debug_read_texture": (I, [VP, I32, I32, VP]),
 }
 
 LIB_NAME = "librt_b200.so"

@@ -226,6 +226,13 @@ int rt_host_mesh_texture_pixels(rt_host_scene* s, int shape, int slot, float* ou
     });
 }
 
+int rt_host_texel_lut(float* out512)
+{
+    if (!out512) { g_error = "rt_host_texel_lut: out512 is null"; return RT_ERR_INVALID; }
+    RTexture::MakeLut(out512);
+    return RT_OK;
+}
+
 int rt_host_decode_png(const char* path, int32_t wh[2], int32_t* channels, uint8_t** out_pixels)
 {
     return guard([&]() -> int {

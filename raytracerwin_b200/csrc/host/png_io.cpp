@@ -119,18 +119,23 @@ std::unique_ptr<RTexture> RTexture::LoadTexturePNG(const std::string& Filename)
         printf("%s\n", err.c_str());
         return nullptr;
     }
-    // Linearise once per 8-bit code instead of once per texel: powf((float)c / 255, 2.2f) only
-    // ever sees 256 inputs, so a table gives the same bits as Texture.cpp:128-131 / ColorBuffer.h:70-78.
     std::unique_ptr<RTexture> t(new RTexture());
-    for (int i = 0; i < 256; i++)
-    {
-        float c = (float)i / 255;
-        t->Lut[i] = powf(c, 2.2f);
-        t->Lut[256 + i] = c;
-    }
+    MakeLut(t->Lut);
     t->Width = w; t->Height = h; t->Channels = ch;
     t->Pixels8 = std::move(px);
     return t;
+}
+
+// Linearise once per 8-bit code instead of once per texel: powf((float)c / 255, 2.2f) only
+// ever sees 256 inputs, so a table gives the same bits as Texture.cpp:128-131 / ColorBuffer.h:70-78.
+void RTexture::MakeLut(float* Out512)
+{
+    for (int i = 0; i < 256; i++)
+    {
+        float c = (float)i / 255;
+        Out512[i] = powf(c, 2.2f);
+        Out512[256 + i] = c;
+    }
 }
 
 void RTexture::ExpandTo(float* OutRGBA) const

@@ -176,6 +176,7 @@ struct RTexture
     float Lut[512];                // [c] = powf(c / 255, 2.2f), [256 + c] = c / 255
     void ExpandTo(float* OutRGBA) const;     // 4 * Width * Height floats
     static std::unique_ptr<RTexture> LoadTexturePNG(const std::string& Filename);
+    static void MakeLut(float* Out512);      // the table above (rt_host_texel_lut hands it to callers)
 };
 
 // Pre-order flattened BVH of one mesh + device-ready triangle/shading records.

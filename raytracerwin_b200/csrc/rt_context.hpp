@@ -126,6 +126,15 @@ struct rt_gpu_ctx
     // update on: an update builds into the spare set and publishes it; the published set becomes the spare.
     std::vector<rt_shape> host_shapes;          // the records as uploaded (materials follow rt_gpu_update_shapes)
     int host_num_materials = 0;
+    // ---- appearance updates (rt_gpu_update_materials / rt_gpu_update_lights / rt_gpu_update_texture) ----
+    std::vector<rt_material> host_materials;    // the graph the device holds (the checks of an update run on its edit)
+    // Room of ctx->scene.materials / .lights in records.  `pooled`: from cudaMallocAsync by an update, released with
+    // cudaFreeAsync when a larger array replaces it; the uploaded arrays (cudaMalloc) stay until the next upload or destroy.
+    int material_cap = 0, light_cap = 0;
+    bool materials_pooled = false, lights_pooled = false;
+    std::vector<std::vector<DevTexture>> mesh_textures;   // per mesh, per slot: the atlas rectangle (0 x 0: no pixels)
+    cudaArray_t atlas_array = nullptr;          // in `arrays`
+    cudaSurfaceObject_t atlas_surface = 0;      // writes into the atlas (8-bit expansion); destroyed with the scene
     // One set of a mesh's arrays: room for `cap` triangles (2 * cap - 1 nodes).  `pooled`: from cudaMallocAsync by an
     // update, released with cudaFreeAsync when a larger set replaces it; the uploaded set (cudaMalloc) stays in
     // scene_allocs until the next upload or destroy.

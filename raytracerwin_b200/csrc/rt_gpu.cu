@@ -293,6 +293,16 @@ __global__ void rt_update_shapes_kernel(rt_shape* shapes, ShapeBatch src, int co
     else shapes[k] = src.rec[k];
 }
 
+// rt_gpu_update_materials / rt_gpu_update_lights: caller records travel the same way (28 B each)
+#define RT_RECORDS_PER_LAUNCH 128                     // 128 x 28 B: within the classic 4 KB parameter space
+template <typename T> struct RecordBatch { T rec[RT_RECORDS_PER_LAUNCH]; };
+template <typename T>
+__global__ void rt_update_records_kernel(T* dst, RecordBatch<T> src, int count)
+{
+    const int k = threadIdx.x;
+    if (k < count) dst[k] = src.rec[k];
+}
+
 // ---- mesh refits (rt_gpu_refit_mesh) ----
 // No host read sees the check's flag, so every later kernel runs on clamped copies of BOTH index arrays (bad ones
 // replaced by 0): nothing reads outside `points` or `normals`; with the flag set the result is thrown away below.
@@ -428,6 +438,8 @@ __global__ void rt_refit_finish_kernel(const int* __restrict__ flag, int* status
 
 static void free_scene(rt_gpu_ctx* ctx)
 {
+    if (ctx->atlas_surface) cudaDestroySurfaceObject(ctx->atlas_surface);
+    ctx->atlas_surface = 0; ctx->atlas_array = nullptr;
     for (cudaTextureObject_t t : ctx->texobjs) cudaDestroyTextureObject(t);
     for (cudaArray_t a : ctx->arrays) cudaFreeArray(a);
     for (void* p : ctx->scene_allocs) cudaFree(p);
@@ -838,6 +850,58 @@ static int enqueue_ray_batch(rt_gpu_ctx* ctx, RenderArgs& a, size_t n, size_t pi
     return RT_OK;
 }
 
+// The material checks of rt_gpu_upload_scene and rt_gpu_update_materials over the n nodes of a graph (for an update: the
+// graph as it will be afterwards); failures carry `prefix` before the upload's messages.  *needs_table: some node is
+// Diffuse or Checker (RandomHemisphereDirection reads the unit-vector table).
+static int check_materials(rt_gpu_ctx* ctx, const rt_material* mats, int n, const std::string& prefix, bool* needs_table)
+{
+    *needs_table = false;
+    for (int i = 0; i < n; i++)
+    {
+        const rt_material& m = mats[i];
+        if (m.type < RT_MAT_DIFFUSE || m.type > RT_MAT_NULL) return fail(ctx, RT_ERR_INVALID, prefix + "unknown material type");
+        if (m.type == RT_MAT_BLEND || m.type == RT_MAT_COMBINE)
+            if (m.child_a < 0 || m.child_a >= n || m.child_b < 0 || m.child_b >= n)
+                return fail(ctx, RT_ERR_INVALID, prefix + "material child index out of range");
+        if (m.type == RT_MAT_DIFFUSE || m.type == RT_MAT_CHECKER) *needs_table = true;
+    }
+    // material_eval walks a graph with no visit bound and holds RT_MAX_MATERIAL_DEPTH Combine frames, so from every
+    // node (rt_gpu_update_shapes may point a shape at any of them) each path down to a leaf must be finite and pass at
+    // most that many Combines.  Depth-first with an explicit stack (it holds exactly the current path) and each
+    // node's depth computed once: O(materials) however deep a caller's graph is.
+    std::vector<int8_t> state((size_t)n, 0);     // 0 unseen, 1 on the current path, 2 done
+    std::vector<int32_t> combines((size_t)n, 0);  // most Combine nodes on a path from the node down to a leaf
+    std::vector<int32_t> path;
+    for (int root = 0; root < n; root++)
+    {
+        if (state[root]) continue;
+        state[root] = 1; path.push_back(root);
+        while (!path.empty())
+        {
+            const int i = path.back();
+            const rt_material& m = mats[i];
+            if (m.type == RT_MAT_BLEND || m.type == RT_MAT_COMBINE)
+            {
+                int next = -1;
+                for (int c : { m.child_a, m.child_b })
+                {
+                    if (state[c] == 1)
+                        return fail(ctx, RT_ERR_INVALID, prefix + "material graph has a cycle through node " + std::to_string(c));
+                    if (state[c] == 0) { next = c; break; }
+                }
+                if (next >= 0) { state[next] = 1; path.push_back(next); continue; }
+                combines[i] = std::max(combines[m.child_a], combines[m.child_b]) + (m.type == RT_MAT_COMBINE);
+                if (combines[i] > RT_MAX_MATERIAL_DEPTH)
+                    return fail(ctx, RT_ERR_INVALID, prefix + "material node " + std::to_string(i) + " nests Combine nodes "
+                                + std::to_string(combines[i]) + " deep (at most "
+                                + std::to_string(RT_MAX_MATERIAL_DEPTH) + ")");
+            }
+            state[i] = 2; path.pop_back();
+        }
+    }
+    return RT_OK;
+}
+
 extern "C" {
 
 int rt_gpu_abi_version(void) { return RT_GPU_ABI_VERSION; }
@@ -959,52 +1023,8 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
             return fail(ctx, RT_ERR_INVALID, "negative count in scene");
         // validate indices before anything is copied
         bool needs_table = false;
-        for (int i = 0; i < s->num_materials; i++)
-        {
-            const rt_material& m = s->materials[i];
-            if (m.type < RT_MAT_DIFFUSE || m.type > RT_MAT_NULL) return fail(ctx, RT_ERR_INVALID, "unknown material type");
-            if (m.type == RT_MAT_BLEND || m.type == RT_MAT_COMBINE)
-                if (m.child_a < 0 || m.child_a >= s->num_materials || m.child_b < 0 || m.child_b >= s->num_materials)
-                    return fail(ctx, RT_ERR_INVALID, "material child index out of range");
-            if (m.type == RT_MAT_DIFFUSE || m.type == RT_MAT_CHECKER) needs_table = true;
-        }
-        // material_eval walks a graph with no visit bound and holds RT_MAX_MATERIAL_DEPTH Combine frames, so from every
-        // node (rt_gpu_update_shapes may point a shape at any of them) each path down to a leaf must be finite and pass at
-        // most that many Combines.  Depth-first with an explicit stack (it holds exactly the current path) and each
-        // node's depth computed once: O(materials) however deep a caller's graph is.
-        {
-            const int n = s->num_materials;
-            std::vector<int8_t> state((size_t)n, 0);     // 0 unseen, 1 on the current path, 2 done
-            std::vector<int32_t> combines((size_t)n, 0);  // most Combine nodes on a path from the node down to a leaf
-            std::vector<int32_t> path;
-            for (int root = 0; root < n; root++)
-            {
-                if (state[root]) continue;
-                state[root] = 1; path.push_back(root);
-                while (!path.empty())
-                {
-                    const int i = path.back();
-                    const rt_material& m = s->materials[i];
-                    if (m.type == RT_MAT_BLEND || m.type == RT_MAT_COMBINE)
-                    {
-                        int next = -1;
-                        for (int c : { m.child_a, m.child_b })
-                        {
-                            if (state[c] == 1)
-                                return fail(ctx, RT_ERR_INVALID, "material graph has a cycle through node " + std::to_string(c));
-                            if (state[c] == 0) { next = c; break; }
-                        }
-                        if (next >= 0) { state[next] = 1; path.push_back(next); continue; }
-                        combines[i] = std::max(combines[m.child_a], combines[m.child_b]) + (m.type == RT_MAT_COMBINE);
-                        if (combines[i] > RT_MAX_MATERIAL_DEPTH)
-                            return fail(ctx, RT_ERR_INVALID, "material node " + std::to_string(i) + " nests Combine nodes "
-                                        + std::to_string(combines[i]) + " deep (at most "
-                                        + std::to_string(RT_MAX_MATERIAL_DEPTH) + ")");
-                    }
-                    state[i] = 2; path.pop_back();
-                }
-            }
-        }
+        int rc = check_materials(ctx, s->materials, s->num_materials, "", &needs_table);
+        if (rc != RT_OK) return rc;
         for (int i = 0; i < s->num_shapes; i++)
         {
             const rt_shape& sh = s->shapes[i];
@@ -1074,11 +1094,10 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
         if (ctx->scene_event_live) RT_CUDA(cudaEventSynchronize(ctx->scene_event));    // an update on a caller's stream
         ctx->scene_event_live = false;
         free_scene(ctx);
-        ctx->host_shapes.clear(); ctx->mesh_state.clear();
+        ctx->host_shapes.clear(); ctx->mesh_state.clear(); ctx->mesh_textures.clear();
 
         DevScene d;
         memset(&d, 0, sizeof d);
-        int rc;
         rt_shape* dshapes; rt_material* dmats; rt_light* dlights;
         if ((rc = upload(ctx, s->shapes, (size_t)s->num_shapes, &dshapes)) != RT_OK) return rc;
         if ((rc = upload(ctx, s->materials, (size_t)s->num_materials, &dmats)) != RT_OK) return rc;
@@ -1091,11 +1110,10 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
         // device copies of 8-bit texels wait here until the expansion kernels have run
         struct TempGuard
         {
-            std::vector<void*> v; cudaSurfaceObject_t* surf;
-            ~TempGuard() { for (void* q : v) cudaFree(q); if (*surf) cudaDestroySurfaceObject(*surf); }
+            std::vector<void*> v;
+            ~TempGuard() { for (void* q : v) cudaFree(q); }
         };
-        cudaSurfaceObject_t atlas_surface = 0;
-        TempGuard temp_guard = { {}, &atlas_surface };
+        TempGuard temp_guard;
         std::vector<void*>& texel_temps = temp_guard.v;
         ctx->texel_upload_bytes = 0;
         struct AtlasRect { int x, y, w, h; };
@@ -1145,6 +1163,9 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
                 RT_CUDA(cudaCreateTextureObject(&obj, &res, &td, nullptr));
                 ctx->texobjs.push_back(obj);
                 d.atlas = obj;
+                // the 8-bit expansion here and in rt_gpu_update_texture writes through it
+                ctx->atlas_array = atlas_array;
+                RT_CUDA(cudaCreateSurfaceObject(&ctx->atlas_surface, &res));
             }
         }
 
@@ -1230,14 +1251,8 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
                     texel_temps.push_back(dlut);
                     RT_CUDA(cudaMemcpyAsync(d8, t.texels8, count * (size_t)t.channels, cudaMemcpyHostToDevice, ctx->stream));
                     RT_CUDA(cudaMemcpyAsync(dlut, t.lut, 512 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-                    if (!atlas_surface)
-                    {
-                        cudaResourceDesc sres; memset(&sres, 0, sizeof sres);
-                        sres.resType = cudaResourceTypeArray; sres.res.array.array = atlas_array;
-                        RT_CUDA(cudaCreateSurfaceObject(&atlas_surface, &sres));
-                    }
                     const dim3 grid((unsigned)((t.width + 31) / 32), (unsigned)((t.height + 7) / 8));
-                    rt_expand_texels_kernel<<<grid, dim3(32, 8), 0, ctx->stream>>>(atlas_surface, d8, dlut, t.width, t.height, t.channels, rc2.x, rc2.y);
+                    rt_expand_texels_kernel<<<grid, dim3(32, 8), 0, ctx->stream>>>(ctx->atlas_surface, d8, dlut, t.width, t.height, t.channels, rc2.x, rc2.y);
                     RT_CUDA(cudaGetLastError());
                     ctx->launches++;
                     ctx->texel_upload_bytes += count * (size_t)t.channels + 512 * sizeof(float);
@@ -1252,6 +1267,7 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
             DevTexture* dtex;
             if ((rc = upload(ctx, texs.data(), texs.size(), &dtex)) != RT_OK) return rc;
             dm.textures = dtex;
+            ctx->mesh_textures.push_back(texs);
             RT_CUDA(cudaStreamSynchronize(ctx->stream));   // texs is a local
         }
         DevMesh* dmeshes;
@@ -1341,6 +1357,9 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
         for (int i = 0; i < s->num_shapes; i++) if (!s->shapes[i].has_bounds) ctx->all_bounded = false;
         ctx->host_shapes.assign(s->shapes, s->shapes + s->num_shapes);
         ctx->host_num_materials = s->num_materials;
+        ctx->host_materials.assign(s->materials, s->materials + s->num_materials);
+        ctx->material_cap = s->num_materials; ctx->light_cap = s->num_lights;
+        ctx->materials_pooled = ctx->lights_pooled = false;
         for (int i = 0; i < s->num_shapes; i++)
             if (s->shapes[i].type == RT_SHAPE_MESH) ctx->mesh_state[s->shapes[i].mesh].users++;
         return RT_OK;
@@ -2213,6 +2232,160 @@ int rt_gpu_update_shapes(rt_gpu_ctx* ctx, const rt_shape* shapes, int32_t first,
         if ((rc = publish_done(ctx, st)) != RT_OK) return rc;
         for (int k = 0; k < count; k++) ctx->host_shapes[first + k].material = shapes[k].material;
         return RT_OK;
+    });
+}
+
+} // extern "C"
+
+// Room for `need` records in a scene array (*ptr: ctx->scene.materials or .lights), enqueued on `st` after the join of
+// an update: a larger array from the pool with the first `keep` records copied over.  One an earlier update allocated
+// is released with cudaFreeAsync; the uploaded one stays until the next upload or destroy.  Kernels enqueued before the
+// update hold the old pointer (DevScene goes to kernels by value) and the join has ordered them before the release.
+template <typename T>
+static int grow_records(rt_gpu_ctx* ctx, const T** ptr, int* cap, bool* pooled, int need, int keep, cudaStream_t st)
+{
+    if (need <= *cap) return RT_OK;
+    void* p = nullptr;
+    int rc = alloc_on(ctx, &p, (size_t)need * sizeof(T), st);
+    if (rc != RT_OK) return rc;
+    ctx->scene_allocs.push_back(p);
+    ctx->scene_bytes += (size_t)need * sizeof(T);
+    if (keep > 0) RT_CUDA(cudaMemcpyAsync(p, *ptr, (size_t)keep * sizeof(T), cudaMemcpyDeviceToDevice, st));
+    if (*pooled)
+    {
+        void* old = (void*)*ptr;
+        RT_CUDA(cudaFreeAsync(old, st));
+        ctx->scene_allocs.erase(std::find(ctx->scene_allocs.begin(), ctx->scene_allocs.end(), old));
+        ctx->scene_bytes -= (size_t)*cap * sizeof(T);
+    }
+    *ptr = (const T*)p; *cap = need; *pooled = true;
+    return RT_OK;
+}
+
+// count caller records into dst[0, count) on `st`, as kernel parameters
+template <typename T>
+static int write_records(rt_gpu_ctx* ctx, T* dst, const T* src, int count, cudaStream_t st)
+{
+    for (int b = 0; b < count; b += RT_RECORDS_PER_LAUNCH)
+    {
+        const int n = count - b < RT_RECORDS_PER_LAUNCH ? count - b : RT_RECORDS_PER_LAUNCH;
+        RecordBatch<T> batch;
+        memset(&batch, 0, sizeof batch);
+        memcpy(batch.rec, src + b, (size_t)n * sizeof(T));
+        rt_update_records_kernel<T><<<1, RT_RECORDS_PER_LAUNCH, 0, st>>>(dst + b, batch, n);
+        RT_CUDA(cudaGetLastError());
+        ctx->launches++;
+    }
+    return RT_OK;
+}
+
+extern "C" {
+
+int rt_gpu_update_materials(rt_gpu_ctx* ctx, const rt_material* materials, int32_t first, int32_t count, void* stream)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_update_materials before rt_gpu_upload_scene");
+        const int num = (int)ctx->host_materials.size();
+        if (first < 0 || count < 0 || first > num || count > 0x7fffffff - first)
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_materials: first must be in [0, node count] and count >= 0");
+        if (count == 0) return RT_OK;
+        if (!materials) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_materials: materials is null");
+        // the checks run on the graph as it will be: an edit can close a cycle through nodes it does not touch
+        const int n = std::max(num, first + count);
+        std::vector<rt_material> next(ctx->host_materials);
+        next.resize((size_t)n);
+        std::copy(materials, materials + count, next.begin() + first);
+        bool needs_table = false;
+        int rc = check_materials(ctx, next.data(), n, "rt_gpu_update_materials: ", &needs_table);
+        if (rc != RT_OK) return rc;
+        RT_CUDA(cudaSetDevice(ctx->device));
+        const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+        RT_CUDA(wait_scene(ctx, st));
+        if ((rc = join_scene_readers(ctx, st)) != RT_OK) return rc;
+        if ((rc = grow_records(ctx, &ctx->scene.materials, &ctx->material_cap, &ctx->materials_pooled, n, num, st)) != RT_OK)
+            return rc;
+        if ((rc = write_records(ctx, const_cast<rt_material*>(ctx->scene.materials) + first, materials, count, st)) != RT_OK)
+            return rc;
+        if ((rc = publish_done(ctx, st)) != RT_OK) return rc;
+        ctx->host_materials.swap(next);
+        ctx->host_num_materials = n;
+        ctx->scene.num_materials = n;
+        ctx->needs_table = needs_table;
+        return RT_OK;
+    });
+}
+
+int rt_gpu_update_lights(rt_gpu_ctx* ctx, const rt_light* lights, int32_t count, void* stream)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_update_lights before rt_gpu_upload_scene");
+        if (count < 0) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_lights: count must be >= 0");
+        if (count > 0 && !lights) return fail(ctx, RT_ERR_INVALID, "rt_gpu_update_lights: lights is null");
+        RT_CUDA(cudaSetDevice(ctx->device));
+        const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+        RT_CUDA(wait_scene(ctx, st));
+        int rc = join_scene_readers(ctx, st);
+        if (rc != RT_OK) return rc;
+        if ((rc = grow_records(ctx, &ctx->scene.lights, &ctx->light_cap, &ctx->lights_pooled, count, 0, st)) != RT_OK) return rc;
+        if ((rc = write_records(ctx, const_cast<rt_light*>(ctx->scene.lights), lights, count, st)) != RT_OK) return rc;
+        if ((rc = publish_done(ctx, st)) != RT_OK) return rc;
+        ctx->scene.num_lights = count;        // later calls size their Whitted rounds and pools by it
+        return RT_OK;
+    });
+}
+
+int rt_gpu_update_texture(rt_gpu_ctx* ctx, int32_t mesh, int32_t slot, const rt_texture_update* t, void* stream)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        const std::string f("rt_gpu_update_texture: ");
+        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_update_texture before rt_gpu_upload_scene");
+        if (!t) return fail(ctx, RT_ERR_INVALID, f + "update is null");
+        if (mesh < 0 || mesh >= (int)ctx->mesh_textures.size()) return fail(ctx, RT_ERR_INVALID, f + "mesh out of range");
+        if (slot < 0 || slot >= (int)ctx->mesh_textures[mesh].size()) return fail(ctx, RT_ERR_INVALID, f + "texture slot out of range");
+        const DevTexture dt = ctx->mesh_textures[mesh][slot];
+        if (dt.width <= 0 || dt.height <= 0) return fail(ctx, RT_ERR_INVALID, f + "the slot had no pixels at upload");
+        if (t->x < 0 || t->y < 0 || t->width < 0 || t->height < 0 || (long long)t->x + t->width > dt.width ||
+            (long long)t->y + t->height > dt.height)
+            return fail(ctx, RT_ERR_INVALID, f + "rectangle outside the slot");
+        if ((t->rgba == nullptr) == (t->texels8 == nullptr)) return fail(ctx, RT_ERR_INVALID, f + "exactly one of rgba and texels8");
+        if (t->rgba)
+        {
+            if (t->pitch < (size_t)t->width * 16 || t->pitch % 4 != 0)
+                return fail(ctx, RT_ERR_INVALID, f + "pitch must be at least width * 16 bytes and a multiple of 4");
+            if ((uintptr_t)t->rgba % 4 != 0) return fail(ctx, RT_ERR_INVALID, f + "rgba must be 4-byte aligned");
+        }
+        else
+        {
+            if (t->channels != 3 && t->channels != 4) return fail(ctx, RT_ERR_INVALID, f + "texels8 needs 3 or 4 channels");
+            if (!t->lut || (uintptr_t)t->lut % 4 != 0) return fail(ctx, RT_ERR_INVALID, f + "texels8 needs a 4-byte aligned 512-entry lut");
+        }
+        RT_CUDA(cudaSetDevice(ctx->device));
+        const void* ptrs[3] = { t->rgba, t->texels8, t->rgba ? nullptr : t->lut };
+        const char* names[3] = { "rgba", "texels8", "lut" };
+        for (int k = 0; k < 3; k++)
+            if (ptrs[k] && !on_device(ctx, ptrs[k]))
+                return fail(ctx, RT_ERR_INVALID, f + names[k] + " is not device memory of the context's GPU");
+        if (t->width == 0 || t->height == 0) return RT_OK;
+        const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+        RT_CUDA(wait_scene(ctx, st));
+        int rc = join_scene_readers(ctx, st);
+        if (rc != RT_OK) return rc;
+        const int ax = dt.x0 + t->x, ay = dt.y0 + t->y;
+        if (t->rgba)
+            RT_CUDA(cudaMemcpy2DToArrayAsync(ctx->atlas_array, (size_t)ax * 16, (size_t)ay, t->rgba, t->pitch, (size_t)t->width * 16,
+                                             (size_t)t->height, cudaMemcpyDeviceToDevice, st));
+        else
+        {
+            const dim3 grid((unsigned)((t->width + 31) / 32), (unsigned)((t->height + 7) / 8));
+            rt_expand_texels_kernel<<<grid, dim3(32, 8), 0, st>>>(ctx->atlas_surface, t->texels8, t->lut, t->width, t->height,
+                                                                  t->channels, ax, ay);
+            RT_CUDA(cudaGetLastError());
+            ctx->launches++;
+        }
+        return publish_done(ctx, st);
     });
 }
 

@@ -196,6 +196,45 @@ int rt_gpu_debug_read_mesh(rt_gpu_ctx* ctx, int32_t mesh, rt_bvh_node* nodes, rt
     });
 }
 
+int rt_gpu_debug_read_appearance(rt_gpu_ctx* ctx, rt_material* materials, int32_t mat_cap, rt_light* lights, int32_t light_cap,
+                                 int32_t* counts2)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_debug_read_appearance before rt_gpu_upload_scene");
+        if (mat_cap < 0 || light_cap < 0) return fail(ctx, RT_ERR_INVALID, "rt_gpu_debug_read_appearance: negative capacity");
+        RT_CUDA(cudaSetDevice(ctx->device));
+        RT_CUDA(wait_scene(ctx, ctx->stream));
+        const DevScene& sc = ctx->scene;
+        const int nm = std::min(mat_cap, sc.num_materials), nl = std::min(light_cap, sc.num_lights);
+        if (materials && nm > 0)
+            RT_CUDA(cudaMemcpyAsync(materials, sc.materials, (size_t)nm * sizeof(rt_material), cudaMemcpyDeviceToHost, ctx->stream));
+        if (lights && nl > 0)
+            RT_CUDA(cudaMemcpyAsync(lights, sc.lights, (size_t)nl * sizeof(rt_light), cudaMemcpyDeviceToHost, ctx->stream));
+        RT_CUDA(cudaStreamSynchronize(ctx->stream));
+        if (counts2) { counts2[0] = sc.num_materials; counts2[1] = sc.num_lights; }
+        return RT_OK;
+    });
+}
+
+int rt_gpu_debug_read_texture(rt_gpu_ctx* ctx, int32_t mesh, int32_t slot, float* rgba)
+{
+    return rt_guard(ctx, [&]() -> int {
+        if (!ctx) return RT_ERR_INVALID;
+        if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_gpu_debug_read_texture before rt_gpu_upload_scene");
+        if (!rgba || mesh < 0 || mesh >= (int)ctx->mesh_textures.size() || slot < 0 || slot >= (int)ctx->mesh_textures[mesh].size())
+            return fail(ctx, RT_ERR_INVALID, "rt_gpu_debug_read_texture: bad arguments");
+        const DevTexture t = ctx->mesh_textures[mesh][slot];
+        if (t.width <= 0 || t.height <= 0) return fail(ctx, RT_ERR_INVALID, "rt_gpu_debug_read_texture: the slot has no pixels");
+        RT_CUDA(cudaSetDevice(ctx->device));
+        RT_CUDA(wait_scene(ctx, ctx->stream));
+        RT_CUDA(cudaMemcpy2DFromArrayAsync(rgba, (size_t)t.width * 16, ctx->atlas_array, (size_t)t.x0 * 16, (size_t)t.y0,
+                                           (size_t)t.width * 16, (size_t)t.height, cudaMemcpyDeviceToHost, ctx->stream));
+        RT_CUDA(cudaStreamSynchronize(ctx->stream));
+        return RT_OK;
+    });
+}
+
 int rt_gpu_trace_rays(rt_gpu_ctx* ctx, const float* rays, int32_t n, int32_t traverse, int32_t* shape, int32_t* tri, float* hit11)
 {
     return rt_guard(ctx, [&]() -> int {
@@ -271,6 +310,7 @@ int rt_gpu_kat_texture(rt_gpu_ctx* ctx, int32_t texture, const float* uv, int32_
         cudaError_t e = cudaMalloc((void**)&duv, (size_t)n * 2 * sizeof(float));
         if (e == cudaSuccess) e = cudaMalloc((void**)&dout, (size_t)n * 4 * sizeof(float));
         if (e == cudaSuccess) e = cudaMemcpyAsync(duv, uv, (size_t)n * 2 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+        if (e == cudaSuccess) e = wait_scene(ctx, ctx->stream);      // after every rt_gpu_update_texture enqueued so far
         if (e == cudaSuccess)
         {
             rt_kat_texture_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->scene.atlas, ctx->host_textures[texture], duv, n, dout);
