@@ -375,18 +375,7 @@ struct Buf
     }
 };
 
-// The scratch block: level counters, then every per-triangle array of the build, each 256-byte aligned
-struct Carve
-{
-    char* base; size_t off;
-    template <typename T> T* take(size_t n)
-    {
-        T* p = (T*)(base + off);
-        off += ((n ? n : 1) * sizeof(T) + 255) & ~(size_t)255;
-        return p;
-    }
-};
-
+// The scratch block: level counters, then every per-triangle array of the build
 struct Scratch
 {
     int* counts;                                             // next_count, max_count, flag, -

@@ -1,11 +1,25 @@
 // rt_bvh_core.hpp — the device BVH builder's core (rt_bvh_build.cu), library-internal: rt_gpu_build_bvh wraps it with
-// host copies, rt_gpu_update_mesh (rt_gpu.cu) runs it on device inputs into a mesh's spare arrays.
+// host copies, rt_gpu_update_mesh and rt_gpu_replace_mesh (rt_scene_edit.cu) run it on device inputs into a mesh's spare
+// arrays.  Carve lays out the builder's scratch block and the scene edits' scratch.
 #pragma once
 #include <cuda_runtime.h>
 #include <float.h>
 #include <stddef.h>
 
 #include "rt_gpu.h"
+
+// Arrays cut one after another from a block whose base is 256-byte aligned, each 256-byte aligned.  On a null base the
+// pointers are meaningless and `off` ends as the block's size.
+struct Carve
+{
+    char* base; size_t off;
+    template <typename T> T* take(size_t n)
+    {
+        T* p = (T*)(base + off);
+        off += ((n ? n : 1) * sizeof(T) + 255) & ~(size_t)255;
+        return p;
+    }
+};
 
 // Device bytes of the scratch block a build of num_tris triangles needs (256-byte aligned base).  Its first 16 bytes
 // are the level counters {next segments, largest child, flag, -}; the flag is the caller's (see below).

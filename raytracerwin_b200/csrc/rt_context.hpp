@@ -1,6 +1,6 @@
-// rt_context.hpp — the opaque context behind include/rt_gpu.h and the error helpers every translation unit of
-// the library uses (rt_gpu.cu: lifetime / upload / render / readback; rt_exchange.cu: multi-GPU tile exchange;
-// rt_hooks.cu: test and tooling hooks; rt_bvh_build.cu: device BVH builder).
+// rt_context.hpp — the opaque context behind include/rt_gpu.h and the error and argument helpers every translation
+// unit of the library uses (rt_gpu.cu: lifetime / upload / render / queries / readback; rt_scene_edit.cu: scene edits;
+// rt_exchange.cu: multi-GPU tile exchange; rt_hooks.cu: test and tooling hooks; rt_bvh_build.cu: device BVH builder).
 #pragma once
 #include "rt_wave_types.hpp"
 
@@ -8,6 +8,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <initializer_list>
 #include <new>
 #include <string>
 #include <vector>
@@ -125,7 +126,6 @@ struct rt_gpu_ctx
     // What the updates check and swap, per uploaded shape and mesh.  A mesh's arrays are double-buffered from its first
     // update on: an update builds into the spare set and publishes it; the published set becomes the spare.
     std::vector<rt_shape> host_shapes;          // the records as uploaded (materials follow rt_gpu_update_shapes)
-    int host_num_materials = 0;
     // ---- appearance updates (rt_gpu_update_materials / rt_gpu_update_lights / rt_gpu_update_texture) ----
     std::vector<rt_material> host_materials;    // the graph the device holds (the checks of an update run on its edit)
     // Room of ctx->scene.materials / .lights in records.  `pooled`: from cudaMallocAsync by an update, released with
@@ -192,3 +192,27 @@ static inline int rt_guard(rt_gpu_ctx* ctx, F&& body) noexcept
     catch (const std::exception& e) { try { return fail(ctx, RT_ERR_INVALID, e.what()); } catch (...) { return RT_ERR_INVALID; } }
     catch (...) { return RT_ERR_INVALID; }
 }
+
+// The caller's arrays of a call that takes device memory (`fn` names the call in the messages): each one given (null:
+// an optional array left out) must be `align`-byte aligned device memory (or managed memory) of the context's GPU.
+struct DeviceArg { const void* ptr; const char* name; size_t align; };
+static inline int check_device_args(rt_gpu_ctx* ctx, const char* fn, std::initializer_list<DeviceArg> args)
+{
+    for (const DeviceArg& a : args)
+    {
+        if (!a.ptr) continue;
+        if ((uintptr_t)a.ptr % a.align != 0)
+            return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": " + a.name + " must be " + std::to_string(a.align) + "-byte aligned");
+        cudaPointerAttributes at;
+        memset(&at, 0, sizeof at);
+        const cudaError_t e = cudaPointerGetAttributes(&at, a.ptr);
+        if (e != cudaSuccess) cudaGetLastError();
+        if (e != cudaSuccess || (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != ctx->device)
+            return fail(ctx, RT_ERR_INVALID, std::string(fn) + ": " + a.name + " is not device memory of the context's GPU");
+    }
+    return RT_OK;
+}
+
+// The material checks of rt_gpu_upload_scene and rt_gpu_update_materials (rt_gpu.cu; library-internal: not exported)
+__attribute__((visibility("hidden"))) int check_materials(rt_gpu_ctx* ctx, const rt_material* mats, int n, const std::string& prefix,
+                                                          bool* needs_table);
