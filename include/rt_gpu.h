@@ -224,7 +224,10 @@ int rt_gpu_destroy(rt_gpu_ctx* ctx);
 const char* rt_gpu_last_error(rt_gpu_ctx* ctx);   /* ctx may be NULL: last create() error */
 
 /* Copies the whole scene to the device; the caller keeps ownership of all host memory and may
- * free it on return.  A second upload replaces the scene. */
+ * free it on return.  A second upload replaces the scene.  RT_ERR_INVALID (the context keeps its scene) for a
+ * malformed description, a material graph it refuses (see rt_material), and a mesh with a non-finite (NaN or
+ * infinite) BVH node bound or triangle corner p0 / p1 / p2; the message names the mesh.  The precomputed face normal
+ * n is not checked: finite corners whose cross product overflows give a NaN n, and the reference computes the same. */
 int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* scene);
 
 /* Frame slots.  A context holds RT_GPU_FRAME_SLOTS independent sets of frame buffers (accuBuffer, bitcolor,
@@ -340,7 +343,8 @@ int rt_gpu_radiance_rays(rt_gpu_ctx* ctx, const rt_radiance_query* q, void* stre
  * on the device once the calls enqueued before it have finished with the old scene, and later calls wait for that on
  * their streams.  Errors (RT_ERR_INVALID) leave the scene exactly as it was. */
 typedef struct rt_mesh_update {
-    const float* points;       /* DEVICE, num_points x 3, 4-byte aligned */
+    const float* points;       /* DEVICE, num_points x 3, 4-byte aligned; every coordinate finite, the points no triangle
+                                  uses too (they widen the shape's bounds); a NaN or infinity is refused */
     int32_t num_points;
     const int32_t* point_idx;  /* DEVICE, num_tris x 3: triangle t = original triangle id t */
     int32_t num_tris;          /* must equal the mesh's num_tris (as uploaded, or as the last rt_gpu_replace_mesh gave it) */
@@ -356,8 +360,9 @@ typedef struct rt_mesh_update {
  * spare set of its arrays (192 B per triangle).  RT_ERR_INVALID for NULL, misaligned or non-device pointers, a shape
  * that is not a mesh or whose mesh another shape also references, num_tris other than the mesh's count, an
  * uploaded mesh whose node count is not 2 * num_tris - 1 (a description the host layer never produces),
- * num_points <= 0, normals without normal_idx or the reverse, and a point or normal index out of range (found on the
- * device, before anything is published); RT_ERR_NO_SCENE before an upload. */
+ * num_points <= 0, normals without normal_idx or the reverse, and a point or normal index out of range or a non-finite
+ * point coordinate (found on the device and read by the host before the build starts; nothing is published);
+ * RT_ERR_NO_SCENE before an upload. */
 int rt_gpu_update_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, void* stream);
 
 /* A REFIT of the mesh of mesh shape `shape` to new points (per-frame deformation: skinning, cloth, physics): the
@@ -373,7 +378,8 @@ int rt_gpu_update_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, 
  * After a refit, every later call returns what a fresh upload of the scene with these arrays returns.  Ordering and
  * the spare set as rt_gpu_update_mesh, but the call RETURNS AT ONCE: no host read, no synchronisation, no blocking
  * allocation.  `status`: DEVICE int32 or NULL, written in `stream`'s order: 0 when the refit was published, otherwise
- * the bits of the index check (1 = a point index out of range, 2 = a normal index out of range).  The mesh's arrays,
+ * the bits of the device check (1 = a point index out of range, 2 = a normal index out of range, 16 = a non-finite
+ * point coordinate, which the upload would refuse).  The mesh's arrays,
  * the shape's bounds and the culling margin are then left as they were, and every later call returns what it returned
  * before.  Such a refit still publishes (a copy of the arrays), so, as after an update, an RT_OCTO mesh walks its binary
  * tree from then on and for mesh 0 RT_TOP_STAGE is turned off; both give the same bits.  RT_ERR_INVALID (nothing
@@ -397,8 +403,9 @@ int rt_gpu_refit_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, i
  * RT_ERR_INVALID (the scene left exactly as it was) for rt_gpu_update_mesh's host-side checks other than the count and
  * node-count tests, num_tris <= 0, texcoords without texcoord_idx or the reverse, num_texcoords <= 0 with texcoords,
  * misaligned or non-device texcoords / texcoord_idx / texture, and, found on the device before anything is published, a
- * point, normal or texcoord index out of range or a texture slot the upload would refuse (>= the mesh's texture count,
- * or a slot without pixels; negative slots are untextured and pass); RT_ERR_NO_SCENE before an upload. */
+ * point, normal or texcoord index out of range, a texture slot the upload would refuse (>= the mesh's texture count,
+ * or a slot without pixels; negative slots are untextured and pass) or a non-finite point coordinate; RT_ERR_NO_SCENE
+ * before an upload. */
 typedef struct rt_mesh_replace {
     rt_mesh_update geometry;      /* rt_mesh_update's rules, except that num_tris is the NEW triangle count (>= 1) */
     const float* texcoords;       /* DEVICE, num_texcoords x 2 {u, v}, 4-byte aligned, or NULL: every corner gets uv (0, 0) */
@@ -553,7 +560,9 @@ int rt_gpu_kernel_class_ms(rt_gpu_ctx* ctx, float* ms, int32_t* launches, int32_
  * KdTree::Build (KdTree.cpp:10-126, 202-220) with the reference's partition rule, emitting the same
  * pre-order rt_bvh_node / leaf-order rt_tri arrays as the host builder, bit for bit.  `points` are xyz
  * triples, `indices` three point indices per triangle (host pointers); out_nodes holds 2*num_tris-1
- * records, out_tris num_tris.  out_depth / out_ms (device time of the build, CUDA events) may be NULL. */
+ * records, out_tris num_tris.  out_depth / out_ms (device time of the build, CUDA events) may be NULL.
+ * RT_ERR_INVALID for a point index out of range and for a non-finite (NaN or infinite) coordinate of any point,
+ * which the upload would refuse too. */
 int rt_gpu_build_bvh(rt_gpu_ctx* ctx, const float* points, int32_t num_points, const int32_t* indices,
                      int32_t num_tris, rt_bvh_node* out_nodes, rt_tri* out_tris, int32_t* out_depth, float* out_ms);
 

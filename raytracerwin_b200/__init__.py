@@ -484,7 +484,8 @@ class GpuContext:
 
         Enqueued on torch.cuda.current_stream(self.device) and returns at once, with no host wait.  Returns the int32
         (1,) status tensor on the device, written in that stream's order: 0 when the refit was published, otherwise
-        1 (a point index out of range) | 2 (a normal index out of range), and the mesh is left as it was.  Reading
+        1 (a point index out of range) | 2 (a normal index out of range) | 16 (a NaN or infinite point coordinate), and
+        the mesh is left as it was.  Reading
         it is the caller's choice (it synchronises)."""
         import torch
         self._mesh_update_tensors(points, point_idx, normals, normal_idx)

@@ -416,7 +416,7 @@ size_t rt_bvh_scratch_bytes(int num_tris) { return carve(nullptr, num_tris, null
 int* rt_bvh_scratch_flag(void* scratch) { return (int*)scratch + 2; }
 
 int rt_bvh_build_core(rt_gpu_ctx* ctx, const float* dP, const int* dI, int T, cudaStream_t st, void* scratch, int* host_counts,
-                      bool check_flag, const char* message, rt_bvh_node* dnodes, rt_tri* dtris, int* out_depth)
+                      rt_bvh_node* dnodes, rt_tri* dtris, int* out_depth)
 {
     Scratch s;
     carve(scratch, T, &s);
@@ -450,11 +450,9 @@ int rt_bvh_build_core(rt_gpu_ctx* ctx, const float* dP, const int* dI, int T, cu
         k_children<<<(num_segs + tb - 1) / tb, tb, 0, st>>>(L);
         k_scatter<<<pg, tb, 0, st>>>(L);
         BV_CUDA(cudaGetLastError());
-        // one read per level: the next level's segment count and largest segment (and, first, the caller's flag)
-        const bool first = depth == 1 && check_flag;
-        BV_CUDA(cudaMemcpyAsync(host_counts, s.counts, (first ? 3 : 2) * sizeof(int), cudaMemcpyDeviceToHost, st));
+        // one read per level: the next level's segment count and largest segment
+        BV_CUDA(cudaMemcpyAsync(host_counts, s.counts, 2 * sizeof(int), cudaMemcpyDeviceToHost, st));
         BV_CUDA(cudaStreamSynchronize(st));
-        if (first && host_counts[2] != 0) { rt_ctx_set_error(ctx, message); return RT_ERR_INVALID; }
         num_segs = host_counts[0]; level_max = host_counts[1];
         cur ^= 1;
         if (depth > 4096) { rt_ctx_set_error(ctx, "rt_gpu_build_bvh: runaway depth"); return RT_ERR_CUDA; }
@@ -483,6 +481,14 @@ extern "C" int rt_gpu_build_bvh(rt_gpu_ctx* ctx, const float* points, int32_t nu
             rt_ctx_set_error(ctx, "rt_gpu_build_bvh: point index out of range");
             return RT_ERR_INVALID;
         }
+    // a NaN or infinite coordinate is refused, as the upload and the mesh edits refuse it: the builder equals the host
+    // builder on every input either of them accepts
+    for (long long k = 0; k < 3ll * num_points; k++)
+        if (!(fabsf(points[k]) <= FLT_MAX))
+        {
+            rt_ctx_set_error(ctx, "rt_gpu_build_bvh: non-finite point");
+            return RT_ERR_INVALID;
+        }
     BV_CUDA(cudaSetDevice(rt_ctx_device(ctx)));
     cudaStream_t st = (cudaStream_t)rt_gpu_stream(ctx);
     const int T = num_tris;
@@ -497,7 +503,7 @@ extern "C" int rt_gpu_build_bvh(rt_gpu_ctx* ctx, const float* points, int32_t nu
     BV_CUDA(cudaEventCreate(&e0)); BV_CUDA(cudaEventCreate(&e1));
     BV_CUDA(cudaEventRecord(e0, st));
     int counts[4] = { 0, 0, 0, 0 }, depth = 0;
-    const int rc = rt_bvh_build_core(ctx, dP, dI, T, st, scratch, counts, false, nullptr, dnodes, dtris, &depth);
+    const int rc = rt_bvh_build_core(ctx, dP, dI, T, st, scratch, counts, dnodes, dtris, &depth);
     if (rc != RT_OK) { cudaEventDestroy(e0); cudaEventDestroy(e1); return rc; }
     BV_CUDA(cudaEventRecord(e1, st));
     BV_CUDA(cudaMemcpyAsync(out_nodes, dnodes, (2 * (size_t)T - 1) * sizeof(rt_bvh_node), cudaMemcpyDeviceToHost, st));

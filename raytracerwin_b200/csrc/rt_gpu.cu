@@ -86,6 +86,12 @@ static void build_octo(const rt_bvh_node* nodes, int n, std::vector<rt_bvh_node>
 }
 
 static inline bool texture_has_pixels(const rt_texture& t) { return t.rgba != nullptr || t.texels8 != nullptr; }
+static inline bool finite_n(const float* v, int n)
+{
+    for (int k = 0; k < n; k++)
+        if (!std::isfinite(v[k])) return false;
+    return true;
+}
 
 // RTexture::LoadTexturePNG's texel loop (Texture.cpp:119-151) on the device: 8-bit code -> table entry.  The
 // table is the host's (glibc powf(c / 255, 2.2f) for rgb, c / 255 for alpha), so the float4 texels written into
@@ -746,6 +752,16 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
                 if (m.tris[k].index < 0 || m.tris[k].index >= m.num_tris) return fail(ctx, RT_ERR_INVALID, "triangle index out of range");
                 if (m.shade[k].texture >= m.num_textures) return fail(ctx, RT_ERR_INVALID, "texture index out of range");
             }
+            // Non-finite geometry is refused: a NaN corner makes the face normal NaN, and triangle_test then accepts the
+            // triangle from any direction, outside the margin of the culled walk; a NaN bound is where slab_fast and the
+            // reference's slab test part.  The face normal `n` is not checked: finite corners whose cross product
+            // overflows give a NaN normal, and the reference computes the same.
+            for (int k = 0; k < m.num_nodes; k++)
+                if (!finite_n(m.nodes[k].bmin, 3) || !finite_n(m.nodes[k].bmax, 3))
+                    return fail(ctx, RT_ERR_INVALID, "mesh " + std::to_string(i) + ": non-finite BVH node bound");
+            for (int k = 0; k < m.num_tris; k++)
+                if (!finite_n(m.tris[k].p0, 3) || !finite_n(m.tris[k].p1, 3) || !finite_n(m.tris[k].p2, 3))
+                    return fail(ctx, RT_ERR_INVALID, "mesh " + std::to_string(i) + ": non-finite triangle corner");
             for (int k = 0; k < m.num_textures; k++)
             {
                 const rt_texture& t = m.textures[k];

@@ -57,13 +57,16 @@ __global__ void rt_kat_kernel(int kind, const float* rays, const float* prims, i
         RayPre pre = ray_pre(r);
         float tlo, thi;
         hit = slab_general(r, pre, ld3(b), ld3(b + 3), tlo, thi);
-        const bool all_axes = pre.ex && pre.ey && pre.ez && finite3(r.o) && finite3(r.d);
+        // the walks run slab_fast where this holds; their boxes are finite because the upload refuses other ones
+        const bool all_axes = pre.ex && pre.ey && pre.ez && finite3(r.o) && finite3(r.d) && finite3(ld3(b)) && finite3(ld3(b + 3));
         if (all_axes)
         {
             float tlo2, thi2;
             const bool hit2 = slab_fast(r, pre, ld3(b), ld3(b + 3), tlo2, thi2);
             if (hit2 != hit) hit = !hit;   // would surface as a mismatch against the oracle
-            if (hit && __float_as_uint(tlo2) != __float_as_uint(tlo)) tlo = __uint_as_float(0x7fc00000u);
+            // by value: where tlo is a zero (an origin on a face of the box), FMNMX and the reference's ternaries can keep
+            // zeros of different sign; no walk can tell them apart (the walks only compare tlo with other values)
+            if (hit && tlo2 != tlo) tlo = __uint_as_float(0x7fc00000u);
         }
         flags[i] = hit ? 1 : 0;
         o[0] = hit ? tlo : 0.0f;

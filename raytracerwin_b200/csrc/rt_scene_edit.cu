@@ -19,19 +19,28 @@ __global__ void rt_patch_right_child(rt_bvh_node* nodes, int n);
 #define RT_UPD_BAD_NORMAL_INDEX 2
 #define RT_UPD_BAD_TEXCOORD_INDEX 4
 #define RT_UPD_BAD_TEXTURE 8
+#define RT_UPD_BAD_POINT_VALUE 16
 
 // Checks every index the call gives and copies the point indices into `safe_p`, the texcoord indices into `safe_t` and,
 // when `safe_n` is given, the normal indices into it, with bad ones replaced by 0: no later kernel reads outside
 // `points`, `normals` or `texcoords` even before the host has seen the flag.  (An update and a replace read normal_idx
 // only once the host has seen it; a refit never waits for it, and throws its result away on the device.)  A replace
 // also gives one texture slot per triangle: one the upload would refuse (>= the mesh's slot count, or a slot without
-// pixels) is bad; negative slots pass.
-__global__ void rt_update_check_kernel(const int* __restrict__ pidx, int num_points, const int* __restrict__ nidx, int num_normals,
-                                       const int* __restrict__ tidx, int num_texcoords, const int* __restrict__ texture,
-                                       const DevMesh* __restrict__ mesh, int n, int* __restrict__ safe_p, int* __restrict__ safe_n,
-                                       int* __restrict__ safe_t, int* __restrict__ flag)
+// pixels) is bad; negative slots pass.  Every point in [0, num_points) must be finite, the ones no triangle uses too:
+// the shape's bounds are RAabb::Expand over all of them, and the upload refuses non-finite geometry for the walks'
+// sake (rt_gpu_upload_scene).  Thread i checks index i (i < n) and point i (i < num_points).
+__global__ void rt_update_check_kernel(const int* __restrict__ pidx, const float* __restrict__ points, int num_points,
+                                       const int* __restrict__ nidx, int num_normals, const int* __restrict__ tidx, int num_texcoords,
+                                       const int* __restrict__ texture, const DevMesh* __restrict__ mesh, int n,
+                                       int* __restrict__ safe_p, int* __restrict__ safe_n, int* __restrict__ safe_t,
+                                       int* __restrict__ flag)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < num_points)
+    {
+        const float* p = points + 3 * (size_t)i;
+        if (!(fabsf(p[0]) <= FLT_MAX && fabsf(p[1]) <= FLT_MAX && fabsf(p[2]) <= FLT_MAX)) atomicOr(flag, RT_UPD_BAD_POINT_VALUE);
+    }
     if (i >= n) return;
     int v = pidx[i], bad = 0;
     if (v < 0 || v >= num_points) { v = 0; bad |= RT_UPD_BAD_POINT_INDEX; }
@@ -514,29 +523,29 @@ static int rebuild_mesh(rt_gpu_ctx* ctx, const char* fn, int32_t shape, int mi, 
     const int n3 = 3 * T;
     const unsigned gT = (unsigned)((T + 255) / 256);
     RT_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), st));
-    rt_update_check_kernel<<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(u->point_idx, u->num_points, u->normal_idx,
-                                                                          u->normals ? u->num_normals : 0, r->texcoord_idx,
-                                                                          r->num_texcoords, r->texture, ctx->scene.meshes + mi,
-                                                                          n3, safe_idx, nullptr, safe_tidx, flag);
+    const int nc = n3 > u->num_points ? n3 : u->num_points;
+    rt_update_check_kernel<<<(unsigned)((nc + 255) / 256), 256, 0, st>>>(u->point_idx, u->points, u->num_points, u->normal_idx,
+                                                                         u->normals ? u->num_normals : 0, r->texcoord_idx,
+                                                                         r->num_texcoords, r->texture, ctx->scene.meshes + mi,
+                                                                         n3, safe_idx, nullptr, safe_tidx, flag);
     RT_CUDA(cudaGetLastError());
     ctx->launches++;
-    const std::string message = std::string(fn) + (replace ? ": point, normal or texcoord index or texture slot out of range"
-                                                           : ": point or normal index out of range");
-    rc = rt_bvh_build_core(ctx, u->points, safe_idx, T, st, build, ctx->update_counts, true, message.c_str(),
-                           ms.spare.nodes, ms.spare.tris, nullptr);
-    if (rc != RT_OK)
+    // the host reads the check before the builder runs: the builder never sees a non-finite key or an unchecked index
+    RT_CUDA(cudaMemcpyAsync(ctx->update_counts + 2, flag, sizeof(int), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaStreamSynchronize(st));
+    if (const int bad = ctx->update_counts[2])
     {
-        if (rc == RT_ERR_INVALID && replace)
-        {
-            const int bad = ctx->update_counts[2];
-            std::string what;
-            for (auto b : { std::make_pair(RT_UPD_BAD_POINT_INDEX, "point index"), std::make_pair(RT_UPD_BAD_NORMAL_INDEX, "normal index"),
-                            std::make_pair(RT_UPD_BAD_TEXCOORD_INDEX, "texcoord index"), std::make_pair(RT_UPD_BAD_TEXTURE, "texture slot") })
-                if (bad & b.first) what += (what.empty() ? " " : ", ") + std::string(b.second);
-            ctx->err = std::string(fn) + ": out of range:" + what;
-        }
-        return rc;
+        std::string what;
+        for (auto b : { std::make_pair(RT_UPD_BAD_POINT_INDEX, "point index"), std::make_pair(RT_UPD_BAD_NORMAL_INDEX, "normal index"),
+                        std::make_pair(RT_UPD_BAD_TEXCOORD_INDEX, "texcoord index"), std::make_pair(RT_UPD_BAD_TEXTURE, "texture slot") })
+            if (bad & b.first) what += (what.empty() ? " " : ", ") + std::string(b.second);
+        std::string msg = std::string(fn) + ":";
+        if (!what.empty()) msg += " out of range:" + what;
+        if (bad & RT_UPD_BAD_POINT_VALUE) msg += std::string(what.empty() ? "" : ";") + " non-finite point";
+        return fail(ctx, RT_ERR_INVALID, msg);
     }
+    rc = rt_bvh_build_core(ctx, u->points, safe_idx, T, st, build, ctx->update_counts, ms.spare.nodes, ms.spare.tris, nullptr);
+    if (rc != RT_OK) return rc;
     rt_patch_right_child<<<(unsigned)((2 * T - 1 + 255) / 256), 256, 0, st>>>(ms.spare.nodes, 2 * T - 1);
     if (replace)
         rt_replace_shade_kernel<<<gT, 256, 0, st>>>(u->points, safe_idx, u->normals, u->normal_idx, r->texcoords, safe_tidx,
@@ -653,9 +662,10 @@ int rt_gpu_refit_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, i
 
         const int n3 = 3 * T;
         RT_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), st));
-        rt_update_check_kernel<<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(u->point_idx, u->num_points, u->normal_idx,
-                                                                              u->normals ? u->num_normals : 0, nullptr, 0, nullptr,
-                                                                              nullptr, n3, safe_p, safe_n, nullptr, flag);
+        const int nc = n3 > u->num_points ? n3 : u->num_points;
+        rt_update_check_kernel<<<(unsigned)((nc + 255) / 256), 256, 0, st>>>(u->point_idx, u->points, u->num_points, u->normal_idx,
+                                                                             u->normals ? u->num_normals : 0, nullptr, 0, nullptr,
+                                                                             nullptr, n3, safe_p, safe_n, nullptr, flag);
         rt_refit_links_kernel<<<gN, 256, 0, st>>>(ms.cur.nodes, N, parent, leaf_node, arrivals);
         rt_refit_kernel<<<gT, 256, 0, st>>>((const float4*)ms.cur.tris, (const float4*)ms.cur.nodes, u->points, safe_p, leaf_node,
                                             parent, arrivals, ms.spare.tris, (float4*)ms.spare.nodes, T);
