@@ -25,6 +25,9 @@
  *                        (levels of detail, procedural and streamed geometry) without a new upload
  *   rt_gpu_update_materials  material nodes edited in place or appended, rt_gpu_update_lights a new light list and
  *   rt_gpu_update_texture    a rectangle of texels from device memory: the scene's appearance without a new upload
+ *   rt_gpu_track_moments     per-pixel moments of the pass colours (the error estimate of each pixel of a frame slot),
+ *   rt_gpu_select_pixels     the pixels whose estimate is above a tolerance, as a device mask, and
+ *   rt_gpu_render_masked     render_tile restricted to a device pixel mask: adaptive sampling
  *
  * Plain C: POD structs, pointers and sizes only.  No C++/STL/torch types cross the boundary.
  * Every entry returns 0 on success or a negative rt_status; rt_gpu_last_error() gives text.
@@ -197,8 +200,10 @@ enum {
     RT_READ_PRIMARY_IDS_I32X2 = 2,/* width*height x {shape index, triangle index} of the primary hit, -1 = none */
     RT_READ_PRIMARY_DIST_F32 = 3, /* width*height x RayHitResult::Distance of the primary hit (0 if none) */
     RT_READ_COUNTERS_U64 = 4,     /* rt_counters */
-    RT_READ_PREVIEW_RGBA_F32 = 5  /* width*height x float4: the linear colour c of the last RT_MODE_PREVIEW pass, the value the
+    RT_READ_PREVIEW_RGBA_F32 = 5, /* width*height x float4: the linear colour c of the last RT_MODE_PREVIEW pass, the value the
                                      reference hands to LinearToGamma before it stores bitcolor (RayTracerProgram.cpp:175-180) */
+    RT_READ_MOMENTS_F32 = 6       /* width*height x float4 {M2.r, M2.g, M2.b, passes}: the moments of rt_gpu_track_moments
+                                     (RT_ERR_NO_SCENE if tracking has never been on for the frame slot) */
 };
 
 typedef struct rt_counters {
@@ -275,6 +280,58 @@ typedef struct rt_camera {
  * RT_ERR_INVALID, with nothing enqueued, for a non-finite field, a basis whose determinant (in double) is 0, and
  * every error of render_tile. */
 int rt_gpu_render_view(rt_gpu_ctx* ctx, const rt_render_params* params, const rt_camera* camera);
+
+/* ---- adaptive sampling -------------------------------------------------------------------------
+ * accuBuffer keeps a sample count per pixel (RayTracerProgram.cpp:57-71), so pixels may hold different numbers of passes.
+ * These calls let a driver spend passes where a pixel's error estimate is high.  A pixel's samples are keyed by
+ * (seed, pixel, pass) (include/rt_rng.h), so a pixel that a masked call renders for passes [b, b + k) receives exactly
+ * the samples a render_tile of those passes gives it.
+ *
+ * rt_gpu_track_moments: on != 0 turns tracking on for the current frame slot: it allocates a width*height float4 moment
+ * buffer for the slot (the first time) and zeroes it, stream-ordered (every call with on != 0 zeroes it).  Without a
+ * frame yet, the buffer comes with the frame.  While tracking is on, the fold of every RT_MODE_PATH and RT_MODE_WHITTED
+ * render on the slot (render_tile, render_view, render_masked) also updates the buffer, per pixel and pass with the
+ * pass colour x that the fold adds to sum (antialiased: the /4 average), channels r, g, b, in fp32 with one rounding per
+ * operation in this order: n = Num before the pass, s0 the sum before and s1 = s0 + x the fold's own sum after it;
+ * if n > 0, M2 += (x - s0 / (float)n) * (x - s1 / (float)(n + 1)); .w += 1 (the passes the moments cover).  PREVIEW and
+ * PRIMARY leave it alone, as they leave accuBuffer.  rt_gpu_reset_accum zeroes it while tracking is on, a frame resize
+ * reallocates it (zeroed), and it is read back with RT_READ_MOMENTS_F32.  on == 0 stops the updates and keeps the buffer.
+ * With tracking off, renders run exactly the code they ran before. */
+int rt_gpu_track_moments(rt_gpu_ctx* ctx, int32_t on);
+
+/* render_tile (camera == NULL) or render_view (camera != NULL) restricted to a mask: a pixel is rendered iff it is inside
+ * [start, end], owned under the tile fields, and mask[pixel] != 0.  `mask`: DEVICE memory of the context's GPU,
+ * width*height bytes, read after everything enqueued on `stream` (a cudaStream_t; NULL = the current frame slot's stream)
+ * before the call; work enqueued on `stream` after the call runs after the mask has been read (so the caller may free
+ * or overwrite it in that stream's order), not after the render.  The work runs on the slot's stream like render_tile's, and every other rule of render_tile applies
+ * unchanged: modes, passes, pass chunks, pipes, frame slot, counters (camera_rays counts the rendered pixels x passes x
+ * rays per pass), last_render_ms and kernel-class timing, errors.  The pixels not rendered keep every frame buffer as it
+ * was.  The mask is compacted on the device into a per-slot list of pixels in 8x4-block order (no host read), and the
+ * grids stay those of the whole task.  RT_ERR_INVALID, with nothing enqueued, for a NULL mask, a mask that is not device
+ * memory of the context's GPU, and every error of render_tile / render_view. */
+int rt_gpu_render_masked(rt_gpu_ctx* ctx, const rt_render_params* params, const rt_camera* camera, const uint8_t* mask,
+                         void* stream);
+
+typedef struct rt_select_params {
+    int32_t min_passes;     /* >= 2: pixels with fewer passes are selected */
+    int32_t max_passes;     /* >= min_passes: pixels with this many passes or more are never selected */
+    float abs_tol;          /* finite, >= 0 */
+    float rel_tol;          /* finite, >= 0: tolerance relative to the pixel's mean luminance */
+} rt_select_params;
+
+/* The pixels of `region` (its frame size, which must equal the current frame slot's, [start, end] and tile fields) whose
+ * error estimate calls for more passes.  With n = Num and m the slot's moments, mask[pixel] = 1 iff the pixel is in the
+ * region, n < max_passes, and one of: n < min_passes; m.w != n (the moments do not cover every pass: error unknown);
+ * se_c > abs_tol + rel_tol * Y for some channel c, where, in fp32 with one rounding per operation,
+ * se_c = sqrtf((M2_c / (float)(n - 1)) / (float)n), Y = (0.2126f*mean_r + 0.7152f*mean_g) + 0.0722f*mean_b and
+ * mean_c = sum_c / (float)n.  A comparison with NaN is false, so a NaN estimate or tolerance selects nothing.  Every other
+ * pixel gets 0.  *count (DEVICE int32) = the number of ones.  `mask`: DEVICE, width*height bytes.  The inputs are read on
+ * the slot's stream after its earlier work, and after everything enqueued on `stream` (NULL = the slot's stream) before
+ * the call; the outputs are complete for work enqueued on `stream` after it.  RT_ERR_INVALID, with nothing enqueued, for
+ * min_passes < 2 or max_passes < min_passes, a non-finite or negative tolerance, a slot on which tracking has never been
+ * on, a region that does not match the frame (size, range, tile fields), and NULL, misaligned or non-device pointers. */
+int rt_gpu_select_pixels(rt_gpu_ctx* ctx, const rt_render_params* region, const rt_select_params* s, uint8_t* mask,
+                         int32_t* count, void* stream);
 
 /* ---- ray queries on device memory -------------------------------------------------------------
  * Batches of the caller's own rays through the same wavefront kernels as render_tile (generate -> packet /

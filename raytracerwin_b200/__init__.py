@@ -14,11 +14,12 @@ import numpy as np
 
 from . import _abi
 from ._abi import (rt_render_params, rt_counters, rt_scene_desc, rt_ray_query, rt_radiance_query, rt_mesh_update,  # noqa: F401
-                   rt_mesh_replace, rt_camera, rt_texture_update, rt_material, rt_light,
+                   rt_mesh_replace, rt_camera, rt_texture_update, rt_material, rt_light, rt_select_params,
                    RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY, RT_QUERY_NEAREST, RT_QUERY_ANY,
                    RT_TRAVERSE_EXACT, RT_TRAVERSE_CULLED,
                    RT_READ_ACCUM_RGBN_F32, RT_READ_DISPLAY_ARGB8, RT_READ_PRIMARY_IDS_I32X2,
-                   RT_READ_PRIMARY_DIST_F32, RT_READ_COUNTERS_U64, RT_READ_PREVIEW_RGBA_F32)
+                   RT_READ_PRIMARY_DIST_F32, RT_READ_COUNTERS_U64, RT_READ_PREVIEW_RGBA_F32, RT_READ_MOMENTS_F32)
+from . import tiles
 
 _lib = None
 
@@ -298,15 +299,81 @@ class GpuContext:
     def reset_counters(self):
         self._check(self._lib.rt_gpu_reset_counters(self._h))
 
-    def render_tile(self, params, camera=None):
+    def render_tile(self, params, camera=None, mask=None):
         """Enqueues one render task (rt_gpu_render_tile); with an rt_camera (look_at, camera) its camera rays are that
-        camera's (rt_gpu_render_view)."""
+        camera's (rt_gpu_render_view).  With `mask`, a contiguous uint8 (height, width) torch tensor on cuda:<self.device>,
+        only the task's pixels where it is nonzero are rendered (rt_gpu_render_masked).  The mask is read in
+        torch.cuda.current_stream's order: it may come from torch work on that stream without a host synchronisation,
+        and that stream's later work (freeing or overwriting the mask) runs after it has been read."""
+        if camera is not None and not isinstance(camera, rt_camera):
+            raise TypeError(f"camera must be an rt_camera (look_at, camera), not {type(camera).__name__}")
+        if mask is not None:
+            import torch
+            dev = torch.device("cuda", self.device)
+            self._device_tensor("mask", mask, torch.uint8, (params.height, params.width))
+            self._check(self._lib.rt_gpu_render_masked(self._h, C.byref(params), None if camera is None else C.byref(camera),
+                                                       mask.data_ptr(), self._torch_stream(dev)))
+            return
         if camera is None:
             self._check(self._lib.rt_gpu_render_tile(self._h, C.byref(params)))
         else:
-            if not isinstance(camera, rt_camera):
-                raise TypeError(f"camera must be an rt_camera (look_at, camera), not {type(camera).__name__}")
             self._check(self._lib.rt_gpu_render_view(self._h, C.byref(params), C.byref(camera)))
+
+    def track_moments(self, on=True):
+        """Per-pixel moments of the pass colours on the current frame slot (rt_gpu_track_moments): True zeroes them and
+        lets every later PATH / WHITTED render on the slot update them; False stops the updates.  Read them with
+        readback(RT_READ_MOMENTS_F32, ...): {M2.r, M2.g, M2.b, passes}."""
+        self._check(self._lib.rt_gpu_track_moments(self._h, 1 if on else 0))
+
+    def select_pixels(self, params, min_passes, max_passes, abs_tol, rel_tol):
+        """The pixels of the region `params` (frame size, [start, end], tiles) that need more passes by their error
+        estimate (rt_gpu_select_pixels): returns (mask uint8 (height, width), count int32 (1,)), torch tensors on
+        cuda:<self.device>, complete in torch.cuda.current_stream's order (reading count synchronises)."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        mask = torch.empty((params.height, params.width), dtype=torch.uint8, device=dev)
+        count = torch.empty(1, dtype=torch.int32, device=dev)
+        s = rt_select_params(int(min_passes), int(max_passes), float(abs_tol), float(rel_tol))
+        self._check(self._lib.rt_gpu_select_pixels(self._h, C.byref(params), C.byref(s), mask.data_ptr(), count.data_ptr(),
+                                                   self._torch_stream(dev)))
+        return mask, count
+
+    def render_adaptive(self, params, camera=None, min_passes=4, max_passes=64, passes_per_round=4, abs_tol=2e-3,
+                        rel_tol=0.02):
+        """Adaptive sampling of the region `params` (frame size, [start, end], tiles, mode, seed, ...; its pass_count is
+        not used).  Turns moment tracking on (zeroed), renders passes [pass_begin, pass_begin + min_passes) on every pixel
+        of the region, then repeats: select_pixels(min_passes, max_passes, abs_tol, rel_tol); stop when it selects no
+        pixel or the pass cursor has reached max_passes; render min(passes_per_round, max_passes - cursor) passes at the
+        cursor on the selected pixels.  The cursor is global, so every pixel holds a subset of the passes a uniform render
+        of [pass_begin, pass_begin + max_passes) gives it, each bit for bit.  Start from a reset frame: passes the frame
+        already holds are not covered by the moments, so such pixels are selected until max_passes.
+        Reading each round's count is ONE HOST SYNCHRONISATION PER ROUND.  Returns dict(rounds=masked rounds,
+        camera_rays=camera rays enqueued, passes=the final cursor relative to pass_begin)."""
+        if not (2 <= min_passes <= max_passes) or passes_per_round < 1:
+            raise ValueError("render_adaptive needs 2 <= min_passes <= max_passes and passes_per_round >= 1")
+        p = rt_render_params.from_buffer_copy(params)
+        spp = 4 if p.antialias and p.mode != RT_MODE_PRIMARY else 1
+        self.track_moments(True)
+        p.pass_count = min_passes
+        self.render_tile(p, camera)
+        if p.tile_count > 1:
+            idx = tiles.dense_index(p.width, p.height, p.tile_size, p.tile_count, p.tile_rank)
+            region = int(((idx >= p.start) & (idx <= p.end)).sum())
+        else:
+            region = max(p.end - p.start + 1, 0)
+        camera_rays, cursor, rounds = region * min_passes * spp, min_passes, 0
+        while cursor < max_passes:
+            mask, count = self.select_pixels(p, min_passes, max_passes, abs_tol, rel_tol)
+            n = int(count.item())
+            if n == 0:
+                break
+            k = min(passes_per_round, max_passes - cursor)
+            p.pass_begin, p.pass_count = params.pass_begin + cursor, k
+            self.render_tile(p, camera, mask=mask)
+            camera_rays += n * k * spp
+            cursor += k
+            rounds += 1
+        return dict(rounds=rounds, camera_rays=camera_rays, passes=cursor)
 
     def synchronize(self):
         self._check(self._lib.rt_gpu_synchronize(self._h))
@@ -354,7 +421,7 @@ class GpuContext:
         return int(self._lib.rt_gpu_launch_count(self._h))
 
     def readback(self, what, width, height, out=None):
-        if what in (RT_READ_ACCUM_RGBN_F32, RT_READ_PREVIEW_RGBA_F32):
+        if what in (RT_READ_ACCUM_RGBN_F32, RT_READ_PREVIEW_RGBA_F32, RT_READ_MOMENTS_F32):
             out = np.empty((height, width, 4), np.float32) if out is None else out
         elif what == RT_READ_DISPLAY_ARGB8:
             out = np.empty((height, width), np.uint32) if out is None else out

@@ -1,6 +1,6 @@
 // rt_context.hpp — the opaque context behind include/rt_gpu.h and the error and argument helpers every translation
 // unit of the library uses (rt_gpu.cu: lifetime / upload / render / queries / readback; rt_scene_edit.cu: scene edits;
-// rt_exchange.cu: multi-GPU tile exchange; rt_hooks.cu: test and tooling hooks; rt_bvh_build.cu: device BVH builder).
+// rt_adaptive.cu: moments, mask compaction and pixel selection; rt_exchange.cu: multi-GPU tile exchange; rt_hooks.cu: test and tooling hooks; rt_bvh_build.cu: device BVH builder).
 #pragma once
 #include "rt_wave_types.hpp"
 
@@ -12,6 +12,17 @@
 #include <new>
 #include <string>
 #include <vector>
+
+// Adaptive sampling state of one frame slot (rt_gpu_track_moments, rt_gpu_render_masked, rt_gpu_select_pixels)
+struct SlotAdaptive
+{
+    float4* moments = nullptr;                  // width*height {M2.r, M2.g, M2.b, passes}; allocated by the first track_moments(on)
+    bool track = false;                         // the folds of PATH / WHITTED renders update `moments`
+    // scratch of a masked render: the device count, the compacted work items of the mask and CUB's temporaries (only grows,
+    // stream-ordered on the slot's stream)
+    void* scratch = nullptr;
+    size_t scratch_cap = 0;
+};
 
 struct rt_gpu_ctx
 {
@@ -43,10 +54,11 @@ struct rt_gpu_ctx
     int2* prim_ids = nullptr;
     float* prim_dist = nullptr;
     float4* preview = nullptr;                  // linear colour of the last preview pass (allocated by the first RT_MODE_PREVIEW call)
+    SlotAdaptive adapt;
     unsigned long long* counters = nullptr;     // rt_counters
-    // Frame slots (rt_gpu_set_frame_slot): the members above — stream, timing events, frame size and the five
-    // frame buffers — are those of the CURRENT slot; the other slots' sets wait here.  Calls that address
-    // different slots are not ordered against each other on the device, so a driver can enqueue frame k+1
+    // Frame slots (rt_gpu_set_frame_slot): the members above — stream, timing events, frame size, the five frame
+    // buffers and the adaptive state — are those of the CURRENT slot; the other slots' sets wait here.  Calls that
+    // address different slots are not ordered against each other on the device, so a driver can enqueue frame k+1
     // while the thin last bounce rounds, the exchange and the read-back of frame k are still running.
     struct FrameSlot
     {
@@ -55,6 +67,7 @@ struct rt_gpu_ctx
         bool timed = false;
         int width = 0, height = 0;
         float4* accum = nullptr; uint32_t* display = nullptr; int2* prim_ids = nullptr; float* prim_dist = nullptr; float4* preview = nullptr;
+        SlotAdaptive adapt;
     };
     FrameSlot parked[RT_FRAME_SLOTS];
     int slot = 0;
@@ -159,6 +172,7 @@ struct rt_gpu_ctx
     void* update_scratch = nullptr;             // the builder's scratch block and the update's temporaries (only grows)
     size_t update_scratch_cap = 0;
     int* update_counts = nullptr;               // PINNED HOST: the builder's per-level read
+    cudaEvent_t order_event = nullptr;          // orders a caller's stream and the slot's stream (render_masked, select_pixels)
 };
 
 // A scene reader enqueued on `st` runs after the last published update
@@ -216,3 +230,21 @@ static inline int check_device_args(rt_gpu_ctx* ctx, const char* fn, std::initia
 // The material checks of rt_gpu_upload_scene and rt_gpu_update_materials (rt_gpu.cu; library-internal: not exported)
 __attribute__((visibility("hidden"))) int check_materials(rt_gpu_ctx* ctx, const rt_material* mats, int n, const std::string& prefix,
                                                           bool* needs_table);
+
+// Work enqueued on `to` after this runs after everything enqueued on `from` before it (no-op when they are one stream)
+static inline cudaError_t order_streams(rt_gpu_ctx* ctx, cudaStream_t from, cudaStream_t to)
+{
+    if (from == to) return cudaSuccess;
+    if (!ctx->order_event)
+    {
+        const cudaError_t e = cudaEventCreateWithFlags(&ctx->order_event, cudaEventDisableTiming);
+        if (e != cudaSuccess) return e;
+    }
+    const cudaError_t e = cudaEventRecord(ctx->order_event, from);
+    return e != cudaSuccess ? e : cudaStreamWaitEvent(to, ctx->order_event, 0);
+}
+
+// The work items of the task `a` (block << 5 | lane, in block order) whose pixel has mask[pixel] != 0, compacted into the
+// slot's scratch on the slot's stream: *list and *count are device addresses (rt_adaptive.cu; library-internal)
+__attribute__((visibility("hidden"))) int compact_mask(rt_gpu_ctx* ctx, const RenderArgs& a, const uint8_t* mask,
+                                                       const unsigned** list, const unsigned** count);

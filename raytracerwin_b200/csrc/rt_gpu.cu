@@ -155,6 +155,7 @@ static void park_slot(rt_gpu_ctx* ctx, rt_gpu_ctx::FrameSlot& f)
     f.stream = ctx->stream; f.ev0 = ctx->ev0; f.ev1 = ctx->ev1; f.timed = ctx->timed;
     f.width = ctx->width; f.height = ctx->height;
     f.accum = ctx->accum; f.display = ctx->display; f.prim_ids = ctx->prim_ids; f.prim_dist = ctx->prim_dist; f.preview = ctx->preview;
+    f.adapt = ctx->adapt;
 }
 
 static void unpark_slot(rt_gpu_ctx* ctx, const rt_gpu_ctx::FrameSlot& f)
@@ -162,6 +163,7 @@ static void unpark_slot(rt_gpu_ctx* ctx, const rt_gpu_ctx::FrameSlot& f)
     ctx->stream = f.stream; ctx->ev0 = f.ev0; ctx->ev1 = f.ev1; ctx->timed = f.timed;
     ctx->width = f.width; ctx->height = f.height;
     ctx->accum = f.accum; ctx->display = f.display; ctx->prim_ids = f.prim_ids; ctx->prim_dist = f.prim_dist; ctx->preview = f.preview;
+    ctx->adapt = f.adapt;
 }
 
 static void free_frame(rt_gpu_ctx* ctx)
@@ -169,6 +171,13 @@ static void free_frame(rt_gpu_ctx* ctx)
     cudaFree(ctx->accum); cudaFree(ctx->display); cudaFree(ctx->prim_ids); cudaFree(ctx->prim_dist); cudaFree(ctx->preview);
     ctx->accum = nullptr; ctx->display = nullptr; ctx->prim_ids = nullptr; ctx->prim_dist = nullptr; ctx->preview = nullptr;
     ctx->width = ctx->height = 0;
+}
+
+// the moment buffer and the masked-render scratch of a slot (its streams are idle)
+static void free_adaptive(SlotAdaptive& s)
+{
+    cudaFree(s.moments); cudaFree(s.scratch);
+    s = SlotAdaptive();
 }
 
 template <typename T>
@@ -185,11 +194,32 @@ static int upload(rt_gpu_ctx* ctx, const T* src, size_t count, T** out)
     return RT_OK;
 }
 
-// view: the basis of a turned camera (rt_gpu_render_view), nullptr for the reference's generator
+// view: the basis of a turned camera (rt_gpu_render_view), nullptr for the reference's generator; list: the pixels of
+// a masked render come from a.list (rt_gpu_render_masked)
+template <bool CULL, bool VIEW>
+static void launch_generate_list(int mode, unsigned grid, cudaStream_t st, const DevScene& sc, const RenderArgs& a, const WaveArgs& w,
+                                 const ViewBasis& view)
+{
+    switch (mode)
+    {
+    case RT_MODE_PATH: rt_generate_list_kernel<CULL, RT_MODE_PATH, VIEW><<<grid, 256, 0, st>>>(sc, a, w, view); break;
+    case RT_MODE_PREVIEW: rt_generate_list_kernel<CULL, RT_MODE_PREVIEW, VIEW><<<grid, 256, 0, st>>>(sc, a, w, view); break;
+    case RT_MODE_WHITTED: rt_generate_list_kernel<CULL, RT_MODE_WHITTED, VIEW><<<grid, 256, 0, st>>>(sc, a, w, view); break;
+    case RT_MODE_PRIMARY: rt_generate_list_kernel<CULL, RT_MODE_PRIMARY, VIEW><<<grid, 256, 0, st>>>(sc, a, w, view); break;
+    }
+}
+
 template <bool CULL>
 static cudaError_t launch_generate(int mode, unsigned grid, cudaStream_t st, const DevScene& sc, const RenderArgs& a, const WaveArgs& w,
-                                   const ViewBasis* view)
+                                   const ViewBasis* view, bool list)
 {
+    if (mode < RT_MODE_PATH || mode > RT_MODE_PRIMARY) return cudaErrorInvalidValue;
+    if (list)
+    {
+        if (view) launch_generate_list<CULL, true>(mode, grid, st, sc, a, w, *view);
+        else launch_generate_list<CULL, false>(mode, grid, st, sc, a, w, ViewBasis());
+        return cudaGetLastError();
+    }
     if (view)
     {
         switch (mode)
@@ -647,14 +677,16 @@ int rt_gpu_destroy(rt_gpu_ctx* ctx)
         if (ctx->scene_event_live) cudaEventSynchronize(ctx->scene_event);
         free_scene(ctx);
         free_frame(ctx);
+        free_adaptive(ctx->adapt);
         cudaFree(ctx->update_scratch);
         if (ctx->update_counts) cudaFreeHost(ctx->update_counts);
-        for (cudaEvent_t e : { ctx->scene_event, ctx->join_event }) if (e) cudaEventDestroy(e);
+        for (cudaEvent_t e : { ctx->scene_event, ctx->join_event, ctx->order_event }) if (e) cudaEventDestroy(e);
         for (int k = 0; k < RT_FRAME_SLOTS; k++)
         {
             if (k == ctx->slot) continue;
             rt_gpu_ctx::FrameSlot& f = ctx->parked[k];
             cudaFree(f.accum); cudaFree(f.display); cudaFree(f.prim_ids); cudaFree(f.prim_dist); cudaFree(f.preview);
+            free_adaptive(f.adapt);
             if (f.ev0) cudaEventDestroy(f.ev0);
             if (f.ev1) cudaEventDestroy(f.ev1);
             if (f.stream) cudaStreamDestroy(f.stream);
@@ -1081,7 +1113,8 @@ int rt_gpu_reset_accum(rt_gpu_ctx* ctx, int32_t width, int32_t height)
         if (width <= 0 || height <= 0 || (long long)width * height > 0x7fffffffLL) return fail(ctx, RT_ERR_INVALID, "bad frame size");
         RT_CUDA(cudaSetDevice(ctx->device));
         const size_t n = (size_t)width * height;
-        if (width != ctx->width || height != ctx->height)
+        const bool resized = width != ctx->width || height != ctx->height;
+        if (resized)
         {
             RT_CUDA(cudaStreamSynchronize(ctx->stream));
             free_frame(ctx);
@@ -1090,7 +1123,15 @@ int rt_gpu_reset_accum(rt_gpu_ctx* ctx, int32_t width, int32_t height)
             RT_CUDA(cudaMalloc((void**)&ctx->prim_ids, n * sizeof(int2)));
             RT_CUDA(cudaMalloc((void**)&ctx->prim_dist, n * sizeof(float)));
             ctx->width = width; ctx->height = height;
+            // the moments follow the frame size (a buffer of the old size, tracked or not, is reallocated)
+            if (ctx->adapt.moments || ctx->adapt.track)
+            {
+                cudaFree(ctx->adapt.moments); ctx->adapt.moments = nullptr;
+                RT_CUDA(cudaMalloc((void**)&ctx->adapt.moments, n * sizeof(float4)));
+            }
         }
+        if (ctx->adapt.moments && (ctx->adapt.track || resized))
+            RT_CUDA(cudaMemsetAsync(ctx->adapt.moments, 0, n * sizeof(float4), ctx->stream));
         RT_CUDA(cudaMemsetAsync(ctx->accum, 0, n * sizeof(float4), ctx->stream));
         RT_CUDA(cudaMemsetAsync(ctx->display, 0, n * sizeof(uint32_t), ctx->stream));
         RT_CUDA(cudaMemsetAsync(ctx->prim_ids, 0xff, n * sizeof(int2), ctx->stream));
@@ -1115,9 +1156,13 @@ static const char* bad_camera(const rt_camera* c)
     return nullptr;
 }
 
-// rt_gpu_render_tile and rt_gpu_render_view: cam == nullptr renders the uploaded view.  A camera replaces the eye,
-// dir_z and distance of the scene the generate kernel reads; a basis other than the identity selects its view variant.
-static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* cam)
+// rt_gpu_render_tile, rt_gpu_render_view and rt_gpu_render_masked: cam == nullptr renders the uploaded view.  A camera
+// replaces the eye, dir_z and distance of the scene the generate kernel reads; a basis other than the identity selects
+// its view variant.  masked: only the task's pixels with mask[pixel] != 0 are rendered (the mask is read after the work
+// enqueued on mask_stream before the call): they are compacted into a list that the list variants of the generate and
+// fold kernels walk.
+static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* cam, bool masked = false,
+                  const uint8_t* mask = nullptr, cudaStream_t mask_stream = nullptr)
 {
     return rt_guard(ctx, [&]() -> int {
         if (!ctx) return RT_ERR_INVALID;
@@ -1137,6 +1182,12 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
         if (p->pass_count < 0 || p->pass_begin < 0) return fail(ctx, RT_ERR_INVALID, "negative pass range");
         if (p->tile_count > 1 && (p->tile_size <= 0 || p->tile_rank < 0 || p->tile_rank >= p->tile_count))
             return fail(ctx, RT_ERR_INVALID, "bad tile ownership fields");
+        if (masked)
+        {
+            if (!mask) return fail(ctx, RT_ERR_INVALID, "rt_gpu_render_masked: mask is null");
+            const int rc = check_device_args(ctx, "rt_gpu_render_masked", { { mask, "mask", 1 } });
+            if (rc != RT_OK) return rc;
+        }
         RT_CUDA(cudaSetDevice(ctx->device));
         if (p->width != ctx->width || p->height != ctx->height)
         {
@@ -1144,6 +1195,7 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
             if (rc != RT_OK) return rc;
         }
         RT_CUDA(wait_scene(ctx, ctx->stream));
+        if (masked && mask_stream) RT_CUDA(order_streams(ctx, mask_stream, ctx->stream));
         RT_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
         ctx->timed = true;
         ctx->kev_used = 0;
@@ -1204,6 +1256,8 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
         a.counters = ctx->counters;
         a.exact = p->traverse == RT_TRAVERSE_EXACT ? 1 : 0;
         a.all_bounded = ctx->all_bounded ? 1 : 0;
+        // moments follow accuBuffer: PREVIEW and PRIMARY leave both alone
+        if (ctx->adapt.track && (p->mode == RT_MODE_PATH || p->mode == RT_MODE_WHITTED)) a.moments = ctx->adapt.moments;
         if (a.num_blocks == 0)
         {
             RT_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
@@ -1315,6 +1369,15 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
         // rounds are not coherent enough: measured slower, see DESIGN.md)
         const int packet_rounds = ctx->tune_packet_rounds >= 0 ? ctx->tune_packet_rounds : 1;
         const unsigned walk_grid = (unsigned)(ctx->num_sms * ctx->walk_blocks_per_sm);
+        // A masked render compacts the mask on the slot's stream before the pipes fork.  The grids, the chunks and the pool
+        // plan stay those of the whole task (the list's length is on the device only): threads past it idle.
+        if (masked)
+        {
+            RT_CUDA(mark(RT_KERNEL_OTHER, ctx->stream));
+            if ((rc = compact_mask(ctx, a, mask, &a.list, &a.list_count)) != RT_OK) return rc;
+            // the mask has been read: the caller's stream may reuse it from here on
+            if (mask_stream) RT_CUDA(order_streams(ctx, ctx->stream, mask_stream));
+        }
 
         // Chunks alternate between the pipes.  Each pipe renders into its own sample buffer and folds it
         // itself; the only cross-pipe order is fold(k) before fold(k+1) (AddPixel sums in pass order), so
@@ -1349,7 +1412,9 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
                 if (retries > 0) RT_CUDA(cudaMemsetAsync(pp.retry_counts, 0, RT_MAX_RETRIES * sizeof(unsigned), pp.stream));
                 // (the shape of a call for this purpose: mode and depth; chunks of a frame differ a little in size, which the
                 // threshold does not care about)
-                const unsigned long long signature = ((unsigned long long)p->mode << 8) ^ (unsigned long long)p->max_bounce ^ ((unsigned long long)(a.tiled ? a.tile_count : 1) << 16);
+                // (masked calls keep their own sizes: their rounds are as thin as their masks)
+                const unsigned long long signature = ((unsigned long long)p->mode << 8) ^ (unsigned long long)p->max_bounce ^
+                                                     ((unsigned long long)(a.tiled ? a.tile_count : 1) << 16) ^ ((unsigned long long)masked << 40);
                 // (a racy read of pinned memory the device may be updating: either batch's sizes will do)
                 const volatile unsigned* seen_counts = (pp.seen_counts && pp.seen_signature == signature && pp.seen_counts[0] != 0u) ? pp.seen_counts : nullptr;
                 for (int pass = 0; pass <= retries; pass++)
@@ -1367,8 +1432,8 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
                     RT_CUDA(mark(RT_KERNEL_OTHER, pp.stream));
                     RT_CUDA(cudaMemsetAsync(pp.round_counters, 0, (6 * RT_MAX_ROUNDS + 1) * sizeof(unsigned), pp.stream));
                     RT_CUDA(mark(RT_KERNEL_GENERATE, pp.stream));
-                    RT_CUDA(cull ? launch_generate<true>(p->mode, small_pass ? sms : gen_grid, pp.stream, gen_scene, a, w, view)
-                                 : launch_generate<false>(p->mode, small_pass ? sms : gen_grid, pp.stream, gen_scene, a, w, view));
+                    RT_CUDA(cull ? launch_generate<true>(p->mode, small_pass ? sms : gen_grid, pp.stream, gen_scene, a, w, view, masked)
+                                 : launch_generate<false>(p->mode, small_pass ? sms : gen_grid, pp.stream, gen_scene, a, w, view, masked));
                     ctx->launches++;
                     // (tooling: RT_FINISH_ROUND = k > 0 runs rounds >= k in the finishing kernel, -1 every round)
                     const int wave_rounds = ctx->tune_finish_round < 0 ? 0
@@ -1410,9 +1475,13 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
             if (p->mode != RT_MODE_PRIMARY)
             {
                 if (last_pipe >= 0 && last_pipe != pipe) RT_CUDA(cudaStreamWaitEvent(pp.stream, ctx->pipes[last_pipe].done, 0));
-                const int n = p->end - p->start + 1;
+                const unsigned n = masked ? a.num_blocks * 32u : (unsigned)(p->end - p->start + 1);
+                const unsigned fold_grid = (n + 255u) / 256u;
                 RT_CUDA(mark(RT_KERNEL_FOLD, pp.stream));
-                rt_resolve_kernel<<<(n + 255) / 256, 256, 0, pp.stream>>>(a, chunk);
+                if (masked && a.moments) rt_fold_kernel<true, true><<<fold_grid, 256, 0, pp.stream>>>(a, chunk);
+                else if (masked) rt_fold_kernel<false, true><<<fold_grid, 256, 0, pp.stream>>>(a, chunk);
+                else if (a.moments) rt_fold_kernel<true, false><<<fold_grid, 256, 0, pp.stream>>>(a, chunk);
+                else rt_resolve_kernel<<<fold_grid, 256, 0, pp.stream>>>(a, chunk);
                 RT_CUDA(cudaGetLastError());
                 ctx->launches++;
             }
@@ -1438,6 +1507,11 @@ int rt_gpu_render_tile(rt_gpu_ctx* ctx, const rt_render_params* p)
 int rt_gpu_render_view(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* camera)
 {
     return render(ctx, p, camera);
+}
+
+int rt_gpu_render_masked(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* camera, const uint8_t* mask, void* stream)
+{
+    return render(ctx, p, camera, true, mask, (cudaStream_t)stream);
 }
 
 // A batch of ray queries runs through the render's wavefront (enqueue_ray_batch): query generate, then one round per
@@ -1583,6 +1657,9 @@ int rt_gpu_readback(rt_gpu_ctx* ctx, int what, void* dst, size_t bytes)
         case RT_READ_PREVIEW_RGBA_F32:
             if (!ctx->preview) return fail(ctx, RT_ERR_NO_SCENE, "no preview pass has been rendered on this frame");
             src = ctx->preview; need = n * sizeof(float4); break;
+        case RT_READ_MOMENTS_F32:
+            if (!ctx->adapt.moments) return fail(ctx, RT_ERR_NO_SCENE, "moments have not been tracked on this frame slot (rt_gpu_track_moments)");
+            src = ctx->adapt.moments; need = n * sizeof(float4); break;
         default: return fail(ctx, RT_ERR_INVALID, "unknown readback selector");
         }
         if (what != RT_READ_COUNTERS_U64 && n == 0) return fail(ctx, RT_ERR_NO_SCENE, "no frame buffers yet (render or reset_accum first)");

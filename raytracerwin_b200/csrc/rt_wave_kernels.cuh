@@ -268,7 +268,9 @@ __device__ __forceinline__ bool shade_query(const DevScene& sc, const RenderArgs
 // hit nothing — most of them: they miss every bound and see the sky — is retired on the spot; the
 // rest become paths: pool record + an entry in the round-0 queue, compacted per warp by ballot.
 // VIEW: the camera rays of rt_gpu_render_view's turned camera (camera_ray_view), everything else unchanged.
-template <bool CULL, int MODE, bool VIEW>
+// LIST: the pixels of a masked render: thread t takes work item a.list[t] of the *a.list_count the compaction kept
+// (threads past the count idle), so "block" below is a group of 32 list entries; everything else unchanged.
+template <bool CULL, int MODE, bool VIEW, bool LIST>
 __device__ __forceinline__ void generate_items(const DevScene& sc, const RenderArgs& a, const WaveArgs& w, const ViewBasis& view)
 {
     Counters cnt = { 0, 0, 0, 0, 0, 0 };
@@ -279,7 +281,7 @@ __device__ __forceinline__ void generate_items(const DevScene& sc, const RenderA
     const unsigned stride = gridDim.x * blockDim.x;
     const bool retry = w.retry_in != nullptr;
     const unsigned nthreads_needed = retry ? (*w.retry_in_count < w.item_count ? *w.retry_in_count : w.item_count)
-                                           : a.num_blocks * 32u;
+                                           : LIST ? *a.list_count : a.num_blocks * 32u;
     if (nthreads_needed == 0) return;
     const unsigned rounded = (nthreads_needed + 31u) & ~31u;
     const int sample_count = retry ? 1 : a.num_samples;
@@ -299,7 +301,12 @@ __device__ __forceinline__ void generate_items(const DevScene& sc, const RenderA
                 lane_in_block = (int)(item & 31u);
             }
             else { bl = t >> 5; lane_in_block = (int)(t & 31u); }
-            px = block_pixel(a, bl, lane_in_block, cx, cy);
+            if (LIST)
+            {
+                const unsigned item = a.list[(bl << 5) | (unsigned)lane_in_block];
+                px = block_pixel(a, item >> 5, (int)(item & 31u), cx, cy);
+            }
+            else px = block_pixel(a, bl, lane_in_block, cx, cy);
         }
         float base_dx = 0.0f, base_dy = 0.0f;
         camera_base(a.width, a.height, cx, cy, base_dx, base_dy);
@@ -441,14 +448,22 @@ template <bool CULL, int MODE>
 __global__ void __launch_bounds__(256, RT_GEN_BLOCKS)
 rt_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w)
 {
-    generate_items<CULL, MODE, false>(sc, a, w, ViewBasis());
+    generate_items<CULL, MODE, false, false>(sc, a, w, ViewBasis());
 }
 
 template <bool CULL, int MODE>
 __global__ void __launch_bounds__(256, RT_GEN_BLOCKS)
 rt_generate_view_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, const ViewBasis view)
 {
-    generate_items<CULL, MODE, true>(sc, a, w, view);
+    generate_items<CULL, MODE, true, false>(sc, a, w, view);
+}
+
+// rt_gpu_render_masked: the generate kernels above over the compacted pixel list (VIEW: with a turned camera)
+template <bool CULL, int MODE, bool VIEW>
+__global__ void __launch_bounds__(256, RT_GEN_BLOCKS)
+rt_generate_list_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, const ViewBasis view)
+{
+    generate_items<CULL, MODE, VIEW, true>(sc, a, w, view);
 }
 
 // ---- kernel Q: generate for a batch of ray queries (rt_gpu_query_rays) ---------------------------------------------
@@ -1621,19 +1636,36 @@ rt_finish_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, int ro
 }
 
 // ---- sample fold: AccumulatePixel::AddPixel + GetGammaSpacePixel ---------------------------------------
-// (RayTracerProgram.cpp:57-71, :155-185).  One thread per pixel of the task; streaming.
-__global__ void rt_resolve_kernel(const RenderArgs a, int pass_count)
+// (RayTracerProgram.cpp:57-71, :155-185).  One thread per pixel of the task (LIST: per entry of the masked render's
+// pixel list; threads past its count idle); streaming.
+// MOMENTS (rt_gpu_track_moments): also the Welford update of the pixel's moments per pass colour x, one fp32 rounding per
+// operation: with n = Num before the pass, s0 the sum before and s1 = s0 + x after it, M2 += (x - s0 / n) * (x - s1 / (n + 1))
+// when n > 0, and .w += 1.
+template <bool MOMENTS, bool LIST>
+__device__ __forceinline__ void fold_items(const RenderArgs& a, int pass_count)
 {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    const int pixel = a.start + idx;
-    if (pixel > a.end) return;
-    const int x = pixel % a.width, y = pixel / a.width;
-    if (!owns_pixel(a, x, y)) return;
+    int pixel;
+    if (LIST)
+    {
+        if ((unsigned)idx >= *a.list_count) return;
+        const unsigned item = a.list[idx];
+        int x, y;
+        pixel = block_pixel(a, item >> 5, (int)(item & 31u), x, y);
+    }
+    else
+    {
+        pixel = a.start + idx;
+        if (pixel > a.end) return;
+        const int x = pixel % a.width, y = pixel / a.width;
+        if (!owns_pixel(a, x, y)) return;
+    }
     const size_t stride = (size_t)a.width * a.height;
     float4 acc = a.accum[pixel];
     float3 sum = V3(acc.x, acc.y, acc.z);
     int num = (int)acc.w;
     float3 last = V3(0, 0, 0);
+    float4 mom = MOMENTS ? a.moments[pixel] : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
     for (int p = 0; p < pass_count; p++)
     {
         float3 col;
@@ -1658,7 +1690,20 @@ __global__ void rt_resolve_kernel(const RenderArgs a, int pass_count)
             const float4 s = a.samples[(size_t)p * stride + pixel];
             col = V3(s.x, s.y, s.z);
         }
-        sum = add3(sum, col); num++;
+        const float3 before = sum;
+        sum = add3(sum, col);
+        if (MOMENTS)
+        {
+            if (num > 0)
+            {
+                const float n0 = (float)num, n1 = (float)(num + 1);
+                mom.x = mom.x + (col.x - before.x / n0) * (col.x - sum.x / n1);
+                mom.y = mom.y + (col.y - before.y / n0) * (col.y - sum.y / n1);
+                mom.z = mom.z + (col.z - before.z / n0) * (col.z - sum.z / n1);
+            }
+            mom.w = mom.w + 1.0f;
+        }
+        num++;
         last = col;
     }
     if (a.mode == RT_MODE_PREVIEW)
@@ -1669,8 +1714,21 @@ __global__ void rt_resolve_kernel(const RenderArgs a, int pass_count)
         return;
     }
     a.accum[pixel] = make_float4(sum.x, sum.y, sum.z, (float)num);
+    if (MOMENTS) a.moments[pixel] = mom;
     const float fn = (float)num;
     a.display[pixel] = make_pixel(V3(sum.x / fn, sum.y / fn, sum.z / fn));
+}
+
+__global__ void rt_resolve_kernel(const RenderArgs a, int pass_count)
+{
+    fold_items<false, false>(a, pass_count);
+}
+
+// the fold of a render that tracks moments (MOMENTS) or renders a pixel list (LIST); <false, false> is rt_resolve_kernel
+template <bool MOMENTS, bool LIST>
+__global__ void rt_fold_kernel(const RenderArgs a, int pass_count)
+{
+    fold_items<MOMENTS, LIST>(a, pass_count);
 }
 
 __global__ void rt_display_kernel(const float4* accum, uint32_t* display, int n)

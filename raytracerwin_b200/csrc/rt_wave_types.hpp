@@ -51,6 +51,11 @@ struct RenderArgs
     uint32_t q_stream_base;
     uint32_t q_sample;
     uint32_t q_first_draw;
+    // masked renders (rt_gpu_render_masked): the task's work items (block << 5 | lane) whose pixel the mask selects, in
+    // block order, and their number (device memory, written by the compaction on the slot's stream)
+    const unsigned* list;
+    const unsigned* list_count;
+    float4* moments;            // rt_gpu_track_moments: {M2.rgb, passes} per pixel, updated by the folds of the *_moments variants
 };
 
 // Internal modes of the wavefront kernels next to the RT_MODE_* of the ABI: a batch of ray queries.  A completed
