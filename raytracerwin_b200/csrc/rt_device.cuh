@@ -675,22 +675,42 @@ __device__ __forceinline__ int trace_scene(const DevScene& sc, const Ray& in, bo
 // ---- materials ----------------------------------------------------------------------------------------
 struct Bounce { float3 att, emi; };                                        // ViewRayBounceResult
 
+// What the material code reads of the scene.  It travels by value: the Combine interpreter (material_eval) is a real
+// call, and an object passed to a call by reference lives in local memory — a `const DevScene&` would make every
+// thread of the shade kernel copy the whole scene parameter to its stack, before even an empty launch returns.
+struct MaterialEnv
+{
+    const rt_material* materials;
+    const float4* unit_vectors;
+    uint32_t num_unit_vectors;
+    float bounce_offset;
+};
+__device__ __forceinline__ MaterialEnv material_env(const DevScene& sc)
+{
+    MaterialEnv e; e.materials = sc.materials; e.unit_vectors = sc.unit_vectors;
+    e.num_unit_vectors = sc.num_unit_vectors; e.bounce_offset = sc.bounce_offset;
+    return e;
+}
+
 // RMath::RandomUnitVector, Math.h:34-40.  sinf/cosf/acosf are CUDA's, not glibc's: results may
 // differ from the CPU in the last ulp (the only non-bit-exact arithmetic on the path).
+// t1 is in [0, 2 PI] and t2 in [0, PI]: told so, the compiler drops sinf/cosf's huge-argument reduction, whose
+// scratch array would otherwise take local memory in the shade kernel (the results are the same).
 __device__ __forceinline__ float3 random_unit_vector(Rng& rng)
 {
     float t1 = 2.0f * RT_PI_REF * rng_random(rng);
     float t2 = acosf(1.0f - 2.0f * rng_random(rng));
+    __builtin_assume(fabsf(t1) <= 7.0f && fabsf(t2) <= 7.0f);
     float sin_t2 = sinf(t2);
     return V3(sinf(t1) * sin_t2, cosf(t1) * sin_t2, cosf(t2));
 }
 
 // RMath::RandomHemisphereDirection, Math.cpp:42-54, table index drawn from the counter RNG
 // (the reference's shared cursor, Math.cpp:33-40, is replaced on both sides; see include/rt_rng.h)
-__device__ __forceinline__ float3 random_hemisphere(const DevScene& sc, float3 n, Rng& rng)
+__device__ __forceinline__ float3 random_hemisphere(MaterialEnv env, float3 n, Rng& rng)
 {
-    uint32_t idx = (uint32_t)rng_rand(rng) % sc.num_unit_vectors;
-    float3 v = xyz(__ldg(sc.unit_vectors + idx));
+    uint32_t idx = (uint32_t)rng_rand(rng) % env.num_unit_vectors;
+    float3 v = xyz(__ldg(env.unit_vectors + idx));
     if (dot3(v, n) > 0.0f) return v;
     return reflect3(v, n);
 }
@@ -708,7 +728,7 @@ __device__ __forceinline__ bool checker_bright(float3 p, float recip)
 
 // One leaf material: BounceViewRay (preview == false) or PreviewColor (preview == true, colour
 // returned in .att).  SurfaceMaterials.cpp:20-38,53-64,98-125,132-143,179-192.
-__device__ __forceinline__ Bounce material_leaf(const DevScene& sc, const rt_material& m, bool preview,
+__device__ __forceinline__ Bounce material_leaf(MaterialEnv env, const rt_material& m, bool preview,
                                                 const Ray& in, const Hit& h, Ray& out, Rng& rng)
 {
     Bounce r; r.att = V3(0, 0, 0); r.emi = V3(0, 0, 0);
@@ -724,8 +744,8 @@ __device__ __forceinline__ Bounce material_leaf(const DevScene& sc, const rt_mat
             return r;
         }
         float remaining = in.dist - h.dist;
-        float3 dir = random_hemisphere(sc, h.nrm, rng);
-        out.o = add3(h.pos, mulf3(dir, sc.bounce_offset)); out.d = dir; out.dist = remaining;
+        float3 dir = random_hemisphere(env, h.nrm, rng);
+        out.o = add3(h.pos, mulf3(dir, env.bounce_offset)); out.d = dir; out.dist = remaining;
         float dp = max_ref(0.0f, dot3(h.nrm, dir));
         r.att = mulf3(rgb, dp);
         if (m.type == RT_MAT_CHECKER) r.att = mulf3(r.att, factor);
@@ -740,7 +760,7 @@ __device__ __forceinline__ Bounce material_leaf(const DevScene& sc, const rt_mat
             nd = add3(nd, mulf3(random_unit_vector(rng), m.scalar));
             nd = normalized3(nd);
         }
-        out.o = add3(h.pos, mulf3(nd, sc.bounce_offset)); out.d = nd; out.dist = remaining;
+        out.o = add3(h.pos, mulf3(nd, env.bounce_offset)); out.d = nd; out.dist = remaining;
         r.att = rgb;
     }
     else if (m.type == RT_MAT_EMISSIVE)
@@ -753,7 +773,7 @@ __device__ __forceinline__ Bounce material_leaf(const DevScene& sc, const rt_mat
     {
         if (preview) return r;
         float remaining = in.dist - h.dist;
-        out.o = add3(h.pos, mulf3(in.d, sc.bounce_offset)); out.d = in.d; out.dist = remaining;
+        out.o = add3(h.pos, mulf3(in.d, env.bounce_offset)); out.d = in.d; out.dist = remaining;
         r.att = V3(1, 1, 1);
     }
     return r;
@@ -763,14 +783,19 @@ __device__ __forceinline__ Bounce material_leaf(const DevScene& sc, const rt_mat
 // and evaluates one child (SurfaceMaterials.cpp:153-161).  Combine evaluates B, then A — the
 // order the compiled reference uses for `A->Bounce(..) + B->Bounce(..)` (:169-177; pinned by
 // tests/test_oracle_vs_ref.py) — so the outgoing ray and the later RNG draws are A's.
-static __device__ __noinline__ Bounce material_eval(const DevScene& sc, int root, bool preview,
-                                             const Ray& in, const Hit& h, Ray& out, Rng& rng)
+// This generic walk holds RT_MAX_MATERIAL_DEPTH Combine frames in local memory, so it is a call of its own, entered
+// only at a Combine node (see material_bounce).  Everything it reads comes by value and everything it writes goes back
+// in the result, so the caller keeps its state in registers.  The outgoing ray starts as `in`: only preview leaves
+// leave it unwritten, and preview reads no outgoing ray.
+struct MaterialResult { Bounce b; Ray out; uint32_t rng_n; };
+static __device__ __noinline__ MaterialResult material_eval(MaterialEnv env, int root, bool preview, Ray in, Hit h, Rng rng)
 {
     int frame_node[RT_MAX_MATERIAL_DEPTH];
     Bounce frame_b[RT_MAX_MATERIAL_DEPTH];
     bool frame_second[RT_MAX_MATERIAL_DEPTH];
     int top = 0;
     int node = root;
+    Ray out = in;
     Bounce r;
     for (;;)
     {
@@ -778,7 +803,7 @@ static __device__ __noinline__ Bounce material_eval(const DevScene& sc, int root
         r.att = V3(0, 0, 0); r.emi = V3(0, 0, 0);
         while (node >= 0)
         {
-            const rt_material m = sc.materials[node];
+            const rt_material m = env.materials[node];
             if (m.type == RT_MAT_BLEND)
             {
                 node = rng_random(rng) > m.scalar ? m.child_a : m.child_b;
@@ -790,7 +815,7 @@ static __device__ __noinline__ Bounce material_eval(const DevScene& sc, int root
                 node = m.child_b;
                 continue;
             }
-            r = material_leaf(sc, m, preview, in, h, out, rng);
+            r = material_leaf(env, m, preview, in, h, out, rng);
             break;
         }
         // ascend through finished Combine frames
@@ -801,7 +826,7 @@ static __device__ __noinline__ Bounce material_eval(const DevScene& sc, int root
             {
                 frame_b[top - 1] = r;
                 frame_second[top - 1] = true;
-                node = sc.materials[frame_node[top - 1]].child_a;
+                node = env.materials[frame_node[top - 1]].child_a;
                 descend = true;
                 break;
             }
@@ -810,8 +835,40 @@ static __device__ __noinline__ Bounce material_eval(const DevScene& sc, int root
             r.emi = add3(r.emi, b.emi);
             top--;
         }
-        if (!descend) return r;
+        if (!descend)
+        {
+            MaterialResult res; res.b = r; res.out = out; res.rng_n = rng.n;
+            return res;
+        }
     }
+}
+
+// The same evaluation, in the caller's registers up to the first Combine node: the Blend nodes above it are walked
+// here with the same draws in the same order (a Blend-only prefix holds no Combine frame), a leaf is evaluated on the
+// spot, and only a Combine hands its subtree to material_eval.  Decided per node at run time, so materials changed on
+// the device (rt_gpu_update_materials) need no extra state.
+__device__ __forceinline__ Bounce material_bounce(const DevScene& sc, int node, bool preview,
+                                                  const Ray& in, const Hit& h, Ray& out, Rng& rng)
+{
+    const MaterialEnv env = material_env(sc);
+    while (node >= 0)
+    {
+        const rt_material m = env.materials[node];
+        if (m.type == RT_MAT_BLEND)
+        {
+            node = rng_random(rng) > m.scalar ? m.child_a : m.child_b;
+            continue;
+        }
+        if (m.type == RT_MAT_COMBINE)
+        {
+            const MaterialResult res = material_eval(env, node, preview, in, h, rng);
+            out = res.out; rng.n = res.rng_n;
+            return res.b;
+        }
+        return material_leaf(env, m, preview, in, h, out, rng);
+    }
+    Bounce r; r.att = V3(0, 0, 0); r.emi = V3(0, 0, 0);
+    return r;
 }
 
 __device__ __forceinline__ bool is_non_zero(float3 a) { return !eq_zero(a.x) && !eq_zero(a.y) && !eq_zero(a.z); }   // RVector.h:142-145

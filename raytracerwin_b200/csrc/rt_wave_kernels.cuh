@@ -202,7 +202,7 @@ __device__ __forceinline__ bool shade_query(const DevScene& sc, const RenderArgs
             if (mat >= 0)
             {
                 Ray unused = in;
-                const Bounce b = material_eval(sc, mat, true, in, q.h, unused, s.rng);
+                const Bounce b = material_bounce(sc, mat, true, in, q.h, unused, s.rng);
                 L = add3(L, mul3(b.att, q.h.color));
             }
             done = true;
@@ -210,7 +210,7 @@ __device__ __forceinline__ bool shade_query(const DevScene& sc, const RenderArgs
         else if (mat < 0) done = true;
         else
         {
-            const Bounce b = material_eval(sc, mat, false, in, q.h, next, s.rng);
+            const Bounce b = material_bounce(sc, mat, false, in, q.h, next, s.rng);
             if (rng_random(s.rng) <= q.h.alpha)
             {
                 if (is_non_zero(b.att))
