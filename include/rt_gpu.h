@@ -28,6 +28,8 @@
  *   rt_gpu_track_moments     per-pixel moments of the pass colours (the error estimate of each pixel of a frame slot),
  *   rt_gpu_select_pixels     the pixels whose estimate is above a tolerance, as a device mask, and
  *   rt_gpu_render_masked     render_tile restricted to a device pixel mask: adaptive sampling
+ *   rt_gpu_denoise           an edge-avoiding a-trous filter of a frame slot's mean colour, guided by the first-hit ids,
+ *                            distances and normals of an RT_MODE_GUIDES render, into the caller's device memory
  *
  * Plain C: POD structs, pointers and sizes only.  No C++/STL/torch types cross the boundary.
  * Every entry returns 0 on success or a negative rt_status; rt_gpu_last_error() gives text.
@@ -168,7 +170,13 @@ enum {
     RT_MODE_PATH = 0,       /* RayTracerScene::RayTrace, RenderOption.UseBaseColor=false */
     RT_MODE_PREVIEW = 1,    /* RenderOption.UseBaseColor=true (RayTracerScene.cpp:54-61) */
     RT_MODE_WHITTED = 2,    /* primary hit + CalculateLightColor per light (RayTracerScene.cpp:127-175) */
-    RT_MODE_PRIMARY = 3     /* nearest hit only: ids + distance, no shading */
+    RT_MODE_PRIMARY = 3,    /* nearest hit only: ids + distance, no shading */
+    RT_MODE_GUIDES = 4      /* RT_MODE_PRIMARY plus the HitNormal of the nearest hit, the guides of rt_gpu_denoise: one
+                               un-jittered camera ray per pixel (antialias and pass_count are ignored), ids and distance
+                               written exactly as RT_MODE_PRIMARY writes them, and {HitNormal.xyz, 0} (zeros on a miss)
+                               into the frame slot's guide buffer (RT_READ_GUIDE_NORMAL_F32).  The buffer is allocated
+                               (zeroed) by the slot's first GUIDES call and reallocated with the frame; accuBuffer,
+                               bitcolor, the preview colour and the moments are left alone. */
 };
 
 enum {
@@ -202,8 +210,10 @@ enum {
     RT_READ_COUNTERS_U64 = 4,     /* rt_counters */
     RT_READ_PREVIEW_RGBA_F32 = 5, /* width*height x float4: the linear colour c of the last RT_MODE_PREVIEW pass, the value the
                                      reference hands to LinearToGamma before it stores bitcolor (RayTracerProgram.cpp:175-180) */
-    RT_READ_MOMENTS_F32 = 6       /* width*height x float4 {M2.r, M2.g, M2.b, passes}: the moments of rt_gpu_track_moments
+    RT_READ_MOMENTS_F32 = 6,      /* width*height x float4 {M2.r, M2.g, M2.b, passes}: the moments of rt_gpu_track_moments
                                      (RT_ERR_NO_SCENE if tracking has never been on for the frame slot) */
+    RT_READ_GUIDE_NORMAL_F32 = 7  /* width*height x float4 {HitNormal.xyz, 0} of the last RT_MODE_GUIDES render (RT_ERR_NO_SCENE
+                                     if the frame slot has none) */
 };
 
 typedef struct rt_counters {
@@ -246,6 +256,8 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* scene);
 #define RT_GPU_FRAME_SLOTS 4
 int rt_gpu_set_frame_slot(rt_gpu_ctx* ctx, int32_t slot);
 int rt_gpu_get_frame_slot(rt_gpu_ctx* ctx);
+/* The frame size of the current frame slot (0 x 0 before its first reset_accum or render); either pointer may be NULL. */
+int rt_gpu_frame_size(rt_gpu_ctx* ctx, int32_t* width, int32_t* height);
 
 /* (Re)allocates width*height accumulation/display/primary buffers and zeroes them. */
 int rt_gpu_reset_accum(rt_gpu_ctx* ctx, int32_t width, int32_t height);
@@ -332,6 +344,52 @@ typedef struct rt_select_params {
  * on, a region that does not match the frame (size, range, tile fields), and NULL, misaligned or non-device pointers. */
 int rt_gpu_select_pixels(rt_gpu_ctx* ctx, const rt_render_params* region, const rt_select_params* s, uint8_t* mask,
                          int32_t* count, void* stream);
+
+/* ---- denoising ------------------------------------------------------------------------------------
+ * An edge-avoiding a-trous wavelet filter (Dammertz et al. 2010) of the current frame slot's mean colour, guided by the
+ * first hit of an RT_MODE_GUIDES render (shape id, distance, normal), with a luminance weight driven by each pixel's
+ * variance carried through the levels (the spatial part of SVGF).  Defined with + - * /, sqrtf and comparisons in fp32,
+ * one rounding per operation, in the order written; Y(v) = (0.2126f*v.r + 0.7152f*v.g) + 0.0722f*v.b.
+ *
+ * Level 0, per pixel p, from acc = accuBuffer, m = the moments, a = the preview colour, the slot's primary ids (shape)
+ * and distance (z) and the guide normal N:
+ *   n = (int)acc.w; c = acc.rgb / (float)n; p is VALID iff n > 0 and acc.r, acc.g, acc.b are finite.
+ *   use_albedo: d_ch = a_ch > 1e-3f ? a_ch : 1e-3f and x = c / d per channel; otherwise d = 1, x = c.
+ *   use_variance, n >= 2 and m.w == (float)n: v = (Y(m.rgb) / (float)(n - 1)) / (float)n, then v = v / (Y(d) * Y(d)) with
+ *   use_albedo; otherwise v = 0.
+ * Level k = 0 .. levels-1, step s = 2^k.  An invalid p keeps x and v.  A valid p sums over the taps q = p + s*(i, j),
+ * i, j in [-2, 2], j outer and i inner, skipping taps outside the frame, invalid taps and taps with shape_q != shape_p:
+ *   centre tap (i = j = 0): w = 0.140625f;
+ *   other taps: h = H[i+2] * H[j+2] with H = {0.0625f, 0.25f, 0.375f, 0.25f, 0.0625f};
+ *     if shape_p >= 0 (a hit): w_n = (N_p.x*N_q.x + N_p.y*N_q.y) + N_p.z*N_q.z, w_n = w_n > 0 ? w_n : 0, then
+ *       w_n = w_n * w_n normal_log2 times; w_z = 1 / (1 + |z_p - z_q| / ((sigma_depth * (float)s) * z_p));
+ *     a miss: w_n = w_z = 1;
+ *     t = |Y(x_p) - Y(x_q)| / (sigma_lum * sqrtf(v_p) + lum_floor); w_l = 1 / (1 + t*t);
+ *     w = ((h * w_n) * w_z) * w_l, and the tap is skipped unless w is finite;
+ *   W += w; X += w * x_q (per channel); V += (w * w) * v_q;  then x = X / W, v = V / (W * W).
+ * Output, per pixel: n <= 0 -> rgba = 0 and argb = 0; non-finite sums -> rgba = {c, (float)n} (the unfiltered mean);
+ * otherwise rgba = {x * d, (float)n}.  argb (if given) = LinearToGamma + MakePixelColor of rgba.rgb, the display's
+ * packing (0 for n <= 0, as bitcolor after rt_gpu_reset_accum).
+ *
+ * The guides are the slot's primary ids, distance and guide normal as last written; render RT_MODE_GUIDES over the
+ * frame (a tiled multi-GPU driver: on the root, after the frame is assembled there) before denoising.  `rgba`: DEVICE,
+ * width*height float4, 16-byte aligned; `argb`: DEVICE width*height uint32, or NULL.  The inputs are read on the slot's
+ * stream after its earlier work, and after everything enqueued on `stream` (a cudaStream_t; NULL = the slot's stream)
+ * before the call; the outputs are complete for work enqueued on `stream` after it.  No host read; no frame buffer of the
+ * slot is written.  RT_ERR_INVALID, with nothing enqueued, for: a slot without a frame or without an RT_MODE_GUIDES
+ * render since its frame was allocated; use_albedo without a preview pass on the slot; use_variance on a slot on which
+ * tracking has never been on; a parameter out of range; NULL, misaligned or non-device pointers. */
+typedef struct rt_denoise_params {
+    int32_t levels;         /* 1..6 */
+    int32_t use_albedo;     /* 0/1: demodulate by the slot's preview colour (RT_MODE_PREVIEW) */
+    int32_t use_variance;   /* 0/1: the variance of each pixel's mean from the slot's moments (rt_gpu_track_moments) */
+    int32_t normal_log2;    /* 0..8: the normal weight is the clamped dot product to the power 2^normal_log2 */
+    float sigma_lum;        /* finite, >= 0 */
+    float sigma_depth;      /* finite, > 0 */
+    float lum_floor;        /* finite, > 0 */
+} rt_denoise_params;
+
+int rt_gpu_denoise(rt_gpu_ctx* ctx, const rt_denoise_params* p, float* rgba, uint32_t* argb, void* stream);
 
 /* ---- ray queries on device memory -------------------------------------------------------------
  * Batches of the caller's own rays through the same wavefront kernels as render_tile (generate -> packet /

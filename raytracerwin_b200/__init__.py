@@ -14,11 +14,12 @@ import numpy as np
 
 from . import _abi
 from ._abi import (rt_render_params, rt_counters, rt_scene_desc, rt_ray_query, rt_radiance_query, rt_mesh_update,  # noqa: F401
-                   rt_mesh_replace, rt_camera, rt_texture_update, rt_material, rt_light, rt_select_params,
-                   RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY, RT_QUERY_NEAREST, RT_QUERY_ANY,
-                   RT_TRAVERSE_EXACT, RT_TRAVERSE_CULLED,
+                   rt_mesh_replace, rt_camera, rt_texture_update, rt_material, rt_light, rt_select_params, rt_denoise_params,
+                   RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY, RT_MODE_GUIDES, RT_QUERY_NEAREST,
+                   RT_QUERY_ANY, RT_TRAVERSE_EXACT, RT_TRAVERSE_CULLED,
                    RT_READ_ACCUM_RGBN_F32, RT_READ_DISPLAY_ARGB8, RT_READ_PRIMARY_IDS_I32X2,
-                   RT_READ_PRIMARY_DIST_F32, RT_READ_COUNTERS_U64, RT_READ_PREVIEW_RGBA_F32, RT_READ_MOMENTS_F32)
+                   RT_READ_PRIMARY_DIST_F32, RT_READ_COUNTERS_U64, RT_READ_PREVIEW_RGBA_F32, RT_READ_MOMENTS_F32,
+                   RT_READ_GUIDE_NORMAL_F32)
 from . import tiles
 
 _lib = None
@@ -324,6 +325,9 @@ class GpuContext:
         lets every later PATH / WHITTED render on the slot update them; False stops the updates.  Read them with
         readback(RT_READ_MOMENTS_F32, ...): {M2.r, M2.g, M2.b, passes}."""
         self._check(self._lib.rt_gpu_track_moments(self._h, 1 if on else 0))
+        if on:
+            # (the slot keeps its moment buffer from here on: denoise(use_variance=None) uses it)
+            self._moment_slots = getattr(self, "_moment_slots", set()) | {self._lib.rt_gpu_get_frame_slot(self._h)}
 
     def select_pixels(self, params, min_passes, max_passes, abs_tol, rel_tol):
         """The pixels of the region `params` (frame size, [start, end], tiles) that need more passes by their error
@@ -352,7 +356,7 @@ class GpuContext:
         if not (2 <= min_passes <= max_passes) or passes_per_round < 1:
             raise ValueError("render_adaptive needs 2 <= min_passes <= max_passes and passes_per_round >= 1")
         p = rt_render_params.from_buffer_copy(params)
-        spp = 4 if p.antialias and p.mode != RT_MODE_PRIMARY else 1
+        spp = 4 if p.antialias and p.mode not in (RT_MODE_PRIMARY, RT_MODE_GUIDES) else 1
         self.track_moments(True)
         p.pass_count = min_passes
         self.render_tile(p, camera)
@@ -374,6 +378,39 @@ class GpuContext:
             cursor += k
             rounds += 1
         return dict(rounds=rounds, camera_rays=camera_rays, passes=cursor)
+
+    def frame_size(self):
+        """(width, height) of the current frame slot's frame ((0, 0) before its first reset_accum or render)."""
+        w, h = C.c_int32(), C.c_int32()
+        self._check(self._lib.rt_gpu_frame_size(self._h, C.byref(w), C.byref(h)))
+        return w.value, h.value
+
+    def denoise(self, levels=5, use_albedo=False, use_variance=None, normal_log2=7, sigma_lum=4.0, sigma_depth=0.1,
+                lum_floor=0.02, out=None, argb=False):
+        """The guided a-trous denoiser (rt_gpu_denoise) on the current frame slot's frame: its mean colour, filtered
+        `levels` times with steps 1, 2, 4, ..., guided by the shape ids, distances and normals of the slot's last
+        RT_MODE_GUIDES render (render_tile(make_params(..., mode=RT_MODE_GUIDES), camera) first).  use_albedo divides by
+        the slot's preview colour (an RT_MODE_PREVIEW pass) before the filter and multiplies after it; use_variance
+        drives the luminance weight by each pixel's variance from the slot's moments (track_moments; None: if the slot
+        has them).  The formula is in include/rt_gpu.h.
+        Enqueued on torch.cuda.current_stream(self.device), after that stream's earlier work; returns at once.  Returns
+        the float32 (H, W, 4) tensor {r, g, b, passes} (`out` if given: contiguous float32 (H, W, 4) on the same device),
+        and with argb=True also the uint32 pixels (H, W) as int32 (the display's gamma and packing)."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        w, h = self.frame_size()
+        if out is None:
+            out = torch.empty((h, w, 4), dtype=torch.float32, device=dev)
+        else:
+            self._device_tensor("out", out, torch.float32, (h, w, 4))
+        pix = torch.empty((h, w), dtype=torch.int32, device=dev) if argb else None
+        if use_variance is None:
+            use_variance = self._lib.rt_gpu_get_frame_slot(self._h) in getattr(self, "_moment_slots", ())
+        p = rt_denoise_params(int(levels), 1 if use_albedo else 0, 1 if use_variance else 0, int(normal_log2),
+                              float(sigma_lum), float(sigma_depth), float(lum_floor))
+        self._check(self._lib.rt_gpu_denoise(self._h, C.byref(p), out.data_ptr() if out.numel() else None,
+                                             None if pix is None or not pix.numel() else pix.data_ptr(), self._torch_stream(dev)))
+        return (out, pix) if argb else out
 
     def synchronize(self):
         self._check(self._lib.rt_gpu_synchronize(self._h))
@@ -421,7 +458,7 @@ class GpuContext:
         return int(self._lib.rt_gpu_launch_count(self._h))
 
     def readback(self, what, width, height, out=None):
-        if what in (RT_READ_ACCUM_RGBN_F32, RT_READ_PREVIEW_RGBA_F32, RT_READ_MOMENTS_F32):
+        if what in (RT_READ_ACCUM_RGBN_F32, RT_READ_PREVIEW_RGBA_F32, RT_READ_MOMENTS_F32, RT_READ_GUIDE_NORMAL_F32):
             out = np.empty((height, width, 4), np.float32) if out is None else out
         elif what == RT_READ_DISPLAY_ARGB8:
             out = np.empty((height, width), np.uint32) if out is None else out

@@ -11,10 +11,10 @@ RT_OK, RT_ERR_INVALID, RT_ERR_CUDA, RT_ERR_NO_SCENE, RT_ERR_SIZE, RT_ERR_NOMEM =
 RT_SHAPE_SPHERE, RT_SHAPE_PLANE, RT_SHAPE_CAPSULE, RT_SHAPE_MESH, RT_SHAPE_TRIANGLE = range(5)
 RT_MAT_DIFFUSE, RT_MAT_CHECKER, RT_MAT_REFLECTIVE, RT_MAT_EMISSIVE, RT_MAT_BLEND, RT_MAT_COMBINE, RT_MAT_NULL = range(7)
 RT_LIGHT_POINT, RT_LIGHT_DIRECTIONAL = 0, 1
-RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY = range(4)
+RT_MODE_PATH, RT_MODE_PREVIEW, RT_MODE_WHITTED, RT_MODE_PRIMARY, RT_MODE_GUIDES = range(5)
 RT_TRAVERSE_EXACT, RT_TRAVERSE_CULLED = 0, 1
 (RT_READ_ACCUM_RGBN_F32, RT_READ_DISPLAY_ARGB8, RT_READ_PRIMARY_IDS_I32X2, RT_READ_PRIMARY_DIST_F32, RT_READ_COUNTERS_U64,
- RT_READ_PREVIEW_RGBA_F32, RT_READ_MOMENTS_F32) = range(7)
+ RT_READ_PREVIEW_RGBA_F32, RT_READ_MOMENTS_F32, RT_READ_GUIDE_NORMAL_F32) = range(8)
 RT_QUERY_NEAREST, RT_QUERY_ANY = 0, 1
 RT_GPU_ABI_VERSION = 2
 RT_GPU_FRAME_SLOTS = 4
@@ -123,6 +123,11 @@ class rt_select_params(C.Structure):
     _fields_ = [("min_passes", C.c_int32), ("max_passes", C.c_int32), ("abs_tol", C.c_float), ("rel_tol", C.c_float)]
 
 
+class rt_denoise_params(C.Structure):
+    _fields_ = [("levels", C.c_int32), ("use_albedo", C.c_int32), ("use_variance", C.c_int32), ("normal_log2", C.c_int32),
+                ("sigma_lum", C.c_float), ("sigma_depth", C.c_float), ("lum_floor", C.c_float)]
+
+
 STRUCT_SIZES = {"rt_shape": 80, "rt_material": 28, "rt_bvh_node": 32, "rt_tri": 64, "rt_shade": 64,
                 "rt_light": 28, "rt_render_params": 56, "rt_counters": 72}
 
@@ -148,6 +153,8 @@ GPU_PROTOTYPES = {
     "rt_gpu_track_moments": (I, [VP, I32]),
     "rt_gpu_render_masked": (I, [VP, C.POINTER(rt_render_params), C.POINTER(rt_camera), VP, VP]),
     "rt_gpu_select_pixels": (I, [VP, C.POINTER(rt_render_params), C.POINTER(rt_select_params), VP, VP, VP]),
+    "rt_gpu_denoise": (I, [VP, C.POINTER(rt_denoise_params), VP, VP, VP]),
+    "rt_gpu_frame_size": (I, [VP, PI32, PI32]),
     "rt_gpu_readback": (I, [VP, I, VP, C.c_size_t]),
     "rt_gpu_synchronize": (I, [VP]),
     "rt_gpu_last_render_ms": (I, [VP, PF]),

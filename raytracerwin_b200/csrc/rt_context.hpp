@@ -1,6 +1,6 @@
 // rt_context.hpp — the opaque context behind include/rt_gpu.h and the error and argument helpers every translation
 // unit of the library uses (rt_gpu.cu: lifetime / upload / render / queries / readback; rt_scene_edit.cu: scene edits;
-// rt_adaptive.cu: moments, mask compaction and pixel selection; rt_exchange.cu: multi-GPU tile exchange; rt_hooks.cu: test and tooling hooks; rt_bvh_build.cu: device BVH builder).
+// rt_adaptive.cu: moments, mask compaction and pixel selection; rt_denoise.cu: the guided denoiser; rt_exchange.cu: multi-GPU tile exchange; rt_hooks.cu: test and tooling hooks; rt_bvh_build.cu: device BVH builder).
 #pragma once
 #include "rt_wave_types.hpp"
 
@@ -20,6 +20,16 @@ struct SlotAdaptive
     bool track = false;                         // the folds of PATH / WHITTED renders update `moments`
     // scratch of a masked render: the device count, the compacted work items of the mask and CUB's temporaries (only grows,
     // stream-ordered on the slot's stream)
+    void* scratch = nullptr;
+    size_t scratch_cap = 0;
+};
+
+// Denoising state of one frame slot (RT_MODE_GUIDES, rt_gpu_denoise)
+struct SlotDenoise
+{
+    float4* guide = nullptr;                    // width*height {HitNormal.xyz, 0} of the nearest hit (allocated by the first GUIDES call)
+    bool guides = false;                        // a GUIDES render has been enqueued since the frame was (re)allocated
+    // the filter's per-pixel records and ping-pong buffers (only grows, stream-ordered on the slot's stream)
     void* scratch = nullptr;
     size_t scratch_cap = 0;
 };
@@ -55,9 +65,10 @@ struct rt_gpu_ctx
     float* prim_dist = nullptr;
     float4* preview = nullptr;                  // linear colour of the last preview pass (allocated by the first RT_MODE_PREVIEW call)
     SlotAdaptive adapt;
+    SlotDenoise den;
     unsigned long long* counters = nullptr;     // rt_counters
     // Frame slots (rt_gpu_set_frame_slot): the members above — stream, timing events, frame size, the five frame
-    // buffers and the adaptive state — are those of the CURRENT slot; the other slots' sets wait here.  Calls that
+    // buffers, the adaptive and the denoising state — are those of the CURRENT slot; the other slots' sets wait here.  Calls that
     // address different slots are not ordered against each other on the device, so a driver can enqueue frame k+1
     // while the thin last bounce rounds, the exchange and the read-back of frame k are still running.
     struct FrameSlot
@@ -68,6 +79,7 @@ struct rt_gpu_ctx
         int width = 0, height = 0;
         float4* accum = nullptr; uint32_t* display = nullptr; int2* prim_ids = nullptr; float* prim_dist = nullptr; float4* preview = nullptr;
         SlotAdaptive adapt;
+        SlotDenoise den;
     };
     FrameSlot parked[RT_FRAME_SLOTS];
     int slot = 0;
@@ -172,7 +184,7 @@ struct rt_gpu_ctx
     void* update_scratch = nullptr;             // the builder's scratch block and the update's temporaries (only grows)
     size_t update_scratch_cap = 0;
     int* update_counts = nullptr;               // PINNED HOST: the builder's per-level read
-    cudaEvent_t order_event = nullptr;          // orders a caller's stream and the slot's stream (render_masked, select_pixels)
+    cudaEvent_t order_event = nullptr;          // orders a caller's stream and the slot's stream (render_masked, select_pixels, denoise)
 };
 
 // A scene reader enqueued on `st` runs after the last published update

@@ -156,6 +156,7 @@ static void park_slot(rt_gpu_ctx* ctx, rt_gpu_ctx::FrameSlot& f)
     f.width = ctx->width; f.height = ctx->height;
     f.accum = ctx->accum; f.display = ctx->display; f.prim_ids = ctx->prim_ids; f.prim_dist = ctx->prim_dist; f.preview = ctx->preview;
     f.adapt = ctx->adapt;
+    f.den = ctx->den;
 }
 
 static void unpark_slot(rt_gpu_ctx* ctx, const rt_gpu_ctx::FrameSlot& f)
@@ -164,12 +165,14 @@ static void unpark_slot(rt_gpu_ctx* ctx, const rt_gpu_ctx::FrameSlot& f)
     ctx->width = f.width; ctx->height = f.height;
     ctx->accum = f.accum; ctx->display = f.display; ctx->prim_ids = f.prim_ids; ctx->prim_dist = f.prim_dist; ctx->preview = f.preview;
     ctx->adapt = f.adapt;
+    ctx->den = f.den;
 }
 
 static void free_frame(rt_gpu_ctx* ctx)
 {
     cudaFree(ctx->accum); cudaFree(ctx->display); cudaFree(ctx->prim_ids); cudaFree(ctx->prim_dist); cudaFree(ctx->preview);
     ctx->accum = nullptr; ctx->display = nullptr; ctx->prim_ids = nullptr; ctx->prim_dist = nullptr; ctx->preview = nullptr;
+    cudaFree(ctx->den.guide); ctx->den.guide = nullptr; ctx->den.guides = false;      // the guides follow the frame size, like the preview colour
     ctx->width = ctx->height = 0;
 }
 
@@ -178,6 +181,13 @@ static void free_adaptive(SlotAdaptive& s)
 {
     cudaFree(s.moments); cudaFree(s.scratch);
     s = SlotAdaptive();
+}
+
+// the guide normals and the denoiser's scratch of a slot (its streams are idle)
+static void free_denoise(SlotDenoise& s)
+{
+    cudaFree(s.guide); cudaFree(s.scratch);
+    s = SlotDenoise();
 }
 
 template <typename T>
@@ -206,6 +216,7 @@ static void launch_generate_list(int mode, unsigned grid, cudaStream_t st, const
     case RT_MODE_PREVIEW: rt_generate_list_kernel<CULL, RT_MODE_PREVIEW, VIEW><<<grid, 256, 0, st>>>(sc, a, w, view); break;
     case RT_MODE_WHITTED: rt_generate_list_kernel<CULL, RT_MODE_WHITTED, VIEW><<<grid, 256, 0, st>>>(sc, a, w, view); break;
     case RT_MODE_PRIMARY: rt_generate_list_kernel<CULL, RT_MODE_PRIMARY, VIEW><<<grid, 256, 0, st>>>(sc, a, w, view); break;
+    case RT_MODE_GUIDES: rt_generate_list_kernel<CULL, RT_MODE_GUIDES, VIEW><<<grid, 256, 0, st>>>(sc, a, w, view); break;
     }
 }
 
@@ -213,7 +224,7 @@ template <bool CULL>
 static cudaError_t launch_generate(int mode, unsigned grid, cudaStream_t st, const DevScene& sc, const RenderArgs& a, const WaveArgs& w,
                                    const ViewBasis* view, bool list)
 {
-    if (mode < RT_MODE_PATH || mode > RT_MODE_PRIMARY) return cudaErrorInvalidValue;
+    if (mode < RT_MODE_PATH || mode > RT_MODE_GUIDES) return cudaErrorInvalidValue;
     if (list)
     {
         if (view) launch_generate_list<CULL, true>(mode, grid, st, sc, a, w, *view);
@@ -228,6 +239,7 @@ static cudaError_t launch_generate(int mode, unsigned grid, cudaStream_t st, con
         case RT_MODE_PREVIEW: rt_generate_view_kernel<CULL, RT_MODE_PREVIEW><<<grid, 256, 0, st>>>(sc, a, w, *view); break;
         case RT_MODE_WHITTED: rt_generate_view_kernel<CULL, RT_MODE_WHITTED><<<grid, 256, 0, st>>>(sc, a, w, *view); break;
         case RT_MODE_PRIMARY: rt_generate_view_kernel<CULL, RT_MODE_PRIMARY><<<grid, 256, 0, st>>>(sc, a, w, *view); break;
+        case RT_MODE_GUIDES: rt_generate_view_kernel<CULL, RT_MODE_GUIDES><<<grid, 256, 0, st>>>(sc, a, w, *view); break;
         default: return cudaErrorInvalidValue;
         }
         return cudaGetLastError();
@@ -238,6 +250,7 @@ static cudaError_t launch_generate(int mode, unsigned grid, cudaStream_t st, con
     case RT_MODE_PREVIEW: rt_generate_kernel<CULL, RT_MODE_PREVIEW><<<grid, 256, 0, st>>>(sc, a, w); break;
     case RT_MODE_WHITTED: rt_generate_kernel<CULL, RT_MODE_WHITTED><<<grid, 256, 0, st>>>(sc, a, w); break;
     case RT_MODE_PRIMARY: rt_generate_kernel<CULL, RT_MODE_PRIMARY><<<grid, 256, 0, st>>>(sc, a, w); break;
+    case RT_MODE_GUIDES: rt_generate_kernel<CULL, RT_MODE_GUIDES><<<grid, 256, 0, st>>>(sc, a, w); break;
     default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();
@@ -252,6 +265,7 @@ static cudaError_t launch_shade(int mode, unsigned grid, cudaStream_t st, const 
     case RT_MODE_PREVIEW: rt_shade_kernel<CULL, RT_MODE_PREVIEW><<<grid, 256, 0, st>>>(sc, a, w, round); break;
     case RT_MODE_WHITTED: rt_shade_kernel<CULL, RT_MODE_WHITTED><<<grid, 256, 0, st>>>(sc, a, w, round); break;
     case RT_MODE_PRIMARY: rt_shade_kernel<CULL, RT_MODE_PRIMARY><<<grid, 256, 0, st>>>(sc, a, w, round); break;
+    case RT_MODE_GUIDES: rt_shade_kernel<CULL, RT_MODE_GUIDES><<<grid, 256, 0, st>>>(sc, a, w, round); break;
     case RT_QMODE_NEAREST: rt_shade_kernel<CULL, RT_QMODE_NEAREST><<<grid, 256, 0, st>>>(sc, a, w, round); break;
     case RT_QMODE_ANY: rt_shade_kernel<CULL, RT_QMODE_ANY><<<grid, 256, 0, st>>>(sc, a, w, round); break;
     default: return cudaErrorInvalidValue;
@@ -283,6 +297,7 @@ static cudaError_t launch_finish(int mode, unsigned grid, cudaStream_t st, const
     case RT_MODE_PREVIEW: rt_finish_kernel<CULL, RT_MODE_PREVIEW><<<grid, 128, 0, st>>>(sc, a, w, round); break;
     case RT_MODE_WHITTED: rt_finish_kernel<CULL, RT_MODE_WHITTED><<<grid, 128, 0, st>>>(sc, a, w, round); break;
     case RT_MODE_PRIMARY: rt_finish_kernel<CULL, RT_MODE_PRIMARY><<<grid, 128, 0, st>>>(sc, a, w, round); break;
+    case RT_MODE_GUIDES: rt_finish_kernel<CULL, RT_MODE_GUIDES><<<grid, 128, 0, st>>>(sc, a, w, round); break;
     default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();
@@ -678,6 +693,7 @@ int rt_gpu_destroy(rt_gpu_ctx* ctx)
         free_scene(ctx);
         free_frame(ctx);
         free_adaptive(ctx->adapt);
+        free_denoise(ctx->den);
         cudaFree(ctx->update_scratch);
         if (ctx->update_counts) cudaFreeHost(ctx->update_counts);
         for (cudaEvent_t e : { ctx->scene_event, ctx->join_event, ctx->order_event }) if (e) cudaEventDestroy(e);
@@ -687,6 +703,7 @@ int rt_gpu_destroy(rt_gpu_ctx* ctx)
             rt_gpu_ctx::FrameSlot& f = ctx->parked[k];
             cudaFree(f.accum); cudaFree(f.display); cudaFree(f.prim_ids); cudaFree(f.prim_dist); cudaFree(f.preview);
             free_adaptive(f.adapt);
+            free_denoise(f.den);
             if (f.ev0) cudaEventDestroy(f.ev0);
             if (f.ev1) cudaEventDestroy(f.ev1);
             if (f.stream) cudaStreamDestroy(f.stream);
@@ -1106,6 +1123,14 @@ int rt_gpu_set_frame_slot(rt_gpu_ctx* ctx, int32_t slot)
 
 int rt_gpu_get_frame_slot(rt_gpu_ctx* ctx) { return ctx ? ctx->slot : -1; }
 
+int rt_gpu_frame_size(rt_gpu_ctx* ctx, int32_t* width, int32_t* height)
+{
+    if (!ctx) return RT_ERR_INVALID;
+    if (width) *width = ctx->width;
+    if (height) *height = ctx->height;
+    return RT_OK;
+}
+
 int rt_gpu_reset_accum(rt_gpu_ctx* ctx, int32_t width, int32_t height)
 {
     return rt_guard(ctx, [&]() -> int {
@@ -1174,7 +1199,7 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
         if (p->width <= 0 || p->height <= 0 || (long long)p->width * p->height > 0x7fffffffLL) return fail(ctx, RT_ERR_INVALID, "bad frame size");
         const int npix = p->width * p->height;
         if (p->start < 0 || p->end >= npix) return fail(ctx, RT_ERR_INVALID, "pixel range outside the frame");
-        if (p->mode < RT_MODE_PATH || p->mode > RT_MODE_PRIMARY) return fail(ctx, RT_ERR_INVALID, "unknown mode");
+        if (p->mode < RT_MODE_PATH || p->mode > RT_MODE_GUIDES) return fail(ctx, RT_ERR_INVALID, "unknown mode");
         if (p->traverse != RT_TRAVERSE_EXACT && p->traverse != RT_TRAVERSE_CULLED) return fail(ctx, RT_ERR_INVALID, "unknown traverse");
         if (p->mode == RT_MODE_PATH && ctx->needs_table && ctx->scene.num_unit_vectors == 0)
             return fail(ctx, RT_ERR_INVALID, "scene has Diffuse materials but no unit-vector table (rt_host_set_unit_vectors)");
@@ -1214,7 +1239,7 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
             ctx->cev_cls[ctx->cev_used] = cls;
             return cudaEventRecord(ctx->cev[ctx->cev_used++], st);
         };
-        if (p->end < p->start || (p->mode != RT_MODE_PRIMARY && p->pass_count == 0))
+        if (p->end < p->start || (!RT_PRIMARY_LIKE(p->mode) && p->pass_count == 0))
         {
             RT_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
             return RT_OK;                                 // empty task
@@ -1224,8 +1249,8 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
         memset(&a, 0, sizeof a);
         a.width = p->width; a.height = p->height; a.start = p->start; a.end = p->end;
         a.mode = p->mode; a.max_bounce = p->max_bounce; a.antialias = p->antialias ? 1 : 0; a.seed = p->seed;
-        a.spp = (a.antialias && p->mode != RT_MODE_PRIMARY) ? 4 : 1;
-        if (p->mode == RT_MODE_PRIMARY) a.antialias = 0;
+        a.spp = (a.antialias && !RT_PRIMARY_LIKE(p->mode)) ? 4 : 1;
+        if (RT_PRIMARY_LIKE(p->mode)) a.antialias = 0;
         a.tiled = (p->tile_count > 1 && p->tile_size > 0) ? 1 : 0;
         a.tile_size = p->tile_size; a.tile_count = p->tile_count; a.tile_rank = p->tile_rank;
         if (a.tiled)
@@ -1253,6 +1278,12 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
         }
         a.accum = ctx->accum; a.display = ctx->display; a.prim_ids = ctx->prim_ids; a.prim_dist = ctx->prim_dist;
         a.preview = ctx->preview;
+        if (p->mode == RT_MODE_GUIDES && !ctx->den.guide)
+        {
+            RT_CUDA(cudaMalloc((void**)&ctx->den.guide, (size_t)npix * sizeof(float4)));
+            RT_CUDA(cudaMemsetAsync(ctx->den.guide, 0, (size_t)npix * sizeof(float4), ctx->stream));
+        }
+        a.guide = ctx->den.guide;
         a.counters = ctx->counters;
         a.exact = p->traverse == RT_TRAVERSE_EXACT ? 1 : 0;
         a.all_bounded = ctx->all_bounded ? 1 : 0;
@@ -1274,7 +1305,7 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
         const int rounds = segments * (mesh_shapes > 0 ? mesh_shapes : 1);
         if (rounds >= RT_MAX_ROUNDS) return fail(ctx, RT_ERR_INVALID, "max_bounce x mesh shapes exceeds the round table");
 
-        const int total_passes = p->mode == RT_MODE_PRIMARY ? 1 : p->pass_count;
+        const int total_passes = RT_PRIMARY_LIKE(p->mode) ? 1 : p->pass_count;
         // sample buffer: whole frames of float4 per sample; split long calls into pass chunks
         // A call with fewer camera rays (one rank's share of a multi-GPU frame) is split in fewer, longer chunks:
         // every chunk pays its thin last rounds once, and there is less dense work to hide them behind.
@@ -1302,7 +1333,7 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
             passes_per_chunk = ((size_t)total_passes + nchunks - 1) / nchunks;
         }
         const int nchunks_total = (int)(((size_t)total_passes + passes_per_chunk - 1) / passes_per_chunk);
-        if (p->mode != RT_MODE_PRIMARY)
+        if (!RT_PRIMARY_LIKE(p->mode))
         {
             const size_t need = passes_per_chunk * (size_t)a.spp * (size_t)npix;
             for (int k = 0; k < RT_PIPES && (k < nchunks_total || ctx->slots_used); k++)
@@ -1472,7 +1503,7 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
             }
             if (retries > 0 && pp.seen_retry)
                 RT_CUDA(cudaMemcpyAsync((void*)pp.seen_retry, pp.retry_counts, RT_MAX_RETRIES * sizeof(unsigned), cudaMemcpyDeviceToHost, pp.stream));
-            if (p->mode != RT_MODE_PRIMARY)
+            if (!RT_PRIMARY_LIKE(p->mode))
             {
                 if (last_pipe >= 0 && last_pipe != pipe) RT_CUDA(cudaStreamWaitEvent(pp.stream, ctx->pipes[last_pipe].done, 0));
                 const unsigned n = masked ? a.num_blocks * 32u : (unsigned)(p->end - p->start + 1);
@@ -1494,6 +1525,7 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
             if (used[k]) RT_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->pipes[k].done, 0));
         guard.joined = true;
         ctx->pipe_cursor = (pipe_base + chunk_index) % npipes;
+        if (p->mode == RT_MODE_GUIDES) ctx->den.guides = true;
         RT_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
         return RT_OK;
     });
@@ -1660,6 +1692,9 @@ int rt_gpu_readback(rt_gpu_ctx* ctx, int what, void* dst, size_t bytes)
         case RT_READ_MOMENTS_F32:
             if (!ctx->adapt.moments) return fail(ctx, RT_ERR_NO_SCENE, "moments have not been tracked on this frame slot (rt_gpu_track_moments)");
             src = ctx->adapt.moments; need = n * sizeof(float4); break;
+        case RT_READ_GUIDE_NORMAL_F32:
+            if (!ctx->den.guide) return fail(ctx, RT_ERR_NO_SCENE, "no RT_MODE_GUIDES render has been made on this frame");
+            src = ctx->den.guide; need = n * sizeof(float4); break;
         default: return fail(ctx, RT_ERR_INVALID, "unknown readback selector");
         }
         if (what != RT_READ_COUNTERS_U64 && n == 0) return fail(ctx, RT_ERR_NO_SCENE, "no frame buffers yet (render or reset_accum first)");

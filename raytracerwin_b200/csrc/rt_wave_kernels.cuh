@@ -148,10 +148,12 @@ __device__ __forceinline__ bool shade_query(const DevScene& sc, const RenderArgs
     float3 L = V3(0, 0, 0);
     const int shape = q.hit_shape;
     Ray in; in.o = q.r.o; in.d = q.r.d; in.dist = s.seg_dist;
-    if (MODE == RT_MODE_PRIMARY)
+    if (RT_PRIMARY_LIKE(MODE))
     {
         a.prim_ids[s.pixel] = make_int2(shape, shape >= 0 ? q.tri : -1);
         a.prim_dist[s.pixel] = shape >= 0 ? q.h.dist : 0.0f;
+        if (MODE == RT_MODE_GUIDES)
+            a.guide[s.pixel] = shape >= 0 ? make_float4(q.h.nrm.x, q.h.nrm.y, q.h.nrm.z, 0.0f) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
         return false;
     }
     else if (MODE == RT_MODE_WHITTED)
@@ -335,8 +337,8 @@ __device__ __forceinline__ void generate_items(const DevScene& sc, const RenderA
                 const int sub = a.antialias ? (int)(smp & 3u) : -1;
                 s.rng.key = rt_rng_key_sample(pixel_key, (uint32_t)(a.antialias ? pass * 4 + sub : pass));
                 s.rng.n = 0;
-                const Ray cam = VIEW ? camera_ray_view(sc, view, a.width, base_dx, base_dy, MODE == RT_MODE_PRIMARY ? -1 : sub, s.rng)
-                                     : camera_ray_from_base(sc, a.width, base_dx, base_dy, MODE == RT_MODE_PRIMARY ? -1 : sub, s.rng);
+                const Ray cam = VIEW ? camera_ray_view(sc, view, a.width, base_dx, base_dy, RT_PRIMARY_LIKE(MODE) ? -1 : sub, s.rng)
+                                     : camera_ray_from_base(sc, a.width, base_dx, base_dy, RT_PRIMARY_LIKE(MODE) ? -1 : sub, s.rng);
                 cnt.camera_rays++;
                 s.depth_left = a.max_bounce; s.sp = 0; s.pass_mask = 0; s.light = 0; s.seg_dist = cam.dist;
                 s.w_pos = s.w_nrm = s.w_surface = s.w_sum = V3(0, 0, 0);
@@ -371,10 +373,11 @@ __device__ __forceinline__ void generate_items(const DevScene& sc, const RenderA
                     if (state == ST_SHADE && q.hit_shape == -1)
                     {
                         // nothing hit and no mesh to walk: RayTrace's miss branch (RayTracerScene.cpp:90-94)
-                        if (MODE == RT_MODE_PRIMARY)
+                        if (RT_PRIMARY_LIKE(MODE))
                         {
                             a.prim_ids[s.pixel] = make_int2(-1, -1);
                             a.prim_dist[s.pixel] = 0.0f;
+                            if (MODE == RT_MODE_GUIDES) a.guide[s.pixel] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
                         }
                         else if (fold_sky)
                         {

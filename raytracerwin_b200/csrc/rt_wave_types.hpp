@@ -56,12 +56,17 @@ struct RenderArgs
     const unsigned* list;
     const unsigned* list_count;
     float4* moments;            // rt_gpu_track_moments: {M2.rgb, passes} per pixel, updated by the folds of the *_moments variants
+    float4* guide;              // RT_MODE_GUIDES: {HitNormal.xyz, 0} of the nearest hit per pixel (zeros on a miss)
 };
 
 // Internal modes of the wavefront kernels next to the RT_MODE_* of the ABI: a batch of ray queries.  A completed
-// query writes its result and ends (no shading); ANY is the shadow query (pool record bit 256).
-#define RT_QMODE_NEAREST 4
-#define RT_QMODE_ANY 5
+// query writes its result and ends (no shading); ANY is the shadow query (pool record bit 256).  Values the ABI's modes
+// do not use.
+#define RT_QMODE_NEAREST 8
+#define RT_QMODE_ANY 9
+
+// The modes that trace one un-jittered camera ray per pixel and write the primary hit (no samples, no fold)
+#define RT_PRIMARY_LIKE(m) ((m) == RT_MODE_PRIMARY || (m) == RT_MODE_GUIDES)
 
 __device__ __forceinline__ bool owns_pixel(const RenderArgs& a, int x, int y)
 {
