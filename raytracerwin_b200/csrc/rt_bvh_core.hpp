@@ -33,6 +33,12 @@ __attribute__((visibility("hidden"))) int rt_bvh_build_core(rt_gpu_ctx* ctx, con
                                                             cudaStream_t st, void* scratch, int* host_counts, rt_bvh_node* nodes,
                                                             rt_tri* tris, int* out_depth);
 
+// v, with a NaN in the bits the host layer's arithmetic gives it.  Finite corners whose edge products overflow make a
+// face normal NaN (inf - inf, inf * 0): x86 writes its default NaN 0xFFC00000 and carries it through every later
+// operation, the device writes 0x7FFFFFFF.  Records written on the device take the host's bits, so that a mesh built or
+// edited here is byte for byte the host build of the same geometry.
+static __device__ __forceinline__ float rt_host_nan(float v) { return v != v ? __uint_as_float(0xFFC00000u) : v; }
+
 // The leaf record of triangle t with corners p0, p1, p2, as the host builder emits it: pads 0 and the face normal
 // exactly as RRay.cpp:138-145 computes it (cross(p1-p0, p2-p0), normalised unless |n|^2 < FLT_EPSILON).  The builder's
 // k_nodes and rt_gpu_refit_mesh both write it.
@@ -51,6 +57,6 @@ static __device__ __forceinline__ rt_tri rt_tri_record(const float* p0, const fl
         const float inv = 1.0f / sqrtf(sqr);
         nx *= inv; ny *= inv; nz *= inv;
     }
-    r.n[0] = nx; r.n[1] = ny; r.n[2] = nz; r.pad2 = 0.0f;
+    r.n[0] = rt_host_nan(nx); r.n[1] = rt_host_nan(ny); r.n[2] = rt_host_nan(nz); r.pad2 = 0.0f;
     return r;
 }

@@ -83,7 +83,7 @@ __device__ __forceinline__ void upd_corner_normals(float* dst, int t, const floa
         const float* p2 = points + 3 * (size_t)pidx[3 * (size_t)t + 2];
         const float ax = p1[0] - p0[0], ay = p1[1] - p0[1], az = p1[2] - p0[2];
         const float bx = p2[0] - p0[0], by = p2[1] - p0[1], bz = p2[2] - p0[2];
-        const float nx = ay * bz - az * by, ny = az * bx - ax * bz, nz = ax * by - ay * bx;
+        const float nx = rt_host_nan(ay * bz - az * by), ny = rt_host_nan(az * bx - ax * bz), nz = rt_host_nan(ax * by - ay * bx);
         for (int k = 0; k < 3; k++) { dst[3 * k] = nx; dst[3 * k + 1] = ny; dst[3 * k + 2] = nz; }
     }
 }
