@@ -496,12 +496,10 @@ int rt_gpu_update_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, 
  * the bits of the device check (1 = a point index out of range, 2 = a normal index out of range, 16 = a non-finite
  * point coordinate, which the upload would refuse).  The mesh's arrays,
  * the shape's bounds and the culling margin are then left as they were, and every later call returns what it returned
- * before.  Such a refit still publishes (a copy of the arrays), so, as after an update, an RT_OCTO mesh walks its binary
- * tree from then on and for mesh 0 RT_TOP_STAGE is turned off; both give the same bits.  RT_ERR_INVALID (nothing
- * enqueued) as rt_gpu_update_mesh's host-side checks, for a misaligned or non-device `status`, and for an uploaded
- * tree that is not a full binary tree over all its nodes whose leaves name every triangle slot exactly once (the host
- * layer always produces one; after an rt_gpu_update_mesh the builder's tree is one); RT_ERR_NO_SCENE before an
- * upload. */
+ * before.  RT_ERR_INVALID (nothing enqueued) as rt_gpu_update_mesh's host-side checks, for a misaligned or non-device
+ * `status`, and for an uploaded tree that is not a full binary tree over all its nodes whose leaves name every
+ * triangle slot exactly once (the host layer always produces one; after an rt_gpu_update_mesh the builder's tree is
+ * one); RT_ERR_NO_SCENE before an upload. */
 int rt_gpu_refit_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, int32_t* status, void* stream);
 
 /* A REPLACE of the mesh of mesh shape `shape`: new geometry of ANY triangle count, with its own texture coordinates and
@@ -510,7 +508,7 @@ int rt_gpu_refit_mesh(rt_gpu_ctx* ctx, int32_t shape, const rt_mesh_update* u, i
  * rt_host_add_mesh_arrays(points, normals, texcoords, point_idx, normal_idx, texcoord_idx, num_tris) with
  * rt_shade.texture of triangle t = texture[t], the mesh keeps its uploaded rt_texture slots, and the shape's bounds are
  * RAabb::Expand over all the points.  Triangle ids that queries return are the new triangle order.  Ordering, blocking
- * (the call returns once the build is complete), RT_OCTO and RT_TOP_STAGE as rt_gpu_update_mesh.  The uploaded mesh must
+ * (the call returns once the build is complete) as rt_gpu_update_mesh.  The uploaded mesh must
  * have at least one triangle; its node count and tree shape do not matter.  Afterwards the mesh is updatable and
  * refittable with the new count, and later updates and refits keep the new uv and slots.
  * Memory: the spare set is reused when it holds at least num_tris triangles, otherwise a set of num_tris is allocated
@@ -666,7 +664,7 @@ enum {
     RT_KERNEL_LONG_WALK = 3,    /* rt_longwalk_kernel */
     RT_KERNEL_SHADE = 4,        /* rt_shade_kernel */
     RT_KERNEL_FOLD = 5,         /* rt_resolve_kernel */
-    RT_KERNEL_OTHER = 6,        /* memsets, rt_finish_kernel */
+    RT_KERNEL_OTHER = 6,        /* memsets */
     RT_KERNEL_CLASSES = 7
 };
 int rt_gpu_kernel_class_ms(rt_gpu_ctx* ctx, float* ms, int32_t* launches, int32_t num_classes);

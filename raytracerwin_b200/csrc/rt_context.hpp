@@ -124,7 +124,6 @@ struct rt_gpu_ctx
     unsigned tune_window = RT_WORK_WINDOW;
     int tune_min_lanes = RT_MIN_LANES;
     int tune_leaf_wait = RT_LEAF_WAIT;
-    int tune_finish_round = RT_FINISH_ROUND;
     bool time_walks = false;                    // record an event pair around every walk launch (rt_gpu_time_kernels)
     bool time_classes = false;                  // rt_gpu_time_kernels(ctx, 2): one event before every launch, by kernel class
     std::vector<cudaEvent_t> cev;
@@ -140,9 +139,6 @@ struct rt_gpu_ctx
     unsigned tune_thin_limit = RT_THIN_LIMIT;
     int tune_thin_from_round = 0;               // RT_THIN_FROM_ROUND: 0 = by the sizes last seen (frames in flight only), k > 0 = from round k, -1 = never
     unsigned tune_thin_grid_count = RT_THIN_GRID_COUNT;   // a round that had fewer entries than this gets quarter grids
-    bool tune_octo = false;                     // RT_OCTO=1: bounce rounds of the culled traversal walk the 8-wide tree (measured slower: opt-in)
-    int octo_blocks_per_sm = 0;
-    bool tune_top_stage = false;                // RT_TOP_STAGE: the walk kernel serves the top of mesh 0's tree from shared memory
     int tune_few_chunks = 0;                    // RT_FEW_CHUNKS: pass chunks of a call of few camera rays (0: 2, or 1 with frame slots)
     size_t tune_sample_budget = 0;              // RT_SAMPLE_BUDGET_MB at create (0: by call size)
     bool tune_time_long = false;                // RT_TIME_LONG at create: timed brackets span walk + long walk

@@ -37,8 +37,6 @@ struct DevMesh
     const float4* tris;         // 4 x float4 per rt_tri: {p0, index} {p1,-} {p2,-} {n,-}
     const float4* shade;        // 4 x float4 per rt_shade, in LEAF order on the device (record k <-> tris[k]; reordered at upload)
     const DevTexture* textures;
-    const float4* octo;         // the tree collapsed to 8-wide nodes for the culled walk: 8 x {bmin.xyz, ref}{bmax.xyz, count}
-                                // per node, children in slot order, ref = child node (>= 0) or ~leaf slot (see rt_walk_octo_kernel)
     int32_t num_nodes, num_tris, num_textures;
     float cull_scale;           // largest |coordinate| of the root bounds (culling margin)
 };
@@ -55,15 +53,12 @@ struct DevScene
     int32_t num_shapes, num_materials, num_meshes, num_lights;
     float eye[3];
     float dir_z, ray_distance, bounce_offset;
-    // Top of the first mesh's tree for the walk kernel's shared-memory stage: RT_TOP_SLOTS hashed slots,
-    // top_tags[s] = node index held by slot s (or -1), top_nodes[2s..2s+1] = that node; built at upload from the
-    // shallowest levels (breadth first).  top_of = the node array they belong to (other meshes bypass the stage).
-    const int* top_tags;
-    const float4* top_nodes;
-    const float4* top_of;
+    // Unused.  Holds the record at 120 bytes, so the kernel parameters after it (RenderArgs, WaveArgs) keep their
+    // constant-bank offsets: at 96 bytes ptxas orders the pool loads of rt_shade_kernel<*, RT_MODE_PRIMARY> differently
+    // and its launch takes 10 % longer on the B200 (0.207 -> 0.228 ms, 4K PRIMARY frame of the default scene).
+    const void* reserved[3];
 };
-#define RT_TOP_SLOTS 512
-__host__ __device__ __forceinline__ unsigned top_slot(int node) { return ((unsigned)node * 0x9E3779B1u) >> 23; }
+static_assert(sizeof(DevScene) == 120, "DevScene: see `reserved`");
 
 struct Ray { float3 o, d; float dist; };                                  // RRay, RRay.h:31-37
 struct Hit { float3 pos, nrm; float dist; float3 color; float alpha; };   // RayHitResult, RRay.h:13-29

@@ -38,53 +38,6 @@ thread_local std::string g_create_error;
 __attribute__((visibility("hidden"))) int rt_ctx_device(rt_gpu_ctx* ctx) { return ctx ? ctx->device : -1; }
 __attribute__((visibility("hidden"))) void rt_ctx_set_error(rt_gpu_ctx* ctx, const char* msg) { if (ctx && msg) ctx->err = msg; }
 
-// The binary tree collapsed into nodes of up to eight children for rt_walk_octo_kernel: out holds 8 records per
-// node, {bmin, ref}{bmax, count} (count in record 0), children in pre-order = slot order; ref >= 0: child node,
-// ref < 0: ~leaf slot.  A node starts with its two children and keeps replacing the inner child with the largest
-// subtree by that child's two children until it has eight (or only leaves).
-static void build_octo(const rt_bvh_node* nodes, int n, std::vector<rt_bvh_node>& out)
-{
-    out.clear();
-    if (n <= 0) return;
-    struct Job { int binary; int slot; };           // wide node `slot` collapses the subtree of binary node `binary`
-    std::vector<Job> jobs;
-    auto new_node = [&]() { const int k = (int)(out.size() / 8); out.resize(out.size() + 8); return k; };
-    jobs.push_back(Job{ 0, new_node() });
-    while (!jobs.empty())
-    {
-        const Job j = jobs.back(); jobs.pop_back();
-        int kids[8], nk = 0;
-        if (nodes[j.binary].tri >= 0) kids[nk++] = j.binary;                 // a tree of one leaf
-        else { kids[nk++] = j.binary + 1; kids[nk++] = nodes[j.binary + 1].escape; }
-        for (;;)
-        {
-            int pick = -1, size = 1;
-            for (int c = 0; c < nk; c++)
-                if (nodes[kids[c]].tri < 0 && nodes[kids[c]].escape - kids[c] > size) { pick = c; size = nodes[kids[c]].escape - kids[c]; }
-            if (pick < 0 || nk == 8) break;
-            const int b = kids[pick];
-            for (int c = nk; c > pick + 1; c--) kids[c] = kids[c - 1];
-            kids[pick] = b + 1; kids[pick + 1] = nodes[b + 1].escape;
-            nk++;
-        }
-        for (int c = 0; c < 8; c++)
-        {
-            rt_bvh_node rec;
-            memset(&rec, 0, sizeof rec);
-            rec.escape = ~0;                                        // (unused slot: a leaf ref that is never looked at)
-            if (c < nk)
-            {
-                const rt_bvh_node& b = nodes[kids[c]];
-                for (int x = 0; x < 3; x++) { rec.bmin[x] = b.bmin[x]; rec.bmax[x] = b.bmax[x]; }
-                if (b.tri >= 0) rec.escape = ~b.tri;
-                else { const int child = new_node(); rec.escape = child; jobs.push_back(Job{ kids[c], child }); }
-            }
-            rec.tri = nk;                                           // every record carries the count; record 0's is read
-            out[(size_t)j.slot * 8 + c] = rec;
-        }
-    }
-}
-
 static inline bool texture_has_pixels(const rt_texture& t) { return t.rgba != nullptr || t.texels8 != nullptr; }
 static inline bool finite_n(const float* v, int n)
 {
@@ -288,25 +241,10 @@ static cudaError_t launch_query_generate(int mode, unsigned grid, cudaStream_t s
     return cudaGetLastError();
 }
 
-template <bool CULL>
-static cudaError_t launch_finish(int mode, unsigned grid, cudaStream_t st, const DevScene& sc, const RenderArgs& a, const WaveArgs& w, int round)
+static cudaError_t launch_walk(bool cull, unsigned grid, cudaStream_t st, const DevScene& sc, const RenderArgs& a, const WaveArgs& w, int round, int resumed)
 {
-    switch (mode)
-    {
-    case RT_MODE_PATH: rt_finish_kernel<CULL, RT_MODE_PATH><<<grid, 128, 0, st>>>(sc, a, w, round); break;
-    case RT_MODE_PREVIEW: rt_finish_kernel<CULL, RT_MODE_PREVIEW><<<grid, 128, 0, st>>>(sc, a, w, round); break;
-    case RT_MODE_WHITTED: rt_finish_kernel<CULL, RT_MODE_WHITTED><<<grid, 128, 0, st>>>(sc, a, w, round); break;
-    case RT_MODE_PRIMARY: rt_finish_kernel<CULL, RT_MODE_PRIMARY><<<grid, 128, 0, st>>>(sc, a, w, round); break;
-    case RT_MODE_GUIDES: rt_finish_kernel<CULL, RT_MODE_GUIDES><<<grid, 128, 0, st>>>(sc, a, w, round); break;
-    default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
-}
-
-static cudaError_t launch_walk(bool cull, bool top, unsigned grid, cudaStream_t st, const DevScene& sc, const RenderArgs& a, const WaveArgs& w, int round, int resumed)
-{
-    if (cull) { if (top) rt_walk_kernel<true, true><<<grid, 256, 0, st>>>(sc, a, w, round, resumed); else rt_walk_kernel<true, false><<<grid, 256, 0, st>>>(sc, a, w, round, resumed); }
-    else { if (top) rt_walk_kernel<false, true><<<grid, 256, 0, st>>>(sc, a, w, round, resumed); else rt_walk_kernel<false, false><<<grid, 256, 0, st>>>(sc, a, w, round, resumed); }
+    if (cull) rt_walk_kernel<true><<<grid, 256, 0, st>>>(sc, a, w, round, resumed);
+    else rt_walk_kernel<false><<<grid, 256, 0, st>>>(sc, a, w, round, resumed);
     return cudaGetLastError();
 }
 
@@ -325,11 +263,9 @@ static int init_walk_grid(rt_gpu_ctx* ctx)
 {
     if (ctx->walk_blocks_per_sm != 0) return RT_OK;
     int b0 = 0, b1 = 0;
-    RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b0, rt_walk_kernel<true, true>, 256, 0));
-    RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b1, rt_walk_kernel<false, true>, 256, 0));
+    RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b0, rt_walk_kernel<true>, 256, 0));
+    RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b1, rt_walk_kernel<false>, 256, 0));
     ctx->walk_blocks_per_sm = b0 < b1 ? b0 : b1;
-    RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->octo_blocks_per_sm, rt_walk_octo_kernel, 256, 0));
-    if (ctx->octo_blocks_per_sm < 1) return fail(ctx, RT_ERR_CUDA, "8-wide walk kernel does not fit on an SM");
     if (ctx->walk_blocks_per_sm < 1) return fail(ctx, RT_ERR_CUDA, "walk kernel does not fit on an SM");
     return RT_OK;
 }
@@ -437,7 +373,7 @@ struct PipeGuard
 };
 
 // One round of the wavefront on a pipe: the mesh walks of the round's queue (rounds below `packet_rounds` as packets,
-// then the walks they hand back lane by lane; later rounds lane by lane or on the 8-wide tree), the long walks parked
+// then the walks they hand back lane by lane; later rounds lane by lane), the long walks parked
 // on the way, then the shade kernel in `mode`.  small_pass / thin: the reduced grids of render_tile's retry passes
 // and of late rounds with frames in flight.  mark(class, stream) tags each launch for rt_gpu_time_kernels(ctx, 2);
 // `timed` lets the walk brackets of rt_gpu_time_kernels(ctx, 1) be recorded.
@@ -468,18 +404,12 @@ static int enqueue_round(rt_gpu_ctx* ctx, rt_gpu_ctx::Pipe& pp, const RenderArgs
             RT_CUDA(cudaGetLastError());
             ctx->launches++;
             RT_CUDA(mark(RT_KERNEL_WALK, pp.stream));
-            RT_CUDA(launch_walk(cull, ctx->tune_top_stage, small_pass ? sms : walk_grid, pp.stream, ctx->scene, a, w, round, 1));
-        }
-        else if (cull && ctx->tune_octo)
-        {
-            // bounce / shadow rounds of the culled traversal: the 8-wide tree
-            RT_CUDA(mark(RT_KERNEL_WALK, pp.stream));
-            rt_walk_octo_kernel<<<(unsigned)(ctx->num_sms * ctx->octo_blocks_per_sm), 256, 0, pp.stream>>>(ctx->scene, a, w, round);
+            RT_CUDA(launch_walk(cull, small_pass ? sms : walk_grid, pp.stream, ctx->scene, a, w, round, 1));
         }
         else
         {
             RT_CUDA(mark(RT_KERNEL_WALK, pp.stream));
-            RT_CUDA(launch_walk(cull, ctx->tune_top_stage, small_pass ? sms : (thin ? walk_grid / 4u : walk_grid), pp.stream, ctx->scene, a, w, round, 0));
+            RT_CUDA(launch_walk(cull, small_pass ? sms : (thin ? walk_grid / 4u : walk_grid), pp.stream, ctx->scene, a, w, round, 0));
         }
         RT_CUDA(cudaGetLastError());
         const bool time_long = ctx->tune_time_long;     // tooling: bracket walk + long walk
@@ -937,19 +867,6 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
             ctx->mesh_state.back().refittable = refittable[i] != 0;
             // room for min(T, (N + 1) / 2) triangles when a replace builds into this set after it has become the spare
             ctx->mesh_state.back().cur = rt_gpu_ctx::MeshArrays{ dn, dt, (rt_shade*)dsh, std::min(m.num_tris, (m.num_nodes + 1) / 2), false };
-            dm.octo = nullptr;
-            if (m.num_nodes > 0 && ctx->tune_octo)
-            {
-                std::vector<rt_bvh_node> octo;
-                build_octo(m.nodes, m.num_nodes, octo);
-                if (octo.size() / 8 < (1u << 24))
-                {
-                    rt_bvh_node* docto = nullptr;
-                    if ((rc = upload(ctx, octo.data(), octo.size(), &docto)) != RT_OK) return rc;
-                    RT_CUDA(cudaStreamSynchronize(ctx->stream));       // octo is a local
-                    dm.octo = (const float4*)docto;
-                }
-            }
             dm.num_nodes = m.num_nodes; dm.num_tris = m.num_tris; dm.num_textures = m.num_textures;
             float scale = 0.0f;
             if (m.num_nodes > 0)
@@ -1005,40 +922,6 @@ int rt_gpu_upload_scene(rt_gpu_ctx* ctx, const rt_scene_desc* s)
         DevMesh* dmeshes;
         if ((rc = upload(ctx, meshes.data(), meshes.size(), &dmeshes)) != RT_OK) return rc;
         d.meshes = dmeshes;
-        std::vector<int> top_tags(RT_TOP_SLOTS, -1);
-        std::vector<rt_bvh_node> top_nodes(RT_TOP_SLOTS);
-        if (s->num_meshes > 0 && s->meshes[0].num_nodes > 0)
-        {
-            // the shallowest levels of mesh 0, breadth first, into hashed slots (a taken slot stays with the shallower
-            // node); children of node k: k + 1 and the escape of k + 1.  The device copy keeps the right child in `tri`.
-            const rt_mesh& m0 = s->meshes[0];
-            std::vector<int> level(1, 0), next_level;
-            int placed = 0;
-            while (!level.empty() && placed < RT_TOP_SLOTS * 3 / 4)
-            {
-                next_level.clear();
-                for (int k : level)
-                {
-                    const unsigned slot = top_slot(k);
-                    if (top_tags[slot] < 0)
-                    {
-                        top_tags[slot] = k; top_nodes[slot] = m0.nodes[k]; placed++;
-                        if (m0.nodes[k].tri < 0) top_nodes[slot].tri = -2 - (k + 1 < m0.num_nodes ? m0.nodes[k + 1].escape : m0.num_nodes);
-                    }
-                    if (m0.nodes[k].tri < 0)
-                    {
-                        next_level.push_back(k + 1);
-                        const int right = m0.nodes[k + 1].escape;
-                        if (right < m0.nodes[k].escape) next_level.push_back(right);
-                    }
-                }
-                level.swap(next_level);
-            }
-            int* dtags; rt_bvh_node* dtop;
-            if ((rc = upload(ctx, top_tags.data(), top_tags.size(), &dtags)) != RT_OK) return rc;
-            if ((rc = upload(ctx, top_nodes.data(), top_nodes.size(), &dtop)) != RT_OK) return rc;
-            d.top_tags = dtags; d.top_nodes = (const float4*)dtop; d.top_of = meshes[0].nodes;
-        }
 
         if (s->num_unit_vectors > 0 && s->unit_vectors)
         {
@@ -1466,10 +1349,7 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
                     RT_CUDA(cull ? launch_generate<true>(p->mode, small_pass ? sms : gen_grid, pp.stream, gen_scene, a, w, view, masked)
                                  : launch_generate<false>(p->mode, small_pass ? sms : gen_grid, pp.stream, gen_scene, a, w, view, masked));
                     ctx->launches++;
-                    // (tooling: RT_FINISH_ROUND = k > 0 runs rounds >= k in the finishing kernel, -1 every round)
-                    const int wave_rounds = ctx->tune_finish_round < 0 ? 0
-                                          : (ctx->tune_finish_round > 0 && ctx->tune_finish_round < rounds) ? ctx->tune_finish_round : rounds;
-                    for (int round = 0; round < wave_rounds; round++)
+                    for (int round = 0; round < rounds; round++)
                     {
                         // Frames in flight: a late round holds a few thousand paths, yet its three launches would each
                         // put a full persistent grid in front of the dense kernels of the frames behind it.  The size
@@ -1490,14 +1370,6 @@ static int render(rt_gpu_ctx* ctx, const rt_render_params* p, const rt_camera* c
                         // this batch's round sizes, for the grids of the next batch on this pipe
                         RT_CUDA(cudaMemcpyAsync(pp.seen_counts, pp.round_counters, RT_SEEN_ROUNDS * sizeof(unsigned), cudaMemcpyDeviceToHost, pp.stream));
                         pp.seen_signature = signature;
-                    }
-                    if (wave_rounds < rounds)
-                    {
-                        // everything still alive after the wavefront rounds runs to its end in one launch
-                        RT_CUDA(mark(RT_KERNEL_OTHER, pp.stream));
-                        RT_CUDA(cull ? launch_finish<true>(p->mode, (unsigned)ctx->num_sms * 4u, pp.stream, ctx->scene, a, w, wave_rounds)
-                                     : launch_finish<false>(p->mode, (unsigned)ctx->num_sms * 4u, pp.stream, ctx->scene, a, w, wave_rounds));
-                        ctx->launches++;
                     }
                 }
             }
@@ -1790,7 +1662,6 @@ uint64_t rt_gpu_launch_count(rt_gpu_ctx* ctx) { return ctx ? ctx->launches : 0; 
 // experiment knobs (tools/, tests that force the long-walk path); the defaults are what ships
 static void tuning_from_env(rt_gpu_ctx* ctx)
 {
-    if (getenv("RT_FINISH_ROUND")) ctx->tune_finish_round = atoi(getenv("RT_FINISH_ROUND"));
     if (getenv("RT_LONG_LIMIT")) ctx->tune_long_limit = (unsigned)atoi(getenv("RT_LONG_LIMIT"));
     if (getenv("RT_SMALL_ROUND")) ctx->tune_small_round = (unsigned)atoi(getenv("RT_SMALL_ROUND"));
     if (getenv("RT_THIN_COUNT")) ctx->tune_thin_count = (unsigned)atoi(getenv("RT_THIN_COUNT"));
@@ -1802,8 +1673,6 @@ static void tuning_from_env(rt_gpu_ctx* ctx)
     if (getenv("RT_SAMPLE_BUDGET_MB")) ctx->tune_sample_budget = (size_t)atoi(getenv("RT_SAMPLE_BUDGET_MB")) << 20;
     ctx->tune_time_long = getenv("RT_TIME_LONG") != nullptr;
     if (getenv("RT_FEW_CHUNKS")) ctx->tune_few_chunks = atoi(getenv("RT_FEW_CHUNKS"));
-    if (getenv("RT_TOP_STAGE")) ctx->tune_top_stage = atoi(getenv("RT_TOP_STAGE")) != 0;
-    if (getenv("RT_OCTO")) ctx->tune_octo = atoi(getenv("RT_OCTO")) != 0;
     if (getenv("RT_THIN_FROM_ROUND")) ctx->tune_thin_from_round = atoi(getenv("RT_THIN_FROM_ROUND"));   // k > 0: from round k; -1: never
     if (getenv("RT_THIN_GRID_COUNT")) ctx->tune_thin_grid_count = (unsigned)atoi(getenv("RT_THIN_GRID_COUNT"));
 }

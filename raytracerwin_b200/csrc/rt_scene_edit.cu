@@ -165,10 +165,10 @@ __global__ void rt_update_bounds_kernel(const float* __restrict__ points, int nu
 }
 
 // The publication of a mesh edit (one thread, after the join): the mesh's record points at the new arrays of num_tris
-// triangles and 2 * num_tris - 1 nodes, with the culling margin of the new root (as upload computes it) and without the
-// 8-wide copy; the shape gets the new bounds.  Kernels read both records at run time.  flag / status: a refit's (null
-// otherwise).  With the flag set the arrays are a copy of the live set (rt_refit_restore_kernel), so the shape's bounds
-// and the mesh's margin stay as they are; the flag goes to *status.
+// triangles and 2 * num_tris - 1 nodes, with the culling margin of the new root (as upload computes it); the shape gets
+// the new bounds.  Kernels read both records at run time.  flag / status: a refit's (null otherwise).  With the flag
+// set the arrays are a copy of the live set (rt_refit_restore_kernel), so the shape's bounds and the mesh's margin stay
+// as they are; the flag goes to *status.
 __global__ void rt_update_publish_kernel(DevMesh* meshes, int mesh, rt_shape* shapes, int shape, const rt_bvh_node* nodes,
                                          const rt_tri* tris, const rt_shade* shade, int num_tris, const unsigned long long* keys,
                                          const float* points, const int* flag, int* status)
@@ -177,7 +177,6 @@ __global__ void rt_update_publish_kernel(DevMesh* meshes, int mesh, rt_shape* sh
     if (status) *status = f;
     DevMesh& m = meshes[mesh];
     m.nodes = (const float4*)nodes; m.tris = (const float4*)tris; m.shade = (const float4*)shade;
-    m.octo = nullptr;
     m.num_tris = num_tris; m.num_nodes = 2 * num_tris - 1;
     if (f) return;
     float scale = 0.0f;
@@ -490,8 +489,6 @@ static int publish_mesh(rt_gpu_ctx* ctx, int32_t shape, int mi, int T, const rt_
     std::swap(ms.cur, ms.spare);
     ms.num_tris = T; ms.num_nodes = 2 * T - 1;
     ms.refittable = true;                   // the builder's tree, or the refitted one
-    // the shared-memory stage holds mesh 0's uploaded top levels; a pointer test cannot tell the ping-pong's arrays apart
-    if (mi == 0) ctx->scene.top_of = nullptr;
     return RT_OK;
 }
 

@@ -1,5 +1,5 @@
 // rt_wave_kernels.cuh — the kernels of the wavefront (generate / walk / packet walk / long walk / shade /
-// finish / fold).  Included by rt_gpu.cu only (it holds non-template __global__ functions).
+// fold).  Included by rt_gpu.cu only (it holds non-template __global__ functions).
 // Compiled with -fmad=false; see rt_device.cuh.
 #pragma once
 #include "rt_wave_types.hpp"
@@ -561,23 +561,10 @@ rt_query_generate_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w
 // escape-threaded node array, see rt_device.cuh — to the end; then it stores (best leaf, position,
 // shrunken Distance) and pops the next id, so a warp's 32 lanes stay on walks of their own length.
 // Rounds of "node steps until the walking lanes hold a leaf, then those triangle tests together".
-// TOP: the shallowest levels of the (first) mesh's tree are staged in shared memory once per CTA and served from
-// there (hashed slots, see DevScene) — the fetches every walk makes leave the L1/TEX path.
-template <bool CULL, bool TOP>
+template <bool CULL>
 __global__ void __launch_bounds__(256, RT_WALK_BLOCKS)
 rt_walk_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, int round, int resumed)
 {
-    __shared__ int s_top_tag[TOP ? RT_TOP_SLOTS : 1];
-    __shared__ float4 s_top_node[TOP ? 2 * RT_TOP_SLOTS : 1];
-    if (TOP)
-    {
-        for (int k = threadIdx.x; k < RT_TOP_SLOTS; k += blockDim.x)
-        {
-            s_top_tag[k] = sc.top_tags ? sc.top_tags[k] : -1;
-            if (sc.top_tags) { s_top_node[2 * k] = sc.top_nodes[2 * k]; s_top_node[2 * k + 1] = sc.top_nodes[2 * k + 1]; }
-        }
-        __syncthreads();
-    }
     const int lane = threadIdx.x & 31;
     const unsigned lt_mask = (1u << lane) - 1u;
     // resumed: the walks the packet kernel handed back (they continue at their cursor); else the round's queue
@@ -595,7 +582,7 @@ rt_walk_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, int roun
     unsigned id = 0;
     Ray r; r.o = V3(0, 0, 0); r.d = V3(0, 0, 1); r.dist = 0.0f;
     RayPre pre = ray_pre(r);
-    bool any = false, weird = false, wide = false, sky_on_miss = false, staged = false;
+    bool any = false, weird = false, wide = false, sky_on_miss = false;
     float3 pad3 = V3(0, 0, 0);
     float growth = 0.0f;
     const float4* __restrict__ nodes = nullptr;
@@ -637,7 +624,6 @@ rt_walk_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, int roun
                     sky_on_miss = (cur.z & 512) != 0;
                     const DevMesh* m = sc.meshes + sc.shapes[cur.x].mesh;
                     nodes = m->nodes; tris = m->tris; n = m->num_nodes;
-                    staged = TOP && nodes == sc.top_of;
                     if (CULL)
                     {
                         pre.cull_pad = cull_pad_for(r, pre, m->cull_scale);
@@ -691,9 +677,7 @@ rt_walk_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, int roun
                     if (have && leaf[RT_LEAF_SLOTS - 1] < 0 && i < n)
                     {
                         float4 na, nb;
-                        const unsigned ts = top_slot(i);
-                        if (TOP && staged && s_top_tag[ts] == i) { na = s_top_node[2 * ts]; nb = s_top_node[2 * ts + 1]; }
-                        else ld32(nodes + 2 * (size_t)i, na, nb);
+                        ld32(nodes + 2 * (size_t)i, na, nb);
                         const int escape = __float_as_int(na.w);
                         const int tri = __float_as_int(nb.w);
                         nodes_seen++;
@@ -785,239 +769,6 @@ rt_walk_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, int roun
     // longest single walk of the batch (tooling: rt_gpu_debug_rounds)
     for (int o = 16; o > 0; o >>= 1) walk_max = max(walk_max, __shfl_xor_sync(RT_FULL_MASK, walk_max, o));
     if (lane == 0 && walk_max > 0) atomicMax(w.counts + RT_MAX_ROUNDS, walk_max);
-}
-
-// ---- kernel O: the culled walk on the 8-wide tree --------------------------------------------------------------
-// Which leaves a walk reaches is decided by the leaf boxes alone: a node's box contains its children's boxes
-// exactly (min / max over the same corners, KdTree.cpp:42-47), and in RRay::TestIntersectionWithAabb's arithmetic
-// — (b - o) * inv, the ternary min / max — every step is monotone in b, so a child whose box the line passes has
-// all its ancestors passing too.  The hierarchy only prunes.  ANY hierarchy over the same leaf boxes that hands the
-// passing leaves over in slot (= the reference's visiting) order therefore produces the reference's sequence of
-// triangle tests, hence its result bit for bit.  The culled traversal (results only; the exact one reproduces the
-// reference's test COUNTS and stays on the binary array) uses that freedom: the binary tree is collapsed at upload
-// into nodes of up to EIGHT children in slot order (DevMesh::octo: 8 x 32-byte records {box, ref} per node,
-// ref = child node | ~leaf slot), and a lane walks it depth first with a small stack of (node, pending children)
-// words in local memory.  One visit fetches and tests 8 boxes (8 independent 256-bit loads) where the binary walk
-// makes ~3.5 DEPENDENT fetches: a bounce ray's ~300 round trips become ~50.  Leaves are held and tested in order
-// as in rt_walk_kernel; rays with a disabled slab axis, nearly axis-parallel ones and non-finite ones (the general
-// slab function and the per-axis culling rule) are handed to the long-walk kernel untouched.
-#define RT_OCTO_STACK 40
-#define RT_OCTO_ROOT 0xffffffffu              // stack word: "expand the root" (node indices stay below 2^24)
-__global__ void __launch_bounds__(256, RT_OCTO_BLOCKS)
-rt_walk_octo_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, int round)
-{
-    const int lane = threadIdx.x & 31;
-    const unsigned lt_mask = (1u << lane) - 1u;
-    const unsigned round_count = w.counts[round] < w.pool.cap ? w.counts[round] : w.pool.cap;
-    const unsigned count = round_count;
-    const unsigned* __restrict__ queue = w.queue[round & 1];
-    unsigned* head = w.heads + round;
-    if (count == 0 || round_count < w.small_round) return;   // empty, or thin: the long-walk kernel takes all of it
-    Counters cnt = { 0, 0, 0, 0, 0, 0 };
-    unsigned win_pos = 0, win_end = 0;
-    bool exhausted = false;
-
-    bool have = false, finished = false;
-    unsigned id = 0;
-    Ray r; r.o = V3(0, 0, 0); r.d = V3(0, 0, 1); r.dist = 0.0f;
-    RayPre pre = ray_pre(r);
-    bool any = false, sky_on_miss = false;
-    const float4* __restrict__ octo = nullptr;
-    const float4* __restrict__ tris = nullptr;
-    unsigned node = 0, mask = 0;
-    int sp = 0, best = -1;
-    unsigned stack[RT_OCTO_STACK];
-    float3 bpos = V3(0, 0, 0);
-    unsigned nodes_seen = 0, tris_seen = 0, visits = 0;
-
-    for (;;)
-    {
-        // ---- refill: lanes without a walk pop ids (ballot -> rank -> window item) ----------------------
-        for (;;)
-        {
-            const unsigned idle = __ballot_sync(RT_FULL_MASK, !have);
-            if (idle == 0) break;
-            if (win_pos >= win_end)
-            {
-                if (exhausted) break;
-                unsigned base = 0;
-                if (lane == 0) base = atomicAdd(head, w.window);
-                base = __shfl_sync(RT_FULL_MASK, base, 0);
-                if (base >= count) { exhausted = true; break; }
-                win_pos = base;
-                win_end = count - base < w.window ? count : base + w.window;
-            }
-            const unsigned item = win_pos + (unsigned)__popc(idle & lt_mask);
-            if (!have && item < win_end)
-            {
-                id = queue[item];
-                const int4 cur = w.pool.cur[id];
-                if ((cur.z & 255) == ST_TRAVERSE)
-                {
-                    const float4 ro = w.pool.ro[id], rd = w.pool.rd[id];
-                    r.o = xyz(ro); r.dist = ro.w; r.d = xyz(rd);
-                    pre = ray_pre(r);
-                    const DevMesh* m = sc.meshes + sc.shapes[cur.x].mesh;
-                    pre.cull_pad = cull_pad_for(r, pre, m->cull_scale);
-                    const float growth = cull_growth(r, m->cull_scale);
-                    const bool plain = pre.ex && pre.ey && pre.ez && finite3(r.o) && finite3(r.d) && pre.cull_pad < FLT_MAX &&
-                                       !(pre.cull_pad > 4096.0f * growth);
-                    if (!plain || m->octo == nullptr)
-                    {
-                        // the general slab function / the per-axis culling rule: the long-walk kernel has both
-                        w.pool.bp[id] = make_float4(0.0f, 0.0f, 0.0f, __int_as_float(0));
-                        w.longq[atomicAdd(w.lcounts + round, 1u)] = id;
-                    }
-                    else
-                    {
-                        any = (cur.z & 256) != 0;
-                        sky_on_miss = (cur.z & 512) != 0;
-                        octo = m->octo; tris = m->tris;
-                        node = 0; mask = 0; sp = 0; best = -1; bpos = V3(0, 0, 0);
-                        stack[0] = RT_OCTO_ROOT;
-                        sp = 1;                 // the root node waits on the stack
-                        visits = 0;
-                        finished = false;
-                        have = true;
-                    }
-                }
-            }
-            const unsigned taken = win_pos + (unsigned)__popc(idle);
-            win_pos = taken < win_end ? taken : win_end;
-        }
-        if (__ballot_sync(RT_FULL_MASK, have) == 0) break;
-
-        const int min_lanes = exhausted ? 1 : w.min_lanes;
-        for (;;)
-        {
-            int leaf[RT_LEAF_SLOTS];
-#pragma unroll
-            for (int k = 0; k < RT_LEAF_SLOTS; k++) leaf[k] = -1;
-            // Node phase: a lane takes its next pending child — a leaf is held, an inner child is expanded (its eight
-            // boxes fetched and tested) — until it holds RT_LEAF_SLOTS leaves or has nothing left.
-            for (;;)
-            {
-                const unsigned stepping = __ballot_sync(RT_FULL_MASK, have && !finished && leaf[RT_LEAF_SLOTS - 1] < 0);
-                if (stepping == 0) break;
-                if (w.leaf_wait > 0 && __popc(stepping) < w.leaf_wait &&
-                    __ballot_sync(RT_FULL_MASK, leaf[0] >= 0) != 0) break;
-                if (have && !finished && leaf[RT_LEAF_SLOTS - 1] < 0)
-                {
-                    // next pending child of the walk, or the walk is over
-                    int expand = -1;
-                    while (mask == 0u && sp > 0)
-                    {
-                        const unsigned e = stack[--sp];
-                        if (e == RT_OCTO_ROOT) { expand = 0; break; }
-                        node = e >> 8; mask = e & 255u;
-                    }
-                    if (expand < 0)
-                    {
-                        if (mask == 0u) finished = true;
-                        else
-                        {
-                            const int k = __ffs((int)mask) - 1;
-                            mask &= mask - 1u;
-                            const int ref = __float_as_int(__ldg(octo + ((size_t)node * 8 + k) * 2).w);
-                            if (ref < 0)
-                            {
-                                bool placed = false;
-#pragma unroll
-                                for (int j = 0; j < RT_LEAF_SLOTS; j++)
-                                    if (!placed && leaf[j] < 0) { leaf[j] = ~ref; placed = true; }
-                            }
-                            else
-                            {
-                                if (mask != 0u && sp < RT_OCTO_STACK) stack[sp++] = (node << 8) | mask;
-                                else if (mask != 0u) { finished = true; visits = 0xffffffffu; }      // (stack overflow: see below)
-                                expand = ref;
-                            }
-                        }
-                    }
-                    if (expand >= 0 && !finished)
-                    {
-                        node = (unsigned)expand;
-                        const float4* __restrict__ rec = octo + (size_t)node * 16;
-                        unsigned m8 = 0u;
-                        int nchild = 8;
-                        const float reach = r.dist * 1.0078125f + pre.cull_pad;
-#pragma unroll
-                        for (int k = 0; k < 8; k++)
-                        {
-                            float4 ba, bb;
-                            ld32(rec + 2 * k, ba, bb);
-                            if (k == 0) nchild = __float_as_int(bb.w);
-                            float tlo, thi;
-                            bool enter = slab_fast(r, pre, xyz(ba), xyz(bb), tlo, thi);
-                            enter = enter && !(thi < -pre.cull_pad) && !(tlo > reach);
-                            m8 |= enter ? (1u << k) : 0u;
-                        }
-                        mask = m8 & ((1u << nchild) - 1u);
-                        nodes_seen += (unsigned)nchild;
-                        visits++;
-                    }
-                }
-            }
-            // Triangle phase: the held leaves, in walk order
-#pragma unroll
-            for (int k = 0; k < RT_LEAF_SLOTS; k++)
-            {
-                const int lf = leaf[k];
-                if (__ballot_sync(RT_FULL_MASK, lf >= 0) == 0) break;
-                if (lf >= 0)
-                {
-                    float4 t0, t1, t2, t3;
-                    ld32(tris + 4 * (size_t)lf, t0, t1);
-                    ld32(tris + 4 * (size_t)lf + 2, t2, t3);
-                    tris_seen++;
-                    float3 hp; float hd;
-                    if (triangle_test(r, xyz(t0), xyz(t1), xyz(t2), xyz(t3), hp, hd))
-                    {
-                        r.dist = hd;
-                        bpos = hp;
-                        best = lf;
-                        if (any)
-                        {
-                            finished = true; mask = 0u; sp = 0;
-#pragma unroll
-                            for (int j = 0; j < RT_LEAF_SLOTS; j++) leaf[j] = -1;
-                        }
-                    }
-                }
-            }
-            if (have && finished)
-            {
-                if (visits == 0xffffffffu)
-                {
-                    // a tree deeper than the stack: the walk starts over in the long-walk kernel (nothing was written)
-                    w.pool.bp[id] = make_float4(0.0f, 0.0f, 0.0f, __int_as_float(0));
-                    w.longq[atomicAdd(w.lcounts + round, 1u)] = id;
-                }
-                else
-                {
-                    int* cur = reinterpret_cast<int*>(w.pool.cur + id);
-                    if (best < 0 && sky_on_miss)
-                    {
-                        const int4 pa = w.pool.pa[id];
-                        const float3 L = sky_color(r.d);
-                        a.samples[(size_t)pa.y * ((size_t)a.width * a.height) + pa.x] = make_float4(L.x, L.y, L.z, 0.0f);
-                        cur[2] = ST_IDLE;           // the shade kernel skips it
-                    }
-                    else
-                    {
-                        w.pool.ro[id].w = r.dist;
-                        cur[1] = best;
-                        cur[2] = ST_MESHDONE | (any ? 256 : 0);
-                        if (best >= 0) w.pool.bp[id] = make_float4(bpos.x, bpos.y, bpos.z, 0.0f);
-                    }
-                }
-                have = false;
-            }
-            if (__popc(__ballot_sync(RT_FULL_MASK, have)) < min_lanes) break;
-        }
-    }
-    cnt.node_visits = nodes_seen; cnt.tri_visits = tris_seen;
-    flush_counters(cnt, a.counters, 0);
 }
 
 // ---- kernel P: packet walk (coherent rounds) ---------------------------------------------------------------
@@ -1551,89 +1302,6 @@ rt_shade_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, int rou
             queue_push(next_queue, next_count, push, id);
         }
         __syncthreads();                        // s_id is rewritten by the next tile
-    }
-    flush_counters(cnt, a.counters, a.exact);
-}
-
-// ---- kernel F: finish ------------------------------------------------------------------------------------------
-// After a few rounds only a percent of the paths is still alive, and a round costs the latency of its
-// longest walk whatever its size.  This kernel takes everything that is left and runs each path to
-// its end in ONE launch: a lane pops a path, then alternates walk (the resumable, warp-collective
-// query_traverse of rt_device.cuh) and shade until the path ends, and pops the next.  Lane efficiency
-// is poor and does not matter here; the critical path drops from (rounds left) x (longest walk) to
-// one path's length.
-template <bool CULL, int MODE>
-__global__ void __launch_bounds__(128)
-rt_finish_kernel(const DevScene sc, const RenderArgs a, const WaveArgs w, int round)
-{
-    const int lane = threadIdx.x & 31;
-    const unsigned lt_mask = (1u << lane) - 1u;
-    const unsigned count = w.counts[round] < w.pool.cap ? w.counts[round] : w.pool.cap;
-    const unsigned* __restrict__ queue = w.queue[round & 1];
-    unsigned* head = w.heads + round;
-    Counters cnt = { 0, 0, 0, 0, 0, 0 };
-    unsigned win_pos = 0, win_end = 0;
-    bool exhausted = count == 0;
-
-    int state = ST_IDLE;
-    unsigned id = 0;
-    Query q;
-    q.r.o = V3(0, 0, 0); q.r.d = V3(0, 0, 1); q.r.dist = 0.0f; q.pre = ray_pre(q.r); q.weird = false;
-    q.h.pos = V3(0, 0, 0); q.h.nrm = V3(0, 0, 0); q.h.dist = 0.0f; q.h.color = V3(1, 1, 1); q.h.alpha = 1.0f;
-    q.bpos = V3(0, 0, 0); q.si = 0; q.node = 0; q.best = -1; q.hit_shape = -1; q.tri = -1; q.any = false;
-    PathState s;
-    s.pixel = 0; s.slot = 0; s.rng.key = 0; s.rng.n = 0; s.depth_left = 0; s.sp = 0; s.pass_mask = 0; s.light = 0; s.seg_dist = 0.0f;
-    s.w_pos = s.w_nrm = s.w_surface = s.w_sum = V3(0, 0, 0);
-
-    for (;;)
-    {
-        for (;;)
-        {
-            const unsigned idle = __ballot_sync(RT_FULL_MASK, state == ST_IDLE);
-            if (idle == 0) break;
-            if (win_pos >= win_end)
-            {
-                if (exhausted) break;
-                unsigned base = 0;
-                if (lane == 0) base = atomicAdd(head, 32u);
-                base = __shfl_sync(RT_FULL_MASK, base, 0);
-                if (base >= count) { exhausted = true; break; }
-                win_pos = base;
-                win_end = count - base < 32u ? count : base + 32u;
-            }
-            const unsigned item = win_pos + (unsigned)__popc(idle & lt_mask);
-            if (state == ST_IDLE && item < win_end)
-            {
-                id = queue[item];
-                pool_load<MODE>(w.pool, id, q, state, s);
-                if (state == ST_TRAVERSE)
-                {
-                    if (CULL) q.pre.cull_pad = cull_pad_for(q.r, q.pre, sc.meshes[sc.shapes[q.si].mesh].cull_scale);
-                    q.node = 0; q.best = -1;
-                }
-                else if (state != ST_SHAPES && state != ST_SHADE && state != ST_MESHDONE) state = ST_IDLE;
-            }
-            const unsigned taken = win_pos + (unsigned)__popc(idle);
-            win_pos = taken < win_end ? taken : win_end;
-        }
-        if (!__any_sync(RT_FULL_MASK, state != ST_IDLE)) break;
-
-        query_traverse<CULL>(sc, q, state, exhausted ? 1 : 12, w.leaf_wait, cnt);
-        query_mesh_done(sc, q, state, cnt);
-        if (state == ST_SHAPES || state == ST_SHADE)
-        {
-            for (;;)
-            {
-                query_shapes<CULL>(sc, q, state, cnt);
-                if (state == ST_TRAVERSE) break;
-                Ray next; next.o = V3(0, 0, 0); next.d = V3(0, 0, 0); next.dist = 0.0f;
-                bool next_any = false;
-                if (!shade_query<MODE>(sc, a, w.pool, id, q, s, next, next_any)) { state = ST_IDLE; break; }
-                query_begin(q, next, next_any, cnt);
-                s.seg_dist = next.dist;
-                state = ST_SHAPES;
-            }
-        }
     }
     flush_counters(cnt, a.counters, a.exact);
 }

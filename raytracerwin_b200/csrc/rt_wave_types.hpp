@@ -214,12 +214,8 @@ struct WaveArgs
 #ifndef RT_LEAF_SLOTS
 #define RT_LEAF_SLOTS 2                     // leaves a lane may hold before its walk has to wait for the triangle phase
 #endif
-#define RT_FINISH_ROUND 0                   // rounds run as walk/shade waves; the rest in one finishing launch (0: never)
 #ifndef RT_STEPS_PER_VOTE
 #define RT_STEPS_PER_VOTE 3                  // node steps of the lane-per-walk kernel between two warp votes
-#endif
-#ifndef RT_OCTO_BLOCKS
-#define RT_OCTO_BLOCKS 3                    // resident 256-thread CTAs per SM of the 8-wide walk kernel (<= 85 registers)
 #endif
 #ifndef RT_WALK_BLOCKS
 #define RT_WALK_BLOCKS 4                    // resident 256-thread CTAs per SM of the walk kernel (64 registers)

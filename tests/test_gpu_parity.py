@@ -562,7 +562,6 @@ def test_frontier_long_walks_are_bit_identical(rt, data_dir, traverse, monkeypat
 @pytest.mark.parametrize("traverse", ["exact", "culled"])
 def test_packet_walk_is_bit_identical(rt, data_dir, traverse, monkeypatch):
     """Round 0 walked as 32-ray packets (rt_walk_packet_kernel) against the lane-per-walk kernel: no packets,
-    (with and without the shared-memory stage for the top of the first mesh's tree, RT_TOP_STAGE),
     packets for round 0, packets for every round, packets that are always given up after their first window
     (every lane resumes lane by lane at its cursor), a probe window of 5 steps — same image bits, same ray and
     hit counts and, in exact mode, the reference's slab / triangle test counts.  Two meshes in the scene, so
@@ -576,12 +575,8 @@ def test_packet_walk_is_bit_identical(rt, data_dir, traverse, monkeypatch):
     trav = rt.RT_TRAVERSE_EXACT if traverse == "exact" else rt.RT_TRAVERSE_CULLED
     p = rt.make_params(W, H, mode=rt.RT_MODE_PATH, max_bounce=6, antialias=1, pass_count=2, seed=21, traverse=trav)
     ref_img, ref_cnt = None, None
-    knobs = ("RT_PACKET_ROUNDS", "RT_PACKET_MIN_LANES", "RT_PACKET_PROBE", "RT_TOP_STAGE", "RT_OCTO")
+    knobs = ("RT_PACKET_ROUNDS", "RT_PACKET_MIN_LANES", "RT_PACKET_PROBE")
     variants = [dict(RT_PACKET_ROUNDS="0"),
-                dict(RT_PACKET_ROUNDS="0", RT_OCTO="1"),           # every round of the culled traversal on the 8-wide tree
-                dict(RT_OCTO="1"),
-                dict(RT_PACKET_ROUNDS="0", RT_TOP_STAGE="1"),      # every round lane by lane, top of mesh 0's tree from shared memory
-                dict(RT_TOP_STAGE="1"),
                 dict(RT_PACKET_ROUNDS="1", RT_PACKET_MIN_LANES="0"),
                 dict(RT_PACKET_ROUNDS="100", RT_PACKET_MIN_LANES="0"),
                 dict(RT_PACKET_ROUNDS="100", RT_PACKET_MIN_LANES="33"),

@@ -545,12 +545,8 @@ def _boundary_rays(sc, scale, seed=0):
     return np.array(rays, F)
 
 
-def _walk_variants(traverse):
-    v = [dict(), dict(RT_LONG_LIMIT="8", RT_SMALL_ROUND="0", RT_THIN_COUNT="0"), dict(RT_TOP_STAGE="1")]
-    return v + ([dict(RT_OCTO="1")] if traverse == "culled" else [])
-
-
-KNOBS = ("RT_LONG_LIMIT", "RT_SMALL_ROUND", "RT_THIN_COUNT", "RT_TOP_STAGE", "RT_OCTO", "RT_PACKET_ROUNDS")
+WALK_VARIANTS = (dict(), dict(RT_LONG_LIMIT="8", RT_SMALL_ROUND="0", RT_THIN_COUNT="0"))
+KNOBS = ("RT_LONG_LIMIT", "RT_SMALL_ROUND", "RT_THIN_COUNT", "RT_PACKET_ROUNDS")
 
 
 @pytest.mark.gpu
@@ -560,7 +556,7 @@ def test_boundary_meshes_through_every_walk(rt, port, monkeypatch, scale, traver
     """Accepted boundary meshes: query_rays (the production wavefront walks) and trace_rays (the hook's walk) == the
     restatement's trace_rays bit for bit (shape, triangle, all 11 hit fields); PRIMARY renders (packets form in the
     camera round) == the restatement's ids and Distance bits; for every walk variant (packets, long walks after 8
-    steps, the shared-memory top stage and, culled, the 8-wide tree) and, exact, the same slab and triangle test counts."""
+    steps) and, exact, the same slab and triangle test counts."""
     import torch
     sc = _boundary_scene(rt, scale)
     d = sc.desc.contents
@@ -574,7 +570,7 @@ def test_boundary_meshes_through_every_walk(rt, port, monkeypatch, scale, traver
     want = port.render(sc.desc, p, nthreads=os.cpu_count() or 1, want_primary=True)
     trav = rt.RT_TRAVERSE_EXACT if traverse == "exact" else rt.RT_TRAVERSE_CULLED
     counts = None
-    for env in _walk_variants(traverse):
+    for env in WALK_VARIANTS:
         for k in KNOBS:
             monkeypatch.delenv(k, raising=False)
         for k, v in env.items():

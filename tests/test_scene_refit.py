@@ -171,15 +171,12 @@ def test_refit_results_equal_fresh_upload(rt, data_dir, name):
 
 
 # ---------------------------------------------------------------------------------------------------
-# 3. sequences with update_mesh in between, also with the top-stage and 8-wide opt-ins
+# 3. sequences with update_mesh in between
 # ---------------------------------------------------------------------------------------------------
 @pytest.mark.gpu
-@pytest.mark.parametrize("env", [None, "RT_TOP_STAGE", "RT_OCTO"])
-def test_refit_sequence(rt, data_dir, monkeypatch, env):
+def test_refit_sequence(rt, data_dir):
     """upload -> refit -> refit -> update_mesh -> refit -> refit back to the uploaded points.  A refit keeps the
     topology it finds: the upload's, then the one update_mesh built (the host builder's for its points)."""
-    if env:
-        monkeypatch.setenv(env, "1")
     sc = make_scene(rt, scenes.c1_torusknot(data_dir))
     dump = sc.mesh_dump(0)
     A, pidx = dump["points"], dump["pidx"]

@@ -257,15 +257,12 @@ def test_replace_results_equal_fresh_upload(rt, data_dir, name):
 
 
 # ---------------------------------------------------------------------------------------------------
-# 3. sequences with refits and updates, also with the top-stage and 8-wide opt-ins
+# 3. sequences with refits and updates
 # ---------------------------------------------------------------------------------------------------
 @pytest.mark.gpu
-@pytest.mark.parametrize("env", [None, "RT_TOP_STAGE", "RT_OCTO"])
-def test_replace_sequence(rt, data_dir, monkeypatch, env):
+def test_replace_sequence(rt, data_dir):
     """replace (grow), refit, update_mesh, replace (shrink), refit, then replaces alternating between two levels of
     detail; arrays and results after every step."""
-    if env:
-        monkeypatch.setenv(env, "1")
     sc = make_scene(rt, scenes.c1_torusknot(data_dir))
     small, mid, big = torus_sizes(sc)
     hi, lo = geometry(grid(big), texcoords=True, slots=[-1]), geometry(grid(mid, seed=1), normals=True)

@@ -248,13 +248,10 @@ def test_update_results_equal_fresh_upload(rt, data_dir, name):
 
 
 # ---------------------------------------------------------------------------------------------------
-# 3. sequences A -> B -> A -> C, also with the top-stage and 8-wide opt-ins
+# 3. sequences A -> B -> A -> C
 # ---------------------------------------------------------------------------------------------------
 @pytest.mark.gpu
-@pytest.mark.parametrize("env", [None, "RT_TOP_STAGE", "RT_OCTO"])
-def test_update_sequence(rt, data_dir, monkeypatch, env):
-    if env:
-        monkeypatch.setenv(env, "1")
+def test_update_sequence(rt, data_dir):
     sc = make_scene(rt, scenes.c1_torusknot(data_dir))
     dump = sc.mesh_dump(0)
     A, pidx = dump["points"], dump["pidx"]

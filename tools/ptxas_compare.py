@@ -1,7 +1,7 @@
 """Per-kernel registers, spills, stack and shared memory of two -Xptxas -v logs (the Makefile keeps them in
 raytracerwin_b200/csrc/build/ptxas*.log), matched by mangled name with nvcc's per-build hash of anonymous namespaces
 removed (it depends on the source's path, so trees built in different directories compare too).  Prints every kernel
-of the first log with its line in the second and whether it changed, then kernels only the second log has.
+of the first log with its line in the second and whether it changed or is gone, then kernels only the second log has.
 
    python tools/ptxas_compare.py OLD.log NEW.log
 """
@@ -23,16 +23,20 @@ def parse(path):
 
 def main(old, new):
     A, B = parse(old), parse(new)
-    changed = 0
+    changed = removed = 0
     for k in A:
-        same = A[k] == B.get(k)
+        if k not in B:
+            removed += 1
+            print(f"removed {k}: {A[k]}")
+            continue
+        same = A[k] == B[k]
         changed += not same
-        print(f"{'same   ' if same else 'CHANGED'} {k}: {A[k]}" + ("" if same else f"  ->  {B.get(k)}"))
+        print(f"{'same   ' if same else 'CHANGED'} {k}: {A[k]}" + ("" if same else f"  ->  {B[k]}"))
     for k in B:
         if k not in A:
             print(f"new     {k}: {B[k]}")
-    print(f"{len(A)} kernels compared, {changed} changed, {sum(k not in A for k in B)} new")
-    return changed
+    print(f"{len(A)} kernels compared, {changed} changed, {removed} removed, {sum(k not in A for k in B)} new")
+    return changed + removed
 
 
 if __name__ == "__main__":

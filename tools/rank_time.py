@@ -18,7 +18,7 @@ ctx.upload_scene(scene)
 variants = os.environ.get("RT_VARIANTS", "").split(";")
 for v in variants:
     os.environ.pop("RT_SAMPLE_BUDGET_MB", None)
-    os.environ.update(RT_FINISH_ROUND="0", RT_LONG_LIMIT="2048", RT_SMALL_ROUND="24000", RT_LONG_GROUP_N="32", RT_THIN_COUNT="200000", RT_THIN_LIMIT="256", RT_PIPES_N="4", RT_PACKET_ROUNDS="-1", RT_PACKET_PROBE="24", RT_PACKET_MIN_LANES="10")
+    os.environ.update(RT_LONG_LIMIT="2048", RT_SMALL_ROUND="24000", RT_LONG_GROUP_N="32", RT_THIN_COUNT="200000", RT_THIN_LIMIT="256", RT_PIPES_N="4", RT_PACKET_ROUNDS="-1", RT_PACKET_PROBE="24", RT_PACKET_MIN_LANES="10")
     for kv in v.split():
         k, x = kv.split("="); os.environ[k] = x
     ctx.set_pipes(int(os.environ.get("RT_PIPES_N", "4")))
